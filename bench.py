@@ -26,11 +26,16 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True  # the bench leaves the source tree as it found it (which may be read-only)
 
 import numpy as np
 
 METRIC = "Mmappings/s filtered (sweep+scaffold)"
 N_HAP = 90
+# --dump-outputs: status (f32) and chain id (f64) of at most this many records over all ranks, 48 MB; the result counts of swg_stats
+DUMP_RECORDS = 4_000_000
+DUMP_STATS = ("n_input", "n_stage1", "n_after_sweep", "n_chains", "n_chains_after_mass", "n_chains_kept", "n_anchors", "n_rescued",
+              "n_kept")
 
 
 def peaks():
@@ -285,6 +290,19 @@ def pinned_copy(table, with_identity):
     return t2
 
 
+def dump_outputs(out_dir, status, chain, stats, world, rank):
+    """What the timed step returned to its caller, as out_dir/<name>.npy (out_dir/<name>_rank<r>.npy for each of several ranks):
+    status and chain id of every record, or of a fixed seeded sample of DUMP_RECORDS / world records (in record order) when the
+    table is larger, and the result counts DUMP_STATS."""
+    os.makedirs(out_dir, exist_ok=True)
+    n, m = len(status), DUMP_RECORDS // world
+    suffix = "" if world == 1 else f"_rank{rank}"
+    idx = np.sort(np.random.default_rng(rank).choice(n, m, replace=False)) if n > m else np.arange(n)
+    np.save(os.path.join(out_dir, f"status{suffix}.npy"), status[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, f"chain_id{suffix}.npy"), chain[idx].astype(np.float64))
+    np.save(os.path.join(out_dir, f"stats{suffix}.npy"), np.array([getattr(stats, k) for k in DUMP_STATS], np.float64))
+
+
 def paf_file_leg(ctx, cfg, n_lines):
     """Extra, informational: PafFilter::filter_paf file to file (text tokenised and tagged output assembled on the GPU,
     swg_filter_paf) and the same call with the host front end, on a synthetic PAF with cg:Z: tags.  Never fails the bench."""
@@ -418,7 +436,14 @@ def main():
     ap.add_argument("--cpu-sample-1t", type=int, default=2_000_000, help="records of the single-thread oracle figure")
     ap.add_argument("--no-parity", action="store_true", help="skip the full-size comparison with the oracle (profiling runs)")
     ap.add_argument("--no-anchor", action="store_true", help="N = 1: skip the configs[3]-shard scaling anchor")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (status and chain id of a fixed seeded sample "
+                         "of the records, the result counts) as DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the result of the b200 arm")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -426,7 +451,7 @@ def main():
 
     import __graft_entry__
     if not os.path.exists(__graft_entry__.LIB) or not os.path.exists(__graft_entry__.ORACLE):
-        __graft_entry__.build(import_package=False)
+        sys.exit("the native libraries are not built: run `python __graft_entry__.py` first")
 
     if args.impl == "reference":
         if rank == 0:
@@ -553,6 +578,8 @@ def main():
         status_dev, chain_dev = status_t.cpu().numpy(), chain_t.cpu().numpy().view(np.uint32)
     else:
         status_dev, chain_dev = ctx.download(n, d_res)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, status_dev, chain_dev, stats, world, rank)
 
     # ---- end to end: pinned host buffers in, host result out, copies inside the timed region ---------------------------
     with gpu_numa_affinity(local_rank) as numa:

@@ -81,22 +81,50 @@ def test_build_rs_compiles_the_same_sources_with_the_same_flags():
     assert "sm_90" not in text and "compute_90" not in text  # one architecture, no fallback
 
 
+def _hunks(patch):
+    """-> [(file, old_start, old_len, new_start, new_len, [body lines])] of a unified diff"""
+    out, path = [], None
+    lines = patch.split("\n")
+    for i, line in enumerate(lines):
+        if line.startswith("+++ "):
+            path = line[4:].split("/", 1)[1]
+        m = re.match(r"@@ -(\d+)(?:,(\d+))? \+(\d+)(?:,(\d+))? @@", line)
+        if m:
+            old, old_n, new, new_n = (int(g) if g is not None else 1 for g in m.groups())
+            body, j = [], i + 1
+            while j < len(lines) and lines[j][:1] in (" ", "-", "+") and not lines[j].startswith(("--- ", "+++ ")):
+                body.append(lines[j])
+                j += 1
+            out.append((path, old, old_n, new, new_n, body))
+    return out
+
+
 def test_patch_applies_to_the_cited_lines():
     """patches/apply_filters.patch replaces the body of PafFilter::apply_filters; its hunk header cites the reference lines it
-    was written against (src/paf_filter.rs:379-382) and its context lines quote the reference verbatim where it is present."""
+    was written against (src/paf_filter.rs:379-382).  Every hunk's line counts agree with its header, its new start follows
+    from the hunks before it in the same file, and the function head sits at the cited lines of the paf_filter.rs hunk.
+    When SWEEPGA_SRC names a sweepga v0.1.1 checkout, every context and removed line of every hunk must also quote that
+    checkout verbatim at the line its header cites (no offset, no fuzz)."""
     patch = open(os.path.join(ROOT, "patches", "apply_filters.patch")).read()
     assert "--- a/src/paf_filter.rs" in patch and "+++ b/src/paf_filter.rs" in patch
     assert "sweepga_cuda_sys" in patch and "swg_filter" in patch
-    ref = "/root/reference"
-    import shutil
-    import subprocess
-    import tempfile
-    if os.path.exists(os.path.join(ref, "src", "paf_filter.rs")) and shutil.which("patch"):
-        # only in the build container (the GPU box has no reference tree): the patch applies cleanly to v0.1.1
-        with tempfile.TemporaryDirectory() as d:
-            os.makedirs(os.path.join(d, "src"))
-            for f in ("Cargo.toml", "src/lib.rs", "src/main.rs", "src/paf_filter.rs"):
-                shutil.copy(os.path.join(ref, f), os.path.join(d, f))
-            r = subprocess.run(["patch", "-p1", "--dry-run", "-i", os.path.join(ROOT, "patches", "apply_filters.patch")], cwd=d,
-                               capture_output=True, text=True)
-            assert r.returncode == 0, r.stdout + r.stderr
+    hunks = _hunks(patch)
+    assert [h[0] for h in hunks] == ["Cargo.toml", "Cargo.toml", "src/lib.rs", "src/main.rs", "src/paf_filter.rs", "src/cuda_filter.rs"]
+    delta = {}
+    for path, old, old_n, new, new_n, body in hunks:
+        assert sum(l[0] in " -" for l in body) == old_n, (path, old)
+        assert sum(l[0] in " +" for l in body) == new_n, (path, old)
+        assert new == (1 if old_n == 0 and old == 0 else old + delta.get(path, 0)), (path, old, new)
+        delta[path] = delta.get(path, 0) + new_n - old_n
+    # the pre-image lines of the paf_filter.rs hunk, at the reference's line numbers: the function head is lines 379-382
+    _, old, _, _, _, body = hunks[4]
+    pre = {old + k: l[1:] for k, l in enumerate(l for l in body if l[0] in " -")}
+    assert pre[379].strip() == "pub fn apply_filters(" and pre[382].strip() == ") -> Result<HashMap<usize, RecordMeta>> {"
+    ref = os.environ.get("SWEEPGA_SRC")
+    if ref:  # the reference sources are not part of this repository: compared where a checkout of them is at hand
+        assert re.search(r'^version\s*=\s*"0\.1\.1"', open(os.path.join(ref, "Cargo.toml")).read(), re.M), "not sweepga v0.1.1"
+        for path, old, old_n, _, _, body in hunks:
+            if old_n:
+                src = open(os.path.join(ref, path)).read().split("\n")
+                want = [l[1:] for l in body if l[0] in " -"]
+                assert src[old - 1:old - 1 + old_n] == want, (path, old)
