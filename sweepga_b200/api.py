@@ -228,7 +228,8 @@ def with_ids16(table: "MappingTable", alloc=None) -> "MappingTable":
     """A copy of the table whose swg_mappings view carries 16-bit id columns (n_seq <= 65536).  alloc(array) -> array lets the
     caller place the two columns (e.g. in pinned memory)."""
     import copy
-    assert table.n_seq <= 65536
+    if table.n_seq > 65536:
+        raise ValueError(f"16-bit id columns hold at most 65536 sequences, the table has {table.n_seq}")
     t = copy.copy(table)
     q, tt = table.query_id.astype(np.uint16), table.target_id.astype(np.uint16)
     t.ids16 = (alloc(q), alloc(tt)) if alloc else (q, tt)

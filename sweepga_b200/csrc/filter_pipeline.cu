@@ -1536,14 +1536,24 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
                        [=] __device__(u32 i, u32 slot, u32 v) { if (v) rlist[slot] = i; }, N, bsum, d_na + 1, st, lc);
             const u32 *avc = av;
             const u32 *d_nr = d_na + 1;
+            // The reference squares in u64 and wraps (a release build): qd^2 + td^2 passes 2^64 once td reaches ~0.866 * 2^32, and the
+            // wrapped sum can put a far anchor inside D.  Every scanned anchor has qd <= D and td <= max(tc, maxcoord - tc) (anchor
+            // centres lie in [0, maxcoord]), so for a candidate with (D^2 + that^2 < 2^64) the sum never wraps and the two shortcuts
+            // below hold; for any other candidate every anchor with qd <= D is measured.  Only target centres beyond 3.7 * 10^9 from
+            // one end of the coordinate range take that path (on a repeat pile it costs O(anchors within +-D) per candidate).
+            const u64 wrap_lim = ~0ull - D * D; // D < 2^31 (checked on entry)
+            const bool may_wrap = (u64)maxcoord * maxcoord > wrap_lim;
+            const u64 maxc = maxcoord;
             launch_for_dev<t_rescue>(d_nr, c->sm_count, st, lc, [=] __device__(u32 x0) {
                 const u32 i = rlist[x0];
                 const u64 pair = ((u64)in.qid[i] << sb) | in.tid[i];
                 const u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2, tc = ((u64)in.ts[i] + in.te[i]) / 2;
+                const u64 td_max = tc > maxc - tc ? tc : maxc - tc;
+                const bool wrap = may_wrap && td_max * td_max > wrap_lim;
                 // first anchor of the pair at or right of the query center; the scan runs outwards from there and stops once
                 // the query-axis distance alone exceeds the best distance found: dist = floor(sqrt(qd^2 + td^2)) >= qd - 1 (the f64
                 // square root of a rounded sum can fall one short), so nothing beyond qd > best + 1 can win or tie.  On a repeat pile
-                // (10^5..10^6 anchors inside +-D) that is a handful of anchors instead of all of them.
+                // (10^5..10^6 anchors inside +-D) that is a handful of anchors instead of all of them.  Not when the sum may wrap.
                 u32 lo = 0, hi = NA;
                 while (lo < hi) {
                     u32 mid = (lo + hi) >> 1;
@@ -1556,20 +1566,20 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
                     const u32 a = avc[x];
                     const u64 atc = ((u64)in.ts[a] + in.te[a]) / 2;
                     const u64 td = atc > tc ? atc - tc : tc - atc;
-                    if (td > D) return; // then floor(sqrt(qd^2+td^2)) > D
-                    const u64 dist = (u64)__dsqrt_rn((double)(qd * qd + td * td));
+                    if (td > D && !wrap) return; // then floor(sqrt(qd^2+td^2)) > D
+                    const u64 dist = (u64)__dsqrt_rn((double)(qd * qd + td * td)); // u64: wraps like the reference
                     if (dist <= D && (dist < best_d || (dist == best_d && a < best_a))) { best_d = dist; best_a = a; }
                 };
                 for (u32 x = lo; x < NA && apair[x] == pair; x++) {
                     const u64 qd = (u64)aqc[x] - qc;
-                    if (qd > D || (best_a != NONE32 && qd > best_d + 1)) break;
+                    if (qd > D || (!wrap && best_a != NONE32 && qd > best_d + 1)) break;
                     visit(x, qd);
                 }
                 for (u32 x = lo; x > 0;) {
                     x--;
                     if (apair[x] != pair) break;
                     const u64 qd = qc - (u64)aqc[x];
-                    if (qd > D || (best_a != NONE32 && qd > best_d + 1)) break;
+                    if (qd > D || (!wrap && best_a != NONE32 && qd > best_d + 1)) break;
                     visit(x, qd);
                 }
                 if (best_a != NONE32) { status[i] = 2; chain_id[i] = chain_id[best_a]; }
