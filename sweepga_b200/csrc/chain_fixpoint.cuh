@@ -16,13 +16,13 @@
 //
 // A round:
 //   1. snapshot: picker lists per successor j (CSR) in position order — the positions sorted by their pick, stable — with the
-//      picker d stored as prefix minima; per successor one 32 B word: minpd[j] = smallest d over all pickers of j, minpi[j] = the
+//      picker d stored as prefix minima; per successor one 32 B word: the smallest d over all pickers of j, minpi[j] = the
 //      first picker holding it, firstp[j] = the first picker at all and its d, the list range.  "d < B(i,j)?" is answered from
 //      that word in all but a few cases (fx_eligible_packed), else by one binary search over the list.
-//   2. k_fx_check (thread per position; a position is skipped outright when no picker list among the successors it can
-//      depend on — up to xhi[i] = max(pick(i), X(i)) — changed in the last round: dirty blocks of 512 successors and their
-//      prefix counts; an entry whose successor's own list did not change — one bit per successor — keeps its verdict): position i
-//      must be re-evaluated iff its pick is now blocked (an earlier picker
+//   2. k_fx_check_warp (lane per position, X(i) lists read by whole warps; a position is skipped outright when no picker list
+//      among the successors it can depend on — up to xhi[i] = max(pick(i), X(i)) — changed in the last round: dirty blocks of
+//      512 successors and their prefix counts; an entry whose successor's own list did not change — one bit per successor —
+//      keeps its verdict): position i must be re-evaluated iff its pick is now blocked (an earlier picker
 //      of the same j with d' <= d) or one of the candidates that rank BEFORE its pick — X(i), all of them ineligible when
 //      the pick was made, remembered explicitly with their d — has become eligible.  This test is exact: a position whose pick
 //      stands and whose X(i) is still blocked would pick the same j again.
@@ -30,8 +30,7 @@
 //      once more by (bucket of the target coordinate the gap rule tests, position); buckets visited outwards from the position's
 //      own, pruned outward scans inside a bucket) with eligibility against the snapshot.  The blocked candidates the search meets
 //      while they still beat the lane's best are recorded in shared memory — a superset of X(i), filtered against the final pick
-//      (fx_filter_seen); only if that record overflows, a second pruned pass collects X(i).  SWG_FX_NO_BUCKETS=1: the pruned
-//      window search of the sequential walk (bb_best_successor_warp) along the query axis instead, from the candidate records.
+//      (fx_filter_seen); only if that record overflows, a second pruned pass collects X(i).
 // A huge group whose picks have not settled after SWG_FIXPOINT_MAX_ROUNDS rounds goes to the sequential walk after all;
 // SWG_FIXPOINT_VERIFY=1 re-evaluates every position from scratch against the final picks (0 of 50 M change on configs[4]).
 // Round 0 evaluates every position against the empty snapshot: the unconstrained arg-min (X(i) is empty there by definition).
@@ -42,7 +41,7 @@
 
 namespace swg {
 
-struct t_fx_init; struct t_fx_skey; struct t_fx_pm; struct t_fx_snap; struct t_fx_hg; struct t_fx_bkey; struct t_fx_brec; struct t_fx_dir; struct t_fx_count; struct t_fx_minpi; struct t_fx_all; struct t_fx_fill; struct t_fx_pred; struct t_fx_jump; struct t_fx_scatter;
+struct t_fx_init; struct t_fx_skey; struct t_fx_pm; struct t_fx_bkey; struct t_fx_brec; struct t_fx_count; struct t_fx_all; struct t_fx_pred; struct t_fx_jump; struct t_fx_scatter;
 
 constexpr u32 FX_XCAP = 1024;     // blocked candidates remembered per position; a position with more is re-evaluated every round
 constexpr u16 FX_XOVER = 0xFFFF; // xcnt value of such a position
@@ -53,32 +52,29 @@ struct FxArrays {
     u32 n;             // positions in huge groups
     uint4 *rec;        // (qs, qe, ts, te)
     u32 *gend;         // end of the position's group (k-space) | FX_REV
-    u32 *c0;           // origin of the outward scans from the candidate pass, NONE32 if its window ended in the linear phase
     u32 *pick;         // current pick (k-space), NONE32 = none
     u64 *pd;           // d of the current pick
-    u32 *cnt, *off;    // picker lists: off[j] .. off[j+1]
-    u64 *minpd;        // smallest d over all pickers of j (NONE64: nobody picks j)
-    u32 *minpi;        // the first picker of j that has that d
+    u32 *cnt, *off;    // picker lists: off[j] .. off[j+1], in position order
+    u32 *minpi;        // the first picker of j that has the smallest d over all pickers of j
     u32 *firstp;       // the first picker of j at all (NONE32: nobody)
     u32 *li;           // picker position
-    u64 *ld;           // picker d (sorted lists: the smallest d of the list up to and including this entry)
+    u64 *ld;           // the smallest picker d of the list up to and including this entry
     u32 force_collect; // testing aid (SWG_FX_FORCE_COLLECT=1): X(i) always from the separate collecting pass
-    u32 sorted;        // 1: every picker list is in position order and ld holds prefix minima (bucket order)
     u32 *xoff;         // X(i) lives at pool[xoff .. xoff + xcnt)
     u16 *xcnt, *xcap;
     u32 *pool;
-    u64 *pool_d;       // bucket order only: d(i, x) of every pool entry (k_fx_check then needs no record gather)
+    u64 *pool_d;       // d(i, x) of every pool entry (k_fx_check_warp then needs no record gather)
     unsigned long long *pool_top; // 64-bit: refused requests keep counting and must never wrap into live slots
     u32 pool_cap;
     u32 *list;         // positions to re-evaluate this round
     u32 *xhi;          // largest position in {pick(i)} U X(i) (i itself if there is none): how far i's verdict can depend
     u32 *dirty, *dps;  // per block of successors: some picker list in it changed in the last round; prefix counts of that
-    u32 use_dirty;     // 0: check every position (first round, or the feature is off)
-    u32 *dbits, *dbits_w; // one bit per successor: its picker list changed in the last round (read by k_fx_check) / in this one
+    u32 use_dirty;     // 0: check every position (first round)
+    u32 *dbits, *dbits_w; // one bit per successor: its picker list changed in the last round (read by k_fx_check_warp) / in this one
     u32 *ctrs;         // [0] list length, [1] picks changed this round, [2] recompute work counter, [3] slots refused (pool full)
     // target-bucket order (fx_bucket_pass): the positions of every huge group once more, ordered by (group, target bucket, k)
     u32 *hg;           // dense number of the position's huge group
-    uint4 *snap;       // 32 B (one sector) per successor: [2j] = (minpd lo, minpd hi, minpi, firstp), [2j+1] = (d of the first picker lo, hi, off[j], list length)
+    uint4 *snap;       // 32 B (one sector) per successor: [2j] = (smallest picker d lo, hi, minpi, firstp), [2j+1] = (d of the first picker lo, hi, off[j], list length)
     uint2 *bq;         // (query_start, t') of the entries in bucket order: all the gap rule reads of a candidate
     u32 *bk;           // their positions k
     u32 *dir;          // dir[hg * dirD + b] .. dir[hg * dirD + b + 1]: the entries of bucket b of the group
@@ -87,23 +83,20 @@ struct FxArrays {
 };
 
 // is some picker of j before position i with d' <= d?  (the caller knows that the list is not empty)
+// Position order + prefix minima: the last picker before i answers for all of them.
 __device__ __forceinline__ bool fx_list_blocks(const FxArrays &f, u32 i, u32 j, u64 d, u32 a = NONE32, u32 b = NONE32) {
     if (a == NONE32) { a = f.off[j]; b = f.off[j + 1]; }
-    if (f.sorted) { // position order + prefix minima: the last picker before i answers for all of them
-        u32 lo = a, hi = b;
-        while (hi - lo > 4) {
-            const u32 mid = (lo + hi) >> 1;
-            if (f.li[mid] < i) lo = mid + 1; else hi = mid;
-        }
-        while (lo < hi && f.li[lo] < i) lo++;
-        return lo > a && f.ld[lo - 1] <= d;
+    u32 lo = a, hi = b;
+    while (hi - lo > 4) {
+        const u32 mid = (lo + hi) >> 1;
+        if (f.li[mid] < i) lo = mid + 1; else hi = mid;
     }
-    for (u32 p = a; p < b; p++)
-        if (f.li[p] < i && f.ld[p] <= d) return true;
-    return false;
+    while (lo < hi && f.li[lo] < i) lo++;
+    return lo > a && f.ld[lo - 1] <= d;
 }
 // smallest d over the pickers of j that precede position i, compared with d: true iff d < B(i,j)
-// (callers have established d >= minpd[j]: if the picker that holds the minimum precedes i, that settles it)
+// (callers have established that d is not below the smallest d over all pickers of j: if the picker that holds that minimum
+// precedes i, that settles it)
 __device__ __forceinline__ bool fx_eligible(const FxArrays &f, u32 i, u32 j, u64 d, u32 mi /* = minpi[j] */) {
     if (mi < i) return false;
     if (mi == i) return true; // i itself holds the minimum and is the first to: every earlier picker has a larger d
@@ -123,23 +116,13 @@ __device__ __forceinline__ bool fx_eligible_packed(const FxArrays &f, u32 i, u32
     return !fx_list_blocks(f, i, j, d, s2.z, s2.z + s2.w);
 }
 struct FxExtra {
-    static constexpr u32 OUTWARD = 128; // wider rounds measured slower (256: 2.3x on the 8 M pile): most searches end within the first rounds
-    static constexpr bool PREFETCH = true;
-    const u32 *pi; // = minpi
     FxArrays f;
     u32 i;
     u32 *seen, *n_seen; // shared memory of the warp: the blocked candidates met by the search (a superset of X(i))
-    // the same verdict from the packed snapshot word of j (mi = minpi[j], fp = firstp[j]); callers have established d >= minpd[j]
+    // the verdict from the packed snapshot word of j (mi = minpi[j], fp = firstp[j]); callers have established that d is not
+    // below the smallest d over all pickers of j
     __device__ __forceinline__ bool packed(u32 j, u64 d, u32 mi, u32 fp) const {
         const bool el = fx_eligible_packed(f, i, j, d, mi, fp);
-        if (!el) {
-            const u32 o = atomicAdd(n_seen, 1u);
-            if (o < FX_XCAP) seen[o] = j;
-        }
-        return el;
-    }
-    __device__ __forceinline__ bool operator()(u32 j, u64 d, u32 mi) const {
-        const bool el = fx_eligible(f, i, j, d, mi);
         if (!el) { // it beat the lane's best so far and is blocked: the only kind of candidate that can belong to X(i)
             const u32 o = atomicAdd(n_seen, 1u);
             if (o < FX_XCAP) seen[o] = j;
@@ -147,56 +130,6 @@ struct FxExtra {
         return el;
     }
 };
-
-// step 2: does position k have to be re-evaluated against the new snapshot?
-__global__ void __launch_bounds__(256) k_fx_check(FxArrays f, u64 G) {
-    const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
-    bool need = false;
-    if (k < f.n) {
-        const u16 xc = f.xcnt[k];
-        const u32 j = f.pick[k];
-        bool untouched = false;
-        if (xc != FX_XOVER && f.use_dirty) { // no picker list this position depends on has changed since its last verdict
-            const u32 hi = f.xhi[k];
-            untouched = hi <= k || f.dps[(hi >> FX_DB) + 1] == f.dps[(k + 1) >> FX_DB];
-        }
-        if (xc == FX_XOVER) need = true;
-        else if (!untouched) {
-            // a successor whose picker list did not change in the last round gives the verdict it gave then: still blocked
-            const bool bits = f.use_dirty && f.dbits;
-            if (j != NONE32 && f.off[j + 1] - f.off[j] > 1 && (!bits || (f.dbits[j >> 5] >> (j & 31) & 1))) need = !fx_eligible(f, k, j, f.pd[k], f.minpi[j]);
-            if (!need && xc) {
-                const uint4 a = f.rec[k];
-                const bool fwd = !(f.gend[k] & FX_REV);
-                const u32 *x = f.pool + f.xoff[k];
-                if (f.pool_d) { // d stored with the entry, the successor's snapshot in one word
-                    const u64 *xd = f.pool_d + f.xoff[k];
-                    for (u32 q = 0; q < xc && !need; q++) {
-                        const u32 jx = x[q];
-                        if (bits && !(f.dbits[jx >> 5] >> (jx & 31) & 1)) continue;
-                        const u64 d = xd[q];
-                        const uint4 sn = f.snap[2 * (size_t)jx];
-                        const u64 mp = ((u64)sn.y << 32) | sn.x;
-                        need = d < mp || fx_eligible_packed(f, k, jx, d, sn.z, sn.w);
-                    }
-                } else
-                for (u32 q = 0; q < xc && !need; q++) {
-                    const u32 jx = x[q];
-                    u64 d;
-                    if (bb_candidate(a, f.rec[jx], fwd, G, G / 5, d)) need = d < f.minpd[jx] || fx_eligible(f, k, jx, d, f.minpi[jx]);
-                }
-            }
-        }
-    }
-    const u32 m = __ballot_sync(0xFFFFFFFFu, need);
-    if (m) {
-        u32 base = 0;
-        const u32 leader = __ffs(m) - 1;
-        if (lane_id() == leader) base = atomicAdd(&f.ctrs[0], (u32)__popc(m));
-        base = __shfl_sync(0xFFFFFFFFu, base, leader);
-        if (need) f.list[base + __popc(m & lanemask_lt())] = k;
-    }
-}
 
 // Round 0 for the positions whose window ends within the next BB_LINEAR successors — every position of a chromosome-scale group of
 // collinear mappings, which is huge and sparse: one thread scans them in order (the unconstrained arg-min, first minimal j), no warp
@@ -226,10 +159,10 @@ __global__ void __launch_bounds__(256) k_fx_round0_linear(FxArrays f, u64 G) {
     }
 }
 
-// step 2 in bucket order: the same test, the X(i) lists read by whole warps.  A lane first judges its own position (skip tests, its
-// pick); the lists that still have to be looked at are then taken one at a time by all 32 lanes — coalesced reads of the pool instead
-// of 32 private strided walks (at 50 M the pool holds 2.7 * 10^9 entries and the thread-per-position loop moved them at a tenth of
-// the HBM rate) — and an entry whose successor's picker list did not change keeps last round's verdict without a further load.
+// step 2: does position k have to be re-evaluated against the new snapshot?  A lane first judges its own position (skip tests, its
+// pick); the X(i) lists that still have to be looked at are then taken one at a time by all 32 lanes — coalesced reads of the pool
+// instead of 32 private strided walks (at 50 M the pool holds 2.7 * 10^9 entries and a thread-per-position loop moved them at a tenth
+// of the HBM rate) — and an entry whose successor's picker list did not change keeps last round's verdict without a further load.
 __global__ void __launch_bounds__(256) k_fx_check_warp(FxArrays f, u64 G) {
     const u32 full = 0xFFFFFFFFu;
     const u32 lane = lane_id();
@@ -295,69 +228,6 @@ __device__ __forceinline__ u32 fx_collect_chunk(const uint4 &a, bool fwd, u64 G,
     }
     return xn + __popc(m);
 }
-__device__ __forceinline__ u32 fx_collect_blocked(const uint4 *__restrict__ rec, u32 i, u32 e, const uint4 &a, bool fwd, u64 G, u64 G5,
-                                                  u64 bd, u32 bj, u32 c0, u32 *xs) {
-    const u32 full = 0xFFFFFFFFu;
-    const u32 lane = lane_id();
-    u32 xn = 0;
-    // the nearest successors, evaluated one by one like the searches do (their origin may lie in here)
-    const u32 lin_end = min(e, i + 1 + 64);
-    const u64 bound = (u64)a.y + G;
-    for (u32 j0 = i + 1; j0 < lin_end; j0 += 32) {
-        const u32 j = j0 + lane;
-        uint4 b = make_uint4(0, 0, 0, 0);
-        bool in = false;
-        if (j < lin_end) { b = rec[j]; in = (u64)b.x <= bound; }
-        xn = fx_collect_chunk(a, fwd, G, G5, bd, bj, j, in, b, xs, xn);
-    }
-    if (c0 == NONE32 || lin_end >= e) return xn; // the window ended in there (k_chain_candidates' linear phase saw its end)
-    c0 = max(c0, lin_end);
-    // four chunks per round, every load issued before the first use (one memory round trip per 128 candidates)
-    constexpr u32 CW = 4;
-    for (u32 r0 = c0; r0 < e; r0 += 32 * CW) { // right of the origin: q_gap = qs - qe >= 0 grows; d >= q_gap^2
-        uint4 b[CW];
-#pragma unroll
-        for (u32 k = 0; k < CW; k++) {
-            const u32 r = r0 + k * 32 + lane;
-            b[k] = r < e ? rec[r] : make_uint4(0, 0, 0, 0);
-        }
-        bool in = false;
-#pragma unroll
-        for (u32 k = 0; k < CW; k++) {
-            const u32 r = r0 + k * 32 + lane;
-            in = false;
-            if (r < e) {
-                const u64 qg = (u64)b[k].x - a.y;
-                in = qg <= G && qg * qg <= bd;
-            }
-            xn = fx_collect_chunk(a, fwd, G, G5, bd, bj, r, in, b[k], xs, xn);
-        }
-        if (!__shfl_sync(full, (int)in, 31)) break; // monotone: once the last candidate is out, so is everything further right
-    }
-    for (u32 top = c0; top > lin_end;) { // left of the origin: overlap = qe - qs > 0 grows going left
-        const u32 cnt = min(32u * CW, top - lin_end);
-        uint4 b[CW];
-#pragma unroll
-        for (u32 k = 0; k < CW; k++) {
-            const u32 off = k * 32 + lane;
-            b[k] = off < cnt ? rec[top - 1 - off] : make_uint4(0, 0, 0, 0);
-        }
-        bool in = false;
-#pragma unroll
-        for (u32 k = 0; k < CW; k++) {
-            const u32 off = k * 32 + lane;
-            in = false;
-            if (off < cnt) {
-                const u64 ov = (u64)a.y - b[k].x;
-                in = ov <= G5 && ov * ov <= bd;
-            }
-            xn = fx_collect_chunk(a, fwd, G, G5, bd, bj, top - 1 - off, in, b[k], xs, xn);
-        }
-        if (cnt < 32 * CW || !__shfl_sync(full, (int)in, 31)) break;
-        top -= 32 * CW;
-    }
-    return xn;
-}
 
 // X(i) out of the search's own record: keep the entries that rank before the final pick (compacted in place)
 __device__ __forceinline__ u32 fx_filter_seen(const uint4 *__restrict__ rec, const uint4 &a, bool fwd, u64 G, u64 G5, u64 bd, u32 bj, u32 *xs,
@@ -386,9 +256,9 @@ __device__ __forceinline__ u32 fx_filter_seen(const uint4 *__restrict__ rec, con
 // those that beat the best so far — independent gathers, one memory round trip — then the verdicts in order.  (Loading the
 // words lazily, candidate by candidate, made a blocked candidate cost two dependent round trips; a position deep in a conflict
 // meets dozens of them before its first eligible one.)
-template <u32 CW, class Extra>
+template <u32 CW>
 __device__ __forceinline__ void fx_eval_round(const FxArrays &f, const uint4 &a, bool fwd, u64 G, u64 G5, const uint2 (&rb)[CW], const u32 (&rj)[CW],
-                                              const bool (&in)[CW], u64 &bd, u32 &bj, const Extra &ex) {
+                                              const bool (&in)[CW], u64 &bd, u32 &bj, const FxExtra &ex) {
     u64 dd[CW];
     bool want[CW];
     uint4 sn[CW];
@@ -428,8 +298,8 @@ __device__ __forceinline__ void fx_eval_round(const FxArrays &f, const uint4 &a,
 // only candidates with q_gap^2 > best d), which is all the blocked-candidate record needs.
 // COLLECT = false: bd / bj receive the pick.  COLLECT = true: bd / bj are the final pick; the valid candidates ranking before
 // it are appended to xs (X(i)); returns their number.
-template <bool COLLECT, class Extra>
-__device__ __forceinline__ u32 fx_bucket_pass(const FxArrays &f, u32 i, const uint4 &a, bool fwd, u64 G, u64 G5, u64 &bd, u32 &bj, Extra ex,
+template <bool COLLECT>
+__device__ __forceinline__ u32 fx_bucket_pass(const FxArrays &f, u32 i, const uint4 &a, bool fwd, u64 G, u64 G5, u64 &bd, u32 &bj, FxExtra ex,
                                               u32 *xs) {
     const u32 full = 0xFFFFFFFFu;
     const u32 lane = lane_id();
@@ -533,8 +403,7 @@ __device__ __forceinline__ u32 fx_bucket_pass(const FxArrays &f, u32 i, const ui
 }
 
 // step 3: one warp per listed position
-template <bool BUCKET>
-__global__ void __launch_bounds__(128, BUCKET ? 8 : 3) k_fx_recompute(FxArrays f, u64 G) {
+__global__ void __launch_bounds__(128, 8) k_fx_recompute(FxArrays f, u64 G) {
     __shared__ u32 s_x[4][FX_XCAP];
     __shared__ u32 s_seen[4];
     const u32 full = 0xFFFFFFFFu;
@@ -549,24 +418,19 @@ __global__ void __launch_bounds__(128, BUCKET ? 8 : 3) k_fx_recompute(FxArrays f
         if (w >= n_list) break;
         const u32 i = f.list[w];
         const uint4 a = f.rec[i];
-        const u32 ge = f.gend[i];
-        const u32 e = ge & ~FX_REV;
-        const bool fwd = !(ge & FX_REV);
-        const u32 c0 = BUCKET ? NONE32 : f.c0[i];
+        const bool fwd = !(f.gend[i] & FX_REV);
         u64 bd;
         u32 bj;
         u32 *n_seen = &s_seen[threadIdx.x >> 5];
         if (lane == 0) *n_seen = 0;
         __syncwarp();
-        FxExtra ex{f.minpi, f, i, xs, n_seen};
-        if (BUCKET) fx_bucket_pass<false>(f, i, a, fwd, G, G5, bd, bj, ex, nullptr);
-        else bb_best_successor_warp(f.rec, f.minpd, i, e, a, fwd, G, G5, bd, bj, c0, ex);
+        FxExtra ex{f, i, xs, n_seen};
+        fx_bucket_pass<false>(f, i, a, fwd, G, G5, bd, bj, ex, nullptr);
         __syncwarp();
         // X(i): normally out of the search's own record of blocked candidates; a separate pruned pass if that overflowed
         const u32 seen = *n_seen;
         const u32 xn = seen <= FX_XCAP && !f.force_collect ? fx_filter_seen(f.rec, a, fwd, G, G5, bd, bj, xs, seen)
-                       : BUCKET    ? fx_bucket_pass<true>(f, i, a, fwd, G, G5, bd, bj, ex, xs)
-                                   : fx_collect_blocked(f.rec, i, e, a, fwd, G, G5, bd, bj, c0, xs);
+                                                           : fx_bucket_pass<true>(f, i, a, fwd, G, G5, bd, bj, ex, xs);
         __syncwarp();
         u32 xo = 0;
         u16 xc = FX_XOVER;
@@ -580,10 +444,8 @@ __global__ void __launch_bounds__(128, BUCKET ? 8 : 3) k_fx_recompute(FxArrays f
                 atomicAdd(&f.ctrs[1], 1u);
                 if (old != NONE32) f.dirty[old >> FX_DB] = 1; // the picker lists of both successors change
                 if (bj != NONE32) f.dirty[bj >> FX_DB] = 1;
-                if (f.dbits_w) {
-                    if (old != NONE32) atomicOr(&f.dbits_w[old >> 5], 1u << (old & 31));
-                    if (bj != NONE32) atomicOr(&f.dbits_w[bj >> 5], 1u << (bj & 31));
-                }
+                if (old != NONE32) atomicOr(&f.dbits_w[old >> 5], 1u << (old & 31));
+                if (bj != NONE32) atomicOr(&f.dbits_w[bj >> 5], 1u << (bj & 31));
             }
             f.xhi[i] = hi;
             f.pick[i] = bj;
@@ -605,25 +467,22 @@ __global__ void __launch_bounds__(128, BUCKET ? 8 : 3) k_fx_recompute(FxArrays f
             for (u32 q = lane; q < xn; q += 32) {
                 const u32 jx = xs[q];
                 f.pool[xo + q] = jx;
-                if (BUCKET) {
-                    u64 d = 0;
-                    bb_candidate(a, f.rec[jx], fwd, G, G5, d); // valid by construction (fx_filter_seen / the collect pass)
-                    f.pool_d[xo + q] = d;
-                }
+                u64 d = 0;
+                bb_candidate(a, f.rec[jx], fwd, G, G5, d); // valid by construction (fx_filter_seen / the collect pass)
+                f.pool_d[xo + q] = d;
             }
         __syncwarp();
     }
 }
 
 // Resolve the huge groups.  hpos[k] = sorted position of k (ascending); gid / gstart / n_groups describe the groups in
-// sorted-position space; cand = k_chain_candidates' result there.  Writes root[] for the positions of huge groups and
-// returns true; returns false (root[] untouched) if the picks have not settled after SWG_FIXPOINT_MAX_ROUNDS rounds (default
-// 256): a dependency chain that long is walked faster sequentially, and the caller hands the groups to k_chain_resolve_warp.
-// cand == nullptr selects the target-bucket order: the first round evaluates every position against an empty snapshot (that IS
-// the unconstrained arg-min of the candidate pass), all searches go through fx_bucket_pass.  maxcoord bounds every coordinate.
+// sorted-position space.  Writes root[] for the positions of huge groups and returns true; returns false (root[] untouched)
+// if the picks have not settled after SWG_FIXPOINT_MAX_ROUNDS rounds (default 256): a dependency chain that long is walked
+// faster sequentially, and the caller hands the groups to k_chain_resolve_warp.  The first round evaluates every position
+// against an empty snapshot (that IS the unconstrained arg-min), all searches go through fx_bucket_pass.  maxcoord bounds
+// every coordinate.
 static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *srec, const u64 *skey, int cb, const u32 *gid, const u32 *gstart,
-                           u32 n_groups, u32 n_m, const Cand *cand, u64 G, u32 *root, u32 *bsum, u32 maxcoord) {
-    const bool bucket = cand == nullptr;
+                           u32 n_groups, u32 n_m, u64 G, u32 *root, u32 *bsum, u32 maxcoord) {
     cudaStream_t st = c->stream;
     LaunchCounter &lc = c->lc;
     Arena &A = c->arena;
@@ -632,16 +491,13 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     f.n = n_h;
     f.rec = A.take<uint4>(n_h);
     f.gend = A.take<u32>(n_h);
-    f.c0 = bucket ? nullptr : A.take<u32>(n_h);
     f.pick = A.take<u32>(n_h);
     f.pd = A.take<u64>(n_h);
     f.cnt = A.take<u32>(n_h);
     f.off = A.take<u32>((size_t)n_h + 1);
-    f.minpd = A.take<u64>(n_h);
     f.minpi = A.take<u32>(n_h);
     f.firstp = A.take<u32>(n_h);
-    f.li = bucket ? nullptr : A.take<u32>(n_h); // bucket order: the sorted positions of the round's sort
-    f.sorted = bucket ? 1 : 0;
+    f.li = nullptr; // the sorted positions of each round's sort
     f.force_collect = getenv("SWG_FX_FORCE_COLLECT") != nullptr;
     f.ld = A.take<u64>(n_h);
     f.xoff = A.take<u32>(n_h);
@@ -651,11 +507,11 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
         // that at 50 M); slots are powers of two and an outgrown slot is abandoned, so be generous where memory allows
         size_t free_b = 0, total_b = 0;
         SWG_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        const u64 want = (u64)n_h * 96 + 4096, fit = free_b / 2 / (bucket ? 12 : 4);
+        const u64 want = (u64)n_h * 96 + 4096, fit = free_b / 2 / 12;
         f.pool_cap = (u32)std::min<u64>(std::min<u64>(want, std::max<u64>(fit, (u64)n_h * 8 + 4096)), 0xF0000000ull);
     }
     f.pool = A.take<u32>(f.pool_cap);
-    f.pool_d = bucket ? A.take<u64>(f.pool_cap) : nullptr;
+    f.pool_d = A.take<u64>(f.pool_cap);
     f.pool_top = A.take<unsigned long long>(1);
     f.list = A.take<u32>(n_h);
     const u32 n_blk = (n_h >> FX_DB) + 1;
@@ -664,9 +520,8 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     f.dps = A.take<u32>((size_t)n_blk + 1);
     f.use_dirty = 0;
     const size_t n_bw = ((size_t)n_h >> 5) + 1;
-    f.dbits = bucket ? A.take<u32>(n_bw) : nullptr;
-    f.dbits_w = bucket ? A.take<u32>(n_bw) : nullptr;
-    const bool dirty_on = getenv("SWG_FX_NO_DIRTY") == nullptr; // testing aid: check every position in every round
+    f.dbits = A.take<u32>(n_bw);
+    f.dbits_w = A.take<u32>(n_bw);
     f.ctrs = A.take<u32>(4);
     u32 *scan_tot = A.take<u32>(1);
     SWG_CUDA(cudaMemsetAsync(f.xcnt, 0, sizeof(u16) * (size_t)n_h, st));
@@ -681,86 +536,79 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
             const bool fwd = ((skey[p] >> cb) & 1) == 0;
             g.rec[k] = srec[p];
             g.gend[k] = (k + (e - p)) | (fwd ? 0u : FX_REV);
-            if (bucket) { g.pick[k] = NONE32; g.xhi[k] = k; g.pd[k] = NONE64; return; }
-            const Cand cd = cand[p];
-            g.pick[k] = cd.j == NONE32 ? NONE32 : k + (cd.j - p);
-            g.xhi[k] = cd.j == NONE32 ? k : k + (cd.j - p);
-            g.pd[k] = cd.d;
-            g.c0[k] = cd.c0 == NONE32 ? NONE32 : k + (cd.c0 - p);
+            g.pick[k] = NONE32;
+            g.xhi[k] = k;
+            g.pd[k] = NONE64;
         });
     }
     u32 *h = reinterpret_cast<u32 *>(c->h_ctr + C_COUNT);
-    f.hg = nullptr; f.snap = nullptr; f.bq = nullptr; f.bk = nullptr; f.dir = nullptr; f.dirD = 0; f.bshift = 0;
-    if (bucket) {
-        // dense numbers of the huge groups (a group starts where the previous position's group ends)
-        f.hg = A.take<u32>(n_h);
-        f.snap = A.take<uint4>(2 * (size_t)n_h);
-        {
-            const FxArrays g = f;
-            scan_apply([=] __device__(u32 k) -> u32 { return (k == 0 || (g.gend[k - 1] & ~FX_REV) == k) ? 1u : 0u; },
-                       [=] __device__(u32 k, u32 ex, u32 v) { g.hg[k] = ex + v - 1; }, n_h, bsum, scan_tot, st, lc);
-        }
-        SWG_CUDA(cudaMemcpyAsync(h, scan_tot, sizeof(u32), cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaStreamSynchronize(st));
-        const u32 n_hg = h[0];
-        // bucket width: 1/32 of the smallest power of two >= G + G/5 + 1 (SWG_FX_BUCKET_NARROW=<log2 of the divisor>: tuning aid).
-        // A search visits the buckets outwards from the one that holds its own target coordinate and stops at the first whose
-        // nearest edge is further than sqrt(best d): narrow buckets keep the scans of the dense diagonal short, wide ones spare
-        // the scattered positions origin searches.  Wider if the directory (one entry per group and bucket) would pass 2^25
-        // entries or 2^20 per group.
-        const int narrow = getenv("SWG_FX_BUCKET_NARROW") ? atoi(getenv("SWG_FX_BUCKET_NARROW")) : 5;
-        int bs = std::max(bits_for(G + G / 5) - narrow, 4);
-        while (((((u64)maxcoord >> bs) + 2) * n_hg > (1ull << 25) || ((u64)maxcoord >> bs) + 2 > (1ull << 20)) && bs < 32) bs++;
-        f.bshift = bs;
-        const u32 nbk = (u32)(((u64)maxcoord >> bs) + 1);
-        f.dirD = nbk + 1;
-        const int tb = bits_for(nbk - 1 ? nbk - 1 : 1);
-        const size_t n_dir = (size_t)n_hg * f.dirD + 1;
-        u64 *bkey = A.take<u64>(n_h), *bkey2 = A.take<u64>(n_h);
-        u32 *bv = A.take<u32>(n_h), *bv2 = A.take<u32>(n_h);
-        {
-            const FxArrays g = f;
-            launch_for<t_fx_bkey>(n_h, st, lc, [=] __device__(u32 k) {
-                const uint4 r = g.rec[k];
-                const u32 t = (g.gend[k] & FX_REV) ? r.w : r.z; // '-' strand: the rule tests the candidate's target_end
-                bkey[k] = ((u64)g.hg[k] << tb) | ((u64)t >> bs);
-                bv[k] = k;
-            });
-        }
-        sort_pairs(c, bkey, bkey2, bv, bv2, n_h, tb + bits_for(n_hg > 1 ? n_hg - 1 : 1)); // stable: positions ascend inside a bucket
-        f.bk = bv;
-        f.bq = A.take<uint2>(n_h);
-        f.dir = A.take<u32>(n_dir);
-        {
-            const FxArrays g = f;
-            const u64 *ks = bkey;
-            const u32 D = f.dirD;
-            launch_for<t_fx_brec>(n_h, st, lc, [=] __device__(u32 m) {
-                {
-                    const u32 k = g.bk[m];
-                    const uint4 r = g.rec[k];
-                    g.bq[m] = make_uint2(r.x, (g.gend[k] & FX_REV) ? r.w : r.z);
-                }
-                // directory: dir[x] = first entry whose (group, bucket) slot is >= x
-                const u64 km = ks[m];
-                const u64 slot = (km >> tb) * D + (km & ((1ull << tb) - 1));
-                u64 from = 0;
-                if (m > 0) { const u64 kp = ks[m - 1]; from = (kp >> tb) * D + (kp & ((1ull << tb) - 1)) + 1; }
-                for (u64 x = from; x <= slot; x++) g.dir[x] = m;
-                if (m + 1 == g.n)
-                    for (u64 x = slot + 1; x < n_dir; x++) g.dir[x] = g.n;
-            });
-        }
-        if (verbose) fprintf(stderr, "[swg fixpoint] target buckets: %u huge groups, 2^%d wide, %u per group\n", n_hg, bs, nbk);
+    // dense numbers of the huge groups (a group starts where the previous position's group ends)
+    f.hg = A.take<u32>(n_h);
+    f.snap = A.take<uint4>(2 * (size_t)n_h);
+    {
+        const FxArrays g = f;
+        scan_apply([=] __device__(u32 k) -> u32 { return (k == 0 || (g.gend[k - 1] & ~FX_REV) == k) ? 1u : 0u; },
+                   [=] __device__(u32 k, u32 ex, u32 v) { g.hg[k] = ex + v - 1; }, n_h, bsum, scan_tot, st, lc);
     }
+    SWG_CUDA(cudaMemcpyAsync(h, scan_tot, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    SWG_CUDA(cudaStreamSynchronize(st));
+    const u32 n_hg = h[0];
+    // bucket width: 1/32 of the smallest power of two >= G + G/5 + 1 (SWG_FX_BUCKET_NARROW=<log2 of the divisor>: tuning aid).
+    // A search visits the buckets outwards from the one that holds its own target coordinate and stops at the first whose
+    // nearest edge is further than sqrt(best d): narrow buckets keep the scans of the dense diagonal short, wide ones spare
+    // the scattered positions origin searches.  Wider if the directory (one entry per group and bucket) would pass 2^25
+    // entries or 2^20 per group.
+    const int narrow = getenv("SWG_FX_BUCKET_NARROW") ? atoi(getenv("SWG_FX_BUCKET_NARROW")) : 5;
+    int bs = std::max(bits_for(G + G / 5) - narrow, 4);
+    while (((((u64)maxcoord >> bs) + 2) * n_hg > (1ull << 25) || ((u64)maxcoord >> bs) + 2 > (1ull << 20)) && bs < 32) bs++;
+    f.bshift = bs;
+    const u32 nbk = (u32)(((u64)maxcoord >> bs) + 1);
+    f.dirD = nbk + 1;
+    const int tb = bits_for(nbk - 1 ? nbk - 1 : 1);
+    const size_t n_dir = (size_t)n_hg * f.dirD + 1;
+    u64 *bkey = A.take<u64>(n_h), *bkey2 = A.take<u64>(n_h);
+    u32 *bv = A.take<u32>(n_h), *bv2 = A.take<u32>(n_h);
+    {
+        const FxArrays g = f;
+        launch_for<t_fx_bkey>(n_h, st, lc, [=] __device__(u32 k) {
+            const uint4 r = g.rec[k];
+            const u32 t = (g.gend[k] & FX_REV) ? r.w : r.z; // '-' strand: the rule tests the candidate's target_end
+            bkey[k] = ((u64)g.hg[k] << tb) | ((u64)t >> bs);
+            bv[k] = k;
+        });
+    }
+    sort_pairs(c, bkey, bkey2, bv, bv2, n_h, tb + bits_for(n_hg > 1 ? n_hg - 1 : 1)); // stable: positions ascend inside a bucket
+    f.bk = bv;
+    f.bq = A.take<uint2>(n_h);
+    f.dir = A.take<u32>(n_dir);
+    {
+        const FxArrays g = f;
+        const u64 *ks = bkey;
+        const u32 D = f.dirD;
+        launch_for<t_fx_brec>(n_h, st, lc, [=] __device__(u32 m) {
+            {
+                const u32 k = g.bk[m];
+                const uint4 r = g.rec[k];
+                g.bq[m] = make_uint2(r.x, (g.gend[k] & FX_REV) ? r.w : r.z);
+            }
+            // directory: dir[x] = first entry whose (group, bucket) slot is >= x
+            const u64 km = ks[m];
+            const u64 slot = (km >> tb) * D + (km & ((1ull << tb) - 1));
+            u64 from = 0;
+            if (m > 0) { const u64 kp = ks[m - 1]; from = (kp >> tb) * D + (kp & ((1ull << tb) - 1)) + 1; }
+            for (u64 x = from; x <= slot; x++) g.dir[x] = m;
+            if (m + 1 == g.n)
+                for (u64 x = slot + 1; x < n_dir; x++) g.dir[x] = g.n;
+        });
+    }
+    if (verbose) fprintf(stderr, "[swg fixpoint] target buckets: %u huge groups, 2^%d wide, %u per group\n", n_hg, bs, nbk);
     int rounds = 0;
     const int max_rounds = getenv("SWG_FIXPOINT_MAX_ROUNDS") ? atoi(getenv("SWG_FIXPOINT_MAX_ROUNDS")) : 256;
     u64 total_recomputed = 0;
     auto t_round = std::chrono::steady_clock::now();
-    if (bucket) {
-        // round 0: every position against the empty snapshot = the unconstrained arg-min (nothing is blocked: X(i) stays empty)
-        const FxArrays g = f;
-        SWG_CUDA(cudaMemsetAsync(f.minpd, 0xFF, sizeof(u64) * (size_t)n_h, st));
+    {
+        // round 0: every position against the empty snapshot = the unconstrained arg-min (nothing is blocked: X(i) stays empty).
+        // A thread scans the next successors of its position first; only a window that goes on is left to the warp search.
         SWG_CUDA(cudaMemsetAsync(f.minpi, 0xFF, sizeof(u32) * (size_t)n_h, st));
         SWG_CUDA(cudaMemsetAsync(f.firstp, 0xFF, sizeof(u32) * (size_t)n_h, st));
         SWG_CUDA(cudaMemsetAsync(f.off, 0, sizeof(u32) * ((size_t)n_h + 1), st));
@@ -768,14 +616,9 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
         SWG_CUDA(cudaMemsetAsync(f.dbits_w, 0, sizeof(u32) * n_bw, st));
         SWG_CUDA(cudaMemsetAsync(f.dirty, 0, sizeof(u32) * (size_t)n_blk, st));
         SWG_CUDA(cudaMemsetAsync(f.ctrs, 0, 4 * sizeof(u32), st));
-        if (getenv("SWG_FX_NO_LINEAR0"))
-            launch_for<t_fx_all>(n_h, st, lc, [=] __device__(u32 k) {
-                g.list[k] = k;
-                if (k == 0) g.ctrs[0] = g.n;
-            });
-        else { k_fx_round0_linear<<<cdiv(n_h, 256), 256, 0, st>>>(f, G); lc.n++; }
-        k_fx_recompute<true><<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
-        lc.n++;
+        k_fx_round0_linear<<<cdiv(n_h, 256), 256, 0, st>>>(f, G);
+        k_fx_recompute<<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
+        lc.n += 2;
         if (verbose) {
             SWG_CUDA(cudaStreamSynchronize(st));
             const auto t1 = std::chrono::steady_clock::now();
@@ -783,18 +626,13 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
             t_round = t1;
         }
     }
-    // bucket order: picker lists in position order (stable sort of the positions by their pick), picker d as prefix minima
-    u64 *sk = nullptr, *sk2 = nullptr;
-    u32 *sv = nullptr, *sv2 = nullptr;
-    void *stmp = nullptr;
-    RadixSortPlan sp;
-    if (bucket) {
-        sk = A.take<u64>(n_h); sk2 = A.take<u64>(n_h); sv = A.take<u32>(n_h); sv2 = A.take<u32>(n_h);
-        sp = rs_plan(n_h, 0, bits_for(n_h));
-        stmp = A.take<char>(sp.temp_bytes);
-    }
+    // picker lists in position order (stable sort of the positions by their pick), picker d as prefix minima
+    u64 *sk = A.take<u64>(n_h), *sk2 = A.take<u64>(n_h);
+    u32 *sv = A.take<u32>(n_h), *sv2 = A.take<u32>(n_h);
+    const RadixSortPlan sp = rs_plan(n_h, 0, bits_for(n_h));
+    void *stmp = A.take<char>(sp.temp_bytes);
     while (true) {
-        if (bucket) {
+        {
             const FxArrays gs = f;
             u64 *kk = sk;
             u32 *vv = sv;
@@ -806,8 +644,8 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
             rs_sort_pairs(sp, sk, sk2, sv, sv2, stmp, st, c->sm_count, lc);
             f.li = sv;
         }
-        // 0. which blocks of successors saw a picker list change in the last round (prefix counts for k_fx_check)
-        if (dirty_on && rounds > 0) {
+        // 0. which blocks of successors saw a picker list change in the last round (prefix counts for k_fx_check_warp)
+        if (rounds > 0) {
             const FxArrays gd = f;
             scan_apply([=] __device__(u32 b) -> u32 { return gd.dirty[b]; },
                        [=] __device__(u32 b, u32 ex, u32 v) {
@@ -818,64 +656,38 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
             f.use_dirty = 1;
         }
         SWG_CUDA(cudaMemsetAsync(f.dirty, 0, sizeof(u32) * (size_t)n_blk, st));
-        if (f.dbits) { // what the last round's re-evaluations marked is read by this round's check
-            std::swap(f.dbits, f.dbits_w);
-            SWG_CUDA(cudaMemsetAsync(f.dbits_w, 0, sizeof(u32) * n_bw, st));
-        }
+        // what the last round's re-evaluations marked is read by this round's check
+        std::swap(f.dbits, f.dbits_w);
+        SWG_CUDA(cudaMemsetAsync(f.dbits_w, 0, sizeof(u32) * n_bw, st));
         // 1. snapshot of the picks
         const FxArrays g = f;
         SWG_CUDA(cudaMemsetAsync(f.cnt, 0, sizeof(u32) * (size_t)n_h, st));
         SWG_CUDA(cudaMemsetAsync(f.ctrs, 0, 4 * sizeof(u32), st));
-        if (!bucket) {
-            SWG_CUDA(cudaMemsetAsync(f.minpd, 0xFF, sizeof(u64) * (size_t)n_h, st));
-            SWG_CUDA(cudaMemsetAsync(f.minpi, 0xFF, sizeof(u32) * (size_t)n_h, st));
-            SWG_CUDA(cudaMemsetAsync(f.firstp, 0xFF, sizeof(u32) * (size_t)n_h, st));
-        }
         launch_for<t_fx_count>(n_h, st, lc, [=] __device__(u32 k) {
             const u32 j = g.pick[k];
-            if (j != NONE32) {
-                atomicAdd(&g.cnt[j], 1u);
-                if (!g.sorted) { // (sorted lists: the per-successor pass below reads both off its list)
-                    atomicMin((unsigned long long *)&g.minpd[j], (unsigned long long)g.pd[k]);
-                    atomicMin(&g.firstp[j], k);
-                }
-            }
+            if (j != NONE32) atomicAdd(&g.cnt[j], 1u);
         });
-        if (!bucket)
-            launch_for<t_fx_minpi>(n_h, st, lc, [=] __device__(u32 k) {
-                const u32 j = g.pick[k];
-                if (j != NONE32 && g.pd[k] == g.minpd[j]) atomicMin(&g.minpi[j], k);
-            });
         scan_apply([=] __device__(u32 k) -> u32 { return g.cnt[k]; },
                    [=] __device__(u32 k, u32 ex, u32 v) {
                        g.off[k] = ex;
                        if (k + 1 == g.n) g.off[g.n] = ex + v;
                    },
                    n_h, bsum, scan_tot, st, lc);
-        if (bucket) // one pass per successor over its list (position order): prefix minima, who holds the minimum first, the packed words
-            launch_for<t_fx_pm>(n_h, st, lc, [=] __device__(u32 j) {
-                const u32 a = g.off[j], b = g.off[j + 1];
-                u64 m = NONE64, fd = NONE64;
-                u32 mi = NONE32, fp = NONE32;
-                for (u32 p = a; p < b; p++) {
-                    const u32 k = g.li[p];
-                    const u64 d = g.pd[k];
-                    if (p == a) { fp = k; fd = d; }
-                    if (d < m) { m = d; mi = k; }
-                    g.ld[p] = m;
-                }
-                g.minpd[j] = m; g.minpi[j] = mi; g.firstp[j] = fp;
-                g.snap[2 * (size_t)j] = make_uint4((u32)m, (u32)(m >> 32), mi, fp);
-                g.snap[2 * (size_t)j + 1] = make_uint4((u32)fd, (u32)(fd >> 32), a, b - a);
-            });
-        else
-        launch_for<t_fx_fill>(n_h, st, lc, [=] __device__(u32 k) {
-            const u32 j = g.pick[k];
-            if (j != NONE32) {
-                const u32 slot = g.off[j] + atomicSub(&g.cnt[j], 1u) - 1;
-                g.li[slot] = k;
-                g.ld[slot] = g.pd[k];
+        // one pass per successor over its list (position order): prefix minima, who holds the minimum first, the packed words
+        launch_for<t_fx_pm>(n_h, st, lc, [=] __device__(u32 j) {
+            const u32 a = g.off[j], b = g.off[j + 1];
+            u64 m = NONE64, fd = NONE64;
+            u32 mi = NONE32, fp = NONE32;
+            for (u32 p = a; p < b; p++) {
+                const u32 k = g.li[p];
+                const u64 d = g.pd[k];
+                if (p == a) { fp = k; fd = d; }
+                if (d < m) { m = d; mi = k; }
+                g.ld[p] = m;
             }
+            g.minpi[j] = mi; g.firstp[j] = fp;
+            g.snap[2 * (size_t)j] = make_uint4((u32)m, (u32)(m >> 32), mi, fp);
+            g.snap[2 * (size_t)j + 1] = make_uint4((u32)fd, (u32)(fd >> 32), a, b - a);
         });
         // 2. + 3.
         double ms_snap = 0, ms_check = 0;
@@ -886,11 +698,9 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
             ms = std::chrono::duration<double, std::milli>(t1 - t_round).count();
         };
         lap(ms_snap);
-        if (bucket) k_fx_check_warp<<<cdiv(n_h, 256), 256, 0, st>>>(f, G);
-        else k_fx_check<<<cdiv(n_h, 256), 256, 0, st>>>(f, G);
+        k_fx_check_warp<<<cdiv(n_h, 256), 256, 0, st>>>(f, G);
         lap(ms_check);
-        if (bucket) k_fx_recompute<true><<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
-        else k_fx_recompute<false><<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
+        k_fx_recompute<<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
         lc.n += 2;
         SWG_CUDA(cudaMemcpyAsync(h, f.ctrs, 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
         if (verbose) SWG_CUDA(cudaMemcpyAsync(h + 4, f.pool_top, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
@@ -912,15 +722,14 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     }
     if (getenv("SWG_FIXPOINT_VERIFY")) {
         // Self-check for sizes no oracle reaches: (*) has exactly one solution, so it suffices that EVERY position, evaluated
-        // from scratch against the final snapshot, reproduces its pick (this bypasses the X(i) bookkeeping of k_fx_check).
+        // from scratch against the final snapshot, reproduces its pick (this bypasses the X(i) bookkeeping of k_fx_check_warp).
         const FxArrays g = f;
         SWG_CUDA(cudaMemsetAsync(f.ctrs, 0, 4 * sizeof(u32), st));
         launch_for<t_fx_all>(n_h, st, lc, [=] __device__(u32 k) {
             g.list[k] = k;
             if (k == 0) g.ctrs[0] = g.n;
         });
-        if (bucket) k_fx_recompute<true><<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
-        else k_fx_recompute<false><<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
+        k_fx_recompute<<<(u32)c->sm_count * 8, 128, 0, st>>>(f, G);
         lc.n++;
         SWG_CUDA(cudaMemcpyAsync(h, f.ctrs, 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
         SWG_CUDA(cudaStreamSynchronize(st));

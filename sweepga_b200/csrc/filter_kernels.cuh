@@ -512,20 +512,9 @@ __device__ __forceinline__ void bb_argmin(u64 &bd, u32 &bj) { // smallest d, the
 #ifndef SWG_RESCAN_WIDTH
 #define SWG_RESCAN_WIDTH 128
 #endif
-// `extra(j, d)` is consulted only for a candidate that fails the plain test d < bps[j]: the sequential walk passes BbNoExtra
-// (never eligible then); the fixed-point resolve (chain_fixpoint.cuh) passes bps = the smallest d over ALL current pickers
-// of j and decides the exact "smallest d over the pickers before i" there.
-// An Extra with PREFETCH = true names a per-successor u32 column `pi` that is loaded together with bps[j] (same index, same
-// round trip) and handed to the call, so that the common verdicts need no dependent load.
-struct BbNoExtra {
-    static constexpr u32 OUTWARD = SWG_RESCAN_WIDTH; // candidates per outward round
-    static constexpr bool PREFETCH = false;
-    const u32 *pi = nullptr;
-    __device__ __forceinline__ bool operator()(u32, u64, u32) const { return false; }
-};
-template <class Extra>
+// The blocked step of the sequential walk: the arg-min over the candidates j that pass the eligibility test d < bps[j].
 __device__ __forceinline__ void bb_best_successor_warp(const uint4 *__restrict__ srec, const u64 *bps, u32 i, u32 e, const uint4 &a,
-                                                       bool fwd, u64 G, u64 G5, u64 &bd, u32 &bj, u32 c0_hint, Extra extra) {
+                                                       bool fwd, u64 G, u64 G5, u64 &bd, u32 &bj, u32 c0_hint) {
     const u32 full = 0xFFFFFFFFu;
     const u32 lane = lane_id();
     const u64 bound = (u64)a.y + G;
@@ -549,7 +538,6 @@ __device__ __forceinline__ void bb_best_successor_warp(const uint4 *__restrict__
         uint4 rb[2 + 2 * (RW / 32)];
         u64 rp[2 + 2 * (RW / 32)];
         u32 rj[2 + 2 * (RW / 32)];
-        u32 rq[2 + 2 * (RW / 32)];
 #pragma unroll
         for (u32 k = 0; k < 2; k++) {
             const u32 j = i + 1 + k * 32 + lane;
@@ -563,10 +551,8 @@ __device__ __forceinline__ void bb_best_successor_warp(const uint4 *__restrict__
             rj[2 + RW / 32 + k] = off < lcnt ? c0 - 1 - off : NONE32;
         }
 #pragma unroll
-        for (u32 k = 0; k < 2 + 2 * (RW / 32); k++) {
-            rq[k] = 0;
-            if (rj[k] != NONE32) { rb[k] = srec[rj[k]]; rp[k] = bps[rj[k]]; if (Extra::PREFETCH) rq[k] = extra.pi[rj[k]]; }
-        }
+        for (u32 k = 0; k < 2 + 2 * (RW / 32); k++)
+            if (rj[k] != NONE32) { rb[k] = srec[rj[k]]; rp[k] = bps[rj[k]]; }
         rnext = c0 + RW < e ? (u64)srec[c0 + RW].x : NONE64; // first candidate of the next right round (pruning test)
         lnext = c0 - lcnt > jl ? (u64)srec[c0 - lcnt - 1].x : NONE64;
 #pragma unroll
@@ -578,7 +564,7 @@ __device__ __forceinline__ void bb_best_successor_warp(const uint4 *__restrict__
             else if (k < 2 + RW / 32) inwin = (u64)b.x - a.y <= G;      // right of the origin: q_gap <= G
             else inwin = true;                                          // left of the origin: overlap, judged by the gap rule
             u64 d;
-            if (inwin && bb_candidate(a, b, fwd, G, G5, d) && (d < ld || (d == ld && rj[k] < lj)) && (d < rp[k] || extra(rj[k], d, rq[k]))) { ld = d; lj = rj[k]; }
+            if (inwin && bb_candidate(a, b, fwd, G, G5, d) && (d < ld || (d == ld && rj[k] < lj)) && d < rp[k]) { ld = d; lj = rj[k]; }
         }
         bb_argmin(ld, lj);
         bd = ld;
@@ -596,7 +582,7 @@ __device__ __forceinline__ void bb_best_successor_warp(const uint4 *__restrict__
                 const uint4 b = srec[j];
                 inwin = (u64)b.x <= bound;
                 u64 d;
-                if (inwin && bb_candidate(a, b, fwd, G, G5, d) && (d < bd || (d == bd && j < bj)) && (d < bps[j] || extra(j, d, Extra::PREFETCH ? extra.pi[j] : 0u))) { bd = d; bj = j; }
+                if (inwin && bb_candidate(a, b, fwd, G, G5, d) && (d < bd || (d == bd && j < bj)) && d < bps[j]) { bd = d; bj = j; }
             }
             exhausted = !__all_sync(full, inwin || j >= lin_end);
         }
@@ -626,58 +612,53 @@ __device__ __forceinline__ void bb_best_successor_warp(const uint4 *__restrict__
     }
     // Outward rounds.  The pruning test looks at the first candidate of a round only; candidates past the exact pruning
     // point have d >= q_gap^2 > best d and cannot win, so reading a few more of them changes nothing.
-    constexpr u32 OW = Extra::OUTWARD; // outward rounds may be wider than the fused first round: one memory round trip per OW candidates
-    for (u32 base = rbase; base < e; base += OW) { // right side, q_gap >= 0 non-decreasing
+    for (u32 base = rbase; base < e; base += RW) { // right side, q_gap >= 0 non-decreasing
         const u64 qg0 = rnext - a.y;
         if (rnext == NONE64 || qg0 > G || qg0 * qg0 > bd) break;
-        uint4 rb[OW / 32];
-        u64 rp[OW / 32];
-        u32 rq[OW / 32];
+        uint4 rb[RW / 32];
+        u64 rp[RW / 32];
 #pragma unroll
-        for (u32 k = 0; k < OW / 32; k++) {
+        for (u32 k = 0; k < RW / 32; k++) {
             const u32 r = base + k * 32 + lane;
-            rq[k] = 0;
-            if (r < e) { rb[k] = srec[r]; rp[k] = bps[r]; if (Extra::PREFETCH) rq[k] = extra.pi[r]; }
+            if (r < e) { rb[k] = srec[r]; rp[k] = bps[r]; }
         }
-        rnext = base + OW < e ? (u64)srec[base + OW].x : NONE64;
+        rnext = base + RW < e ? (u64)srec[base + RW].x : NONE64;
         u64 ld = bd; // every lane starts from the best so far: only a candidate that beats it is tested for eligibility
         u32 lj = bj;
 #pragma unroll
-        for (u32 k = 0; k < OW / 32; k++) {
+        for (u32 k = 0; k < RW / 32; k++) {
             const u32 r = base + k * 32 + lane;
             if (r < e) {
                 const u64 qg = (u64)rb[k].x - a.y;
                 u64 d;
-                if (qg <= G && bb_candidate(a, rb[k], fwd, G, G5, d) && d < ld && (d < rp[k] || extra(r, d, rq[k]))) { ld = d; lj = r; } // r ascends: ties keep the smaller j
+                if (qg <= G && bb_candidate(a, rb[k], fwd, G, G5, d) && d < ld && d < rp[k]) { ld = d; lj = r; } // r ascends: ties keep the smaller j
             }
         }
         bb_argmin(ld, lj);
         bd = ld;
         bj = lj;
     }
-    for (u32 top = ltop; top > jl;) { // left side, overlap > 0 non-decreasing going left; round = [top-OW, top)
+    for (u32 top = ltop; top > jl;) { // left side, overlap > 0 non-decreasing going left; round = [top-RW, top)
         const u64 ov0 = (u64)a.y - lnext;
         if (lnext == NONE64 || ov0 > G5 || ov0 * ov0 > bd) break;
-        const u32 cnt = min(OW, top - jl);
-        uint4 rb[OW / 32];
-        u64 rp[OW / 32];
-        u32 rq[OW / 32];
+        const u32 cnt = min(RW, top - jl);
+        uint4 rb[RW / 32];
+        u64 rp[RW / 32];
 #pragma unroll
-        for (u32 k = 0; k < OW / 32; k++) {
+        for (u32 k = 0; k < RW / 32; k++) {
             const u32 off = k * 32 + lane;
-            rq[k] = 0;
-            if (off < cnt) { rb[k] = srec[top - 1 - off]; rp[k] = bps[top - 1 - off]; if (Extra::PREFETCH) rq[k] = extra.pi[top - 1 - off]; }
+            if (off < cnt) { rb[k] = srec[top - 1 - off]; rp[k] = bps[top - 1 - off]; }
         }
         lnext = top - cnt > jl ? (u64)srec[top - cnt - 1].x : NONE64;
         u64 ld = bd;
         u32 lj = bj;
 #pragma unroll
-        for (u32 k = 0; k < OW / 32; k++) {
+        for (u32 k = 0; k < RW / 32; k++) {
             const u32 off = k * 32 + lane;
             if (off < cnt) {
                 const u32 l = top - 1 - off;
                 u64 d;
-                if (bb_candidate(a, rb[k], fwd, G, G5, d) && (d < ld || (d == ld && l < lj)) && (d < rp[k] || extra(l, d, rq[k]))) { ld = d; lj = l; }
+                if (bb_candidate(a, rb[k], fwd, G, G5, d) && (d < ld || (d == ld && l < lj)) && d < rp[k]) { ld = d; lj = l; }
             }
         }
         bb_argmin(ld, lj);
@@ -728,7 +709,7 @@ k_chain_resolve_warp(const Cand *__restrict__ cand, const uint4 *__restrict__ sr
                 if (cd < bt) { wd = cd; wj = cj; }
                 else {
                     const uint4 a = srec[i];
-                    bb_best_successor_warp(srec, bps, i, e, a, fwd, G, G5, wd, wj, __shfl_sync(full, ck.c0, t), BbNoExtra{});
+                    bb_best_successor_warp(srec, bps, i, e, a, fwd, G, G5, wd, wj, __shfl_sync(full, ck.c0, t));
                 }
                 if (wj != NONE32) {
                     if (lane == 0) { bps[wj] = wd; pred[wj] = i; }
@@ -1059,8 +1040,8 @@ __device__ __forceinline__ bool act_less(const ActEntry &a, const ActEntry &b) {
 // looks at its neighbours in start order: to the right while start_k < end_m, to the left while some item at or left of k
 // still reaches start_m — one load of the group's running maximum of the interval ends (pmax[k] = max end over the group's
 // items up to k, scan_segmax): on collinear data the scan stops after a step or two however long the longest item of the group
-// is.  S(p) changes only at the starts and ends of those neighbours.  Groups where a scan gets long (deep piles, one very long item) go to the warp-per-group kernel, which
-// redoes the whole group and k_sweep_keep_big overwrites the keep bytes of its items.
+// is.  S(p) changes only at the starts and ends of those neighbours.  Groups where a scan gets long (deep piles, one very long item)
+// are listed and go through the position-parallel tree sweep (sweep_tree.cuh), which decides the keep bytes of their items.
 constexpr u32 SWF_LEFT = 48, SWF_RIGHT = 48;
 // the verdict of one item (sorted position u): everything k_sweep_flat1's header describes
 __device__ __forceinline__ void sweep_flat1_item(u32 u, const u32 *__restrict__ sitem, const SweepItem *__restrict__ sdata, const u32 *__restrict__ gid,
@@ -1172,21 +1153,6 @@ k_sweep_flat1_rest(const u32 *__restrict__ rest, const u32 *__restrict__ rest_co
     const u32 n = *rest_count;
     for (u32 x = blockIdx.x * blockDim.x + threadIdx.x; x < n; x += gridDim.x * blockDim.x)
         sweep_flat1_item(rest[x], sitem, sdata, gid, gstart, pmax, n_groups, n_sorted, thr, keep, gflag, big_list, big_count, ctr, scan_limit);
-}
-
-// keep = good && !flagged for the items of the groups the warp kernel redid (n_keep == 1 path)
-__global__ void __launch_bounds__(128) k_sweep_keep_big(const u32 *__restrict__ sitem, const u32 *__restrict__ gstart, u32 n_groups, u32 n_sorted,
-                                                        const u32 *__restrict__ big_list, const u32 *__restrict__ big_count,
-                                                        const u8 *__restrict__ good, const u8 *__restrict__ flagged, u8 *__restrict__ keep) {
-    const u32 n_big = *big_count;
-    for (u32 w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_big; w += (gridDim.x * blockDim.x) >> 5) {
-        const u32 g = big_list[w];
-        const u32 gs = gstart[g], ge = (g + 1 < n_groups) ? gstart[g + 1] : n_sorted;
-        for (u32 k = gs + lane_id(); k < ge; k += 32) {
-            const u32 i = sitem[k];
-            keep[i] = (good[i] && !flagged[i]) ? 1 : 0;
-        }
-    }
 }
 
 // sort keys of the included items: (group << pbits) | start, payload = item (pbits == 64: the start alone, the group id

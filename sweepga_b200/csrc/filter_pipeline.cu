@@ -118,42 +118,33 @@ struct Arena {
 namespace swg {
 // Environment knobs (diagnostics and tests, DESIGN 7b).  Read once per entry point, never cached across calls.
 struct Knobs {
-    bool force_wide = false, sweep_no_flat = false, no_fixpoint = false, fx_no_buckets = false, inv_grid = false, inv_no_grid = false, inv_no_diag = false, inv_wide = false, inv_narrow = false, cuda_log = false;
-    bool pairs_sort = false;   // SWG_SORT_PAIRS=1: the record sort keeps (key, payload) pairs through every pass
+    bool force_wide = false, no_fixpoint = false, inv_grid = false, inv_no_diag = false, inv_wide = false, inv_narrow = false, cuda_log = false;
     bool no_fused_keys = false; // SWG_NO_FUSED_KEYS=1: the chain sort keys always come from k_chain_keys
     bool no_group_sort = false; // SWG_NO_GROUP_SORT=1: the record sort always runs the LSD passes (radix_sort.cuh)
-    bool sweep_no_tree = false, sweep_tree_all = false; // SWG_SWEEP_NO_TREE=1: piles of an n = 1 sweep go through the warp walk; SWG_SWEEP_TREE_ALL=1: every group through the tree (tests)
+    bool sweep_tree_all = false; // SWG_SWEEP_TREE_ALL=1: every group of an n = 1 sweep through the tree (tests)
     bool group_sort_always = false; // SWG_GROUP_SORT_ALWAYS=1: ... never because the rows look ungrouped (tests)
     u32 group_sort_max = 0;     // SWG_GROUP_SORT_MAX: largest group the group sort accepts (default GS_CTA_MAX; tests lower it)
     u32 fixpoint_min = 0;      // 0 = default
     double max_pair_evals = 0; // 0 = no limit (SWG_MAX_PAIR_EVALS)
-    int sweep_mult = 8, resolve_mult = 4;
     int exact_scores = 0;      // SWG_EXACT_SCORES: 0 auto, 1 always, 2 never
 };
 static Knobs read_knobs() {
     Knobs k;
     auto on = [](const char *n) { const char *v = getenv(n); return v != nullptr && *v && strcmp(v, "0") != 0; };
     k.force_wide = on("SWG_FORCE_WIDE_KEYS");
-    k.sweep_no_flat = on("SWG_SWEEP_NO_FLAT");
     k.no_fixpoint = on("SWG_NO_FIXPOINT");
-    k.fx_no_buckets = on("SWG_FX_NO_BUCKETS");
     k.inv_grid = on("SWG_INV_GRID");
     k.inv_no_diag = on("SWG_INV_NO_DIAG");
     k.inv_wide = on("SWG_INV_WIDE");
     k.inv_narrow = on("SWG_INV_NARROW");
-    k.inv_no_grid = on("SWG_INV_NO_GRID");
-    k.pairs_sort = on("SWG_SORT_PAIRS");
     k.no_fused_keys = on("SWG_NO_FUSED_KEYS");
     k.no_group_sort = on("SWG_NO_GROUP_SORT");
     k.group_sort_always = on("SWG_GROUP_SORT_ALWAYS");
-    k.sweep_no_tree = on("SWG_SWEEP_NO_TREE");
     k.sweep_tree_all = on("SWG_SWEEP_TREE_ALL");
     if (const char *v = getenv("SWG_GROUP_SORT_MAX")) k.group_sort_max = (u32)atoi(v);
     if (const char *v = getenv("SWG_LOG_IMPL")) k.cuda_log = strcmp(v, "cuda") == 0;
     if (const char *v = getenv("SWG_FIXPOINT_MIN")) k.fixpoint_min = (u32)atoi(v);
     if (const char *v = getenv("SWG_MAX_PAIR_EVALS")) k.max_pair_evals = atof(v);
-    if (const char *v = getenv("SWG_SWEEP_MULT")) k.sweep_mult = std::max(1, atoi(v));
-    if (const char *v = getenv("SWG_RESOLVE_MULT")) k.resolve_mult = std::max(1, atoi(v));
     if (const char *v = getenv("SWG_EXACT_SCORES")) k.exact_scores = strcmp(v, "always") == 0 ? 1 : strcmp(v, "never") == 0 ? 2 : 0;
     return k;
 }
@@ -506,11 +497,7 @@ static void general_sweep_impl(swg_ctx *c, u32 n_items, const u8 *include, u8 in
                    n_inc, bsum, d_ng, st, c->lc);
         n_groups = read_u32(c, d_ng);
     }
-    const bool no_flat = c->knobs.sweep_no_flat; // testing aid: the sequential kernels for every n
-    u32 *ends = (n_keep == 1 && !no_flat) ? c->arena.take<u32>(n_inc) : nullptr; // interval ends in sorted order (for the running maximum)
-    u8 *good = c->arena.take<u8>(n_items), *flagged = c->arena.take<u8>(n_items);
-    SWG_CUDA(cudaMemsetAsync(good, 0, n_items, st));
-    SWG_CUDA(cudaMemsetAsync(flagged, 0, n_items, st));
+    u32 *ends = n_keep == 1 ? c->arena.take<u32>(n_inc) : nullptr; // interval ends in sorted order (for the running maximum)
     // per-item copies (score key, axis interval) in sorted order: a group becomes one contiguous stream
     SweepItem *sdata = c->arena.take<SweepItem>(n_inc);
     u32 *gflag = c->arena.take<u32>(n_groups);
@@ -529,7 +516,7 @@ static void general_sweep_impl(swg_ctx *c, u32 n_items, const u8 *include, u8 in
         });
     }
     u32 *pmax = nullptr;
-    if (n_keep == 1 && !no_flat) { // running maximum of the interval ends inside every group (bounds the leftward scan of k_sweep_flat1)
+    if (n_keep == 1) { // running maximum of the interval ends inside every group (bounds the leftward scan of k_sweep_flat1)
         pmax = c->arena.take<u32>(n_inc);
         u32 *tmp = c->arena.take<u32>(scan_temp_u32(n_inc));
         const u32 *gidc = gid;
@@ -541,41 +528,33 @@ static void general_sweep_impl(swg_ctx *c, u32 n_items, const u8 *include, u8 in
     u32 *sw_ctr = c->arena.take<u32>(4); // [0] thread-kernel group counter, [1] deep groups, [2] warp-kernel work counter
     SWG_CUDA(cudaMemsetAsync(sw_ctr, 0, 4 * sizeof(u32), st));
     stage_mark(c, "gs_sweep");
-    if (n_keep == 1 && !no_flat) {
+    if (n_keep == 1) {
         u32 *rest = c->arena.take<u32>(n_inc);
         const u32 limit = c->knobs.sweep_tree_all ? 0u : SWF_LEFT;
         k_sweep_flat1<<<cdiv(n_inc, 1024), 256, 0, st>>>(ev, sdata, gid, gstart, pmax, n_groups, n_inc, keep, rest, sw_ctr + 3, limit);
         k_sweep_flat1_rest<<<(u32)c->sm_count * 8, 256, 0, st>>>(rest, sw_ctr + 3, ev, sdata, gid, gstart, pmax, n_groups, n_inc, thr, keep, gflag,
                                                                   big_list, sw_ctr + 1, ctr, limit);
-        c->lc.n++;
-    } else {
-        const int sweep_mult = c->knobs.sweep_mult;
-        k_sweep_small<<<(u32)c->sm_count * sweep_mult, 128, 0, st>>>(ev, sdata, gstart, n_groups, n_inc, n_keep, thr, good, flagged, big_list,
-                                                                    sw_ctr + 1, sw_ctr, ctr);
-    }
-    const bool tree = n_keep == 1 && !no_flat && !c->knobs.sweep_no_tree;
-    if (tree) {
-        // n = 1: the groups whose neighbour scans got long (piles) go through the position-parallel tree sweep (sweep_tree.cuh)
+        c->lc.n += 2;
+        // the groups whose neighbour scans got long (piles) go through the position-parallel tree sweep (sweep_tree.cuh)
         const u32 n_big = read_u32(c, sw_ctr + 1);
         if (n_big) sweep_piles_n1(c, ev, sdata, gstart, n_groups, n_inc, big_list, n_big, thr, keep);
     } else {
+        u8 *good = c->arena.take<u8>(n_items), *flagged = c->arena.take<u8>(n_items);
+        SWG_CUDA(cudaMemsetAsync(good, 0, n_items, st));
+        SWG_CUDA(cudaMemsetAsync(flagged, 0, n_items, st));
+        k_sweep_small<<<(u32)c->sm_count * 8, 128, 0, st>>>(ev, sdata, gstart, n_groups, n_inc, n_keep, thr, good, flagged, big_list,
+                                                           sw_ctr + 1, sw_ctr, ctr);
         // groups whose pile is deeper than the per-thread array: one warp each, active set in global scratch
         ActEntry *act = c->arena.take<ActEntry>(n_inc + 1);
         k_sweep_groups<<<(u32)c->sm_count * 4, 128, 0, st>>>(ev, sdata, gstart, n_groups, n_inc, n_keep, thr, act, good, flagged, big_list,
                                                             sw_ctr + 1, sw_ctr + 2, ctr);
-        if (n_keep == 1 && !no_flat) {
-            k_sweep_keep_big<<<(u32)c->sm_count, 128, 0, st>>>(ev, gstart, n_groups, n_inc, big_list, sw_ctr + 1, good, flagged, keep);
-            c->lc.n++;
-        } else {
-            const u32 *evc = ev;
-            launch_for<t_sweep_keep>(n_inc, st, c->lc, [=] __device__(u32 u) {
-                const u32 i = evc[u];
-                keep[i] = (good[i] && !flagged[i]) ? 1 : 0;
-            });
-        }
-        c->lc.n += 1;
+        c->lc.n += 2;
+        const u32 *evc = ev;
+        launch_for<t_sweep_keep>(n_inc, st, c->lc, [=] __device__(u32 u) {
+            const u32 i = evc[u];
+            keep[i] = (good[i] && !flagged[i]) ? 1 : 0;
+        });
     }
-    c->lc.n += 1;
     stage_mark(c, "gs_done");
     SWG_CUDA(cudaGetLastError());
 }
@@ -697,14 +676,14 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     case SWG_ONE_TO_MANY: qlim0 = cfg.mapping_max_per_query != SWG_NO_LIMIT ? cfg.mapping_max_per_query : 1; tlim0 = cfg.mapping_max_per_target; break;
     default: qlim0 = cfg.mapping_max_per_query; tlim0 = cfg.mapping_max_per_target;
     }
-    bool fused_keys = cfg.scaffold_gap != 0 && qlim0 == SWG_KEEP_ALL && tlim0 == SWG_KEEP_ALL && !K.force_wide && !K.pairs_sort &&
+    bool fused_keys = cfg.scaffold_gap != 0 && qlim0 == SWG_KEEP_ALL && tlim0 == SWG_KEEP_ALL && !K.force_wide &&
                       2 * sb0 + 1 <= 32 && !K.no_fused_keys;
     u64 *keys = nullptr, *keys2 = nullptr;
     u32 *vals = nullptr, *vals2 = nullptr;
     if (cfg.scaffold_gap != 0) { keys = A.take<u64>(N); keys2 = A.take<u64>(N); vals = A.take<u32>(N); vals2 = A.take<u32>(N); }
     // The record sort as a counting sort by group (group_sort.cuh) when the table of all possible groups fits.
     const u64 g_entries = 2ull * in.n_seq * in.n_seq;
-    bool gsort = cfg.scaffold_gap != 0 && !K.force_wide && !K.pairs_sort && !K.no_group_sort && g_entries <= GS_MAX_TABLE && 2 * sb0 + 1 <= 31;
+    bool gsort = cfg.scaffold_gap != 0 && !K.force_wide && !K.no_group_sort && g_entries <= GS_MAX_TABLE && 2 * sb0 + 1 <= 31;
     if (gsort) {
         try { group_table(c, g_entries); } // (up to 512 MB for ~5800 sequences) no room: the LSD passes need no table
         catch (const OomError &) { gsort = false; }
@@ -844,15 +823,7 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
                 lc.n++;
             }
         }
-        if (!lsd) {
-            // done above
-        } else if (K.pairs_sort) {
-            read_counters_begin(c);
-            sort_pairs(c, keys, keys2, vals, vals2, N, kb, true);
-            skey = keys;
-            sidx.v = vals;
-            read_counters_end(c);
-        } else {
+        if (lsd) {
             read_counters_begin(c); // the survivor count is final here; the host picks it up while the sort runs
             // the packed sort (radix_sort.cuh): once the key bits still to be sorted and the index fit one word, the passes
             // move 8 B per record instead of 12 B; the result holds the index and the key from bit c0 upwards
@@ -977,8 +948,8 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         lc.n++;
         stage_mark(c, "ch_resolve");
         // enough threads to hide the dependent-load latency of a step, few enough that every group's lines stay in L1/L2
-        k_chain_resolve<<<(u32)c->sm_count * K.resolve_mult, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work, bb_ctr, gshift, cfg.scaffold_gap,
-                                                                             bps, pred, bb_ctr + 1);
+        k_chain_resolve<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work, bb_ctr, gshift, cfg.scaffold_gap,
+                                                              bps, pred, bb_ctr + 1);
         k_chain_resolve_warp<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work_big, bb_ctr + 2, gshift,
                                                                   cfg.scaffold_gap, bps, pred, bb_ctr + 3);
         lc.n += 2;
@@ -990,19 +961,13 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
             SWG_CUDA(cudaMemsetAsync(root_preset, 0xFF, sizeof(u32) * (size_t)n_m, st));
             scan_flags([=] __device__(u32 p) -> u32 { return is_huge(gid[p]) ? 1u : 0u; },
                        [=] __device__(u32 p, u32 ex, u32 v) { if (v) hpos[ex] = p; }, n_m, bsum, d_tot + 3, st, lc);
-            // searches in target-bucket order (default; SWG_FX_NO_BUCKETS=1: along the query axis, from the candidate records)
-            const bool fx_buckets = !K.fx_no_buckets;
-            auto huge_candidates = [&] {
-                k_chain_candidates<true><<<(u32)c->sm_count * 16, 256, 0, st>>>(srec, skey, gid, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, cand, nullptr,
-                                                                                 nullptr, hpos, d_tot + 3); // their candidate records (position-parallel)
-                lc.n++;
-            };
-            if (!fx_buckets) huge_candidates();
-            if (!chain_fixpoint(c, n_huge, hpos, srec, skey, gshift, gid, gstart, n_groups, n_m, fx_buckets ? nullptr : cand, cfg.scaffold_gap, root_preset,
-                                bsum, maxcoord)) {
+            if (!chain_fixpoint(c, n_huge, hpos, srec, skey, gshift, gid, gstart, n_groups, n_m, cfg.scaffold_gap, root_preset, bsum, maxcoord)) {
                 // a dependency chain longer than the round limit: the huge groups go through the sequential warp walk after all
-                // (it resets the groups' pred / best_pred_score itself; root_preset is untouched)
-                if (fx_buckets) huge_candidates(); // the walk starts from the candidate records
+                // (it resets the groups' pred / best_pred_score itself; root_preset is untouched).  The walk starts from the
+                // candidate records of their positions (position-parallel).
+                k_chain_candidates<true><<<(u32)c->sm_count * 16, 256, 0, st>>>(srec, skey, gid, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, cand, nullptr,
+                                                                                 nullptr, hpos, d_tot + 3);
+                lc.n++;
                 SWG_CUDA(cudaMemsetAsync(bb_ctr + 2, 0, 2 * sizeof(u32), st));
                 scan_flags([=] __device__(u32 g) -> u32 { return is_huge(g) ? 1u : 0u; },
                            [=] __device__(u32 g, u32 ex, u32 v) { if (v) work_big[ex] = g; }, n_groups, bsum, bb_ctr + 2, st, lc);
@@ -1278,7 +1243,7 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         // A chromosome pair that holds a huge group can hold 10^5..10^6 kept chains; walking all of them for every
         // reverse mapping is O(n * chains).  Then (or with SWG_INV_GRID=1) chains and mappings meet in buckets of the query axis.
         const int wb0 = std::max(17, bits_for(2 * cfg.scaffold_gap + 1)); // widest bucket: 2^wb0 > 2 * jump
-        const bool inv_grid = (n_huge > 0 || K.inv_grid) && !K.inv_no_grid && 2 * sb + (cb > wb0 ? cb - wb0 : 1) + 1 <= 64;
+        const bool inv_grid = (n_huge > 0 || K.inv_grid) && 2 * sb + (cb > wb0 ? cb - wb0 : 1) + 1 <= 64;
         if (inv_grid) {
             stage_mark(c, "inversion_grid");
             const u64 G = cfg.scaffold_gap;

@@ -4,7 +4,7 @@
     pick(i) = first arg-min_j { d(i,j) : d(i,j) < B(i,j) },   B(i,j) = min { d(i',j) : i' < i, pick(i') = j }
 
 and re-evaluating all positions against a snapshot of the picks (Jacobi rounds), starting from the unconstrained arg-min,
-ends exactly there.  Also the re-evaluation test of k_fx_check: a position has to be re-evaluated iff its pick is now
+ends exactly there.  Also the re-evaluation test of k_fx_check_warp: a position has to be re-evaluated iff its pick is now
 blocked or a candidate ranking before its pick has become eligible.  No GPU, no product code: a model of the algorithm."""
 import numpy as np
 import pytest

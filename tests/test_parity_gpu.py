@@ -88,15 +88,6 @@ def test_yeast_configs(ctx, yeast, case):
     check(ctx, swg.FilterConfig.from_cli(**CLI_CASES[case]), yeast, case)
 
 
-@pytest.mark.parametrize("case", ["1:1_1:1", "mass0", "1:1_rescue"])
-def test_sequential_sweep_kernels_for_n1(ctx, yeast, case, monkeypatch):
-    """n = 1 normally runs the thread-per-item sweep (k_sweep_flat1); SWG_SWEEP_NO_FLAT routes it through the sequential
-    thread-per-group / warp-per-group kernels that every other n uses: both must agree with the oracle."""
-    monkeypatch.setenv("SWG_SWEEP_NO_FLAT", "1")
-    check(ctx, swg.FilterConfig.from_cli(**CLI_CASES[case]), yeast, case)
-    check(ctx, swg.FilterConfig.from_cli(**CLI_CASES[case]), synth.pansn(200_000, seed=8, n_hap=10), case)
-
-
 @pytest.mark.parametrize("case", ["defaults", "rescue100k", "1:1_1:1"])
 def test_pansn_400k(ctx, case):
     """configs[2]/[3] generator at a size the oracle finishes in seconds."""
@@ -170,21 +161,17 @@ def test_fixpoint_everywhere(ctx, yeast, what, monkeypatch):
             check(ctx, cfg, t, f"fixpoint-fuzz{seed}")
 
 
-@pytest.mark.parametrize("variant", ["query_axis", "query_axis_collect", "narrow0", "narrow6", "narrow12", "narrow5_collect"])
+@pytest.mark.parametrize("variant", ["narrow0", "narrow6", "narrow12", "narrow5_collect"])
 def test_fixpoint_search_orders(ctx, yeast, variant, monkeypatch):
-    """The fixed point's searches: along the query axis from the candidate records (SWG_FX_NO_BUCKETS=1, the round-1 form) and
-    in target-bucket order with buckets from G + G/5 wide (at most two per search) down to a few bases (dozens per search)."""
+    """The fixed point's searches in target-bucket order with buckets from G + G/5 wide (at most two per search) down to a few
+    bases (dozens per search).  Short windows reach the warp search too: the windows that go on past round 0's linear scan,
+    every later re-evaluation and the verify pass."""
     monkeypatch.setenv("SWG_FIXPOINT_MIN", "2")
     monkeypatch.setenv("SWG_FIXPOINT_VERIFY", "1")
     if variant.endswith("_collect"):  # X(i) from the separate collecting pass (otherwise only after 1024 blocked candidates)
         monkeypatch.setenv("SWG_FX_FORCE_COLLECT", "1")
         variant = variant[:-8]
-    if variant == "query_axis":
-        monkeypatch.setenv("SWG_FX_NO_BUCKETS", "1")
-    else:
-        monkeypatch.setenv("SWG_FX_BUCKET_NARROW", variant[6:])
-        if variant == "narrow6":  # round 0 entirely through the warp search (default: a thread scans the next 48 successors first)
-            monkeypatch.setenv("SWG_FX_NO_LINEAR0", "1")
+    monkeypatch.setenv("SWG_FX_BUCKET_NARROW", variant[6:])
     check(ctx, swg.FilterConfig(), synth.skew(n_pile=20_000, n_tiny_groups=3_000, seed=5, window=3_000_000), variant)
     check(ctx, swg.FilterConfig.from_cli(**CLI_CASES["1:1_rescue"]), yeast, variant)
     for seed in (500, 503, 505, 506):
@@ -361,10 +348,10 @@ def test_wide_key_paths(ctx, yeast, case, monkeypatch):
                                             scaffold_dist="300"), t, f"wide fuzz{seed}")
 
 
-@pytest.mark.parametrize("knob", ["SWG_SORT_PAIRS", "SWG_NO_FUSED_KEYS", None])
+@pytest.mark.parametrize("knob", ["SWG_NO_FUSED_KEYS", None])
 def test_record_sort_variants(ctx, yeast, knob, monkeypatch):
-    """The three forms of the record sort give the same result: (default) keys written by the prefilter pass in the gap layout
-    and packed into one word by the third pass; keys from k_chain_keys, packed; key + payload pairs through every pass.
+    """The two forms of the record sort give the same result: (default) keys written by the prefilter pass in the gap layout
+    and packed into one word by the third pass; keys from k_chain_keys, packed.
     The default only takes the fused-key path when the key plus the index exceed 64 bits, i.e. on a large table: the PanSN
     table below (12 + 12 + 1 + 28 key bits, 21 index bits) qualifies, the yeast table exercises the other branch."""
     if knob:
