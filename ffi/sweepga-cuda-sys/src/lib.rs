@@ -24,6 +24,14 @@ pub const SWG_SCAFFOLD: u8 = 1;
 pub const SWG_RESCUED: u8 = 2;
 pub const SWG_UNASSIGNED: u8 = 3;
 
+/// Columns of the per-table counts of `swg_filter_batch` (row k, column SWG_TC_*; n_tables * SWG_TC_COUNT u64, row-major).
+pub const SWG_TC_STAGE1: usize = 0;
+pub const SWG_TC_KEPT: usize = 1;
+pub const SWG_TC_SCAFFOLD: usize = 2;
+pub const SWG_TC_RESCUED: usize = 3;
+pub const SWG_TC_CHAINS_KEPT: usize = 4;
+pub const SWG_TC_COUNT: usize = 5;
+
 pub const SWG_OK: c_int = 0;
 pub const SWG_ERR_ARG: c_int = -1;
 pub const SWG_ERR_RANGE: c_int = -2;
@@ -150,6 +158,8 @@ extern "C" {
     pub fn swg_stream(ctx: *mut swg_ctx) -> *mut c_void;
     pub fn swg_prefetch(ctx: *mut swg_ctx, host_in: *const swg_mappings) -> c_int;
     pub fn swg_prefetch_drop(ctx: *mut swg_ctx);
+    pub fn swg_filter_batch(ctx: *mut swg_ctx, cfg: *const swg_config, n_tables: u64, host_in: *const swg_mappings,
+                            host_out: *mut swg_result, table_counts: *mut u64, stats: *mut swg_stats) -> c_int;
     pub fn swg_upload(ctx: *mut swg_ctx, host_in: *const swg_mappings, dev_out: *mut swg_mappings, dev_res: *mut swg_result) -> c_int;
     pub fn swg_release(ctx: *mut swg_ctx, dev: *mut swg_mappings, dev_res: *mut swg_result);
     pub fn swg_download_result(ctx: *mut swg_ctx, n: u64, dev_res: *const swg_result, host_out: *mut swg_result) -> c_int;

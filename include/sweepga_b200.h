@@ -196,6 +196,21 @@ void *swg_stream(swg_ctx *ctx);
 int swg_prefetch(swg_ctx *ctx, const swg_mappings *host_in);
 void swg_prefetch_drop(swg_ctx *ctx);
 
+/* Many independent tables in one call (one PAF per sample, per chromosome, per batch): host_out[k] receives byte for byte
+ * what swg_filter writes for host_in[k] alone, chain numbers starting at chain_1 in every table, whatever else shares the
+ * batch.  The tables travel as one union (ids made disjoint per table) through one run of the pipeline: one upload, one
+ * kernel chain and one download instead of K, so a loop of small tables stops paying the per-call floor.  Every table may
+ * use 16- or 32-bit ids and may lack `identity`; `score` is given for every table or for none (else SWG_ERR_ARG).  Tables
+ * with n == 0 contribute nothing, n_tables == 0 is SWG_OK.  A NULL column (swg_last_error names the table), or more than
+ * 0x7FFFFFF0 records or 2^31 sequences in all: SWG_ERR_ARG; a range error in any table fails the whole call
+ * (SWG_ERR_RANGE).  table_counts (may be NULL): n_tables rows of SWG_TC_COUNT u64, row-major: records that pass the
+ * stage-1 retain, records kept (status != SWG_DROPPED), SWG_SCAFFOLD, SWG_RESCUED, and the table's largest chain
+ * number.  stats (may be NULL) describes the whole call (the union's stage counts, launches, phase times).  Outstanding
+ * prefetches stay outstanding; afterwards the last-call chain queries report no chains.                               */
+enum { SWG_TC_STAGE1 = 0, SWG_TC_KEPT = 1, SWG_TC_SCAFFOLD = 2, SWG_TC_RESCUED = 3, SWG_TC_CHAINS_KEPT = 4, SWG_TC_COUNT = 5 };
+int swg_filter_batch(swg_ctx *ctx, const swg_config *cfg, uint64_t n_tables, const swg_mappings *host_in,
+                     swg_result *host_out, uint64_t *table_counts, swg_stats *stats);
+
 /* Upload a host table once / free it; lets a caller time swg_filter_device on
  * resident data without touching CUDA itself.                                   */
 int swg_upload(swg_ctx *ctx, const swg_mappings *host_in, swg_mappings *dev_out, swg_result *dev_res);

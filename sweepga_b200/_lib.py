@@ -17,6 +17,8 @@ ONE_TO_ONE, ONE_TO_MANY, MANY_TO_MANY = 0, 1, 2
 SCORE_IDENTITY, SCORE_LENGTH, SCORE_LENGTH_IDENTITY, SCORE_LOG_LENGTH_IDENTITY, SCORE_MATCHES = range(5)
 DROPPED, SCAFFOLD, RESCUED, UNASSIGNED = range(4)
 OK, ERR_ARG, ERR_RANGE, ERR_CUDA, ERR_OOM, ERR_IO, ERR_PARSE, ERR_UNSUPPORTED = 0, -1, -2, -3, -4, -5, -6, -7
+# columns of swg_filter_batch's per-table counts
+TC_STAGE1, TC_KEPT, TC_SCAFFOLD, TC_RESCUED, TC_CHAINS_KEPT, TC_COUNT = range(6)
 
 
 class swg_config(C.Structure):
@@ -71,6 +73,7 @@ SYMBOLS = [
     ("swg_stream", _vp, [_vp]),
     ("swg_prefetch", C.c_int, [_vp, _mapp]),
     ("swg_prefetch_drop", None, [_vp]),
+    ("swg_filter_batch", C.c_int, [_vp, _cfgp, C.c_uint64, _mapp, _resp, u64p, _statp]),
     ("swg_upload", C.c_int, [_vp, _mapp, _mapp, _resp]),
     ("swg_release", None, [_vp, _mapp, _resp]),
     ("swg_download_result", C.c_int, [_vp, C.c_uint64, _resp, _resp]),

@@ -276,6 +276,21 @@ class Context:
         self._check(lib.swg_filter(self._h, C.byref(cc), C.byref(cm), C.byref(res), C.byref(stats)))
         return status, chain_id, stats
 
+    def filter_batch(self, cfg: FilterConfig, tables):
+        """Many independent tables in one call (swg_filter_batch): every table's result is what filter() returns for it alone.
+        Returns (results, counts, stats): results[k] = (status u8[n_k], chain_id u32[n_k]); counts = uint64 (K, TC_COUNT), columns
+        TC_STAGE1, TC_KEPT, TC_SCAFFOLD, TC_RESCUED, TC_CHAINS_KEPT; stats describes the whole call."""
+        tables = list(tables)
+        k = len(tables)
+        results = [(np.zeros(t.n, np.uint8), np.zeros(t.n, np.uint32)) for t in tables]
+        cms = (_lib.swg_mappings * max(k, 1))(*[t.to_c() for t in tables])
+        outs = (_lib.swg_result * max(k, 1))(*[_lib.swg_result(_ptr(s, C.c_uint8), _ptr(c, C.c_uint32)) for s, c in results])
+        counts = np.zeros((k, _lib.TC_COUNT), np.uint64)
+        stats = _lib.swg_stats()
+        cc = cfg.to_c()
+        self._check(lib.swg_filter_batch(self._h, C.byref(cc), k, cms, outs, _ptr(counts, C.c_uint64), C.byref(stats)))
+        return results, counts, stats
+
     def prefetch(self, table: MappingTable):
         """Start uploading `table` now (swg_prefetch); the next filter() of the same table (same arrays) finds it on the device."""
         cm = table.to_c()

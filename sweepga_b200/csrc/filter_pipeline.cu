@@ -171,6 +171,8 @@ struct swg_ctx {
     const u32 *last_keyA = nullptr, *last_keyB = nullptr; // order keys of the kept chains of the last call (in `keys`, not in the scratch arena)
     u64 last_n_chains = 0;
     Arena keys;       // owns last_keyA / last_keyB: they survive later calls that rewind the scratch arena
+    const u8 *last_flags = nullptr; // flags[] of the last run_filter (F_ALIVE = passed the stage-1 retain); in the scratch arena
+    Arena batch;      // swg_filter_batch: the union of the tables and its results
     bool log_matches_host = false; // swg_create: the device's glibc_log agrees with the host libm's log on the probe set
     bool cudalog_matches_host = false; // ... and CUDA's log() (SWG_LOG_IMPL=cuda) does
     Knobs knobs;      // environment knobs, re-read at the start of every entry point (read_knobs)
@@ -607,6 +609,7 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     c->stage_used = 0;
     c->last_n_chains = 0;
     c->last_keyA = c->last_keyB = nullptr;
+    c->last_flags = nullptr;
     auto finish = [&]() {
         stage_mark(c, "end");
         stage_report(c);
@@ -639,6 +642,7 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     stage_mark(c, "prefilter");
     // ---- K0 ------------------------------------------------------------------------------
     u8 *flags = A.take<u8>(N);
+    c->last_flags = flags;
     // distinct genome pairs <= min(N, nP^2); table of 2x that, power of two
     u32 *d_maxp = A.take<u32>(2);
     SWG_CUDA(cudaMemsetAsync(d_maxp, 0, 2 * sizeof(u32), st));
@@ -757,7 +761,9 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     stage_mark(c, "keys+sort");
     int gshift = cb; // group id of a sorted position = skey >> gshift
     const int kb = 2 * sb + 1 + cb;
-    const bool wide = kb > 64 || K.force_wide;
+    // The packed LSD sort keeps the key from bit c0 upwards; the group key starts at bit cb, so c0 > cb (many sequences, narrow
+    // coordinates, 2^24 or more records) would cut group bits: such inputs take the two-stage path as well.
+    const bool wide = kb > 64 || K.force_wide || rs_packed_c0(kb, bits_for(N - 1)) > cb;
     SortedIdx sidx{nullptr, nullptr, 0};
     const u64 *skey = nullptr;
     bool kept_is_alive = false;   // the keys came from k_prefilter: kept == alive, nobody counted C_KEPT_M
@@ -1728,13 +1734,43 @@ static void ensure_pinned(swg_ctx *c) {
 }
 struct CopyJob { const char *src; char *dst; size_t bytes; int fd; }; // fd >= 0: the source is that file (pread), src its mapping
 
-// host -> device on c->copy_stream; returns when every piece is QUEUED (the last DMAs may still be in flight)
-static void staged_h2d(swg_ctx *c, const std::vector<CopyJob> &jobs) {
-    ensure_pinned(c);
-    struct Piece { const CopyJob *j; size_t off, len; };
-    std::vector<Piece> pieces;
+// The general form: one column is one contiguous device range whose bytes come from (or go to) several host slices, e.g. the
+// same column of many tables (swg_filter_batch).  seg.off is the slice's byte offset inside the column; slices are ascending
+// and disjoint.  A piece is PIN_PIECE bytes of ONE column and one DMA, however many slices it covers.
+struct PinSeg { char *host; size_t off, len; int fd = -1; }; // fd >= 0: host -> device reads the slice from that file (pread)
+struct PinCol { char *dev; size_t bytes; std::vector<PinSeg> segs; };
+struct PinPiece { const PinCol *col; size_t off, len, seg0; };
+static std::vector<PinPiece> pin_pieces(const std::vector<PinCol> &cols) {
+    std::vector<PinPiece> pieces;
+    for (const PinCol &col : cols) {
+        size_t s = 0;
+        for (size_t o = 0; o < col.bytes; o += PIN_PIECE) {
+            while (s < col.segs.size() && col.segs[s].off + col.segs[s].len <= o) s++;
+            pieces.push_back(PinPiece{&col, o, std::min(PIN_PIECE, col.bytes - o), s});
+        }
+    }
+    return pieces;
+}
+// fn(slice, byte offset inside the slice, byte offset inside the piece, length) for every slice the piece overlaps
+template <class F> static void piece_slices(const PinPiece &p, F fn) {
+    const std::vector<PinSeg> &segs = p.col->segs;
+    for (size_t s = p.seg0; s < segs.size() && segs[s].off < p.off + p.len; s++) {
+        const size_t a = std::max(segs[s].off, p.off), b = std::min(segs[s].off + segs[s].len, p.off + p.len);
+        if (a < b) fn(segs[s], a - segs[s].off, a - p.off, b - a);
+    }
+}
+static std::vector<PinCol> jobs_as_cols(const std::vector<CopyJob> &jobs, bool h2d) {
+    std::vector<PinCol> cols;
     for (const CopyJob &j : jobs)
-        for (size_t o = 0; o < j.bytes; o += PIN_PIECE) pieces.push_back(Piece{&j, o, std::min(PIN_PIECE, j.bytes - o)});
+        cols.push_back(h2d ? PinCol{j.dst, j.bytes, {PinSeg{(char *)j.src, 0, j.bytes, j.fd}}} : PinCol{(char *)j.src, j.bytes, {PinSeg{j.dst, 0, j.bytes, -1}}});
+    return cols;
+}
+
+// host -> device on c->copy_stream; returns when every piece is QUEUED (the last DMAs may still be in flight).  Bytes of a piece
+// that no slice covers carry whatever the pinned buffer held.
+static void staged_h2d_cols(swg_ctx *c, const std::vector<PinCol> &cols) {
+    ensure_pinned(c);
+    const std::vector<PinPiece> pieces = pin_pieces(cols);
     std::atomic<size_t> next{0};
     std::atomic<int> failed{0};
     auto worker = [&](int t) {
@@ -1742,20 +1778,23 @@ static void staged_h2d(swg_ctx *c, const std::vector<CopyJob> &jobs) {
         while (!failed.load()) {
             const size_t k = next.fetch_add(1);
             if (k >= pieces.size()) break;
-            const Piece &pc = pieces[k];
+            const PinPiece &pc = pieces[k];
             if (cudaEventSynchronize(c->pin_ev[t]) != cudaSuccess) { failed = 1; break; }
-            bool filled = false;
-            if (pc.j->fd >= 0) { // plain file: pread skips the page-table work of touching a fresh mapping
-                size_t got = 0;
-                while (got < pc.len) {
-                    const ssize_t r = pread(pc.j->fd, c->pin[t] + got, pc.len - got, (off_t)(pc.off + got));
-                    if (r <= 0) break;
-                    got += (size_t)r;
+            char *buf = c->pin[t];
+            piece_slices(pc, [&](const PinSeg &sg, size_t so, size_t po, size_t len) {
+                bool filled = false;
+                if (sg.fd >= 0) { // plain file: pread skips the page-table work of touching a fresh mapping
+                    size_t got = 0;
+                    while (got < len) {
+                        const ssize_t r = pread(sg.fd, buf + po + got, len - got, (off_t)(so + got));
+                        if (r <= 0) break;
+                        got += (size_t)r;
+                    }
+                    filled = got == len;
                 }
-                filled = got == pc.len;
-            }
-            if (!filled) memcpy(c->pin[t], pc.j->src + pc.off, pc.len);
-            if (cudaMemcpyAsync(pc.j->dst + pc.off, c->pin[t], pc.len, cudaMemcpyHostToDevice, c->copy_stream) != cudaSuccess ||
+                if (!filled) memcpy(buf + po, sg.host + so, len);
+            });
+            if (cudaMemcpyAsync(pc.col->dev + pc.off, buf, pc.len, cudaMemcpyHostToDevice, c->copy_stream) != cudaSuccess ||
                 cudaEventRecord(c->pin_ev[t], c->copy_stream) != cudaSuccess) { failed = 1; break; }
         }
     };
@@ -1766,18 +1805,16 @@ static void staged_h2d(swg_ctx *c, const std::vector<CopyJob> &jobs) {
     for (auto &t : th) t.join();
     if (failed.load()) { cudaGetLastError(); throw CudaError{cudaErrorUnknown, __FILE__, __LINE__}; }
 }
+static void staged_h2d(swg_ctx *c, const std::vector<CopyJob> &jobs) { staged_h2d_cols(c, jobs_as_cols(jobs, true)); }
 // host text -> device, through the pinned pieces, one reader thread per piece buffer
 static void upload_text(swg_ctx *c, const char *src, int fd, size_t bytes, char *dst) {
     staged_h2d(c, std::vector<CopyJob>{CopyJob{src, dst, bytes, fd}});
 }
-// device -> pageable host memory: DMA per piece into a pinned buffer, the team copies the pieces out; returns when done.
+// device -> pageable host memory: DMA per piece into a pinned buffer, the team copies the slices out; returns when done.
 // The device data must be complete on c->copy_stream's view (the caller makes copy_stream wait for the producing stream).
-static void staged_d2h(swg_ctx *c, const std::vector<CopyJob> &jobs /* src = device, dst = host */) {
+static void staged_d2h_cols(swg_ctx *c, const std::vector<PinCol> &cols) {
     ensure_pinned(c);
-    struct Piece { const CopyJob *j; size_t off, len; };
-    std::vector<Piece> pieces;
-    for (const CopyJob &j : jobs)
-        for (size_t o = 0; o < j.bytes; o += PIN_PIECE) pieces.push_back(Piece{&j, o, std::min(PIN_PIECE, j.bytes - o)});
+    const std::vector<PinPiece> pieces = pin_pieces(cols);
     std::atomic<size_t> next{0};
     std::atomic<int> failed{0};
     auto worker = [&](int t) {
@@ -1785,10 +1822,11 @@ static void staged_d2h(swg_ctx *c, const std::vector<CopyJob> &jobs /* src = dev
         while (!failed.load()) {
             const size_t k = next.fetch_add(1);
             if (k >= pieces.size()) break;
-            const Piece &pc = pieces[k];
-            if (cudaMemcpyAsync(c->pin[t], pc.j->src + pc.off, pc.len, cudaMemcpyDeviceToHost, c->copy_stream) != cudaSuccess ||
+            const PinPiece &pc = pieces[k];
+            char *buf = c->pin[t];
+            if (cudaMemcpyAsync(buf, pc.col->dev + pc.off, pc.len, cudaMemcpyDeviceToHost, c->copy_stream) != cudaSuccess ||
                 cudaEventRecord(c->pin_ev[t], c->copy_stream) != cudaSuccess || cudaEventSynchronize(c->pin_ev[t]) != cudaSuccess) { failed = 1; break; }
-            memcpy(pc.j->dst + pc.off, c->pin[t], pc.len);
+            piece_slices(pc, [&](const PinSeg &sg, size_t so, size_t po, size_t len) { memcpy(sg.host + so, buf + po, len); });
         }
     };
     std::vector<std::thread> th;
@@ -1798,6 +1836,7 @@ static void staged_d2h(swg_ctx *c, const std::vector<CopyJob> &jobs /* src = dev
     for (auto &t : th) t.join();
     if (failed.load()) { cudaGetLastError(); throw CudaError{cudaErrorUnknown, __FILE__, __LINE__}; }
 }
+static void staged_d2h(swg_ctx *c, const std::vector<CopyJob> &jobs /* src = device, dst = host */) { staged_d2h_cols(c, jobs_as_cols(jobs, false)); }
 static bool is_pageable(const void *p) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return true; }
@@ -1978,6 +2017,7 @@ static void do_sweep_core(void *p) {
 
 #include "paf_device.cuh"
 #include "ani_device.cuh"
+#include "batch.cuh"
 
 // =================================================================================================
 // C ABI
@@ -2035,6 +2075,7 @@ void swg_destroy(swg_ctx *c) {
     c->arena.release();
     c->io.release();
     c->keys.release();
+    c->batch.release();
     c->score_arena.release();
     if (c->h_ctr) cudaFreeHost(c->h_ctr);
     for (char *p : c->pin) cudaFreeHost(p);
@@ -2142,6 +2183,31 @@ int swg_filter(swg_ctx *c, const swg_config *cfg, const swg_mappings *host_in, s
         if (pf) { pf->valid = false; c->pf_head ^= 1; c->pf_count--; }
         if (a->stats) *a->stats = local;
     }, &a);
+}
+
+int swg_filter_batch(swg_ctx *c, const swg_config *cfg, uint64_t n_tables, const swg_mappings *host_in, swg_result *host_out,
+                     uint64_t *table_counts, swg_stats *stats) {
+    if (!c) return SWG_ERR_ARG;
+    if (!check_cfg(c, cfg)) return SWG_ERR_ARG;
+    if (n_tables && (!host_in || !host_out)) { set_err(c, "swg_filter_batch: NULL table or result array"); return SWG_ERR_ARG; }
+    if (n_tables >= (1ull << 31)) { set_err(c, "swg_filter_batch: too many tables (must be < 2^31)"); return SWG_ERR_ARG; }
+    u64 n = 0, n_seq = 0;
+    int score = -1; // of the first non-empty table: every non-empty table has a score column, or none has
+    for (u64 k = 0; k < n_tables; k++) {
+        const swg_mappings &m = host_in[k];
+        const std::string at = "swg_filter_batch: table " + std::to_string(k) + ": ";
+        if (!check_maps(c, &m)) { set_err(c, at + c->err); return SWG_ERR_ARG; }
+        if (m.n == 0) continue;
+        if (!host_out[k].status || !host_out[k].chain_id) { set_err(c, at + "NULL result column"); return SWG_ERR_ARG; }
+        if (score < 0) score = m.score != nullptr;
+        if (score != (m.score != nullptr)) { set_err(c, at + "a score column must be given for every table or for none"); return SWG_ERR_ARG; }
+        n += m.n;
+        n_seq += m.n_seq;
+        if (n >= 0x7FFFFFF0ull) { set_err(c, at + "the tables hold too many records together (must be < 2^31 per context)"); return SWG_ERR_ARG; }
+        if (n_seq >= (1ull << 31)) { set_err(c, at + "the tables hold too many sequences together (must be < 2^31)"); return SWG_ERR_ARG; }
+    }
+    BatchArgs a{c, cfg, n_tables, host_in, host_out, table_counts, stats};
+    return guarded(c, "swg_filter_batch", do_filter_batch, &a);
 }
 
 int swg_prefetch(swg_ctx *c, const swg_mappings *host_in) {
