@@ -486,7 +486,7 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     cudaStream_t st = c->stream;
     LaunchCounter &lc = c->lc;
     Arena &A = c->arena;
-    static const bool verbose = getenv("SWG_STAGE_TIMING") != nullptr;
+    const bool verbose = c->knobs.stage_timing;
     FxArrays f;
     f.n = n_h;
     f.rec = A.take<uint4>(n_h);
@@ -498,7 +498,7 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     f.minpi = A.take<u32>(n_h);
     f.firstp = A.take<u32>(n_h);
     f.li = nullptr; // the sorted positions of each round's sort
-    f.force_collect = getenv("SWG_FX_FORCE_COLLECT") != nullptr;
+    f.force_collect = c->knobs.fx_force_collect;
     f.ld = A.take<u64>(n_h);
     f.xoff = A.take<u32>(n_h);
     f.xcnt = A.take<u16>(n_h);
@@ -558,8 +558,7 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     // nearest edge is further than sqrt(best d): narrow buckets keep the scans of the dense diagonal short, wide ones spare
     // the scattered positions origin searches.  Wider if the directory (one entry per group and bucket) would pass 2^25
     // entries or 2^20 per group.
-    const int narrow = getenv("SWG_FX_BUCKET_NARROW") ? atoi(getenv("SWG_FX_BUCKET_NARROW")) : 5;
-    int bs = std::max(bits_for(G + G / 5) - narrow, 4);
+    int bs = std::max(bits_for(G + G / 5) - c->knobs.fx_bucket_narrow, 4);
     while (((((u64)maxcoord >> bs) + 2) * n_hg > (1ull << 25) || ((u64)maxcoord >> bs) + 2 > (1ull << 20)) && bs < 32) bs++;
     f.bshift = bs;
     const u32 nbk = (u32)(((u64)maxcoord >> bs) + 1);
@@ -603,7 +602,6 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
     }
     if (verbose) fprintf(stderr, "[swg fixpoint] target buckets: %u huge groups, 2^%d wide, %u per group\n", n_hg, bs, nbk);
     int rounds = 0;
-    const int max_rounds = getenv("SWG_FIXPOINT_MAX_ROUNDS") ? atoi(getenv("SWG_FIXPOINT_MAX_ROUNDS")) : 256;
     u64 total_recomputed = 0;
     auto t_round = std::chrono::steady_clock::now();
     {
@@ -715,12 +713,12 @@ static bool chain_fixpoint(swg_ctx *c, u32 n_h, const u32 *hpos, const uint4 *sr
             t_round = t1;
         }
         if (h[1] == 0) break; // the snapshot of this round equals the picks: it is the fixed point
-        if (rounds >= max_rounds) {
+        if (rounds >= c->knobs.fixpoint_max_rounds) {
             if (verbose) fprintf(stderr, "[swg fixpoint] not settled after %d rounds (%u picks still changing): sequential walk instead\n", rounds, h[1]);
             return false;
         }
     }
-    if (getenv("SWG_FIXPOINT_VERIFY")) {
+    if (c->knobs.fixpoint_verify) {
         // Self-check for sizes no oracle reaches: (*) has exactly one solution, so it suffices that EVERY position, evaluated
         // from scratch against the final snapshot, reproduces its pick (this bypasses the X(i) bookkeeping of k_fx_check_warp).
         const FxArrays g = f;

@@ -1,17 +1,17 @@
 // filter_pipeline.cu — swg_ctx, the device pipeline that replaces the body of
 // PafFilter::apply_filters (reference src/paf_filter.rs:379-747) and its C ABI.
 //
-// Stage order mirrors the reference (SURVEY.md §8a rows 2..11):
-//   K0  stage-1 retain                                   paf_filter.rs:384-388
-//   GS  primary plane sweep (closed form when n = inf)   paf_filter.rs:972-1123, plane_sweep_exact.rs
-//   K1+sort+K2  (q,t,strand) grouping + stable sort      paf_filter.rs:761-777
-//   K3  best-buddy chaining + roots + aggregates         paf_filter.rs:780-928, union_find.rs
-//   K4  chain table, mass/identity filter                paf_filter.rs:449-455
-//   O*  insertion-order reproduction -> chain_N          SURVEY Appendix B
-//   GS  scaffold plane sweep (closed form when n = inf)  plane_sweep_scaffold.rs:47-251
-//   K5  anchors                                          paf_filter.rs:517-528
-//   K6  inversion capture                                paf_filter.rs:535-597
-//   K7  rescue                                           paf_filter.rs:613-732
+// Stage order mirrors the reference (SURVEY.md §8a rows 2..11); run_filter calls one function per stage:
+//   K0  prefilter           stage-1 retain                                   paf_filter.rs:384-388
+//   GS  primary_sweep       primary plane sweep (closed form when n = inf)   paf_filter.rs:972-1123, plane_sweep_exact.rs
+//   K1+sort+K2  order_records  (q,t,strand) grouping + stable sort          paf_filter.rs:761-777
+//   K3  chain_groups        best-buddy chaining (huge groups: fixed point)   paf_filter.rs:780-928, union_find.rs
+//   K4  chain_table         roots, aggregates, mass/identity filter          paf_filter.rs:449-455
+//   O*  order_chains        insertion-order reproduction -> chain_N          SURVEY Appendix B
+//   GS                      ... with the scaffold plane sweep                plane_sweep_scaffold.rs:47-251
+//   K5  assign_anchors      anchors                                          paf_filter.rs:517-528
+//   K6  capture_inversions  inversion capture (inversion_grid: bucketed)     paf_filter.rs:535-597
+//   K7  rescue              rescue                                           paf_filter.rs:613-732
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -127,6 +127,12 @@ struct Knobs {
     u32 fixpoint_min = 0;      // 0 = default
     double max_pair_evals = 0; // 0 = no limit (SWG_MAX_PAIR_EVALS)
     int exact_scores = 0;      // SWG_EXACT_SCORES: 0 auto, 1 always, 2 never
+    bool stage_timing = false; // SWG_STAGE_TIMING (set, whatever its value): stage events and diagnostic prints
+    bool fx_force_collect = false, fixpoint_verify = false; // SWG_FX_FORCE_COLLECT, SWG_FIXPOINT_VERIFY (set, whatever the value)
+    int fx_bucket_narrow = 5;        // SWG_FX_BUCKET_NARROW
+    int fixpoint_max_rounds = 256;   // SWG_FIXPOINT_MAX_ROUNDS
+    u32 tok_long = 4096;             // SWG_TOK_LONG
+    bool paf_host_frontend = false;  // SWG_PAF_FRONTEND=host
 };
 static Knobs read_knobs() {
     Knobs k;
@@ -146,6 +152,13 @@ static Knobs read_knobs() {
     if (const char *v = getenv("SWG_FIXPOINT_MIN")) k.fixpoint_min = (u32)atoi(v);
     if (const char *v = getenv("SWG_MAX_PAIR_EVALS")) k.max_pair_evals = atof(v);
     if (const char *v = getenv("SWG_EXACT_SCORES")) k.exact_scores = strcmp(v, "always") == 0 ? 1 : strcmp(v, "never") == 0 ? 2 : 0;
+    k.stage_timing = getenv("SWG_STAGE_TIMING") != nullptr;
+    k.fx_force_collect = getenv("SWG_FX_FORCE_COLLECT") != nullptr;
+    k.fixpoint_verify = getenv("SWG_FIXPOINT_VERIFY") != nullptr;
+    if (const char *v = getenv("SWG_FX_BUCKET_NARROW")) k.fx_bucket_narrow = atoi(v);
+    if (const char *v = getenv("SWG_FIXPOINT_MAX_ROUNDS")) k.fixpoint_max_rounds = atoi(v);
+    if (const char *v = getenv("SWG_TOK_LONG")) k.tok_long = (u32)atoi(v);
+    if (const char *v = getenv("SWG_PAF_FRONTEND")) k.paf_host_frontend = strcmp(v, "host") == 0;
     return k;
 }
 } // namespace swg
@@ -204,8 +217,7 @@ namespace swg {
 static void set_err(swg_ctx *c, const std::string &m) { if (c) c->err = m; else g_create_error = m; }
 
 static void stage_mark(swg_ctx *c, const char *name) {
-    static const bool on = getenv("SWG_STAGE_TIMING") != nullptr;
-    if (!on) return;
+    if (!c->knobs.stage_timing) return;
     if (c->stage_used == c->stage_ev.size()) {
         cudaEvent_t e;
         SWG_CUDA(cudaEventCreate(&e));
@@ -256,6 +268,25 @@ static void sort_pairs(swg_ctx *c, u64 *&k, u64 *&k2, u32 *&v, u32 *&v2, u32 n, 
         if (timed) { c->sort_passes = p.passes; c->sort_pairs = n; }
     }
 }
+// a key wider than 64 bits as two chained stable sorts, least significant field first: k holds the low field (lo_bits);
+// hi(i) = the high field (hi_bits) of item i replaces it for the second sort.  timed: as sort_pairs, for the first sort.
+template <class Hi>
+static void sort_pairs_wide(swg_ctx *c, u64 *&k, u64 *&k2, u32 *&v, u32 *&v2, u32 n, int lo_bits, int hi_bits, Hi hi, bool timed = false) {
+    sort_pairs(c, k, k2, v, v2, n, lo_bits, timed);
+    u64 *kk = k;
+    const u32 *vv = v;
+    launch_for<t_gather>(n, c->stream, c->lc, [=] __device__(u32 p) { kk[p] = hi(vv[p]); });
+    sort_pairs(c, k, k2, v, v2, n, hi_bits);
+}
+// groups of a sorted key: gstart[g] = first position of group g, gid[p] = group of position p, group count to *d_count
+static void group_bounds(swg_ctx *c, const u64 *key, int shift, u32 n, u32 *gstart, u32 *gid, u32 *temp, u32 *d_count) {
+    scan_flags([=] __device__(u32 p) -> u32 { return (p == 0 || (key[p] >> shift) != (key[p - 1] >> shift)) ? 1u : 0u; },
+               [=] __device__(u32 p, u32 ex, u32 v) {
+                   if (v) gstart[ex] = p;
+                   gid[p] = ex + v - 1;
+               },
+               n, temp, d_count, c->stream, c->lc);
+}
 
 // ---- the group sort (csrc/group_sort.cuh) as one call ---------------------------------------------------------------------
 // keys[i] = (group key << shift) | secondary key (< 2^shift); excluded items carry the group key `dead`.  Orders the items by
@@ -281,6 +312,8 @@ static u32 *group_table(swg_ctx *c, u64 entries) { // counters (cleared per use)
     }
     return c->gtable;
 }
+// largest group the group sort takes (SWG_GROUP_SORT_MAX lowers it)
+static u32 group_sort_limit(const Knobs &K) { return K.group_sort_max ? std::min(K.group_sort_max, GS_CTA_MAX) : GS_CTA_MAX; }
 static GroupSorted group_sort(swg_ctx *c, const u64 *keys, u64 *scratch, u64 *out, u32 *run_of, u32 n, int shift, GsIndex ix, u32 dead,
                               u64 table_entries, int ib, u32 limit, bool with_counters, u32 *sec_out = nullptr /* n u32: the secondary keys in sorted order */) {
     cudaStream_t st = c->stream;
@@ -324,7 +357,7 @@ static GroupSorted group_sort(swg_ctx *c, const u64 *keys, u64 *scratch, u64 *ou
     read_counters_end(c);
     r.n_groups = h[0]; r.n_rec = h[1]; r.gmax = h[2]; r.n_runs = h[3];
     r.d_n_groups = gs_ctr;
-    if (getenv("SWG_STAGE_TIMING")) fprintf(stderr, "[swg group sort] records %u runs %u groups %u largest %u\n", r.n_rec, r.n_runs, r.n_groups, r.gmax);
+    if (c->knobs.stage_timing) fprintf(stderr, "[swg group sort] records %u runs %u groups %u largest %u\n", r.n_rec, r.n_runs, r.n_groups, r.gmax);
     if (r.n_groups == 0) { r.done = true; return r; }
     if (r.gmax > limit) return r;
     stage_mark(c, "gs_order");
@@ -449,25 +482,17 @@ static void general_sweep_impl(swg_ctx *c, u32 n_items, const u8 *include, u8 in
     GroupSorted gs;
     if (!wide && !c->knobs.no_group_sort && gb <= 22 && pbits <= 32 && pbits + ib <= 64 && gb + ib <= 64 && n_items >= (1u << 18) &&
         (c->rows_grouped || c->knobs.group_sort_always)) {
-        const u32 limit = c->knobs.group_sort_max ? std::min(c->knobs.group_sort_max, GS_CTA_MAX) : GS_CTA_MAX;
-        gs = group_sort(c, ek, ek2, ek, ev2, n_items, pbits, GsIndex{0, 0, 0}, 0xFFFFFFFFu, 1ull << gb, ib, limit, true);
+        gs = group_sort(c, ek, ek2, ek, ev2, n_items, pbits, GsIndex{0, 0, 0}, 0xFFFFFFFFu, 1ull << gb, ib, group_sort_limit(c->knobs), true);
     }
     if (gs.done) {
         // (sorted item indices: the low bits of ek; t_sweep_gather below writes them to ev)
     } else if (!wide) {
         sort_pairs(c, ek, ek2, ev, ev2, n_items, gb + pbits);
     } else {
-        sort_pairs(c, ek, ek2, ev, ev2, n_items, pbits);
-        {
-            u64 *kk = ek;
-            const u32 *vv = ev;
-            launch_for<t_gather>(n_items, st, c->lc, [=] __device__(u32 u) {
-                const u32 i = vv[u];
-                const bool inc = include ? (include[i] & include_mask) != 0 : true;
-                kk[u] = inc ? gkey[i] : NONE64;
-            });
-        }
-        sort_pairs(c, ek, ek2, ev, ev2, n_items, gb + 1);
+        sort_pairs_wide(c, ek, ek2, ev, ev2, n_items, pbits, gb + 1, [=] __device__(u32 i) {
+            const bool inc = include ? (include[i] & include_mask) != 0 : true;
+            return inc ? gkey[i] : NONE64;
+        });
         eshift = 0;
     }
     stage_mark(c, "gs_groups");
@@ -490,13 +515,7 @@ static void general_sweep_impl(swg_ctx *c, u32 n_items, const u8 *include, u8 in
         gid = c->arena.take<u32>(n_inc);
         u32 *bsum = c->arena.take<u32>(scan_temp_u32(n_inc));
         u32 *d_ng = c->arena.take<u32>(2);
-        const u64 *ekc = ek;
-        scan_flags([=] __device__(u32 u) -> u32 { return (u == 0 || (ekc[u] >> eshift) != (ekc[u - 1] >> eshift)) ? 1u : 0u; },
-                   [=] __device__(u32 u, u32 ex, u32 v) {
-                       if (v) gstart[ex] = u;
-                       gid[u] = ex + v - 1;
-                   },
-                   n_inc, bsum, d_ng, st, c->lc);
+        group_bounds(c, ek, eshift, n_inc, gstart, gid, bsum, d_ng);
         n_groups = read_u32(c, d_ng);
     }
     u32 *ends = n_keep == 1 ? c->arena.take<u32>(n_inc) : nullptr; // interval ends in sorted order (for the running maximum)
@@ -587,62 +606,80 @@ static inline double host_score(int scoring, double identity, u32 qs, u32 qe) {
 }
 
 // ================================================================================================
-// the pipeline
+// the pipeline: one function per stage of the list at the top of the file, driven by run_filter
 // ================================================================================================
-// exact_host: every logarithm on the path comes from the HOST libm (in.score carries the record scores; the chain-level
-// logs are computed on the host from small downloads) — the exact re-rank of DESIGN 4d, not the normal path.
-static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *status, u32 *chain_id, swg_stats *stats,
-                       cudaEvent_t ev_matches = nullptr /* recorded when in.matches has arrived (swg_filter overlaps that copy) */,
-                       bool exact_host = false) {
+// per-query / per-target limits of the primary sweep (paf_filter.rs:972-1123)
+struct Limits { u64 q, t; };
+static Limits mapping_limits(const swg_config &cfg) {
+    switch (cfg.mapping_filter_mode) {
+    case SWG_ONE_TO_ONE: return {1, 1};
+    case SWG_ONE_TO_MANY: return {cfg.mapping_max_per_query != SWG_NO_LIMIT ? cfg.mapping_max_per_query : 1, cfg.mapping_max_per_target};
+    default: return {cfg.mapping_max_per_query, cfg.mapping_max_per_target};
+    }
+}
+
+// first-appearance table (hash_insert_min / hash_lookup) for n keys: open addressing over a power of two >= 2n slots (at least
+// 1024), every key and value all ones (empty).  Returns the slot mask.
+static u32 first_index_table(swg_ctx *c, u64 n, u64 *&hk, u32 *&hv) {
+    u32 cap = 1024;
+    while ((u64)cap < n * 2) cap <<= 1;
+    hk = c->arena.take<u64>(cap);
+    hv = c->arena.take<u32>(cap);
+    SWG_CUDA(cudaMemsetAsync(hk, 0xFF, sizeof(u64) * cap, c->stream));
+    SWG_CUDA(cudaMemsetAsync(hv, 0xFF, sizeof(u32) * cap, c->stream));
+    return cap - 1;
+}
+
+// the end of every run_filter: stage report, launch count, timings of the record sort and of k_prefilter, the caller's stats
+static void finish(swg_ctx *c, swg_stats &S, u64 launches0, swg_stats *stats) {
+    stage_mark(c, "end");
+    stage_report(c);
+    S.gpu_launches = c->lc.n - launches0;
+    if (c->sort_passes) { // all work has been synchronised by the last counter read
+        float ms = 0;
+        cudaStreamSynchronize(c->stream);
+        if (cudaEventElapsedTime(&ms, c->ev_sort[0], c->ev_sort[1]) == cudaSuccess) S.ms_sort_passes = ms;
+        S.n_sort_passes = (u64)c->sort_passes;
+        S.n_sort_pairs = c->sort_pairs;
+        S.sort_bytes_per_pair = c->sort_bytes_per_pair;
+    }
+    if (S.prefilter_bytes_per_record) {
+        float ms = 0;
+        cudaStreamSynchronize(c->stream);
+        if (cudaEventElapsedTime(&ms, c->ev_pre[0], c->ev_pre[1]) == cudaSuccess) S.ms_prefilter = ms;
+    }
+    if (stats) *stats = S;
+}
+
+// ---- K0: stage-1 retain (k_prefilter) ----------------------------------------------------------
+struct Prefiltered {
+    u8 *flags;
+    u64 *hk; u32 *hv; u32 hmask;                 // genome pair -> first record index
+    uint4 *rec4 = nullptr;                       // packed coordinates (scaffolding only, like the sort buffers)
+    u64 *keys = nullptr, *keys2 = nullptr;
+    u32 *vals = nullptr, *vals2 = nullptr;
+    bool fused_keys;           // k_prefilter wrote the chain sort keys into keys / vals
+    bool gsort;                // the record sort may take the group sort: its table of g_entries groups fits
+    u64 g_entries;
+    u64 n_alive, zlq, zlt;     // records alive; ... with an empty query / target interval
+    u32 maxcoord;
+    int sb, cb, pb;            // bits of a sequence id, a coordinate, a genome-prefix id
+};
+static Prefiltered prefilter(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Limits &lim, u8 *status, u32 *chain_id,
+                             cudaEvent_t ev_matches, swg_stats &S) {
     cudaStream_t st = c->stream;
     const Knobs &K = c->knobs;
-    const bool cuda_log = K.cuda_log;
     LaunchCounter &lc = c->lc;
     const u32 N = in.n;
-    u64 launches0 = lc.n;
-    swg_stats S;
-    std::memset(&S, 0, sizeof S);
-    S.n_input = N;
-    c->sort_passes = 0;
-    c->sort_pairs = 0;
-    c->sort_bytes_per_pair = 24;
-    c->stage_used = 0;
-    c->last_n_chains = 0;
-    c->last_keyA = c->last_keyB = nullptr;
-    c->last_flags = nullptr;
-    auto finish = [&]() {
-        stage_mark(c, "end");
-        stage_report(c);
-        S.gpu_launches = lc.n - launches0;
-        if (c->sort_passes) { // all work has been synchronised by the last counter read
-            float ms = 0;
-            cudaStreamSynchronize(st);
-            if (cudaEventElapsedTime(&ms, c->ev_sort[0], c->ev_sort[1]) == cudaSuccess) S.ms_sort_passes = ms;
-            S.n_sort_passes = (u64)c->sort_passes;
-            S.n_sort_pairs = c->sort_pairs;
-            S.sort_bytes_per_pair = c->sort_bytes_per_pair;
-        }
-        if (S.prefilter_bytes_per_record) {
-            float ms = 0;
-            cudaStreamSynchronize(st);
-            if (cudaEventElapsedTime(&ms, c->ev_pre[0], c->ev_pre[1]) == cudaSuccess) S.ms_prefilter = ms;
-        }
-        if (stats) *stats = S;
-    };
-    if (N == 0) { SWG_CUDA(cudaStreamSynchronize(st)); finish(); return; }
-    // (status / chain_id are cleared below, while the host waits for the first small read)
-    if (cfg.scaffold_gap >= (1ull << 31) || cfg.scaffold_max_deviation >= (1ull << 31))
-        throw RangeError{"scaffold_gap / scaffold_max_deviation must be < 2^31"};
-
     c->arena.reserve((size_t)N * 400 + (64u << 20));
     Arena &A = c->arena;
     u64 *ctr = c->d_ctr;
     SWG_CUDA(cudaMemsetAsync(ctr, 0, sizeof(u64) * C_COUNT, st));
 
     stage_mark(c, "prefilter");
-    // ---- K0 ------------------------------------------------------------------------------
-    u8 *flags = A.take<u8>(N);
-    c->last_flags = flags;
+    Prefiltered P;
+    P.flags = A.take<u8>(N);
+    c->last_flags = P.flags;
     // distinct genome pairs <= min(N, nP^2); table of 2x that, power of two
     u32 *d_maxp = A.take<u32>(2);
     SWG_CUDA(cudaMemsetAsync(d_maxp, 0, 2 * sizeof(u32), st));
@@ -659,105 +696,106 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         maxP2 = h[1];
     }
     if (maxP >= in.n_seq || maxP2 >= in.n_seq) throw RangeError{"genome prefix id >= n_seq (prefix ids must be dense)"};
-    u64 npairs = std::min<u64>((u64)N, (u64)(maxP + 1) * (maxP + 1));
-    u32 hcap = 1024;
-    while ((u64)hcap < npairs * 2) hcap <<= 1;
-    u64 *hk = A.take<u64>(hcap);
-    u32 *hv = A.take<u32>(hcap);
-    SWG_CUDA(cudaMemsetAsync(hk, 0xFF, sizeof(u64) * hcap, st));
-    SWG_CUDA(cudaMemsetAsync(hv, 0xFF, sizeof(u32) * hcap, st));
-    uint4 *rec4 = nullptr;
-    if (cfg.scaffold_gap != 0) rec4 = A.take<uint4>(N);
+    P.hmask = first_index_table(c, std::min<u64>((u64)N, (u64)(maxP + 1) * (maxP + 1)), P.hk, P.hv);
+    if (cfg.scaffold_gap != 0) P.rec4 = A.take<uint4>(N);
     // swg_filter sends `matches` — and `block_length`, when the retain does not test it — behind the other columns: k_prefilter waits
     // for them only if it derives the identity from them
     if (ev_matches && !in.identity && !(cfg.min_identity <= 0.0)) SWG_CUDA(cudaStreamWaitEvent(st, ev_matches, 0));
     // The chain sort keys can be written by the same pass when the primary sweep is the closed form (no per-axis limit): then
     // kept == alive unless an alive record has an empty interval (checked below; k_chain_keys redoes the keys in that case).
-    const int sb0 = bits_for(in.n_seq);
-    u64 qlim0, tlim0;
-    switch (cfg.mapping_filter_mode) {
-    case SWG_ONE_TO_ONE: qlim0 = tlim0 = 1; break;
-    case SWG_ONE_TO_MANY: qlim0 = cfg.mapping_max_per_query != SWG_NO_LIMIT ? cfg.mapping_max_per_query : 1; tlim0 = cfg.mapping_max_per_target; break;
-    default: qlim0 = cfg.mapping_max_per_query; tlim0 = cfg.mapping_max_per_target;
-    }
-    bool fused_keys = cfg.scaffold_gap != 0 && qlim0 == SWG_KEEP_ALL && tlim0 == SWG_KEEP_ALL && !K.force_wide &&
-                      2 * sb0 + 1 <= 32 && !K.no_fused_keys;
-    u64 *keys = nullptr, *keys2 = nullptr;
-    u32 *vals = nullptr, *vals2 = nullptr;
-    if (cfg.scaffold_gap != 0) { keys = A.take<u64>(N); keys2 = A.take<u64>(N); vals = A.take<u32>(N); vals2 = A.take<u32>(N); }
+    P.sb = bits_for(in.n_seq); // ids < n_seq <= 2^sb - 1: the all-ones pattern stays free for dead keys
+    P.fused_keys = cfg.scaffold_gap != 0 && lim.q == SWG_KEEP_ALL && lim.t == SWG_KEEP_ALL && !K.force_wide && 2 * P.sb + 1 <= 32 &&
+                   !K.no_fused_keys;
+    if (cfg.scaffold_gap != 0) { P.keys = A.take<u64>(N); P.keys2 = A.take<u64>(N); P.vals = A.take<u32>(N); P.vals2 = A.take<u32>(N); }
     // The record sort as a counting sort by group (group_sort.cuh) when the table of all possible groups fits.
-    const u64 g_entries = 2ull * in.n_seq * in.n_seq;
-    bool gsort = cfg.scaffold_gap != 0 && !K.force_wide && !K.no_group_sort && g_entries <= GS_MAX_TABLE && 2 * sb0 + 1 <= 31;
-    if (gsort) {
-        try { group_table(c, g_entries); } // (up to 512 MB for ~5800 sequences) no room: the LSD passes need no table
-        catch (const OomError &) { gsort = false; }
+    P.g_entries = 2ull * in.n_seq * in.n_seq;
+    P.gsort = cfg.scaffold_gap != 0 && !K.force_wide && !K.no_group_sort && P.g_entries <= GS_MAX_TABLE && 2 * P.sb + 1 <= 31;
+    if (P.gsort) {
+        try { group_table(c, P.g_entries); } // (up to 512 MB for ~5800 sequences) no room: the LSD passes need no table
+        catch (const OomError &) { P.gsort = false; }
     }
     SWG_CUDA(cudaEventRecord(c->ev_pre[0], st));
-    if (fused_keys) k_prefilter<true><<<cdiv(N, 256), 256, 0, st>>>(in, cfg.min_block_length, cfg.min_identity, cfg.keep_self, flags, ctr, hk, hv, hcap - 1, rec4, sb0, keys, vals);
-    else k_prefilter<false><<<cdiv(N, 256), 256, 0, st>>>(in, cfg.min_block_length, cfg.min_identity, cfg.keep_self, flags, ctr, hk, hv, hcap - 1, rec4);
+    if (P.fused_keys)
+        k_prefilter<true><<<cdiv(N, 256), 256, 0, st>>>(in, cfg.min_block_length, cfg.min_identity, cfg.keep_self, P.flags, ctr, P.hk, P.hv,
+                                                        P.hmask, P.rec4, P.sb, P.keys, P.vals);
+    else k_prefilter<false><<<cdiv(N, 256), 256, 0, st>>>(in, cfg.min_block_length, cfg.min_identity, cfg.keep_self, P.flags, ctr, P.hk, P.hv,
+                                                          P.hmask, P.rec4);
     SWG_CUDA(cudaEventRecord(c->ev_pre[1], st));
     {   // algorithmic bytes of the launch per record: ids 8, coordinates 16, block length 4, strand 1 (+ matches 4 / identity 8 when
         // the identity test needs them) read; flags 1 (+ packed coordinates 16, + key 8 and index 4 when the pass writes the keys) written
         const bool need_id = in.identity != nullptr || !(cfg.min_identity <= 0.0);
-        S.prefilter_bytes_per_record = 29 + (need_id ? (in.identity ? 8 : 4) : 0) + 1 + (rec4 ? 16 : 0) + (fused_keys ? 12 : 0);
+        S.prefilter_bytes_per_record = 29 + (need_id ? (in.identity ? 8 : 4) : 0) + 1 + (P.rec4 ? 16 : 0) + (P.fused_keys ? 12 : 0);
     }
     lc.n++;
     read_counters(c);
     if (c->h_ctr[C_BAD])
         throw RangeError{"a record that passes the length / self / identity retain has end < start, a coordinate beyond the u32 table, or a sequence id >= n_seq"};
-    const u64 n_alive = c->h_ctr[C_ALIVE], zlq = c->h_ctr[C_ZLQ], zlt = c->h_ctr[C_ZLT];
+    P.n_alive = c->h_ctr[C_ALIVE], P.zlq = c->h_ctr[C_ZLQ], P.zlt = c->h_ctr[C_ZLT];
     c->rows_grouped = (c->h_ctr[C_RUNS] - std::min<u64>(c->h_ctr[C_RUNS], N / 32)) * 2 <= (u64)N;
-    const u32 maxcoord = (u32)c->h_ctr[C_MAXCOORD];
-    S.n_stage1 = n_alive;
-    const int sb = bits_for(in.n_seq);      // ids < n_seq <= 2^sb - 1: the all-ones pattern stays free for dead keys
-    const int cb = bits_for(maxcoord);
-    const int pb = bits_for(maxP); // genome-prefix ids of the partner: usually far fewer bits than a sequence id, and one sort pass less
+    P.maxcoord = (u32)c->h_ctr[C_MAXCOORD];
+    S.n_stage1 = P.n_alive;
+    P.cb = bits_for(P.maxcoord);
+    P.pb = bits_for(maxP); // genome-prefix ids of the partner: usually far fewer bits than a sequence id, and one sort pass less
+    return P;
+}
 
+// ---- GS: primary plane sweep (paf_filter.rs:972-1123) ------------------------------------------
+struct Kept { u8 *q = nullptr, *t = nullptr; }; // per record: kept by the query / target axis sweep; nullptr: that sweep keeps all
+static Kept primary_sweep(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, const Limits &lim,
+                          cudaEvent_t ev_matches) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const bool cuda_log = c->knobs.cuda_log;
+    const u32 N = in.n;
+    const int pb = P.pb;
     stage_mark(c, "primary_sweep");
-    // ---- primary plane sweep (paf_filter.rs:972-1123) ----------------------------------------
-    u64 qlim, tlim;
-    switch (cfg.mapping_filter_mode) {
-    case SWG_ONE_TO_ONE: qlim = 1; tlim = 1; break;
-    case SWG_ONE_TO_MANY: qlim = cfg.mapping_max_per_query != SWG_NO_LIMIT ? cfg.mapping_max_per_query : 1; tlim = cfg.mapping_max_per_target; break;
-    default: qlim = cfg.mapping_max_per_query; tlim = cfg.mapping_max_per_target;
-    }
-    u8 *keep_q = nullptr, *keep_t = nullptr;
-    const bool need_q = n_alive > 1 && (qlim != SWG_KEEP_ALL || zlq > 0);
-    const bool need_t = n_alive > 1 && (tlim != SWG_KEEP_ALL || zlt > 0);
-    double *rscore = nullptr;
-    if (need_q || need_t) {
-        rscore = A.take<double>(N);
-        const int scoring = cfg.scoring_function;
-        if (ev_matches && !in.identity && !in.score) SWG_CUDA(cudaStreamWaitEvent(st, ev_matches, 0));
-        launch_for<t_scores>(N, st, lc, [=] __device__(u32 i) {
-            rscore[i] = in.score ? in.score[i] : score_fn(scoring, rec_identity(in, i), in.qs[i], in.qe[i], cuda_log);
+    Kept kept;
+    const bool need_q = P.n_alive > 1 && (lim.q != SWG_KEEP_ALL || P.zlq > 0);
+    const bool need_t = P.n_alive > 1 && (lim.t != SWG_KEEP_ALL || P.zlt > 0);
+    if (!need_q && !need_t) return kept;
+    double *rscore = A.take<double>(N);
+    const int scoring = cfg.scoring_function;
+    if (ev_matches && !in.identity && !in.score) SWG_CUDA(cudaStreamWaitEvent(st, ev_matches, 0));
+    launch_for<t_scores>(N, st, lc, [=] __device__(u32 i) {
+        rscore[i] = in.score ? in.score[i] : score_fn(scoring, rec_identity(in, i), in.qs[i], in.qe[i], cuda_log);
+    });
+    u64 *gk = A.take<u64>(N);
+    for (int axis = 0; axis < 2; axis++) {
+        if (axis == 0 ? !need_q : !need_t) continue;
+        launch_for<t_gkey>(N, st, lc, [=] __device__(u32 i) {
+            u32 a = axis == 0 ? in.qid[i] : in.tid[i], b = axis == 0 ? in.tid[i] : in.qid[i];
+            gk[i] = ((u64)a << pb) | in.P[b];
         });
-        u64 *gk = A.take<u64>(N);
-        for (int axis = 0; axis < 2; axis++) {
-            if (axis == 0 ? !need_q : !need_t) continue;
-            launch_for<t_gkey>(N, st, lc, [=] __device__(u32 i) {
-                u32 a = axis == 0 ? in.qid[i] : in.tid[i], b = axis == 0 ? in.tid[i] : in.qid[i];
-                gk[i] = ((u64)a << pb) | in.P[b];
-            });
-            u8 *keep = A.take<u8>(N);
-            general_sweep(c, N, flags, F_ALIVE, gk, sb + pb, cb, axis == 0 ? in.qs : in.ts, axis == 0 ? in.qe : in.te, rscore,
-                          axis == 0 ? qlim : tlim, cfg.overlap_threshold, keep);
-            (axis == 0 ? keep_q : keep_t) = keep;
-        }
+        u8 *keep = A.take<u8>(N);
+        general_sweep(c, N, P.flags, F_ALIVE, gk, P.sb + pb, P.cb, axis == 0 ? in.qs : in.ts, axis == 0 ? in.qe : in.te, rscore,
+                      axis == 0 ? lim.q : lim.t, cfg.overlap_threshold, keep);
+        (axis == 0 ? kept.q : kept.t) = keep;
     }
+    return kept;
+}
 
-    // ---- no-scaffold exit (paf_filter.rs:409-434) -----------------------------------------------
-    if (cfg.scaffold_gap == 0) {
-        k_unassigned<<<cdiv(N, 256), 256, 0, st>>>(N, flags, keep_q, keep_t, status, ctr);
-        lc.n++;
-        read_counters(c);
-        S.n_after_sweep = S.n_kept = c->h_ctr[C_KEPT];
-        S.score_near_ties = c->h_ctr[C_NEAR_TIES];
-        finish();
-        return;
-    }
-
-    // ---- K1 + sort + K2: group by (q,t,strand), stable order by query_start ------------------------
+// ---- K1 + sort + K2: group by (q,t,strand), stable order by query_start; the packed coordinates in that order -------------
+struct Ordered {
+    u32 n_m = 0;                         // records kept by the primary sweep = sorted positions
+    const u64 *skey = nullptr;           // group key of a sorted position = skey >> gshift
+    int gshift = 0;
+    SortedIdx sidx{nullptr, nullptr, 0}; // record index of a sorted position
+    u32 n_groups = 0;
+    const u32 *gstart = nullptr, *gid = nullptr;
+    const uint4 *srec = nullptr;         // packed coordinates of the sorted positions
+    const u32 *gs_lists = nullptr;       // group sort: [3] groups that had to be ordered, by size class (diagnostic)
+    u32 fx_min = 0;                      // groups of at least fx_min positions are chained by the fixed-point iteration
+};
+static Ordered order_records(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, const Kept &kept, swg_stats &S) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const Knobs &K = c->knobs;
+    const u32 N = in.n;
+    u64 *ctr = c->d_ctr;
+    u8 *flags = P.flags;
+    const uint4 *rec4 = P.rec4;
+    const u8 *keep_q = kept.q, *keep_t = kept.t;
+    u64 *keys = P.keys, *keys2 = P.keys2;
+    u32 *vals = P.vals, *vals2 = P.vals2;
+    const int sb = P.sb, cb = P.cb;
     stage_mark(c, "keys+sort");
     int gshift = cb; // group id of a sorted position = skey >> gshift
     const int kb = 2 * sb + 1 + cb;
@@ -768,38 +806,36 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     const u64 *skey = nullptr;
     bool kept_is_alive = false;   // the keys came from k_prefilter: kept == alive, nobody counted C_KEPT_M
     bool groups_done = false;     // gid / gstart / group count already produced (group sort)
-    const u32 *gs_lists = nullptr; // group sort: [3] groups that had to be ordered, by size class (diagnostic)
-    u32 gs_gmax = 0;               // ... its largest group
+    u32 gs_gmax = 0;              // group sort: its largest group
+    const u32 *gs_lists = nullptr; // ... the groups it had to order, by size class
     u32 n_groups = 0;
     u32 *gstart = nullptr, *gid = nullptr;
-    u32 *d_tot = A.take<u32>(4);
+    u32 *d_ng = A.take<u32>(1);   // group count (k_chain_work_estimate)
     if (!wide) {
         const int ib = bits_for(N - 1);
         // the keys written by k_prefilter<true> stand if no sweep ran (kept == alive)
-        const bool fused_ok = fused_keys && !keep_q && !keep_t && zlq == 0 && zlt == 0;
+        const bool fused_ok = P.fused_keys && !keep_q && !keep_t && P.zlq == 0 && P.zlt == 0;
         // ... for the LSD passes additionally every digit consumed up to the packing pass must lie inside the coordinate field
         // (the gap of the layout is closed by the packing pass)
         const bool fused_lsd_ok = fused_ok && rs_packed_c0(kb, ib) > 0 && rs_packed_c0(kb, ib) <= cb;
-        bool lsd = true;
+        bool lsd = true, fused_keys = fused_lsd_ok;
         int key_shift = cb; // keys[] = (group key << key_shift) | query_start
         // rows in no particular order (runs of ~1 record: every step of the group sort turns into random accesses, ~1.6x the
         // LSD passes on a shuffled 20 M table) go through the LSD passes
         const bool grouped_rows = c->rows_grouped || K.group_sort_always;
-        if (gsort && grouped_rows) {
+        if (P.gsort && grouped_rows) {
             if (fused_ok) { key_shift = 32; kept_is_alive = true; }
             else {
                 k_chain_keys<<<cdiv(N, 256), 256, 0, st>>>(in, flags, keep_q, keep_t, sb, cb, keys, vals, ctr);
                 lc.n++;
-                fused_keys = false;
             }
-            const u32 limit = K.group_sort_max ? std::min(K.group_sort_max, GS_CTA_MAX) : GS_CTA_MAX;
             const GroupSorted gs = group_sort(c, keys, keys2, keys /* the keys have done their duty by then */, vals2, N, key_shift,
-                                              GsIndex{1, sb, in.n_seq}, (1u << (2 * sb + 1)) - 1, g_entries, ib, limit, true);
-            if (gs.n_rec != (kept_is_alive ? (u32)n_alive : (u32)c->h_ctr[C_KEPT_M])) throw RangeError{"group sort: the table counted " + std::to_string(gs.n_rec) + " records"};
+                                              GsIndex{1, sb, in.n_seq}, (1u << (2 * sb + 1)) - 1, P.g_entries, ib, group_sort_limit(K), true);
+            if (gs.n_rec != (kept_is_alive ? (u32)P.n_alive : (u32)c->h_ctr[C_KEPT_M])) throw RangeError{"group sort: the table counted " + std::to_string(gs.n_rec) + " records"};
             if (gs.done) {
                 lsd = false;
                 if (gs.n_groups) {
-                    SWG_CUDA(cudaMemcpyAsync(d_tot, gs.d_n_groups, sizeof(u32), cudaMemcpyDeviceToDevice, st)); // d_tot[0] = group count (k_chain_work_estimate)
+                    SWG_CUDA(cudaMemcpyAsync(d_ng, gs.d_n_groups, sizeof(u32), cudaMemcpyDeviceToDevice, st));
                     n_groups = gs.n_groups;
                     gstart = gs.gstart;
                     gid = gs.gid;
@@ -822,7 +858,6 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
                 } else fused_keys = key_shift == 32;
             }
         } else {
-            fused_keys = fused_lsd_ok;
             kept_is_alive = fused_keys;
             if (!fused_keys) {
                 k_chain_keys<<<cdiv(N, 256), 256, 0, st>>>(in, flags, keep_q, keep_t, sb, cb, keys, vals, ctr);
@@ -847,8 +882,8 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
             read_counters_end(c);
         }
     } else {
-        // key wider than 64 bits (hundreds of thousands of sequences): two chained stable sorts, least significant
-        // field first: by query_start, then by the (query,target,strand) group id; skey then holds the group id alone
+        // key wider than 64 bits (hundreds of thousands of sequences): sorted by query_start, then by the (query,target,strand)
+        // group id; skey then holds the group id alone
         u64 *gk = A.take<u64>(N);
         {
             u64 *kk = keys;
@@ -864,35 +899,22 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
                 if (cnt && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd((unsigned long long *)&ctr[C_KEPT_M], (unsigned long long)cnt);
             });
         }
-        fused_keys = false;
-        sort_pairs(c, keys, keys2, vals, vals2, N, cb, true);
-        {
-            u64 *kk = keys;
-            const u32 *vv = vals;
-            launch_for<t_gather>(N, st, lc, [=] __device__(u32 p) { kk[p] = gk[vv[p]]; });
-        }
-        sort_pairs(c, keys, keys2, vals, vals2, N, 2 * sb + 2);
+        sort_pairs_wide(c, keys, keys2, vals, vals2, N, cb, 2 * sb + 2, [=] __device__(u32 i) { return gk[i]; }, true);
         gshift = 0;
         skey = keys;
         sidx.v = vals;
         read_counters(c);
     }
-    const u32 n_m = kept_is_alive ? (u32)n_alive : (u32)c->h_ctr[C_KEPT_M]; // keys of k_prefilter: kept == alive (nobody counted)
+    const u32 n_m = kept_is_alive ? (u32)P.n_alive : (u32)c->h_ctr[C_KEPT_M]; // keys of k_prefilter: kept == alive (nobody counted)
     S.n_after_sweep = n_m;
     S.score_near_ties = c->h_ctr[C_NEAR_TIES];
-    if (n_m == 0) { finish(); return; }
+    if (n_m == 0) return Ordered{};
     stage_mark(c, "groups+gather");
     uint4 *srec = A.take<uint4>(n_m);
-    u32 *bsum = A.take<u32>(scan_temp_u32(N));
     if (!groups_done) {
         gstart = A.take<u32>(n_m + 1);
         gid = A.take<u32>(n_m);
-        scan_flags([=] __device__(u32 p) -> u32 { return (p == 0 || (skey[p] >> gshift) != (skey[p - 1] >> gshift)) ? 1u : 0u; },
-                   [=] __device__(u32 p, u32 ex, u32 v) {
-                       if (v) gstart[ex] = p;
-                       gid[p] = ex + v - 1;
-                   },
-                   n_m, bsum, d_tot, st, lc);
+        group_bounds(c, skey, gshift, n_m, gstart, gid, A.take<u32>(scan_temp_u32(n_m)), d_ng);
     }
     // groups of at least fx_min positions are chained by the fixed-point iteration (SWG_NO_FIXPOINT=1: by the warp walk)
     const u32 fx_min = K.no_fixpoint ? NONE32 : (K.fixpoint_min ? K.fixpoint_min : FX_MIN_GROUP);
@@ -903,11 +925,11 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         // group count, positions in huge groups and a rough count of the candidate evaluations ahead (SWG_MAX_PAIR_EVALS, if
         // set, refuses an input beyond it; by default nothing is refused: the reference runs such piles to completion too).
         // The host picks the numbers up while the gather below runs.
-        if (K.max_pair_evals > 0) k_chain_work_estimate<true><<<(u32)c->sm_count * 8, 256, 0, st>>>(rec4, sidx, gstart, d_tot, n_m, cfg.scaffold_gap, fx_min, ctr);
-        else k_chain_work_estimate<false><<<(u32)c->sm_count * 8, 256, 0, st>>>(rec4, sidx, gstart, d_tot, n_m, cfg.scaffold_gap, fx_min, ctr);
+        if (K.max_pair_evals > 0) k_chain_work_estimate<true><<<(u32)c->sm_count * 8, 256, 0, st>>>(rec4, sidx, gstart, d_ng, n_m, cfg.scaffold_gap, fx_min, ctr);
+        else k_chain_work_estimate<false><<<(u32)c->sm_count * 8, 256, 0, st>>>(rec4, sidx, gstart, d_ng, n_m, cfg.scaffold_gap, fx_min, ctr);
         lc.n++;
         u32 *h = reinterpret_cast<u32 *>(c->h_ctr + C_COUNT);
-        SWG_CUDA(cudaMemcpyAsync(h, d_tot, sizeof(u32), cudaMemcpyDeviceToHost, st)); // group count and estimate in one round trip
+        SWG_CUDA(cudaMemcpyAsync(h, d_ng, sizeof(u32), cudaMemcpyDeviceToHost, st)); // group count and estimate in one round trip
         read_counters_begin(c);
         // post-sort gather of the packed coordinates (flat, one thread per position: all gathers of a warp in flight at once;
         // fused into the scan above it ran 5x slower: a scan thread owns eight CONSECUTIVE positions, so neither side coalesces).
@@ -919,77 +941,111 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
             throw RangeError{"chaining would need ~" + std::to_string((double)c->h_ctr[C_WORK]) +
                              " candidate evaluations (dense pile), more than SWG_MAX_PAIR_EVALS"};
     }
+    return Ordered{n_m, skey, gshift, sidx, n_groups, gstart, gid, srec, gs_lists, fx_min};
+}
 
-    u32 n_huge = 0; // positions in huge groups (fixed-point chaining; also selects the bucketed inversion capture)
+// ---- K3: best-buddy chaining (claims -> sequential resolve of the dirty groups; huge groups: the fixed point) -------------
+struct Chained {
+    const u32 *pred;        // best predecessor of every sorted position
+    const u32 *root_preset; // roots of the positions of huge groups (fixed-point chaining), NONE32 elsewhere; nullptr: none
+    u32 n_huge;             // positions in huge groups (also selects the bucketed inversion capture)
+    const u32 *bb_ctr;      // [0] ordinary dirty groups, [2] large/dense dirty groups (diagnostic)
+};
+static Chained chain_groups(swg_ctx *c, const swg_config &cfg, const Ordered &O, u32 maxcoord) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const u32 n_m = O.n_m, n_groups = O.n_groups, fx_min = O.fx_min;
+    const u32 *gstart = O.gstart, *gid = O.gid;
+    const uint4 *srec = O.srec;
+    const u64 *skey = O.skey;
+    const int gshift = O.gshift;
     stage_mark(c, "chaining");
-    // ---- K3: best-buddy chaining (claims -> sequential resolve of the dirty groups -> chain numbers -> aggregates) ----
     u64 *bps = A.take<u64>(n_m);     // best_pred_score: only the dirty groups touch it
     u32 *pred = A.take<u32>(n_m);    // best_pred_idx
-    Cand *cand = nullptr;            // unconstrained arg-min of every position of the groups that are redone (dirty / huge)
-    u32 *grp_minidx = A.take<u32>(n_groups); // per GROUP: min original index over its members (first appearance of the group)
     u32 *grp_dirty = A.take<u32>(n_groups);
     u32 *work = A.take<u32>(n_groups), *work_big = A.take<u32>(n_groups);
     u32 *bb_ctr = A.take<u32>(4); // [0] #ordinary dirty groups, [1] their work counter, [2] #large/dense dirty groups, [3] their work counter
-    u32 *root_preset = nullptr;   // roots of the positions of huge groups (fixed-point chaining), NONE32 elsewhere
+    u32 *root_preset = nullptr;
     SWG_CUDA(cudaMemsetAsync(bb_ctr, 0, 4 * sizeof(u32), st));
     SWG_CUDA(cudaMemsetAsync(grp_dirty, 0, sizeof(u32) * (size_t)n_groups, st));
-    SWG_CUDA(cudaMemsetAsync(grp_minidx, 0xFF, sizeof(u32) * (size_t)n_groups, st));
     SWG_CUDA(cudaMemsetAsync(pred, 0xFF, sizeof(u32) * (size_t)n_m, st));
-    {
-        // claims; a group with a conflict puts itself on a work list: ordinary (thread per group) or large/dense (warp per group:
-        // more than RES_THREAD_MAX positions or an expected window > 64 candidates)
-        k_chain_candidates<false><<<cdiv(n_m, 256), 256, 0, st>>>(srec, skey, gid, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, nullptr, pred, grp_dirty,
-                                                                   nullptr, nullptr, c->h_ctr[C_HUGE] ? fx_min : NONE32, work, work_big, bb_ctr);
-        lc.n++;
-        stage_mark(c, "ch_worklists");
-        auto is_huge = [=] __device__(u32 g) -> bool {
-            const u32 s0 = gstart[g], e0 = (g + 1 < n_groups) ? gstart[g + 1] : n_m;
-            return e0 - s0 >= fx_min;
-        };
-        // the redone groups need their candidate records: a second candidate pass over the listed groups only (ordinary data: a
-        // few hundred groups; writing all 16 B records in the first pass cost more than it saved)
-        cand = A.take<Cand>(n_m);
-        k_chain_candidates_groups<<<(u32)c->sm_count * 4, 256, 0, st>>>(srec, skey, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, cand, work, bb_ctr,
-                                                                       work_big, bb_ctr + 2);
-        lc.n++;
-        stage_mark(c, "ch_resolve");
-        // enough threads to hide the dependent-load latency of a step, few enough that every group's lines stay in L1/L2
-        k_chain_resolve<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work, bb_ctr, gshift, cfg.scaffold_gap,
-                                                              bps, pred, bb_ctr + 1);
-        k_chain_resolve_warp<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work_big, bb_ctr + 2, gshift,
-                                                                  cfg.scaffold_gap, bps, pred, bb_ctr + 3);
-        lc.n += 2;
-        n_huge = (u32)c->h_ctr[C_HUGE];
-        if (n_huge) {
-            stage_mark(c, "ch_fixpoint");
-            u32 *hpos = A.take<u32>(n_huge);
-            root_preset = A.take<u32>(n_m);
-            SWG_CUDA(cudaMemsetAsync(root_preset, 0xFF, sizeof(u32) * (size_t)n_m, st));
-            scan_flags([=] __device__(u32 p) -> u32 { return is_huge(gid[p]) ? 1u : 0u; },
-                       [=] __device__(u32 p, u32 ex, u32 v) { if (v) hpos[ex] = p; }, n_m, bsum, d_tot + 3, st, lc);
-            if (!chain_fixpoint(c, n_huge, hpos, srec, skey, gshift, gid, gstart, n_groups, n_m, cfg.scaffold_gap, root_preset, bsum, maxcoord)) {
-                // a dependency chain longer than the round limit: the huge groups go through the sequential warp walk after all
-                // (it resets the groups' pred / best_pred_score itself; root_preset is untouched).  The walk starts from the
-                // candidate records of their positions (position-parallel).
-                k_chain_candidates<true><<<(u32)c->sm_count * 16, 256, 0, st>>>(srec, skey, gid, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, cand, nullptr,
-                                                                                 nullptr, hpos, d_tot + 3);
-                lc.n++;
-                SWG_CUDA(cudaMemsetAsync(bb_ctr + 2, 0, 2 * sizeof(u32), st));
-                scan_flags([=] __device__(u32 g) -> u32 { return is_huge(g) ? 1u : 0u; },
-                           [=] __device__(u32 g, u32 ex, u32 v) { if (v) work_big[ex] = g; }, n_groups, bsum, bb_ctr + 2, st, lc);
-                k_chain_resolve_warp<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work_big, bb_ctr + 2, gshift,
-                                                                          cfg.scaffold_gap, bps, pred, bb_ctr + 3);
-                lc.n++;
-            }
+    // claims; a group with a conflict puts itself on a work list: ordinary (thread per group) or large/dense (warp per group:
+    // more than RES_THREAD_MAX positions or an expected window > 64 candidates)
+    k_chain_candidates<false><<<cdiv(n_m, 256), 256, 0, st>>>(srec, skey, gid, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, nullptr, pred, grp_dirty,
+                                                               nullptr, nullptr, c->h_ctr[C_HUGE] ? fx_min : NONE32, work, work_big, bb_ctr);
+    lc.n++;
+    stage_mark(c, "ch_worklists");
+    auto is_huge = [=] __device__(u32 g) -> bool {
+        const u32 s0 = gstart[g], e0 = (g + 1 < n_groups) ? gstart[g + 1] : n_m;
+        return e0 - s0 >= fx_min;
+    };
+    // the redone groups need their candidate records: a second candidate pass over the listed groups only (ordinary data: a
+    // few hundred groups; writing all 16 B records in the first pass cost more than it saved)
+    Cand *cand = A.take<Cand>(n_m); // unconstrained arg-min of every position of the groups that are redone (dirty / huge)
+    k_chain_candidates_groups<<<(u32)c->sm_count * 4, 256, 0, st>>>(srec, skey, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, cand, work, bb_ctr,
+                                                                   work_big, bb_ctr + 2);
+    lc.n++;
+    stage_mark(c, "ch_resolve");
+    // enough threads to hide the dependent-load latency of a step, few enough that every group's lines stay in L1/L2
+    k_chain_resolve<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work, bb_ctr, gshift, cfg.scaffold_gap,
+                                                          bps, pred, bb_ctr + 1);
+    k_chain_resolve_warp<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work_big, bb_ctr + 2, gshift,
+                                                              cfg.scaffold_gap, bps, pred, bb_ctr + 3);
+    lc.n += 2;
+    const u32 n_huge = (u32)c->h_ctr[C_HUGE];
+    if (n_huge) {
+        stage_mark(c, "ch_fixpoint");
+        u32 *hpos = A.take<u32>(n_huge);
+        u32 *d_nh = A.take<u32>(1);
+        u32 *bsum = A.take<u32>(scan_temp_u32(n_m));
+        root_preset = A.take<u32>(n_m);
+        SWG_CUDA(cudaMemsetAsync(root_preset, 0xFF, sizeof(u32) * (size_t)n_m, st));
+        scan_flags([=] __device__(u32 p) -> u32 { return is_huge(gid[p]) ? 1u : 0u; },
+                   [=] __device__(u32 p, u32 ex, u32 v) { if (v) hpos[ex] = p; }, n_m, bsum, d_nh, st, lc);
+        if (!chain_fixpoint(c, n_huge, hpos, srec, skey, gshift, gid, gstart, n_groups, n_m, cfg.scaffold_gap, root_preset, bsum, maxcoord)) {
+            // a dependency chain longer than the round limit: the huge groups go through the sequential warp walk after all
+            // (it resets the groups' pred / best_pred_score itself; root_preset is untouched).  The walk starts from the
+            // candidate records of their positions (position-parallel).
+            k_chain_candidates<true><<<(u32)c->sm_count * 16, 256, 0, st>>>(srec, skey, gid, gstart, n_groups, n_m, gshift, cfg.scaffold_gap, cand, nullptr,
+                                                                             nullptr, hpos, d_nh);
+            lc.n++;
+            SWG_CUDA(cudaMemsetAsync(bb_ctr + 2, 0, 2 * sizeof(u32), st));
+            scan_flags([=] __device__(u32 g) -> u32 { return is_huge(g) ? 1u : 0u; },
+                       [=] __device__(u32 g, u32 ex, u32 v) { if (v) work_big[ex] = g; }, n_groups, bsum, bb_ctr + 2, st, lc);
+            k_chain_resolve_warp<<<(u32)c->sm_count * 4, 128, 0, st>>>(cand, srec, skey, gstart, n_groups, n_m, work_big, bb_ctr + 2, gshift,
+                                                                      cfg.scaffold_gap, bps, pred, bb_ctr + 3);
+            lc.n++;
         }
     }
+    return Chained{pred, root_preset, n_huge, bb_ctr};
+}
+
+// ---- K4: roots + dense chain numbers (k_chain_number), aggregates, the mass/identity filter, the passing chains sorted -----
+struct Chains {
+    const u32 *chain_of; // chain number of every sorted position
+    ChainTable ct;       // C rows
+    u32 C, C1;           // chains; chains that pass the mass/identity filter
+    const u64 *okey;     // the C1 passing chains in order: their order keys (first index of the genome pair, of the group) ...
+    const u32 *oval;     // ... and chain numbers
+    u64 pass_zero;       // passing chains with an empty query or target interval
+};
+static Chains chain_table(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, const Ordered &O, const Chained &chained,
+                          cudaEvent_t ev_matches, bool exact_host, swg_stats &S) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const bool cuda_log = c->knobs.cuda_log;
+    u64 *ctr = c->d_ctr;
+    const u32 n_m = O.n_m;
+    const u64 *skey = O.skey;
+    const int gshift = O.gshift;
+    const u32 *gid = O.gid;
+    const int sb = P.sb;
     stage_mark(c, "ch_number");
-    // ---- roots + dense chain numbers in one pass (k_chain_number), then the chain table ---------------
     // The table is sized for the worst case (every position its own chain) and each row is cleared by the kernel that numbers
     // its chain, so the aggregate pass can start before the host knows the chain count (it reads it while that pass runs).
     u32 *chain_of = A.take<u32>(n_m);  // chain number of every sorted position
     u32 *head_pos = A.take<u32>(n_m);  // compacted head positions (C of them)
-    u32 *d_nch = d_tot + 2;
+    u32 *grp_minidx = A.take<u32>(O.n_groups); // per GROUP: min original index over its members (first appearance of the group)
+    u32 *d_cnt = A.take<u32>(2);       // [0] chains, [1] passing chains
+    SWG_CUDA(cudaMemsetAsync(grp_minidx, 0xFF, sizeof(u32) * (size_t)O.n_groups, st));
     ChainTable ct;
     ct.pos = head_pos; ct.qid = A.take<u32>(n_m); ct.tid = A.take<u32>(n_m); ct.fwd = A.take<u8>(n_m);
     ct.qs = A.take<u32>(n_m); ct.qe = A.take<u32>(n_m); ct.ts = A.take<u32>(n_m); ct.te = A.take<u32>(n_m);
@@ -1004,19 +1060,19 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         SWG_CUDA(cudaMemsetAsync(cn_status, 0, sizeof(u64) * (size_t)(tiles + 1), st));
         SWG_CUDA(cudaMemsetAsync(cn_ctr, 0, 2 * sizeof(u32), st));
         SWG_CUDA(cudaMemsetAsync(chain_of, 0xFF, sizeof(u32) * (size_t)n_m, st));
-        if (root_preset) k_chain_number<true><<<tiles, CR_THREADS, 0, st>>>(pred, root_preset, n_m, chain_of, head_pos, cn_status, cn_ctr, d_nch, cd);
-        else k_chain_number<false><<<tiles, CR_THREADS, 0, st>>>(pred, nullptr, n_m, chain_of, head_pos, cn_status, cn_ctr, d_nch, cd);
+        if (chained.root_preset) k_chain_number<true><<<tiles, CR_THREADS, 0, st>>>(chained.pred, chained.root_preset, n_m, chain_of, head_pos, cn_status, cn_ctr, d_cnt, cd);
+        else k_chain_number<false><<<tiles, CR_THREADS, 0, st>>>(chained.pred, nullptr, n_m, chain_of, head_pos, cn_status, cn_ctr, d_cnt, cd);
         lc.n++;
     }
     {   // the chain count (and, as diagnostics, how many groups had to be redone sequentially) travels while the aggregate runs
         u32 *h = reinterpret_cast<u32 *>(c->h_ctr + C_COUNT);
-        SWG_CUDA(cudaMemcpyAsync(h, d_nch, sizeof(u32), cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaMemcpyAsync(h + 2, bb_ctr, 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
-        if (gs_lists) SWG_CUDA(cudaMemcpyAsync(h + 6, gs_lists, 3 * sizeof(u32), cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaMemcpyAsync(h, d_cnt, sizeof(u32), cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaMemcpyAsync(h + 2, chained.bb_ctr, 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
+        if (O.gs_lists) SWG_CUDA(cudaMemcpyAsync(h + 6, O.gs_lists, 3 * sizeof(u32), cudaMemcpyDeviceToHost, st));
         SWG_CUDA(cudaEventRecord(c->ev_ctr, st));
     }
     if (ev_matches) SWG_CUDA(cudaStreamWaitEvent(st, ev_matches, 0)); // first use of in.matches
-    k_chain_aggregate<<<cdiv(n_m, 256), 256, 0, st>>>(srec, in.blen, in.matches, sidx, gid, chain_of, n_m, cd, grp_minidx);
+    k_chain_aggregate<<<cdiv(n_m, 256), 256, 0, st>>>(O.srec, in.blen, in.matches, O.sidx, gid, chain_of, n_m, cd, grp_minidx);
     lc.n++;
     SWG_CUDA(cudaEventSynchronize(c->ev_ctr));
     u32 C;
@@ -1024,7 +1080,7 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         const u32 *h = reinterpret_cast<const u32 *>(c->h_ctr + C_COUNT);
         C = h[0];
         S.n_dirty_groups = (u64)h[2] + h[4];
-        if (gs_lists) S.n_unsorted_groups = (u64)h[6] + h[7] + h[8];
+        if (O.gs_lists) S.n_unsorted_groups = (u64)h[6] + h[7] + h[8];
     }
     stage_mark(c, "chain_table");
     S.n_chains = C;
@@ -1047,14 +1103,16 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         SWG_CUDA(cudaMemcpyAsync(host_lg, lg.data(), sizeof(double) * (size_t)C, cudaMemcpyHostToDevice, st));
         SWG_CUDA(cudaStreamSynchronize(st)); // lg lives on this stack frame
     }
-    const int nb = bits_for(N);
+    const int nb = bits_for(in.n);
     if (2 * nb > 63) throw RangeError{"too many records for the chain order key"};
     u64 *okey_all = A.take<u64>(C);
     {
         const u64 min_len = cfg.min_scaffold_length;
         const double min_sid = cfg.min_scaffold_identity;
         const u32 seqmask = (u32)((1ull << sb) - 1);
-        const u32 hmask = hcap - 1;
+        u64 *hk = P.hk;
+        u32 *hv = P.hv;
+        const u32 hmask = P.hmask;
         launch_for<t_chain_order>(C, st, lc, [=] __device__(u32 ci) {
             const u32 p = head_pos[ci];
             u64 k = skey[p] >> gshift;
@@ -1081,134 +1139,144 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     // only the chains that pass the mass/identity filter take part in the ordering
     u64 *okey = A.take<u64>(C), *okey2 = A.take<u64>(C);
     u32 *oval = A.take<u32>(C), *oval2 = A.take<u32>(C);
+    u32 *bsum = A.take<u32>(scan_temp_u32(C));
     scan_flags([=] __device__(u32 ci) -> u32 { return ct.pass[ci] ? 1u : 0u; },
-               [=] __device__(u32 ci, u32 ex, u32 v) { if (v) { okey[ex] = okey_all[ci]; oval[ex] = ci; } }, C, bsum, d_tot + 3, st, lc);
+               [=] __device__(u32 ci, u32 ex, u32 v) { if (v) { okey[ex] = okey_all[ci]; oval[ex] = ci; } }, C, bsum, d_cnt + 1, st, lc);
     u32 C1;
     {   // the count and the counters in one round trip
         u32 *h = reinterpret_cast<u32 *>(c->h_ctr + C_COUNT);
-        SWG_CUDA(cudaMemcpyAsync(h, d_tot + 3, sizeof(u32), cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaMemcpyAsync(h, d_cnt + 1, sizeof(u32), cudaMemcpyDeviceToHost, st));
         read_counters(c);
         C1 = *h;
     }
-    const u64 pass_zero = c->h_ctr[C_PASS_ZEROSPAN];
     sort_pairs(c, okey, okey2, oval, oval2, C1, 2 * nb); // stable: ties (same group) keep head-position order
     S.n_chains_after_mass = C1;
+    return Chains{chain_of, ct, C, C1, okey, oval, c->h_ctr[C_PASS_ZEROSPAN]};
+}
 
+// ---- O* + GS: t-space = passing chains in the reference's `filtered_chains` order, scaffold sweep, final order ------------
+struct KeptChains {
+    u32 C2 = 0;                   // kept chains, numbered u + 1 = 1 .. C2 in chain_N order
+    const u32 *fin_t = nullptr;   // fin_t[u] = t of the chain numbered u + 1
+    const u32 *t_qs = nullptr, *t_qe = nullptr, *t_ts = nullptr; // t-space columns (t = rank among the passing chains)
+    const u64 *t_c2key = nullptr; // chromosome pair
+    const u8 *t_fwd = nullptr;
+};
+static KeptChains order_chains(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, const Chains &chains, bool exact_host,
+                                swg_stats &S) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const bool cuda_log = c->knobs.cuda_log;
+    u64 *ctr = c->d_ctr;
+    const u32 C1 = chains.C1;
+    const ChainTable ct = chains.ct;
+    const int sb = P.sb, nb = bits_for(in.n);
     stage_mark(c, "chain_order");
-    // ---- O*: t-space = passing chains in the reference's `filtered_chains` order ------------------
+    if (C1 == 0) return KeptChains{};
     // oc_chain[t] = dense chain id of the t-th filtered chain
-    const u32 *oc_chain = oval;
-    u32 C2 = 0;
-    u32 *fin_t = nullptr; // fin_t[u] = t of the chain numbered u+1
-    u32 *t_qs = nullptr, *t_qe = nullptr, *t_ts = nullptr, *t_te = nullptr;
-    u64 *t_c2key = nullptr;
-    u8 *t_fwd = nullptr;
-    if (C1 > 0) {
-        t_qs = A.take<u32>(C1); t_qe = A.take<u32>(C1); t_ts = A.take<u32>(C1); t_te = A.take<u32>(C1);
-        t_c2key = A.take<u64>(C1);
-        u64 *t_g2key = A.take<u64>(C1);
-        t_fwd = A.take<u8>(C1);
-        double *t_score = A.take<double>(C1);
-        const int scoring = cfg.scoring_function;
-        // first appearance (smallest t) of every chromosome pair and genome pair among the filtered chains: two open-addressing
-        // tables with atomicMin (one insert per chain; round 1 sorted the chains twice for this)
-        u32 hcap2 = 1024;
-        while ((u64)hcap2 < (u64)C1 * 2) hcap2 <<= 1;
-        u64 *hk2 = A.take<u64>(hcap2), *hk3 = A.take<u64>(hcap2);
-        u32 *hv2 = A.take<u32>(hcap2), *hv3 = A.take<u32>(hcap2);
-        SWG_CUDA(cudaMemsetAsync(hk2, 0xFF, sizeof(u64) * hcap2, st));
-        SWG_CUDA(cudaMemsetAsync(hk3, 0xFF, sizeof(u64) * hcap2, st));
-        SWG_CUDA(cudaMemsetAsync(hv2, 0xFF, sizeof(u32) * hcap2, st));
-        SWG_CUDA(cudaMemsetAsync(hv3, 0xFF, sizeof(u32) * hcap2, st));
-        const u32 hmask2 = hcap2 - 1;
-        launch_for<t_tspace>(C1, st, lc, [=] __device__(u32 t) {
-            u32 ci = oc_chain[t];
-            u32 q = ct.qid[ci], tt = ct.tid[ci];
-            t_qs[t] = ct.qs[ci]; t_qe[t] = ct.qe[ci]; t_ts[t] = ct.ts[ci]; t_te[t] = ct.te[ci];
-            const u64 c2 = ((u64)q << sb) | tt, g2 = ((u64)in.P2[q] << sb) | in.P2[tt];
-            t_c2key[t] = c2;
-            t_g2key[t] = g2;
-            t_fwd[t] = ct.fwd[ci];
-            t_score[t] = score_fn(scoring, ct.wid[ci], ct.qs[ci], ct.qe[ci], cuda_log);
-            hash_insert_min(hk2, hv2, hmask2, c2, t);
-            hash_insert_min(hk3, hv3, hmask2, g2, t);
+    const u32 *oc_chain = chains.oval;
+    u32 *t_qs = A.take<u32>(C1), *t_qe = A.take<u32>(C1), *t_ts = A.take<u32>(C1), *t_te = A.take<u32>(C1);
+    u64 *t_c2key = A.take<u64>(C1);
+    u64 *t_g2key = A.take<u64>(C1);
+    u8 *t_fwd = A.take<u8>(C1);
+    double *t_score = A.take<double>(C1);
+    const int scoring = cfg.scoring_function;
+    // first appearance (smallest t) of every chromosome pair and genome pair among the filtered chains: two open-addressing
+    // tables with atomicMin (one insert per chain; round 1 sorted the chains twice for this)
+    u64 *hk2, *hk3;
+    u32 *hv2, *hv3;
+    const u32 hmask2 = first_index_table(c, C1, hk2, hv2);
+    first_index_table(c, C1, hk3, hv3);
+    launch_for<t_tspace>(C1, st, lc, [=] __device__(u32 t) {
+        u32 ci = oc_chain[t];
+        u32 q = ct.qid[ci], tt = ct.tid[ci];
+        t_qs[t] = ct.qs[ci]; t_qe[t] = ct.qe[ci]; t_ts[t] = ct.ts[ci]; t_te[t] = ct.te[ci];
+        const u64 c2 = ((u64)q << sb) | tt, g2 = ((u64)in.P2[q] << sb) | in.P2[tt];
+        t_c2key[t] = c2;
+        t_g2key[t] = g2;
+        t_fwd[t] = ct.fwd[ci];
+        t_score[t] = score_fn(scoring, ct.wid[ci], ct.qs[ci], ct.qe[ci], cuda_log);
+        hash_insert_min(hk2, hv2, hmask2, c2, t);
+        hash_insert_min(hk3, hv3, hmask2, g2, t);
+    });
+    if (exact_host) { // exact re-rank: the chain scores from the host libm as well
+        std::vector<double> hw(C1), hs(C1);
+        std::vector<u32> hq0(C1), hq1(C1);
+        double *d_w = A.take<double>(C1);
+        launch_for<t_tspace>(C1, st, lc, [=] __device__(u32 t) { d_w[t] = ct.wid[oc_chain[t]]; });
+        SWG_CUDA(cudaMemcpyAsync(hw.data(), d_w, sizeof(double) * (size_t)C1, cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaMemcpyAsync(hq0.data(), t_qs, sizeof(u32) * (size_t)C1, cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaMemcpyAsync(hq1.data(), t_qe, sizeof(u32) * (size_t)C1, cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaStreamSynchronize(st));
+        for (u32 t = 0; t < C1; t++) hs[t] = host_score(scoring, hw[t], hq0[t], hq1[t]);
+        SWG_CUDA(cudaMemcpyAsync(t_score, hs.data(), sizeof(double) * (size_t)C1, cudaMemcpyHostToDevice, st));
+        SWG_CUDA(cudaStreamSynchronize(st)); // hs lives on this stack frame
+    }
+    u32 *g2min = A.take<u32>(C1);
+    u64 *sk = A.take<u64>(C1), *sk2 = A.take<u64>(C1);
+    u32 *sv = A.take<u32>(C1), *sv2 = A.take<u32>(C1);
+    // scaffold plane sweep (plane_sweep_scaffold.rs:47-251)
+    u8 *t_keep = nullptr;
+    u64 nq, nt;
+    if (cfg.scaffold_filter_mode == SWG_ONE_TO_ONE) { nq = 1; nt = 1; }
+    else { nq = cfg.scaffold_max_per_query; nt = cfg.scaffold_max_per_target; }
+    const bool need_sweep = C1 > 1 && (nq != SWG_KEEP_ALL || nt != SWG_KEEP_ALL || chains.pass_zero > 0);
+    if (need_sweep) {
+        u8 *k1 = A.take<u8>(C1);
+        t_keep = A.take<u8>(C1);
+        general_sweep(c, C1, nullptr, 0, t_c2key, 2 * sb, P.cb, t_qs, t_qe, t_score, nq, cfg.scaffold_overlap_threshold, k1);
+        general_sweep(c, C1, k1, 1, t_c2key, 2 * sb, P.cb, t_ts, t_te, t_score, nt, cfg.scaffold_overlap_threshold, t_keep);
+    }
+    // final order: (g2min, c2min, t) in ONE stable sort (t is the input order); dropped chains sort last
+    const int ob = bits_for(C1);
+    if (2 * ob + 1 > 64) throw RangeError{"too many chains for the final order key"};
+    {
+        u64 *skw = sk;
+        u32 *svw = sv;
+        launch_for<t_keys_g2min>(C1, st, lc, [=] __device__(u32 t) {
+            const bool kept = t_keep ? t_keep[t] != 0 : true;
+            const u32 gm = hash_lookup(hk3, hv3, hmask2, t_g2key[t]), cm = hash_lookup(hk2, hv2, hmask2, t_c2key[t]);
+            g2min[t] = gm;
+            skw[t] = kept ? (((u64)gm << ob) | cm) : (1ull << (2 * ob));
+            svw[t] = t;
+            const u32 am = __activemask();
+            const u32 nk = __popc(__ballot_sync(am, kept));
+            if (nk && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd((unsigned long long *)&ctr[C_KEPT_CHAINS], (unsigned long long)nk);
         });
-        if (exact_host) { // exact re-rank: the chain scores from the host libm as well
-            std::vector<double> hw(C1), hs(C1);
-            std::vector<u32> hq0(C1), hq1(C1);
-            double *d_w = A.take<double>(C1);
-            launch_for<t_tspace>(C1, st, lc, [=] __device__(u32 t) { d_w[t] = ct.wid[oc_chain[t]]; });
-            SWG_CUDA(cudaMemcpyAsync(hw.data(), d_w, sizeof(double) * (size_t)C1, cudaMemcpyDeviceToHost, st));
-            SWG_CUDA(cudaMemcpyAsync(hq0.data(), t_qs, sizeof(u32) * (size_t)C1, cudaMemcpyDeviceToHost, st));
-            SWG_CUDA(cudaMemcpyAsync(hq1.data(), t_qe, sizeof(u32) * (size_t)C1, cudaMemcpyDeviceToHost, st));
-            SWG_CUDA(cudaStreamSynchronize(st));
-            for (u32 t = 0; t < C1; t++) hs[t] = host_score(scoring, hw[t], hq0[t], hq1[t]);
-            SWG_CUDA(cudaMemcpyAsync(t_score, hs.data(), sizeof(double) * (size_t)C1, cudaMemcpyHostToDevice, st));
-            SWG_CUDA(cudaStreamSynchronize(st)); // hs lives on this stack frame
-        }
-        u32 *g2min = A.take<u32>(C1);
-        u64 *sk = A.take<u64>(C1), *sk2 = A.take<u64>(C1);
-        u32 *sv = A.take<u32>(C1), *sv2 = A.take<u32>(C1);
-        // scaffold plane sweep (plane_sweep_scaffold.rs:47-251)
-        u8 *t_keep = nullptr;
-        u64 nq, nt;
-        if (cfg.scaffold_filter_mode == SWG_ONE_TO_ONE) { nq = 1; nt = 1; }
-        else { nq = cfg.scaffold_max_per_query; nt = cfg.scaffold_max_per_target; }
-        const bool need_sweep = C1 > 1 && (nq != SWG_KEEP_ALL || nt != SWG_KEEP_ALL || pass_zero > 0);
-        if (need_sweep) {
-            u8 *k1 = A.take<u8>(C1);
-            t_keep = A.take<u8>(C1);
-            general_sweep(c, C1, nullptr, 0, t_c2key, 2 * sb, cb, t_qs, t_qe, t_score, nq, cfg.scaffold_overlap_threshold, k1);
-            general_sweep(c, C1, k1, 1, t_c2key, 2 * sb, cb, t_ts, t_te, t_score, nt, cfg.scaffold_overlap_threshold, t_keep);
-        }
-        // final order: (g2min, c2min, t) in ONE stable sort (t is the input order); dropped chains sort last
-        const int ob = bits_for(C1);
-        if (2 * ob + 1 > 64) throw RangeError{"too many chains for the final order key"};
-        {
-            u64 *skw = sk;
-            u32 *svw = sv;
-            launch_for<t_keys_g2min>(C1, st, lc, [=] __device__(u32 t) {
-                const bool kept = t_keep ? t_keep[t] != 0 : true;
-                const u32 gm = hash_lookup(hk3, hv3, hmask2, t_g2key[t]), cm = hash_lookup(hk2, hv2, hmask2, t_c2key[t]);
-                g2min[t] = gm;
-                skw[t] = kept ? (((u64)gm << ob) | cm) : (1ull << (2 * ob));
-                svw[t] = t;
-                const u32 am = __activemask();
-                const u32 nk = __popc(__ballot_sync(am, kept));
-                if (nk && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd((unsigned long long *)&ctr[C_KEPT_CHAINS], (unsigned long long)nk);
-            });
-        }
-        read_counters_begin(c); // the kept-chain count is final here; the host picks it up while the sort runs
-        sort_pairs(c, sk, sk2, sv, sv2, C1, 2 * ob + 1);
-        read_counters_end(c);
-        C2 = (u32)c->h_ctr[C_KEPT_CHAINS];
-        S.score_near_ties = c->h_ctr[C_NEAR_TIES];
-        fin_t = sv;
-        {
-            const u32 *fin = sv;
-            // chain number + the order key of its genome-pair group (first-appearance indices A, B of the group's first
-            // filtered chain): what a multi-GPU driver needs to merge the per-shard numberings (swg_last_chain_keys)
-            c->keys.reserve(((size_t)C2 + 1) * 8 + 1024); // context-owned: later calls that rewind the scratch arena do not touch it
-            u32 *keyA = c->keys.take<u32>(C2 + 1), *keyB = c->keys.take<u32>(C2 + 1);
-            const u64 *okc = okey;
-            const u64 bmask = (1ull << nb) - 1;
-            launch_for<t_final_k>(C2, st, lc, [=] __device__(u32 u) {
-                const u32 t = fin[u];
-                ct.k[oc_chain[t]] = u + 1;
-                const u64 gk = okc[g2min[t]];
-                keyA[u] = (u32)(gk >> nb);
-                keyB[u] = (u32)(gk & bmask);
-            });
-            c->last_keyA = keyA;
-            c->last_keyB = keyB;
-        }
+    }
+    read_counters_begin(c); // the kept-chain count is final here; the host picks it up while the sort runs
+    sort_pairs(c, sk, sk2, sv, sv2, C1, 2 * ob + 1);
+    read_counters_end(c);
+    const u32 C2 = (u32)c->h_ctr[C_KEPT_CHAINS];
+    S.score_near_ties = c->h_ctr[C_NEAR_TIES];
+    {
+        const u32 *fin = sv;
+        // chain number + the order key of its genome-pair group (first-appearance indices A, B of the group's first
+        // filtered chain): what a multi-GPU driver needs to merge the per-shard numberings (swg_last_chain_keys)
+        c->keys.reserve(((size_t)C2 + 1) * 8 + 1024); // context-owned: later calls that rewind the scratch arena do not touch it
+        u32 *keyA = c->keys.take<u32>(C2 + 1), *keyB = c->keys.take<u32>(C2 + 1);
+        const u64 *okc = chains.okey;
+        const u64 bmask = (1ull << nb) - 1;
+        launch_for<t_final_k>(C2, st, lc, [=] __device__(u32 u) {
+            const u32 t = fin[u];
+            ct.k[oc_chain[t]] = u + 1;
+            const u64 gk = okc[g2min[t]];
+            keyA[u] = (u32)(gk >> nb);
+            keyB[u] = (u32)(gk & bmask);
+        });
+        c->last_keyA = keyA;
+        c->last_keyB = keyB;
     }
     c->last_n_chains = C2;
     S.n_chains_kept = C2;
+    return KeptChains{C2, sv, t_qs, t_qe, t_ts, t_c2key, t_fwd};
+}
 
-    stage_mark(c, "assign+inversion+rescue");
-    // ---- K5: anchors = members of kept chains (paf_filter.rs:517-528) ---------------------------------
-    launch_for<t_assign>(n_m, st, lc, [=] __device__(u32 p) {
+// ---- K5: anchors = members of kept chains (paf_filter.rs:517-528) ---------------------------------
+static void assign_anchors(swg_ctx *c, const Ordered &O, const Chains &chains, u8 *flags, u8 *status, u32 *chain_id) {
+    const u32 *chain_of = chains.chain_of;
+    const SortedIdx sidx = O.sidx;
+    const ChainTable ct = chains.ct;
+    launch_for<t_assign>(O.n_m, c->stream, c->lc, [=] __device__(u32 p) {
         u32 ci = chain_of[p];
         u32 i = sidx[p];
         u32 kk = ct.k[ci];
@@ -1216,358 +1284,412 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
         const u8 add = (u8)((kk ? F_ANCHOR : 0) | (ct.pass[ci] ? F_PREMEM : 0));
         if (add) flags[i] |= add;
     });
+}
 
-    if (!cfg.scaffolds_only && C2 > 0) {
-        // ---- K6: inversion capture (paf_filter.rs:535-597) ------------------------------------------
-        // kept chains in chain_N order u; ik[u] = chromosome pair of a '+' chain, NONE64 for a '-' chain; u_c2[u] = the pair of
-        // either.  The final order groups the chains by chromosome pair, so a pair's chains are one run of u: the table below
-        // maps a pair to the start of its run (atomicMin of u).
-        u64 *ik = A.take<u64>(C2), *ik2 = A.take<u64>(C2);
-        u32 *iv = A.take<u32>(C2), *iv2 = A.take<u32>(C2);
-        u32 *u_qs = A.take<u32>(C2), *u_qe = A.take<u32>(C2), *u_ts = A.take<u32>(C2);
-        u64 *u_c2 = A.take<u64>(C2);
-        u32 hcap4 = 1024;
-        while ((u64)hcap4 < (u64)C2 * 2) hcap4 <<= 1;
-        u64 *hk4 = A.take<u64>(hcap4);
-        u32 *hv4 = A.take<u32>(hcap4);
-        const u32 hmask4 = hcap4 - 1;
-        SWG_CUDA(cudaMemsetAsync(hk4, 0xFF, sizeof(u64) * hcap4, st));
-        SWG_CUDA(cudaMemsetAsync(hv4, 0xFF, sizeof(u32) * hcap4, st));
-        {
-            const u32 *fin = fin_t;
-            launch_for<t_invkeys>(C2, st, lc, [=] __device__(u32 u) {
-                u32 t = fin[u];
-                bool f = t_fwd[t] != 0;
-                const u64 c2 = t_c2key[t];
-                ik[u] = f ? c2 : NONE64;
-                iv[u] = u;
-                u_c2[u] = c2;
-                u_qs[u] = t_qs[t]; u_qe[u] = t_qe[t]; u_ts[u] = t_ts[t];
-                hash_insert_min(hk4, hv4, hmask4, c2, u);
-            });
-        }
-        // A chromosome pair that holds a huge group can hold 10^5..10^6 kept chains; walking all of them for every
-        // reverse mapping is O(n * chains).  Then (or with SWG_INV_GRID=1) chains and mappings meet in buckets of the query axis.
-        const int wb0 = std::max(17, bits_for(2 * cfg.scaffold_gap + 1)); // widest bucket: 2^wb0 > 2 * jump
-        const bool inv_grid = (n_huge > 0 || K.inv_grid) && 2 * sb + (cb > wb0 ? cb - wb0 : 1) + 1 <= 64;
-        if (inv_grid) {
-            stage_mark(c, "inversion_grid");
-            const u64 G = cfg.scaffold_gap;
-            const u64 maxc = maxcoord;
-            u32 *d_cnt = A.take<u32>(2); // [0] entries, [1] candidate mappings
-            u32 *inv_list = A.take<u32>(N);
-            scan_flags([=] __device__(u32 i) -> u32 { return (flags[i] & (F_ALIVE | F_REV | F_ANCHOR)) == (F_ALIVE | F_REV) ? 1u : 0u; },
-                       [=] __device__(u32 i, u32 ex, u32 v) { if (v) inv_list[ex] = i; }, N, bsum, d_cnt + 1, st, lc);
-            // Bucket width of the query axis.  The chains of a (pair, '+') group are numbered in query order, so the entries of a bucket
-            // ascend along the query axis and a mapping in the middle of a wide bucket walks every chain that ends more than a jump to
-            // its left before the first it can belong to (20 M pile, 2^17: 1560 entries per mapping).  Narrow buckets make nearly every
-            // entry of a cell a hit on the query axis; they cost entries (a chain enters every bucket its extended interval touches)
-            // and cells per mapping.  Both are counted for the widths 2^wb0 .. 2^12 and the narrowest width within budget is taken.
-            constexpr int NW = 6;
-            unsigned long long *wcnt = (unsigned long long *)A.take<u64>(2 * NW);
-            SWG_CUDA(cudaMemsetAsync(wcnt, 0, 2 * NW * sizeof(u64), st));
-            launch_for<t_invw>(C2, st, lc, [=] __device__(u32 u) {
-                const bool f = ik[u] != NONE64;
-                const u64 a0 = u_qs[u] > G ? (u64)u_qs[u] - G : 0, e0 = (u64)u_qe[u] + G < maxc ? (u64)u_qe[u] + G : maxc;
-                const u32 am = __activemask();
-#pragma unroll
-                for (int k = 0; k < NW; k++) {
-                    const int w = wb0 - k;
-                    const u32 v = f && w >= 12 ? (u32)((e0 >> w) - (a0 >> w) + 1) : 0u;
-                    const u32 sum = __reduce_add_sync(am, v);
-                    if (sum && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd(&wcnt[k], (unsigned long long)sum);
-                }
-            });
-            launch_for_dev<t_invw2>(d_cnt + 1, c->sm_count, st, lc, [=] __device__(u32 x) {
-                const u32 i = inv_list[x];
-                const u64 qs0 = in.qs[i], qe0 = in.qe[i];
-                const u32 am = __activemask();
-#pragma unroll
-                for (int k = 0; k < NW; k++) {
-                    const int w = wb0 - k;
-                    const u32 v = w >= 12 ? (u32)((qe0 >> w) - (qs0 >> w) + 1) : 0u;
-                    const u32 sum = __reduce_add_sync(am, v);
-                    if (sum && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd(&wcnt[NW + k], (unsigned long long)sum);
-                }
-            });
-            u32 *h2 = reinterpret_cast<u32 *>(c->h_ctr + C_COUNT);
-            unsigned long long hw[2 * NW];
-            SWG_CUDA(cudaMemcpyAsync(h2 + 1, d_cnt + 1, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            SWG_CUDA(cudaMemcpyAsync(hw, wcnt, sizeof hw, cudaMemcpyDeviceToHost, st));
-            SWG_CUDA(cudaStreamSynchronize(st));
-            int wb = wb0;
-            // (only where chains are many: a pair with a pile holds 10^5 and more; a few hundred chromosome-scale chains would just be cut
-            // into thousands of entries each)
-            for (int k = NW - 1; k > 0; k--) {
-                const int w = wb0 - k;
-                if (w < 12 || K.inv_wide || (C2 < 65536 && !K.inv_narrow)) continue;
-                const bool fits = 2 * sb + (cb > w ? cb - w : 1) + 1 <= 64;
-                if (fits && hw[k] <= std::max<u64>(1ull << 25, 8ull * C2) && hw[k] < (1ull << 31) && hw[NW + k] <= 3ull * h2[1] + 1024) { wb = w; break; }
-            }
-            const int bb = cb > wb ? cb - wb : 1;
-            // ... and in buckets of the diagonal (target_start - query_start of a chain against the centre diagonal of a mapping): the
-            // deviation test floor(|dev| / sqrt 2) <= G admits |dev| <= R only, so a mapping meets the chains of the diagonal buckets
-            // that [dm - R, dm + R] touches.  Width: an eighth of 2 R + 1 (a mapping walks up to ten narrow cells, but a cell it can only
-            // fail in is small); wider while the key would pass 64 bits, no diagonal buckets if it still does.
-            const u64 R = (u64)std::ceil((double)(G + 1) * 1.4142135623730951) + 1; // |dev| > R  =>  perp > G
-            int wd = std::max(bits_for(2 * R + 1) - 3, 8);
-            const u64 doff = maxc + 1; // diagonals are shifted to be non-negative: they lie in [-maxc, maxc]
-            int db = bits_for((2 * maxc + 2) >> wd);
-            while (2 * sb + bb + db > 64 && wd < bits_for(2 * R + 1)) { wd++; db = bits_for((2 * maxc + 2) >> wd); }
-            if (2 * sb + bb + db > 64 || K.inv_no_diag) db = 0;
-            // entries: every kept '+' chain once per bucket its extended query interval [qs - G, qe + G] touches
-            u32 *e_off = A.take<u32>(C2);
-            auto first_b = [=] __device__(u32 u) -> u32 { const u64 a = u_qs[u]; return (u32)((a > G ? a - G : 0) >> wb); };
-            auto last_b = [=] __device__(u32 u) -> u32 { const u64 e = (u64)u_qe[u] + G; return (u32)((e < maxc ? e : maxc) >> wb); };
-            scan_apply([=] __device__(u32 u) -> u32 { return ik[u] != NONE64 ? last_b(u) - first_b(u) + 1 : 0u; },
-                       [=] __device__(u32 u, u32 ex, u32) { e_off[u] = ex; }, C2, bsum, d_cnt, st, lc);
-            SWG_CUDA(cudaMemcpyAsync(h2, d_cnt, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            SWG_CUDA(cudaStreamSynchronize(st));
-            if (getenv("SWG_STAGE_TIMING")) fprintf(stderr, "[swg inversion] query buckets 2^%d (widest 2^%d), diagonal buckets 2^%d (%d bits)\n", wb, wb0, wd, db);
-            const u32 n_ent = h2[0], n_inv = h2[1];
-            if (n_ent && n_inv) {
-                u64 *ek = A.take<u64>(n_ent), *ek2 = A.take<u64>(n_ent);
-                u32 *ev = A.take<u32>(n_ent), *ev2 = A.take<u32>(n_ent);
-                launch_for<t_invent>(C2, st, lc, [=] __device__(u32 u) {
-                    if (ik[u] == NONE64) return;
-                    const u32 b0 = first_b(u), b1 = last_b(u);
-                    u32 o = e_off[u];
-                    const u64 dg = db ? ((u64)((i64)u_ts[u] - (i64)u_qs[u] + (i64)doff) >> wd) : 0;
-                    for (u32 b = b0; b <= b1; b++, o++) { ek[o] = (((ik[u] << bb) | b) << db) | dg; ev[o] = u; }
-                });
-                sort_pairs(c, ek, ek2, ev, ev2, n_ent, 2 * sb + bb + db); // stable: chains stay in k order inside a bucket
-                uint4 *ent = A.take<uint4>(n_ent);
-                {
-                    const u32 *evc = ev;
-                    launch_for<t_gather>(n_ent, st, lc, [=] __device__(u32 x) { const u32 u = evc[x]; ent[x] = make_uint4(u_qs[u], u_qe[u], u_ts[u], u); });
-                }
-                // the candidates ordered by (pair, first bucket): neighbouring threads walk the same entries
-                u64 *qk = A.take<u64>(n_inv), *qk2 = A.take<u64>(n_inv);
-                u32 *qv = A.take<u32>(n_inv), *qv2 = A.take<u32>(n_inv);
-                launch_for<t_invkeys>(n_inv, st, lc, [=] __device__(u32 x) {
-                    const u32 i = inv_list[x];
-                    qk[x] = (((((u64)in.qid[i] << sb) | in.tid[i])) << bb) | ((u64)in.qs[i] >> wb);
-                    qv[x] = i;
-                });
-                sort_pairs(c, qk, qk2, qv, qv2, n_inv, 2 * sb + bb);
-                const u64 *ekc = ek, *qkc = qk;
-                const u32 *qvc = qv;
-                unsigned long long *inv_dbg = (unsigned long long *)A.take<u64>(4);
-                SWG_CUDA(cudaMemsetAsync(inv_dbg, 0, 4 * sizeof(u64), st));
-                const bool dbg = getenv("SWG_STAGE_TIMING") != nullptr;
-                launch_for<t_inversion>(n_inv, st, lc, [=] __device__(u32 x0) {
-                    u32 n_walk = 0, n_cells = 0;
-                    const u32 i = qvc[x0];
-                    const u64 mqs = in.qs[i], mqe = in.qe[i], mts = in.ts[i], mte = in.te[i];
-                    const u64 qc = (mqs + mqe) / 2, tc = (mts + mte) / 2;
-                    const u64 pairkey = qkc[x0] >> bb;
-                    u32 best = NONE32; // smallest u = the first chain in the reference's order (paf_filter.rs:553-596)
-                    const u64 dm = (u64)((i64)tc - (i64)qc + (i64)doff);
-                    const u64 d0 = db ? (dm > R ? dm - R : 0) >> wd : 0, d1 = db ? (dm + R) >> wd : 0;
-                    for (u64 b = mqs >> wb; b <= (mqe >> wb); b++)
-                    for (u64 dg = d0; dg <= d1; dg++) {
-                        const u64 key = (((pairkey << bb) | b) << db) | dg;
-                        u32 lo = 0, hi = n_ent;
-                        while (lo < hi) { const u32 mid = (lo + hi) >> 1; if (ekc[mid] < key) lo = mid + 1; else hi = mid; }
-                        n_cells++;
-                        for (u32 x = lo; x < n_ent && ekc[x] == key; x++) {
-                            n_walk++;
-                            const uint4 ch = ent[x];
-                            if (ch.w >= best) break; // entries of a bucket ascend in u
-                            const u64 cqs = ch.x, cqe = ch.y, cts = ch.z;
-                            const u64 ext_s = cqs > G ? cqs - G : 0, ext_e = cqe + G;
-                            if (mqe < ext_s || mqs > ext_e) continue;
-                            const i64 dv = (i64)tc - (i64)qc - ((i64)cts - (i64)cqs);
-                            const u64 dev = dv < 0 ? (u64)(-dv) : (u64)dv;
-                            const u64 perp = (u64)__ddiv_rn((double)dev, 1.4142135623730951);
-                            if (perp <= G) { best = ch.w; break; }
-                        }
-                    }
-                    if (best != NONE32) { status[i] = 1; chain_id[i] = best + 1; flags[i] |= F_ANCHOR; }
-                    if (dbg) { atomicAdd(&inv_dbg[0], (unsigned long long)n_walk); atomicAdd(&inv_dbg[1], (unsigned long long)n_cells); atomicMax(&inv_dbg[2], (unsigned long long)n_walk); if (best != NONE32) atomicAdd(&inv_dbg[3], 1ull); }
-                });
-                if (dbg) {
-                    unsigned long long hd[4];
-                    SWG_CUDA(cudaMemcpyAsync(hd, inv_dbg, sizeof hd, cudaMemcpyDeviceToHost, st));
-                    SWG_CUDA(cudaStreamSynchronize(st));
-                    fprintf(stderr, "[swg inversion] %u candidates, %u entries, %llu entries walked (max %llu per candidate), %llu cells, %llu captured\n", n_inv, n_ent, hd[0], hd[2], hd[1], hd[3]);
-                }
-            }
-        } else {
-        {
-            // the candidates (reverse strand, alive, not yet an anchor: a few per cent of the records) are compacted first, in
-            // no particular order (each is judged on its own); a candidate looks its chromosome pair up and walks the pair's run
-            // of chains in chain_N order — the reference's loop over the kept '+' chains "in order", first hit wins
-            // (paf_filter.rs:553-596)
-            const u64 G = cfg.scaffold_gap;
-            const u64 *ikc = ik;
-            u32 *inv_list = A.take<u32>(N);
-            u32 *d_ninv = A.take<u32>(1);
-            scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & (F_ALIVE | F_REV | F_ANCHOR)) == (F_ALIVE | F_REV); },
-                       [=] __device__(u32 i, u32 slot, u32 v) { if (v) inv_list[slot] = i; }, N, bsum, d_ninv, st, lc);
-            launch_for_dev<t_inversion>(d_ninv, c->sm_count, st, lc, [=] __device__(u32 x0) {
-                const u32 i = inv_list[x0];
-                const u64 key = ((u64)in.qid[i] << sb) | in.tid[i];
-                const u32 u0 = hash_lookup(hk4, hv4, hmask4, key);
-                if (u0 == NONE32) return;
-                u64 mqs = in.qs[i], mqe = in.qe[i], mts = in.ts[i], mte = in.te[i];
-                u64 qc = (mqs + mqe) / 2, tc = (mts + mte) / 2;
-                for (u32 u = u0; u < C2 && u_c2[u] == key; u++) {
-                    if (ikc[u] == NONE64) continue; // a '-' chain
-                    u64 cqs = u_qs[u], cqe = u_qe[u], cts = u_ts[u];
-                    u64 ext_s = cqs > G ? cqs - G : 0, ext_e = cqe + G;
-                    if (mqe < ext_s || mqs > ext_e) continue;
-                    i64 dv = (i64)tc - (i64)qc - ((i64)cts - (i64)cqs);
-                    u64 dev = dv < 0 ? (u64)(-dv) : (u64)dv;
-                    u64 perp = (u64)__ddiv_rn((double)dev, 1.4142135623730951);
-                    if (perp <= G) { status[i] = 1; chain_id[i] = u + 1; flags[i] |= F_ANCHOR; break; }
-                }
-            });
-        }
-        } // !inv_grid
+// ---- K6: inversion capture (paf_filter.rs:535-597) ------------------------------------------------
+// Does a reverse mapping (query interval [mqs, mqe], centres qc / tc) belong to the '+' chain that starts at (cqs, cts) and ends at
+// query cqe?  Its query interval must touch the chain's, extended by G on both sides, and its centre must lie within
+// floor(|dev| / sqrt 2) <= G of the chain's diagonal.
+static __device__ __forceinline__ bool inversion_hit(u64 mqs, u64 mqe, u64 qc, u64 tc, u64 cqs, u64 cqe, u64 cts, u64 G) {
+    const u64 ext_s = cqs > G ? cqs - G : 0, ext_e = cqe + G;
+    if (mqe < ext_s || mqs > ext_e) return false;
+    const i64 dv = (i64)tc - (i64)qc - ((i64)cts - (i64)cqs);
+    const u64 dev = dv < 0 ? (u64)(-dv) : (u64)dv;
+    return (u64)__ddiv_rn((double)dev, 1.4142135623730951) <= G;
+}
 
-        // ---- K7: rescue (paf_filter.rs:613-732) -----------------------------------------------------
-        const u64 D = cfg.scaffold_max_deviation;
-        if (D > 0) {
-            // anchor list (status == 1) ordered by (chromosome pair, query center); one sort when the key fits 64 bits,
-            // else two chained stable sorts (center first, then the pair)
-            const bool wide_a = (2 * sb + cb > 63) || K.force_wide;
-            u64 *ak = A.take<u64>(N), *ak2 = A.take<u64>(N);
-            u32 *av = A.take<u32>(N), *av2 = A.take<u32>(N);
-            u32 *d_na = A.take<u32>(2);
-            u32 NA = 0;
-            u64 *apair = nullptr;
-            u32 *aqc = nullptr;
-            bool a_done = false;
-            const int ibN = bits_for(N - 1);
-            if (gsort && !wide_a && c->rows_grouped && cb + ibN <= 64 && 2 * sb + 1 + ibN <= 64) {
-                // the group sort with the chromosome pair as group (the strand bit of the table index stays 0) and the query centre as
-                // secondary key: anchors come grouped like the records and nearly in centre order
-                const u32 dead = (1u << (2 * sb + 1)) - 1;
-                {
-                    u64 *kk = ak;
-                    launch_for<t_anchor_keys>(N, st, lc, [=] __device__(u32 i) {
-                        const bool anchor = (flags[i] & F_ANCHOR) != 0;
-                        const u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2;
-                        kk[i] = anchor ? ((((((u64)in.qid[i] << sb) | in.tid[i]) << 1) << cb) | qc) : (((u64)dead << cb) | ((1ull << cb) - 1));
-                    });
-                }
-                aqc = A.take<u32>((size_t)N + 1);
-                const u32 limit = K.group_sort_max ? std::min(K.group_sort_max, GS_CTA_MAX) : GS_CTA_MAX;
-                const GroupSorted gs = group_sort(c, ak, ak2, ak, av2, N, cb, GsIndex{1, sb, in.n_seq}, dead, g_entries, ibN, limit, false, aqc);
-                if (gs.done) {
-                    a_done = true;
-                    NA = gs.n_rec;
-                    apair = A.take<u64>((size_t)NA + 1);
-                    const u64 *w = ak;
-                    const u64 imask = (1ull << ibN) - 1;
-                    u64 *ap = apair;
-                    u32 *avw = av;
-                    launch_for<t_gather>(NA, st, lc, [=] __device__(u32 x) { ap[x] = w[x] >> (ibN + 1); avw[x] = (u32)(w[x] & imask); });
-                }
+// A chromosome pair that holds a huge group can hold 10^5..10^6 kept chains; walking all of them for every reverse mapping is
+// O(n * chains).  Then chains and mappings meet in buckets of the query axis (2^wb0: the widest bucket) and of the diagonal.
+// ik[u] = chromosome pair of the kept chain u if it is a '+' chain, NONE64 for a '-' chain; u_qs / u_qe / u_ts its coordinates.
+static void inversion_grid(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, u32 C2, const u64 *ik, const u32 *u_qs,
+                           const u32 *u_qe, const u32 *u_ts, int wb0, u8 *status, u32 *chain_id) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const Knobs &K = c->knobs;
+    const u32 N = in.n;
+    u8 *flags = P.flags;
+    const int sb = P.sb, cb = P.cb;
+    stage_mark(c, "inversion_grid");
+    const u64 G = cfg.scaffold_gap;
+    const u64 maxc = P.maxcoord;
+    u32 *d_cnt = A.take<u32>(2); // [0] entries, [1] candidate mappings
+    u32 *inv_list = A.take<u32>(N);
+    u32 *bsum = A.take<u32>(scan_temp_u32(N));
+    scan_flags([=] __device__(u32 i) -> u32 { return (flags[i] & (F_ALIVE | F_REV | F_ANCHOR)) == (F_ALIVE | F_REV) ? 1u : 0u; },
+               [=] __device__(u32 i, u32 ex, u32 v) { if (v) inv_list[ex] = i; }, N, bsum, d_cnt + 1, st, lc);
+    // Bucket width of the query axis.  The chains of a (pair, '+') group are numbered in query order, so the entries of a bucket
+    // ascend along the query axis and a mapping in the middle of a wide bucket walks every chain that ends more than a jump to
+    // its left before the first it can belong to (20 M pile, 2^17: 1560 entries per mapping).  Narrow buckets make nearly every
+    // entry of a cell a hit on the query axis; they cost entries (a chain enters every bucket its extended interval touches)
+    // and cells per mapping.  Both are counted for the widths 2^wb0 .. 2^12 and the narrowest width within budget is taken.
+    constexpr int NW = 6;
+    unsigned long long *wcnt = (unsigned long long *)A.take<u64>(2 * NW);
+    SWG_CUDA(cudaMemsetAsync(wcnt, 0, 2 * NW * sizeof(u64), st));
+    launch_for<t_invw>(C2, st, lc, [=] __device__(u32 u) {
+        const bool f = ik[u] != NONE64;
+        const u64 a0 = u_qs[u] > G ? (u64)u_qs[u] - G : 0, e0 = (u64)u_qe[u] + G < maxc ? (u64)u_qe[u] + G : maxc;
+        const u32 am = __activemask();
+#pragma unroll
+        for (int k = 0; k < NW; k++) {
+            const int w = wb0 - k;
+            const u32 v = f && w >= 12 ? (u32)((e0 >> w) - (a0 >> w) + 1) : 0u;
+            const u32 sum = __reduce_add_sync(am, v);
+            if (sum && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd(&wcnt[k], (unsigned long long)sum);
+        }
+    });
+    launch_for_dev<t_invw2>(d_cnt + 1, c->sm_count, st, lc, [=] __device__(u32 x) {
+        const u32 i = inv_list[x];
+        const u64 qs0 = in.qs[i], qe0 = in.qe[i];
+        const u32 am = __activemask();
+#pragma unroll
+        for (int k = 0; k < NW; k++) {
+            const int w = wb0 - k;
+            const u32 v = w >= 12 ? (u32)((qe0 >> w) - (qs0 >> w) + 1) : 0u;
+            const u32 sum = __reduce_add_sync(am, v);
+            if (sum && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd(&wcnt[NW + k], (unsigned long long)sum);
+        }
+    });
+    u32 *h2 = reinterpret_cast<u32 *>(c->h_ctr + C_COUNT);
+    unsigned long long hw[2 * NW];
+    SWG_CUDA(cudaMemcpyAsync(h2 + 1, d_cnt + 1, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    SWG_CUDA(cudaMemcpyAsync(hw, wcnt, sizeof hw, cudaMemcpyDeviceToHost, st));
+    SWG_CUDA(cudaStreamSynchronize(st));
+    int wb = wb0;
+    // (only where chains are many: a pair with a pile holds 10^5 and more; a few hundred chromosome-scale chains would just be cut
+    // into thousands of entries each)
+    for (int k = NW - 1; k > 0; k--) {
+        const int w = wb0 - k;
+        if (w < 12 || K.inv_wide || (C2 < 65536 && !K.inv_narrow)) continue;
+        const bool fits = 2 * sb + (cb > w ? cb - w : 1) + 1 <= 64;
+        if (fits && hw[k] <= std::max<u64>(1ull << 25, 8ull * C2) && hw[k] < (1ull << 31) && hw[NW + k] <= 3ull * h2[1] + 1024) { wb = w; break; }
+    }
+    const int bb = cb > wb ? cb - wb : 1;
+    // ... and in buckets of the diagonal (target_start - query_start of a chain against the centre diagonal of a mapping): the
+    // deviation test floor(|dev| / sqrt 2) <= G admits |dev| <= R only, so a mapping meets the chains of the diagonal buckets
+    // that [dm - R, dm + R] touches.  Width: an eighth of 2 R + 1 (a mapping walks up to ten narrow cells, but a cell it can only
+    // fail in is small); wider while the key would pass 64 bits, no diagonal buckets if it still does.
+    const u64 R = (u64)std::ceil((double)(G + 1) * 1.4142135623730951) + 1; // |dev| > R  =>  perp > G
+    int wd = std::max(bits_for(2 * R + 1) - 3, 8);
+    const u64 doff = maxc + 1; // diagonals are shifted to be non-negative: they lie in [-maxc, maxc]
+    int db = bits_for((2 * maxc + 2) >> wd);
+    while (2 * sb + bb + db > 64 && wd < bits_for(2 * R + 1)) { wd++; db = bits_for((2 * maxc + 2) >> wd); }
+    if (2 * sb + bb + db > 64 || K.inv_no_diag) db = 0;
+    // entries: every kept '+' chain once per bucket its extended query interval [qs - G, qe + G] touches
+    u32 *e_off = A.take<u32>(C2);
+    auto first_b = [=] __device__(u32 u) -> u32 { const u64 a = u_qs[u]; return (u32)((a > G ? a - G : 0) >> wb); };
+    auto last_b = [=] __device__(u32 u) -> u32 { const u64 e = (u64)u_qe[u] + G; return (u32)((e < maxc ? e : maxc) >> wb); };
+    scan_apply([=] __device__(u32 u) -> u32 { return ik[u] != NONE64 ? last_b(u) - first_b(u) + 1 : 0u; },
+               [=] __device__(u32 u, u32 ex, u32) { e_off[u] = ex; }, C2, bsum, d_cnt, st, lc);
+    SWG_CUDA(cudaMemcpyAsync(h2, d_cnt, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    SWG_CUDA(cudaStreamSynchronize(st));
+    const bool dbg = K.stage_timing;
+    if (dbg) fprintf(stderr, "[swg inversion] query buckets 2^%d (widest 2^%d), diagonal buckets 2^%d (%d bits)\n", wb, wb0, wd, db);
+    const u32 n_ent = h2[0], n_inv = h2[1];
+    if (!n_ent || !n_inv) return;
+    u64 *ek = A.take<u64>(n_ent), *ek2 = A.take<u64>(n_ent);
+    u32 *ev = A.take<u32>(n_ent), *ev2 = A.take<u32>(n_ent);
+    launch_for<t_invent>(C2, st, lc, [=] __device__(u32 u) {
+        if (ik[u] == NONE64) return;
+        const u32 b0 = first_b(u), b1 = last_b(u);
+        u32 o = e_off[u];
+        const u64 dg = db ? ((u64)((i64)u_ts[u] - (i64)u_qs[u] + (i64)doff) >> wd) : 0;
+        for (u32 b = b0; b <= b1; b++, o++) { ek[o] = (((ik[u] << bb) | b) << db) | dg; ev[o] = u; }
+    });
+    sort_pairs(c, ek, ek2, ev, ev2, n_ent, 2 * sb + bb + db); // stable: chains stay in k order inside a bucket
+    uint4 *ent = A.take<uint4>(n_ent);
+    {
+        const u32 *evc = ev;
+        launch_for<t_gather>(n_ent, st, lc, [=] __device__(u32 x) { const u32 u = evc[x]; ent[x] = make_uint4(u_qs[u], u_qe[u], u_ts[u], u); });
+    }
+    // the candidates ordered by (pair, first bucket): neighbouring threads walk the same entries
+    u64 *qk = A.take<u64>(n_inv), *qk2 = A.take<u64>(n_inv);
+    u32 *qv = A.take<u32>(n_inv), *qv2 = A.take<u32>(n_inv);
+    launch_for<t_invkeys>(n_inv, st, lc, [=] __device__(u32 x) {
+        const u32 i = inv_list[x];
+        qk[x] = (((((u64)in.qid[i] << sb) | in.tid[i])) << bb) | ((u64)in.qs[i] >> wb);
+        qv[x] = i;
+    });
+    sort_pairs(c, qk, qk2, qv, qv2, n_inv, 2 * sb + bb);
+    const u64 *ekc = ek, *qkc = qk;
+    const u32 *qvc = qv;
+    unsigned long long *inv_dbg = (unsigned long long *)A.take<u64>(4);
+    SWG_CUDA(cudaMemsetAsync(inv_dbg, 0, 4 * sizeof(u64), st));
+    launch_for<t_inversion>(n_inv, st, lc, [=] __device__(u32 x0) {
+        u32 n_walk = 0, n_cells = 0;
+        const u32 i = qvc[x0];
+        const u64 mqs = in.qs[i], mqe = in.qe[i], mts = in.ts[i], mte = in.te[i];
+        const u64 qc = (mqs + mqe) / 2, tc = (mts + mte) / 2;
+        const u64 pairkey = qkc[x0] >> bb;
+        u32 best = NONE32; // smallest u = the first chain in the reference's order (paf_filter.rs:553-596)
+        const u64 dm = (u64)((i64)tc - (i64)qc + (i64)doff);
+        const u64 d0 = db ? (dm > R ? dm - R : 0) >> wd : 0, d1 = db ? (dm + R) >> wd : 0;
+        for (u64 b = mqs >> wb; b <= (mqe >> wb); b++)
+        for (u64 dg = d0; dg <= d1; dg++) {
+            const u64 key = (((pairkey << bb) | b) << db) | dg;
+            u32 lo = 0, hi = n_ent;
+            while (lo < hi) { const u32 mid = (lo + hi) >> 1; if (ekc[mid] < key) lo = mid + 1; else hi = mid; }
+            n_cells++;
+            for (u32 x = lo; x < n_ent && ekc[x] == key; x++) {
+                n_walk++;
+                const uint4 ch = ent[x];
+                if (ch.w >= best) break; // entries of a bucket ascend in u
+                if (inversion_hit(mqs, mqe, qc, tc, ch.x, ch.y, ch.z, G)) { best = ch.w; break; }
             }
-            if (!a_done) {
-            scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & F_ANCHOR) != 0; },
-                       [=] __device__(u32 i, u32 ex, u32 v) {
-                           if (!v) return;
-                           u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2;
-                           ak[ex] = wide_a ? qc : (((((u64)in.qid[i] << sb) | in.tid[i]) << cb) | qc);
-                           av[ex] = i;
-                       },
-                       N, bsum, d_na, st, lc);
-            NA = read_u32(c, d_na);
-            if (!wide_a) {
-                sort_pairs(c, ak, ak2, av, av2, NA, 2 * sb + cb);
-            } else {
-                sort_pairs(c, ak, ak2, av, av2, NA, cb);
-                {
-                    u64 *kk = ak;
-                    const u32 *vv = av;
-                    launch_for<t_gather>(NA, st, lc, [=] __device__(u32 x) { const u32 i = vv[x]; kk[x] = ((u64)in.qid[i] << sb) | in.tid[i]; });
-                }
-                sort_pairs(c, ak, ak2, av, av2, NA, 2 * sb);
-            }
-            apair = A.take<u64>(NA + 1);
-            aqc = A.take<u32>(NA + 1);
-            {
-                const u64 *akc = ak;
-                const u32 *avc = av;
-                const u64 cmask = (1ull << cb) - 1;
-                u64 *ap = apair;
-                u32 *aq = aqc;
-                launch_for<t_anchor_keys>(NA, st, lc, [=] __device__(u32 x) {
-                    if (wide_a) { const u32 i = avc[x]; ap[x] = akc[x]; aq[x] = (u32)(((u64)in.qs[i] + in.qe[i]) / 2); }
-                    else { ap[x] = akc[x] >> cb; aq[x] = (u32)(akc[x] & cmask); }
-                });
-            }
-            }
-            // candidates (alive, not an anchor, not a member of a swept-away scaffold), compacted so the searches run dense
-            u32 *rlist = A.take<u32>(N);
-            scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & (F_ALIVE | F_ANCHOR | F_PREMEM)) == F_ALIVE; },
-                       [=] __device__(u32 i, u32 slot, u32 v) { if (v) rlist[slot] = i; }, N, bsum, d_na + 1, st, lc);
-            const u32 *avc = av;
-            const u32 *d_nr = d_na + 1;
-            // The reference squares in u64 and wraps (a release build): qd^2 + td^2 passes 2^64 once td reaches ~0.866 * 2^32, and the
-            // wrapped sum can put a far anchor inside D.  Every scanned anchor has qd <= D and td <= max(tc, maxcoord - tc) (anchor
-            // centres lie in [0, maxcoord]), so for a candidate with (D^2 + that^2 < 2^64) the sum never wraps and the two shortcuts
-            // below hold; for any other candidate every anchor with qd <= D is measured.  Only target centres beyond 3.7 * 10^9 from
-            // one end of the coordinate range take that path (on a repeat pile it costs O(anchors within +-D) per candidate).
-            const u64 wrap_lim = ~0ull - D * D; // D < 2^31 (checked on entry)
-            const bool may_wrap = (u64)maxcoord * maxcoord > wrap_lim;
-            const u64 maxc = maxcoord;
-            launch_for_dev<t_rescue>(d_nr, c->sm_count, st, lc, [=] __device__(u32 x0) {
-                const u32 i = rlist[x0];
-                const u64 pair = ((u64)in.qid[i] << sb) | in.tid[i];
-                const u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2, tc = ((u64)in.ts[i] + in.te[i]) / 2;
-                const u64 td_max = tc > maxc - tc ? tc : maxc - tc;
-                const bool wrap = may_wrap && td_max * td_max > wrap_lim;
-                // first anchor of the pair at or right of the query center; the scan runs outwards from there and stops once
-                // the query-axis distance alone exceeds the best distance found: dist = floor(sqrt(qd^2 + td^2)) >= qd - 1 (the f64
-                // square root of a rounded sum can fall one short), so nothing beyond qd > best + 1 can win or tie.  On a repeat pile
-                // (10^5..10^6 anchors inside +-D) that is a handful of anchors instead of all of them.  Not when the sum may wrap.
-                u32 lo = 0, hi = NA;
-                while (lo < hi) {
-                    u32 mid = (lo + hi) >> 1;
-                    const u64 mp = apair[mid];
-                    if (mp < pair || (mp == pair && (u64)aqc[mid] < qc)) lo = mid + 1; else hi = mid;
-                }
-                u64 best_d = NONE64;
-                u32 best_a = NONE32;
-                auto visit = [&](u32 x, u64 qd) {
-                    const u32 a = avc[x];
-                    const u64 atc = ((u64)in.ts[a] + in.te[a]) / 2;
-                    const u64 td = atc > tc ? atc - tc : tc - atc;
-                    if (td > D && !wrap) return; // then floor(sqrt(qd^2+td^2)) > D
-                    const u64 dist = (u64)__dsqrt_rn((double)(qd * qd + td * td)); // u64: wraps like the reference
-                    if (dist <= D && (dist < best_d || (dist == best_d && a < best_a))) { best_d = dist; best_a = a; }
-                };
-                for (u32 x = lo; x < NA && apair[x] == pair; x++) {
-                    const u64 qd = (u64)aqc[x] - qc;
-                    if (qd > D || (!wrap && best_a != NONE32 && qd > best_d + 1)) break;
-                    visit(x, qd);
-                }
-                for (u32 x = lo; x > 0;) {
-                    x--;
-                    if (apair[x] != pair) break;
-                    const u64 qd = qc - (u64)aqc[x];
-                    if (qd > D || (!wrap && best_a != NONE32 && qd > best_d + 1)) break;
-                    visit(x, qd);
-                }
-                if (best_a != NONE32) { status[i] = 2; chain_id[i] = chain_id[best_a]; }
+        }
+        if (best != NONE32) { status[i] = 1; chain_id[i] = best + 1; flags[i] |= F_ANCHOR; }
+        if (dbg) { atomicAdd(&inv_dbg[0], (unsigned long long)n_walk); atomicAdd(&inv_dbg[1], (unsigned long long)n_cells); atomicMax(&inv_dbg[2], (unsigned long long)n_walk); if (best != NONE32) atomicAdd(&inv_dbg[3], 1ull); }
+    });
+    if (dbg) {
+        unsigned long long hd[4];
+        SWG_CUDA(cudaMemcpyAsync(hd, inv_dbg, sizeof hd, cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaStreamSynchronize(st));
+        fprintf(stderr, "[swg inversion] %u candidates, %u entries, %llu entries walked (max %llu per candidate), %llu cells, %llu captured\n", n_inv, n_ent, hd[0], hd[2], hd[1], hd[3]);
+    }
+}
+
+// kept chains in chain_N order u; ik[u] = chromosome pair of a '+' chain, NONE64 for a '-' chain; u_c2[u] = the pair of either.  The
+// final order groups the chains by chromosome pair, so a pair's chains are one run of u: the table below maps a pair to the start
+// of its run (atomicMin of u).
+static void capture_inversions(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, u32 n_huge, const KeptChains &kc,
+                               u8 *status, u32 *chain_id) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const u32 N = in.n, C2 = kc.C2;
+    u8 *flags = P.flags;
+    const int sb = P.sb, cb = P.cb;
+    const u32 *t_qs = kc.t_qs, *t_qe = kc.t_qe, *t_ts = kc.t_ts;
+    const u64 *t_c2key = kc.t_c2key;
+    const u8 *t_fwd = kc.t_fwd;
+    u64 *ik = A.take<u64>(C2), *ik2 = A.take<u64>(C2);
+    u32 *iv = A.take<u32>(C2), *iv2 = A.take<u32>(C2);
+    u32 *u_qs = A.take<u32>(C2), *u_qe = A.take<u32>(C2), *u_ts = A.take<u32>(C2);
+    u64 *u_c2 = A.take<u64>(C2);
+    u64 *hk4;
+    u32 *hv4;
+    const u32 hmask4 = first_index_table(c, C2, hk4, hv4);
+    {
+        const u32 *fin = kc.fin_t;
+        launch_for<t_invkeys>(C2, st, lc, [=] __device__(u32 u) {
+            u32 t = fin[u];
+            bool f = t_fwd[t] != 0;
+            const u64 c2 = t_c2key[t];
+            ik[u] = f ? c2 : NONE64;
+            iv[u] = u;
+            u_c2[u] = c2;
+            u_qs[u] = t_qs[t]; u_qe[u] = t_qe[t]; u_ts[u] = t_ts[t];
+            hash_insert_min(hk4, hv4, hmask4, c2, u);
+        });
+    }
+    // a huge group (or SWG_INV_GRID=1) takes the buckets of inversion_grid
+    const int wb0 = std::max(17, bits_for(2 * cfg.scaffold_gap + 1)); // widest bucket: 2^wb0 > 2 * jump
+    if ((n_huge > 0 || c->knobs.inv_grid) && 2 * sb + (cb > wb0 ? cb - wb0 : 1) + 1 <= 64) {
+        inversion_grid(c, cfg, in, P, C2, ik, u_qs, u_qe, u_ts, wb0, status, chain_id);
+        return;
+    }
+    // the candidates (reverse strand, alive, not yet an anchor: a few per cent of the records) are compacted first, in
+    // no particular order (each is judged on its own); a candidate looks its chromosome pair up and walks the pair's run
+    // of chains in chain_N order — the reference's loop over the kept '+' chains "in order", first hit wins
+    // (paf_filter.rs:553-596)
+    const u64 G = cfg.scaffold_gap;
+    const u64 *ikc = ik;
+    u32 *inv_list = A.take<u32>(N);
+    u32 *d_ninv = A.take<u32>(1);
+    u32 *bsum = A.take<u32>(scan_temp_u32(N));
+    scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & (F_ALIVE | F_REV | F_ANCHOR)) == (F_ALIVE | F_REV); },
+               [=] __device__(u32 i, u32 slot, u32 v) { if (v) inv_list[slot] = i; }, N, bsum, d_ninv, st, lc);
+    launch_for_dev<t_inversion>(d_ninv, c->sm_count, st, lc, [=] __device__(u32 x0) {
+        const u32 i = inv_list[x0];
+        const u64 key = ((u64)in.qid[i] << sb) | in.tid[i];
+        const u32 u0 = hash_lookup(hk4, hv4, hmask4, key);
+        if (u0 == NONE32) return;
+        u64 mqs = in.qs[i], mqe = in.qe[i], mts = in.ts[i], mte = in.te[i];
+        u64 qc = (mqs + mqe) / 2, tc = (mts + mte) / 2;
+        for (u32 u = u0; u < C2 && u_c2[u] == key; u++) {
+            if (ikc[u] == NONE64) continue; // a '-' chain
+            if (inversion_hit(mqs, mqe, qc, tc, u_qs[u], u_qe[u], u_ts[u], G)) { status[i] = 1; chain_id[i] = u + 1; flags[i] |= F_ANCHOR; break; }
+        }
+    });
+}
+
+// ---- K7: rescue (paf_filter.rs:613-732) -----------------------------------------------------
+static void rescue(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, u8 *status, u32 *chain_id) {
+    cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
+    const Knobs &K = c->knobs;
+    const u32 N = in.n;
+    u8 *flags = P.flags;
+    const int sb = P.sb, cb = P.cb;
+    const u64 D = cfg.scaffold_max_deviation;
+    // anchor list (status == 1) ordered by (chromosome pair, query center); one sort when the key fits 64 bits,
+    // else two chained stable sorts (center first, then the pair)
+    const bool wide_a = (2 * sb + cb > 63) || K.force_wide;
+    u64 *ak = A.take<u64>(N), *ak2 = A.take<u64>(N);
+    u32 *av = A.take<u32>(N), *av2 = A.take<u32>(N);
+    u32 *d_na = A.take<u32>(2);
+    u32 *bsum = A.take<u32>(scan_temp_u32(N));
+    u32 NA = 0;
+    u64 *apair = nullptr;
+    u32 *aqc = nullptr;
+    bool a_done = false;
+    const int ibN = bits_for(N - 1);
+    if (P.gsort && !wide_a && c->rows_grouped && cb + ibN <= 64 && 2 * sb + 1 + ibN <= 64) {
+        // the group sort with the chromosome pair as group (the strand bit of the table index stays 0) and the query centre as
+        // secondary key: anchors come grouped like the records and nearly in centre order
+        const u32 dead = (1u << (2 * sb + 1)) - 1;
+        {
+            u64 *kk = ak;
+            launch_for<t_anchor_keys>(N, st, lc, [=] __device__(u32 i) {
+                const bool anchor = (flags[i] & F_ANCHOR) != 0;
+                const u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2;
+                kk[i] = anchor ? ((((((u64)in.qid[i] << sb) | in.tid[i]) << 1) << cb) | qc) : (((u64)dead << cb) | ((1ull << cb) - 1));
             });
         }
+        aqc = A.take<u32>((size_t)N + 1);
+        const GroupSorted gs = group_sort(c, ak, ak2, ak, av2, N, cb, GsIndex{1, sb, in.n_seq}, dead, P.g_entries, ibN, group_sort_limit(K), false, aqc);
+        if (gs.done) {
+            a_done = true;
+            NA = gs.n_rec;
+            apair = A.take<u64>((size_t)NA + 1);
+            const u64 *w = ak;
+            const u64 imask = (1ull << ibN) - 1;
+            u64 *ap = apair;
+            u32 *avw = av;
+            launch_for<t_gather>(NA, st, lc, [=] __device__(u32 x) { ap[x] = w[x] >> (ibN + 1); avw[x] = (u32)(w[x] & imask); });
+        }
+    }
+    if (!a_done) {
+        scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & F_ANCHOR) != 0; },
+                   [=] __device__(u32 i, u32 ex, u32 v) {
+                       if (!v) return;
+                       u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2;
+                       ak[ex] = wide_a ? qc : (((((u64)in.qid[i] << sb) | in.tid[i]) << cb) | qc);
+                       av[ex] = i;
+                   },
+                   N, bsum, d_na, st, lc);
+        NA = read_u32(c, d_na);
+        if (!wide_a) sort_pairs(c, ak, ak2, av, av2, NA, 2 * sb + cb);
+        else sort_pairs_wide(c, ak, ak2, av, av2, NA, cb, 2 * sb, [=] __device__(u32 i) { return ((u64)in.qid[i] << sb) | in.tid[i]; });
+        apair = A.take<u64>(NA + 1);
+        aqc = A.take<u32>(NA + 1);
+        const u64 *akc = ak;
+        const u32 *avc = av;
+        const u64 cmask = (1ull << cb) - 1;
+        u64 *ap = apair;
+        u32 *aq = aqc;
+        launch_for<t_anchor_keys>(NA, st, lc, [=] __device__(u32 x) {
+            if (wide_a) { const u32 i = avc[x]; ap[x] = akc[x]; aq[x] = (u32)(((u64)in.qs[i] + in.qe[i]) / 2); }
+            else { ap[x] = akc[x] >> cb; aq[x] = (u32)(akc[x] & cmask); }
+        });
+    }
+    // candidates (alive, not an anchor, not a member of a swept-away scaffold), compacted so the searches run dense
+    u32 *rlist = A.take<u32>(N);
+    scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & (F_ALIVE | F_ANCHOR | F_PREMEM)) == F_ALIVE; },
+               [=] __device__(u32 i, u32 slot, u32 v) { if (v) rlist[slot] = i; }, N, bsum, d_na + 1, st, lc);
+    const u32 *avc = av;
+    const u32 *d_nr = d_na + 1;
+    // The reference squares in u64 and wraps (a release build): qd^2 + td^2 passes 2^64 once td reaches ~0.866 * 2^32, and the
+    // wrapped sum can put a far anchor inside D.  Every scanned anchor has qd <= D and td <= max(tc, maxcoord - tc) (anchor
+    // centres lie in [0, maxcoord]), so for a candidate with (D^2 + that^2 < 2^64) the sum never wraps and the two shortcuts
+    // below hold; for any other candidate every anchor with qd <= D is measured.  Only target centres beyond 3.7 * 10^9 from
+    // one end of the coordinate range take that path (on a repeat pile it costs O(anchors within +-D) per candidate).
+    const u64 wrap_lim = ~0ull - D * D; // D < 2^31 (checked on entry)
+    const bool may_wrap = (u64)P.maxcoord * P.maxcoord > wrap_lim;
+    const u64 maxc = P.maxcoord;
+    launch_for_dev<t_rescue>(d_nr, c->sm_count, st, lc, [=] __device__(u32 x0) {
+        const u32 i = rlist[x0];
+        const u64 pair = ((u64)in.qid[i] << sb) | in.tid[i];
+        const u64 qc = ((u64)in.qs[i] + in.qe[i]) / 2, tc = ((u64)in.ts[i] + in.te[i]) / 2;
+        const u64 td_max = tc > maxc - tc ? tc : maxc - tc;
+        const bool wrap = may_wrap && td_max * td_max > wrap_lim;
+        // first anchor of the pair at or right of the query center; the scan runs outwards from there and stops once
+        // the query-axis distance alone exceeds the best distance found: dist = floor(sqrt(qd^2 + td^2)) >= qd - 1 (the f64
+        // square root of a rounded sum can fall one short), so nothing beyond qd > best + 1 can win or tie.  On a repeat pile
+        // (10^5..10^6 anchors inside +-D) that is a handful of anchors instead of all of them.  Not when the sum may wrap.
+        u32 lo = 0, hi = NA;
+        while (lo < hi) {
+            u32 mid = (lo + hi) >> 1;
+            const u64 mp = apair[mid];
+            if (mp < pair || (mp == pair && (u64)aqc[mid] < qc)) lo = mid + 1; else hi = mid;
+        }
+        u64 best_d = NONE64;
+        u32 best_a = NONE32;
+        auto visit = [&](u32 x, u64 qd) {
+            const u32 a = avc[x];
+            const u64 atc = ((u64)in.ts[a] + in.te[a]) / 2;
+            const u64 td = atc > tc ? atc - tc : tc - atc;
+            if (td > D && !wrap) return; // then floor(sqrt(qd^2+td^2)) > D
+            const u64 dist = (u64)__dsqrt_rn((double)(qd * qd + td * td)); // u64: wraps like the reference
+            if (dist <= D && (dist < best_d || (dist == best_d && a < best_a))) { best_d = dist; best_a = a; }
+        };
+        for (u32 x = lo; x < NA && apair[x] == pair; x++) {
+            const u64 qd = (u64)aqc[x] - qc;
+            if (qd > D || (!wrap && best_a != NONE32 && qd > best_d + 1)) break;
+            visit(x, qd);
+        }
+        for (u32 x = lo; x > 0;) {
+            x--;
+            if (apair[x] != pair) break;
+            const u64 qd = qc - (u64)aqc[x];
+            if (qd > D || (!wrap && best_a != NONE32 && qd > best_d + 1)) break;
+            visit(x, qd);
+        }
+        if (best_a != NONE32) { status[i] = 2; chain_id[i] = chain_id[best_a]; }
+    });
+}
+
+// exact_host: every logarithm on the path comes from the HOST libm (in.score carries the record scores; the chain-level
+// logs are computed on the host from small downloads) — the exact re-rank of DESIGN 4d, not the normal path.
+static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *status, u32 *chain_id, swg_stats *stats,
+                       cudaEvent_t ev_matches = nullptr /* recorded when in.matches has arrived (swg_filter overlaps that copy) */,
+                       bool exact_host = false) {
+    const u32 N = in.n;
+    const u64 launches0 = c->lc.n;
+    swg_stats S;
+    std::memset(&S, 0, sizeof S);
+    S.n_input = N;
+    c->sort_passes = 0;
+    c->sort_pairs = 0;
+    c->sort_bytes_per_pair = 24;
+    c->stage_used = 0;
+    c->last_n_chains = 0;
+    c->last_keyA = c->last_keyB = nullptr;
+    c->last_flags = nullptr;
+    if (N == 0) { SWG_CUDA(cudaStreamSynchronize(c->stream)); finish(c, S, launches0, stats); return; }
+    // (status / chain_id are cleared by prefilter, while the host waits for the first small read)
+    if (cfg.scaffold_gap >= (1ull << 31) || cfg.scaffold_max_deviation >= (1ull << 31))
+        throw RangeError{"scaffold_gap / scaffold_max_deviation must be < 2^31"};
+
+    const Limits lim = mapping_limits(cfg);
+    const Prefiltered P = prefilter(c, cfg, in, lim, status, chain_id, ev_matches, S);
+    const Kept kept = primary_sweep(c, cfg, in, P, lim, ev_matches);
+    if (cfg.scaffold_gap == 0) { // no-scaffold exit (paf_filter.rs:409-434)
+        k_unassigned<<<cdiv(N, 256), 256, 0, c->stream>>>(N, P.flags, kept.q, kept.t, status, c->d_ctr);
+        c->lc.n++;
+        read_counters(c);
+        S.n_after_sweep = S.n_kept = c->h_ctr[C_KEPT];
+        S.score_near_ties = c->h_ctr[C_NEAR_TIES];
+        finish(c, S, launches0, stats);
+        return;
+    }
+    const Ordered O = order_records(c, cfg, in, P, kept, S);
+    if (O.n_m == 0) { finish(c, S, launches0, stats); return; }
+    const Chained chained = chain_groups(c, cfg, O, P.maxcoord);
+    const Chains chains = chain_table(c, cfg, in, P, O, chained, ev_matches, exact_host, S);
+    const KeptChains kc = order_chains(c, cfg, in, P, chains, exact_host, S);
+
+    stage_mark(c, "assign+inversion+rescue");
+    assign_anchors(c, O, chains, P.flags, status, chain_id);
+    if (!cfg.scaffolds_only && kc.C2 > 0) {
+        capture_inversions(c, cfg, in, P, chained.n_huge, kc, status, chain_id);
+        if (cfg.scaffold_max_deviation > 0) rescue(c, cfg, in, P, status, chain_id);
     }
 
     stage_mark(c, "stats");
-    // ---- stats ---------------------------------------------------------------------------------
-    k_count_status<<<std::min<u32>(cdiv(N, 256), (u32)c->sm_count * 8), 256, 0, st>>>(N, status, ctr);
-    lc.n++;
+    k_count_status<<<std::min<u32>(cdiv(N, 256), (u32)c->sm_count * 8), 256, 0, c->stream>>>(N, status, c->d_ctr);
+    c->lc.n++;
     read_counters(c);
     S.n_anchors = c->h_ctr[C_ANCHORS];
     S.n_rescued = c->h_ctr[C_RESCUED];
     S.n_kept = S.n_anchors + S.n_rescued;
     S.score_near_ties = c->h_ctr[C_NEAR_TIES];
-    finish();
+    finish(c, S, launches0, stats);
 }
 
 // ---- does the device's ln() produce the host libm's bits? ------------------------------------------
@@ -2632,10 +2754,8 @@ swg_paf *swg_paf_parse_device(swg_ctx *c, const char *path) {
 int swg_filter_paf(swg_ctx *c, const swg_config *cfg, const char *in_path, const char *out_path, swg_stats *stats) {
     if (!c || !cfg || !in_path || !out_path) return SWG_ERR_ARG;
     if (!check_cfg(c, cfg)) return SWG_ERR_ARG;
-    {
-        const char *fe = getenv("SWG_PAF_FRONTEND");
-        if (fe && strcmp(fe, "host") == 0) return swg_filter_paf_host(c, cfg, in_path, out_path, stats);
-    }
+    c->knobs = read_knobs();
+    if (c->knobs.paf_host_frontend) return swg_filter_paf_host(c, cfg, in_path, out_path, stats);
     swg_paf hp;
     {
         std::string err;

@@ -678,7 +678,7 @@ static NameTable intern_names(swg_ctx *c, const char *text, const char *host_tex
 
 // Tokenise hp.text on the device.  All device memory comes from c->io and stays valid until the next front-end call.
 static void tokenize_device(swg_ctx *c, const swg_paf &hp, DevPaf &dp) {
-    const u32 long_thresh = getenv("SWG_TOK_LONG") ? (u32)atoi(getenv("SWG_TOK_LONG")) : 4096u; // read per call: the tests vary it
+    const u32 long_thresh = c->knobs.tok_long;
     const u64 B = hp.text_len;
     cudaStream_t st = c->stream;
     LaunchCounter &lc = c->lc;
@@ -823,7 +823,7 @@ static DevIn devin_of(const DevPaf &dp) {
 // Tagged output, assembled on the device window by window (1 GiB of input text per window keeps every offset in u32),
 // copied back through the pinned pieces and written with plain write()s.
 static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u32 *chain_id, const char *out_path) {
-    const bool trace = getenv("SWG_STAGE_TIMING") != nullptr;
+    const bool trace = c->knobs.stage_timing;
     const auto t_begin = std::chrono::steady_clock::now();
     auto lap = [&](const char *what) {
         if (trace) fprintf(stderr, "[swg write] %s at %.1f ms\n", what, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count());
