@@ -7,7 +7,9 @@
 // f64, alignment by alignment — in file order (method "all") or in the order of a stable descending sort by block
 // length / identity / score (method "nX"), cut where the cumulative block length reaches X % of the genome size.
 // With dv:f: tags the addends are not integers, so the order of the additions is part of the result.  Here:
-//   1. the text is tokenised on the device (k_ani_parse; same line scan, hashing and interning as the filter front end)
+//   1. the text is tokenised on the device (k_ani_parse, built from the line grammar of paf_device.cuh; the lines it
+//      lists are patched by the host reader through patch_lines, records compacted by take_records, names interned as
+//      in the filter front end: ani_records)
 //   2. "nX": one stable radix sort on the order-preserving bit pattern of the f64 key; the cut is found from per-tile
 //      integer sums (exact while the block lengths are integers, which a PAF column always is; otherwise the host
 //      walks the sorted column)
@@ -18,34 +20,24 @@
 
 namespace swg {
 
-struct t_ani_pairs; struct t_ani_first; struct t_ani_sizes; struct t_ani_keys; struct t_ani_gather; struct t_ani_fixgather; struct t_ani_patch;
-struct t_ani_tiles;
+struct t_ani_pairs; struct t_ani_first; struct t_ani_sizes; struct t_ani_keys; struct t_ani_gather; struct t_ani_tiles;
 
-enum : u8 { AK_SKIP = 0, AK_OK = 1, AK_FIX = 2 };
-enum { AC_OK = 0, AC_NFIX, AC_NAN, AC_NONINT, AC_INTER, AC_MAXLEN, AC_COUNT };
-
-struct AniCols { // per line, then per record
-    TokCols names;  // off, qh, th, qlen, trel, tlen are used
-    double *m, *b;  // final matches, block length
-    u64 *ql, *tl;   // sequence lengths (columns 2 and 7)
-    u8 *kind;
-};
 struct AniPatch { u32 line; u32 kind; double m, b; u64 ql, tl; };
 
 // One thread per line.  MODE 0: the ANI reader (main.rs:412-460 / :538-604): columns 2 / 7 as u64 into ql / tl, columns
 // 10 / 11 as f64, the first dv:f: tag that parses.  MODE 1: the tree-filter reader (tree_filter.rs:219-245): columns
-// 10 / 11 as u64 (unwrap_or 0 / 1) into ql / tl, no tags; the line length is kept for the output.
+// 10 / 11 as u64 (unwrap_or 0 / 1) into ql / tl, no tags; the line length is kept for the output.  Both skip empty and
+// '#' lines; the longest line is measured before the '\r' is stripped.
 template <int MODE>
-__global__ void __launch_bounds__(256) k_ani_parse(const char *__restrict__ text, const u64 *__restrict__ line_start, u32 n_lines, AniCols L,
-                                                   u32 *__restrict__ fix_list, u64 *__restrict__ ac) {
+__global__ void __launch_bounds__(256) k_ani_parse(const char *__restrict__ text, const u64 *__restrict__ line_start, u32 n_lines, TokCols L,
+                                                   u32 *__restrict__ fix_list, u64 *__restrict__ tc) {
     const u32 l = blockIdx.x * blockDim.x + threadIdx.x;
     bool ok = false;
     if (l < n_lines) {
         const u64 s = line_start[l];
-        u32 len = (u32)min(line_start[l + 1] - 1 - s, (u64)0xFFFFFFF0u);
         const char *line = text + s;
-        if (len > 0 && line[len - 1] == '\r') len--;
-        u8 kind = AK_SKIP;
+        const u32 len = strip_cr(line, line_len_raw(line_start, l));
+        u8 kind = TK_SKIP;
         if (len > 0 && line[0] != '#') {
             u32 a = 0;
             bool fix = false, enough = true;
@@ -56,32 +48,11 @@ __global__ void __launch_bounds__(256) k_ani_parse(const char *__restrict__ text
             for (int nf = 0; nf < 11; nf++) {
                 u32 e = a;
                 if (nf == 0 || nf == 5) {
-                    u64 hh = 0xcbf29ce484222325ull;
-                    while (e < len) {
-                        const u8 ch = (u8)line[e];
-                        if (ch == '\t') break;
-                        hh = (hh ^ ch) * 0x100000001B3ull;
-                        e++;
-                    }
-                    hh = name_hash_finish(hh, e - a);
+                    const u64 hh = name_field(line, a, e, len);
                     if (nf == 0) { qh = hh; qlen = e - a; }
                     else { th = hh; trel = a; tlen = e - a; }
                 } else if (MODE == 0 ? (nf == 1 || nf == 6) : (nf == 9 || nf == 10)) { // parse::<u64>().unwrap_or(0 | 1)
-                    u64 v = 0;
-                    u32 nd = 0;
-                    bool bad = false;
-                    while (e < len) {
-                        const u8 ch = (u8)line[e];
-                        if (ch == '\t') break;
-                        if (!(e == a && ch == '+')) {
-                            const u32 d = (u32)ch - '0';
-                            if (d > 9) bad = true;
-                            else { if (nd < 19) v = v * 10 + d; nd++; }
-                        }
-                        e++;
-                    }
-                    if (bad || nd == 0) v = (MODE == 1 && nf == 10) ? 1 : 0;
-                    else if (nd > 19) fix = true;
+                    const u64 v = u64_field(line, a, e, len, (MODE == 1 && nf == 10) ? 1 : 0, fix);
                     if (nf == 1 || nf == 9) ql = v; else tl = v;
                 } else {
                     while (e < len && line[e] != '\t') e++;
@@ -101,7 +72,7 @@ __global__ void __launch_bounds__(256) k_ani_parse(const char *__restrict__ text
             }
             if (enough) {
                 double fm = m;
-                if (MODE == 1) L.names.len[l] = len;
+                if (MODE == 1) L.len[l] = len;
                 while (MODE == 0 && a <= len && !fix) { // the first dv:f: tag that parses
                     u32 e = a;
                     while (e < len && line[e] != '\t') e++;
@@ -114,28 +85,23 @@ __global__ void __launch_bounds__(256) k_ani_parse(const char *__restrict__ text
                     if (e >= len) break;
                     a = e + 1;
                 }
-                L.names.off[l] = s;
-                L.names.qh[l] = qh; L.names.th[l] = th;
-                L.names.qlen[l] = qlen; L.names.trel[l] = trel; L.names.tlen[l] = tlen;
+                L.off[l] = s;
+                L.qh[l] = qh; L.th[l] = th;
+                L.qlen[l] = qlen; L.trel[l] = trel; L.tlen[l] = tlen;
                 if (MODE == 0) { L.m[l] = fm; L.b[l] = b; }
                 L.ql[l] = ql; L.tl[l] = tl;
                 if (fix) {
-                    kind = AK_FIX;
-                    fix_list[atomicAdd((unsigned long long *)&ac[AC_NFIX], 1ull)] = l;
-                } else kind = AK_OK;
+                    kind = TK_FIX;
+                    fix_list[atomicAdd((unsigned long long *)&tc[TC_NFIX], 1ull)] = l;
+                } else kind = TK_OK;
             }
         }
         L.kind[l] = kind;
-        ok = kind == AK_OK;
+        ok = kind == TK_OK;
     }
-    const u32 nok = __syncthreads_count(ok);
-    if (threadIdx.x == 0 && nok) atomicAdd((unsigned long long *)&ac[AC_OK], (unsigned long long)nok);
-    { // the longest line: sizes the output window of write_device (MODE 1); lines of 256 MiB and more are declined
-        u32 mylen = 0;
-        if (l < n_lines) mylen = (u32)min(line_start[l + 1] - 1 - line_start[l], (u64)0xFFFFFFF0u);
-        const u32 mx = __reduce_max_sync(0xFFFFFFFFu, mylen);
-        if (lane_id() == 0 && mx > (u32)ac[AC_MAXLEN]) atomicMax((unsigned long long *)&ac[AC_MAXLEN], (unsigned long long)mx);
-    }
+    count_records(ok, tc);
+    // the longest line sizes the output window of write_device (MODE 1); lines of 256 MiB and more are declined
+    raise_maxlen(l < n_lines ? line_len_raw(line_start, l) : 0, tc);
 }
 
 // one thread per genome pair: the pair's addends are contiguous and in the reference's order
@@ -159,6 +125,66 @@ __global__ void __launch_bounds__(128) k_ani_pair_sums(const double *__restrict_
 struct AniResult { double ani50 = 0.0; u64 n_pairs = 0; u64 n_alignments = 0; };
 struct NanError {};
 
+// The host readers of the lines k_ani_parse lists, as patch records.
+static bool ani_reparse(const char *line, size_t len, AniPatch &p) {
+    AniLine al;
+    const bool ok = paf_ani_line(line, len, &al);
+    p.kind = ok ? TK_OK : TK_SKIP; p.m = al.matches; p.b = al.block; p.ql = al.qlen; p.tl = al.tlen;
+    return ok;
+}
+static bool tree_reparse(const char *line, size_t len, AniPatch &p) {
+    AniLine al;
+    p.ql = 0; p.tl = 1;
+    const bool ok = paf_tree_line(line, len, &al, &p.ql, &p.tl);
+    p.kind = ok ? TK_OK : TK_SKIP;
+    return ok;
+}
+
+// The records of the ANI (MODE 0) or tree (MODE 1) reader: k_ani_parse, the host reader for the lines it lists, the
+// compaction, and the names interned (*nt).  tc: the zeroed TC_COUNT counter block.  Returns 0 records (nothing else
+// is set) when no line is an alignment.
+template <int MODE>
+static u32 ani_records(swg_ctx *c, const swg_paf &hp, const DevLines &dl, u64 *tc, TokCols *R, NameTable *nt) {
+    constexpr u32 READER = MODE == 0 ? RD_ANI : RD_TREE;
+    const TokCols L = take_cols<READER>(c->io, dl.n_lines);
+    u32 *fix_list = c->io.take<u32>(dl.n_lines);
+    u64 h_tc[TC_COUNT];
+    k_ani_parse<MODE><<<cdiv(dl.n_lines, 256), 256, 0, c->stream>>>(dl.text, dl.line_start, dl.n_lines, L, fix_list, tc);
+    c->lc.n++;
+    tok_read(c, tc, h_tc);
+    if (h_tc[TC_MAXLEN] > ((u64)256 << 20)) throw FrontEndFallback{"a line longer than 256 MiB"};
+    c->tok_maxlen = (u32)h_tc[TC_MAXLEN];
+    u64 n_ok = h_tc[TC_OK];
+    if (h_tc[TC_NFIX]) // numbers outside the plain grammar: the host's line reader decides
+        n_ok += patch_lines<AniPatch>(
+            c, hp, dl, fix_list, (u32)h_tc[TC_NFIX],
+            MODE == 0 ? ani_reparse : tree_reparse,
+            [=] __device__(const AniPatch &p) {
+                L.kind[p.line] = (u8)p.kind;
+                if (MODE == 0) { L.m[p.line] = p.m; L.b[p.line] = p.b; }
+                L.ql[p.line] = p.ql; L.tl[p.line] = p.tl;
+            });
+    const u32 n = (u32)n_ok;
+    if (n == 0) return 0;
+    *R = take_records<READER>(c, dl, L, n);
+    *nt = intern_names(c, dl.text, hp.text, *R, n, tc, dl.d_cnt);
+    return n;
+}
+
+// Genome of every sequence under `prefix`, as its rank among the sorted distinct genomes (*genomes): equal ranks <=> same
+// genome, and min / max of two ranks orders a pair as the reference's (String, String) key does (main.rs:455-459).
+static std::vector<u32> genome_ranks(const std::vector<std::string> &names, std::string (*prefix)(const std::string &),
+                                     std::vector<std::string> *genomes) {
+    std::vector<std::string> pre(names.size());
+    for (size_t s = 0; s < names.size(); s++) pre[s] = prefix(names[s]);
+    *genomes = pre;
+    std::sort(genomes->begin(), genomes->end());
+    genomes->erase(std::unique(genomes->begin(), genomes->end()), genomes->end());
+    std::vector<u32> rank(names.size());
+    for (size_t s = 0; s < names.size(); s++) rank[s] = (u32)(std::lower_bound(genomes->begin(), genomes->end(), pre[s]) - genomes->begin());
+    return rank;
+}
+
 // method: SWG_ANI_ALL or SWG_ANI_NPERCENTILE (Orthogonal = the 1:1 filter first, then ALL; done by the caller).
 static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double percentile, int sort) {
     cudaStream_t st = c->stream;
@@ -167,99 +193,18 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
     AniResult res;
     const DevLines dl = load_lines(c, hp);
     if (hp.text_len == 0) return res;
-    const char *text = dl.text;
-    const u32 n_lines = dl.n_lines;
     u32 *bsum = dl.bsum, *d_cnt = dl.d_cnt;
-    auto take_cols = [&](u32 n) {
-        AniCols L;
-        memset(&L, 0, sizeof L);
-        L.names.off = A.take<u64>(n);
-        L.names.qh = A.take<u64>(n); L.names.th = A.take<u64>(n);
-        L.names.qlen = A.take<u32>(n); L.names.trel = A.take<u32>(n); L.names.tlen = A.take<u32>(n);
-        L.m = A.take<double>(n); L.b = A.take<double>(n);
-        L.ql = A.take<u64>(n); L.tl = A.take<u64>(n);
-        L.kind = A.take<u8>(n);
-        return L;
-    };
-    AniCols L = take_cols(n_lines);
-    u32 *fix_list = A.take<u32>(n_lines);
-    u64 *ac = A.take<u64>(AC_COUNT);
     u64 *tc = A.take<u64>(TC_COUNT);
-    u64 h_ac[AC_COUNT];
-    auto read_ac = [&]() {
-        SWG_CUDA(cudaMemcpyAsync(h_ac, ac, sizeof(u64) * AC_COUNT, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaStreamSynchronize(st));
-    };
-    SWG_CUDA(cudaMemsetAsync(ac, 0, sizeof(u64) * AC_COUNT, st));
+    u64 h_tc[TC_COUNT];
     SWG_CUDA(cudaMemsetAsync(tc, 0, sizeof(u64) * TC_COUNT, st));
-    k_ani_parse<0><<<cdiv(n_lines, 256), 256, 0, st>>>(text, dl.line_start, n_lines, L, fix_list, ac);
-    lc.n++;
-    read_ac();
-    if (h_ac[AC_MAXLEN] > ((u64)256 << 20)) throw FrontEndFallback{"a line longer than 256 MiB"};
-    u64 n_ok = h_ac[AC_OK];
-    if (h_ac[AC_NFIX]) { // lines outside the plain number grammar: the host's line reader decides
-        const u32 nfix = (u32)h_ac[AC_NFIX];
-        std::vector<u32> lines(nfix);
-        std::vector<u64> offs(nfix + 1);
-        u64 *d_off = A.take<u64>(2 * (size_t)nfix);
-        const u64 *ls = dl.line_start;
-        launch_for<t_ani_fixgather>(nfix, st, lc, [=] __device__(u32 i) { const u32 l = fix_list[i]; d_off[2 * i] = ls[l]; d_off[2 * i + 1] = ls[l + 1] - 1; });
-        std::vector<u64> se(2 * (size_t)nfix);
-        SWG_CUDA(cudaMemcpyAsync(lines.data(), fix_list, nfix * 4, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaMemcpyAsync(se.data(), d_off, nfix * 16, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaStreamSynchronize(st));
-        std::vector<AniPatch> patches(nfix);
-        for (u32 i = 0; i < nfix; i++) {
-            size_t len = (size_t)(se[2 * i + 1] - se[2 * i]);
-            const char *line = hp.text + se[2 * i];
-            if (len > 0 && line[len - 1] == '\r') len--;
-            AniLine al;
-            const bool ok = paf_ani_line(line, len, &al);
-            patches[i] = AniPatch{lines[i], ok ? (u32)AK_OK : (u32)AK_SKIP, al.matches, al.block, al.qlen, al.tlen};
-            if (ok) n_ok++;
-        }
-        AniPatch *d_p = A.take<AniPatch>(nfix);
-        SWG_CUDA(cudaMemcpyAsync(d_p, patches.data(), sizeof(AniPatch) * nfix, cudaMemcpyHostToDevice, st));
-        launch_for<t_ani_patch>(nfix, st, lc, [=] __device__(u32 i) {
-            const AniPatch p = d_p[i];
-            L.kind[p.line] = (u8)p.kind;
-            L.m[p.line] = p.m; L.b[p.line] = p.b; L.ql[p.line] = p.ql; L.tl[p.line] = p.tl;
-        });
-        SWG_CUDA(cudaStreamSynchronize(st));
-    }
-    const u32 n = (u32)n_ok;
+    TokCols R;
+    NameTable nt;
+    const u32 n = ani_records<0>(c, hp, dl, tc, &R, &nt);
     if (n == 0) return res;
-    // ---- records = lines that are alignments ------------------------------------------------------------
-    AniCols R = L;
-    if (n != n_lines) {
-        R = take_cols(n);
-        const AniCols Rc = R;
-        scan_apply([=] __device__(u32 l) -> u32 { return L.kind[l] == AK_OK ? 1u : 0u; },
-                   [=] __device__(u32 l, u32 r, u32 v) {
-                       if (!v) return;
-                       Rc.names.off[r] = L.names.off[l];
-                       Rc.names.qh[r] = L.names.qh[l]; Rc.names.th[r] = L.names.th[l];
-                       Rc.names.qlen[r] = L.names.qlen[l]; Rc.names.trel[r] = L.names.trel[l]; Rc.names.tlen[r] = L.names.tlen[l];
-                       Rc.m[r] = L.m[l]; Rc.b[r] = L.b[l]; Rc.ql[r] = L.ql[l]; Rc.tl[r] = L.tl[l];
-                       Rc.kind[r] = AK_OK;
-                   },
-                   n_lines, bsum, d_cnt, st, lc);
-    }
-    NameTable nt = intern_names(c, text, hp.text, R.names, n, tc, d_cnt);
     const u32 n_seq = nt.n_seq;
-    // genome prefix of every sequence, as its rank in the lexicographic order of the distinct prefixes: equal ranks <=>
-    // same genome, and min / max of two ranks is the reference's ordered (String, String) key (main.rs:455-459)
-    std::vector<u32> seq_rank(n_seq);
-    u32 nP = 0;
-    {
-        std::vector<std::string> pre(n_seq);
-        for (u32 s = 0; s < n_seq; s++) pre[s] = paf_prefix_P(nt.names[s]);
-        std::vector<std::string> uniq = pre;
-        std::sort(uniq.begin(), uniq.end());
-        uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
-        nP = (u32)uniq.size();
-        for (u32 s = 0; s < n_seq; s++) seq_rank[s] = (u32)(std::lower_bound(uniq.begin(), uniq.end(), pre[s]) - uniq.begin());
-    }
+    std::vector<std::string> genomes;
+    const std::vector<u32> seq_rank = genome_ranks(nt.names, paf_prefix_P, &genomes);
+    const u32 nP = (u32)genomes.size();
     u32 *d_rank = A.take<u32>(n_seq);
     SWG_CUDA(cudaMemcpyAsync(d_rank, seq_rank.data(), (size_t)n_seq * 4, cudaMemcpyHostToDevice, st));
     // ---- inter-genome alignments, pair keys, sort keys -------------------------------------------------------
@@ -269,7 +214,6 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
     const u32 *qid = nt.qid, *tid = nt.tid;
     const u64 nP64 = nP;
     const bool npct = method == SWG_ANI_NPERCENTILE;
-    SWG_CUDA(cudaMemsetAsync(ac, 0, sizeof(u64) * AC_COUNT, st));
     {
         u64 *sk = skey;
         u32 *sv = sval;
@@ -294,17 +238,17 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
             const u32 full = __activemask();
             const u32 c_inter = __popc(__ballot_sync(full, inter)), c_nan = __popc(__ballot_sync(full, isnan_)), c_non = __popc(__ballot_sync(full, nonint));
             if ((threadIdx.x & 31) == (u32)(__ffs(full) - 1)) {
-                if (c_inter) atomicAdd((unsigned long long *)&ac[AC_INTER], (unsigned long long)c_inter);
-                if (c_nan) atomicAdd((unsigned long long *)&ac[AC_NAN], (unsigned long long)c_nan);
-                if (c_non) atomicAdd((unsigned long long *)&ac[AC_NONINT], (unsigned long long)c_non);
+                if (c_inter) atomicAdd((unsigned long long *)&tc[TC_INTER], (unsigned long long)c_inter);
+                if (c_nan) atomicAdd((unsigned long long *)&tc[TC_NAN], (unsigned long long)c_nan);
+                if (c_non) atomicAdd((unsigned long long *)&tc[TC_NONINT], (unsigned long long)c_non);
             }
         });
     }
-    read_ac();
-    const u32 n_inter = (u32)h_ac[AC_INTER];
+    tok_read(c, tc, h_tc);
+    const u32 n_inter = (u32)h_tc[TC_INTER];
     res.n_alignments = n_inter;
     if (n_inter == 0) return res; // main.rs:468-471 / :606-609
-    if (h_ac[AC_NAN]) throw NanError{};
+    if (h_tc[TC_NAN]) throw NanError{};
     // order[k] = record of the k-th alignment in the reference's accumulation order; the first `take` are used
     u32 take = n_inter;
     const u32 *order = nullptr; // nullptr: record order
@@ -337,7 +281,7 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
             const u32 *ord = order;
             launch_for<t_ani_gather>(n_inter, st, lc, [=] __device__(u32 k) { bsorted[k] = R.b[ord[k]]; });
         }
-        if (h_ac[AC_NONINT] == 0) {
+        if (h_tc[TC_NONINT] == 0) {
             const u32 TILE = 1024;
             const u32 ntiles = cdiv(n_inter, TILE);
             u64 *tsum = A.take<u64>(ntiles);
@@ -373,7 +317,7 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
                 }
             } else take = 0; // fall through to the sequential walk
         }
-        if (h_ac[AC_NONINT] != 0 || take == 0) { // non-integer block lengths: the rounding of the running sum is order dependent
+        if (h_tc[TC_NONINT] != 0 || take == 0) { // non-integer block lengths: the rounding of the running sum is order dependent
             std::vector<double> hb(n_inter);
             SWG_CUDA(cudaMemcpyAsync(hb.data(), bsorted, (size_t)n_inter * 8, cudaMemcpyDeviceToHost, st));
             SWG_CUDA(cudaStreamSynchronize(st));
@@ -451,97 +395,18 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
     dp.text = dl.text;
     dp.text_len = hp.text_len;
     if (hp.text_len == 0) { write_device(c, dp, nullptr, nullptr, out_path); return res; }
-    const char *text = dl.text;
-    const u32 n_lines = dl.n_lines;
     u32 *bsum = dl.bsum, *d_cnt = dl.d_cnt;
-    auto take_cols = [&](u32 n) {
-        AniCols L;
-        memset(&L, 0, sizeof L);
-        L.names.off = A.take<u64>(n); L.names.len = A.take<u32>(n);
-        L.names.qh = A.take<u64>(n); L.names.th = A.take<u64>(n);
-        L.names.qlen = A.take<u32>(n); L.names.trel = A.take<u32>(n); L.names.tlen = A.take<u32>(n);
-        L.ql = A.take<u64>(n); L.tl = A.take<u64>(n); // matches, block length
-        L.kind = A.take<u8>(n);
-        return L;
-    };
-    AniCols L = take_cols(n_lines);
-    u32 *fix_list = A.take<u32>(n_lines);
-    u64 *ac = A.take<u64>(AC_COUNT);
     u64 *tc = A.take<u64>(TC_COUNT);
-    u64 h_ac[AC_COUNT];
-    auto read_ac = [&]() {
-        SWG_CUDA(cudaMemcpyAsync(h_ac, ac, sizeof(u64) * AC_COUNT, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaStreamSynchronize(st));
-    };
-    SWG_CUDA(cudaMemsetAsync(ac, 0, sizeof(u64) * AC_COUNT, st));
+    u64 h_tc[TC_COUNT];
     SWG_CUDA(cudaMemsetAsync(tc, 0, sizeof(u64) * TC_COUNT, st));
-    k_ani_parse<1><<<cdiv(n_lines, 256), 256, 0, st>>>(text, dl.line_start, n_lines, L, fix_list, ac);
-    lc.n++;
-    read_ac();
-    u64 n_ok = h_ac[AC_OK];
-    if (h_ac[AC_MAXLEN] > ((u64)256 << 20)) throw FrontEndFallback{"a line longer than 256 MiB"};
-    c->tok_maxlen = (u32)h_ac[AC_MAXLEN];
-    if (h_ac[AC_NFIX]) { // integer columns with more than 19 digits: the host's line reader decides
-        const u32 nfix = (u32)h_ac[AC_NFIX];
-        std::vector<u32> lines(nfix);
-        u64 *d_off = A.take<u64>(2 * (size_t)nfix);
-        const u64 *ls = dl.line_start;
-        launch_for<t_ani_fixgather>(nfix, st, lc, [=] __device__(u32 i) { const u32 l = fix_list[i]; d_off[2 * i] = ls[l]; d_off[2 * i + 1] = ls[l + 1] - 1; });
-        std::vector<u64> se(2 * (size_t)nfix);
-        SWG_CUDA(cudaMemcpyAsync(lines.data(), fix_list, nfix * 4, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaMemcpyAsync(se.data(), d_off, nfix * 16, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaStreamSynchronize(st));
-        std::vector<AniPatch> patches(nfix);
-        for (u32 i = 0; i < nfix; i++) {
-            size_t len = (size_t)(se[2 * i + 1] - se[2 * i]);
-            const char *line = hp.text + se[2 * i];
-            if (len > 0 && line[len - 1] == '\r') len--;
-            AniLine al;
-            u64 m = 0, b = 1;
-            const bool ok = paf_tree_line(line, len, &al, &m, &b);
-            patches[i] = AniPatch{lines[i], ok ? (u32)AK_OK : (u32)AK_SKIP, 0.0, 0.0, m, b};
-            if (ok) n_ok++;
-        }
-        AniPatch *d_p = A.take<AniPatch>(nfix);
-        SWG_CUDA(cudaMemcpyAsync(d_p, patches.data(), sizeof(AniPatch) * nfix, cudaMemcpyHostToDevice, st));
-        launch_for<t_ani_patch>(nfix, st, lc, [=] __device__(u32 i) {
-            const AniPatch p = d_p[i];
-            L.kind[p.line] = (u8)p.kind;
-            L.ql[p.line] = p.ql; L.tl[p.line] = p.tl;
-        });
-        SWG_CUDA(cudaStreamSynchronize(st));
-    }
-    const u32 n = (u32)n_ok;
+    TokCols R;
+    NameTable nt;
+    const u32 n = ani_records<1>(c, hp, dl, tc, &R, &nt);
     if (n == 0) { write_device(c, dp, nullptr, nullptr, out_path); return res; }
-    AniCols R = L;
-    if (n != n_lines) {
-        R = take_cols(n);
-        const AniCols Rc = R;
-        scan_apply([=] __device__(u32 l) -> u32 { return L.kind[l] == AK_OK ? 1u : 0u; },
-                   [=] __device__(u32 l, u32 r, u32 v) {
-                       if (!v) return;
-                       Rc.names.off[r] = L.names.off[l]; Rc.names.len[r] = L.names.len[l];
-                       Rc.names.qh[r] = L.names.qh[l]; Rc.names.th[r] = L.names.th[l];
-                       Rc.names.qlen[r] = L.names.qlen[l]; Rc.names.trel[r] = L.names.trel[l]; Rc.names.tlen[r] = L.names.tlen[l];
-                       Rc.ql[r] = L.ql[l]; Rc.tl[r] = L.tl[l];
-                       Rc.kind[r] = AK_OK;
-                   },
-                   n_lines, bsum, d_cnt, st, lc);
-    }
-    NameTable nt = intern_names(c, text, hp.text, R.names, n, tc, d_cnt);
     const u32 n_seq = nt.n_seq;
-    // genome of every sequence under extract_genome_prefix (tree_filter.rs:15-25, the P2 rule), as its rank among the
-    // sorted distinct genomes
-    std::vector<u32> seq_rank(n_seq);
+    // genome of every sequence under extract_genome_prefix (tree_filter.rs:15-25, the P2 rule)
     std::vector<std::string> genomes;
-    {
-        std::vector<std::string> pre(n_seq);
-        for (u32 s = 0; s < n_seq; s++) pre[s] = paf_prefix_P2(nt.names[s]);
-        genomes = pre;
-        std::sort(genomes.begin(), genomes.end());
-        genomes.erase(std::unique(genomes.begin(), genomes.end()), genomes.end());
-        for (u32 s = 0; s < n_seq; s++) seq_rank[s] = (u32)(std::lower_bound(genomes.begin(), genomes.end(), pre[s]) - genomes.begin());
-    }
+    const std::vector<u32> seq_rank = genome_ranks(nt.names, paf_prefix_P2, &genomes);
     const u64 nG = genomes.size();
     u32 *d_rank = A.take<u32>(n_seq);
     SWG_CUDA(cudaMemcpyAsync(d_rank, seq_rank.data(), (size_t)n_seq * 4, cudaMemcpyHostToDevice, st));
@@ -551,7 +416,6 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
     u64 *pk = A.take<u64>(n), *pk2 = A.take<u64>(n);
     u32 *pv = A.take<u32>(n), *pv2 = A.take<u32>(n);
     const u32 *qid = nt.qid, *tid = nt.tid;
-    SWG_CUDA(cudaMemsetAsync(ac, 0, sizeof(u64) * AC_COUNT, st));
     {
         u64 *k = pk;
         u32 *v = pv;
@@ -562,18 +426,18 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
             v[r] = r;
             const u32 am = __activemask();
             const u32 cnt = __popc(__ballot_sync(am, inter));
-            if (cnt && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd((unsigned long long *)&ac[AC_INTER], (unsigned long long)cnt);
+            if (cnt && (threadIdx.x & 31) == (u32)(__ffs(am) - 1)) atomicAdd((unsigned long long *)&tc[TC_INTER], (unsigned long long)cnt);
         });
     }
     sort_pairs(c, pk, pk2, pv, pv2, n, pbits);
-    read_ac();
-    const u32 n_inter = (u32)h_ac[AC_INTER];
+    tok_read(c, tc, h_tc);
+    const u32 n_inter = (u32)h_tc[TC_INTER];
     u8 *status = A.take<u8>(n);
     u32 *chain = A.take<u32>(n);
     SWG_CUDA(cudaMemsetAsync(status, 0, n, st));
     SWG_CUDA(cudaMemsetAsync(chain, 0, sizeof(u32) * (size_t)n, st));
     dp.n = n;
-    dp.rec = R.names;
+    dp.rec = R;
     if (n_inter == 0) { write_device(c, dp, status, chain, out_path); return res; }
     u32 *gid = A.take<u32>(n_inter), *seg_start = A.take<u32>(n_inter);
     {

@@ -2141,6 +2141,36 @@ static void do_sweep_core(void *p) {
 #include "ani_device.cuh"
 #include "batch.cuh"
 
+namespace swg {
+
+// Opens the text of a PAF input for the entry point `who`.  On failure the error is set and the code returned:
+// SWG_ERR_RANGE when the file is readable (so its contents are at fault), SWG_ERR_IO otherwise.
+static int open_paf_text(swg_ctx *c, const char *who, const char *path, swg_paf *hp) {
+    std::string err;
+    if (paf_open_text(path, hp, &err)) return SWG_OK;
+    set_err(c, std::string(who) + ": " + err);
+    return access(path, R_OK) == 0 ? SWG_ERR_RANGE : SWG_ERR_IO;
+}
+
+// The device readers without a host front end (swg_ani_stats, swg_tree_filter_paf): run() catches their declines, rc()
+// turns them into the return code.
+struct Declines {
+    bool fallback = false, nan = false;
+    template <class F> void run(F &&f) {
+        try { f(); } catch (const FrontEndFallback &) { fallback = true; } catch (const NanError &) { nan = true; }
+    }
+    int rc(swg_ctx *c, const char *who, const char *nan_what) const {
+        if (nan) { set_err(c, std::string(who) + ": " + nan_what + " (the reference panics here)"); return SWG_ERR_RANGE; }
+        if (fallback) {
+            set_err(c, std::string(who) + ": input not supported by the device front end (> 64 GiB, or a sequence-name hash collision)");
+            return SWG_ERR_UNSUPPORTED;
+        }
+        return SWG_OK;
+    }
+};
+
+} // namespace swg
+
 // =================================================================================================
 // C ABI
 // =================================================================================================
@@ -2757,13 +2787,7 @@ int swg_filter_paf(swg_ctx *c, const swg_config *cfg, const char *in_path, const
     c->knobs = read_knobs();
     if (c->knobs.paf_host_frontend) return swg_filter_paf_host(c, cfg, in_path, out_path, stats);
     swg_paf hp;
-    {
-        std::string err;
-        if (!paf_open_text(in_path, &hp, &err)) {
-            set_err(c, "swg_filter_paf: " + err);
-            return access(in_path, R_OK) == 0 ? SWG_ERR_RANGE : SWG_ERR_IO;
-        }
-    }
+    if (const int orc = open_paf_text(c, "swg_filter_paf", in_path, &hp)) return orc;
     struct Args { swg_ctx *c; const swg_config *cfg; const swg_paf *hp; const char *out; swg_stats *stats; bool fallback; } a{c, cfg, &hp, out_path, stats, false};
     const int rc = guarded(c, "swg_filter_paf", [](void *q) {
         Args *a = (Args *)q;
@@ -2825,26 +2849,19 @@ int swg_ani_stats(swg_ctx *c, const char *paf_path, int method, double percentil
         method = SWG_ANI_ALL;
     }
     swg_paf hp;
-    {
-        std::string err;
-        if (!paf_open_text(input.c_str(), &hp, &err)) {
-            set_err(c, "swg_ani_stats: " + err);
-            if (!tmp.empty()) unlink(tmp.c_str());
-            return access(input.c_str(), R_OK) == 0 ? SWG_ERR_RANGE : SWG_ERR_IO;
-        }
+    if (const int orc = open_paf_text(c, "swg_ani_stats", input.c_str(), &hp)) {
+        if (!tmp.empty()) unlink(tmp.c_str());
+        return orc;
     }
-    struct Args { swg_ctx *c; const swg_paf *hp; int method; double pct; int sort; AniResult res; bool fallback, nan; } a{c, &hp, method, percentile, sort, {}, false, false};
+    struct Args { swg_ctx *c; const swg_paf *hp; int method; double pct; int sort; AniResult res; Declines d; } a{c, &hp, method, percentile, sort, {}, {}};
     int rc = guarded(c, "swg_ani_stats", [](void *q) {
         Args *a = (Args *)q;
         SWG_CUDA(cudaSetDevice(a->c->device));
-        try { a->res = ani_device(a->c, *a->hp, a->method, a->pct, a->sort); }
-        catch (const FrontEndFallback &) { a->fallback = true; }
-        catch (const NanError &) { a->nan = true; }
+        a->d.run([&] { a->res = ani_device(a->c, *a->hp, a->method, a->pct, a->sort); });
     }, &a);
     if (!tmp.empty()) unlink(tmp.c_str());
+    if (rc == SWG_OK) rc = a.d.rc(c, "swg_ani_stats", "NaN among the sort keys or pair ANI values");
     if (rc != SWG_OK) return rc;
-    if (a.nan) { set_err(c, "swg_ani_stats: NaN among the sort keys or pair ANI values (the reference panics here)"); return SWG_ERR_RANGE; }
-    if (a.fallback) { set_err(c, "swg_ani_stats: input not supported by the device front end (> 64 GiB, or a sequence-name hash collision)"); return SWG_ERR_UNSUPPORTED; }
     *ani50 = a.res.ani50;
     if (n_pairs) *n_pairs = a.res.n_pairs;
     return SWG_OK;
@@ -2855,24 +2872,15 @@ int swg_tree_filter_paf(swg_ctx *c, const char *in_path, const char *out_path, u
                         double random_fraction, uint64_t *n_kept, uint64_t *n_pairs_selected) {
     if (!c || !in_path || !out_path) return SWG_ERR_ARG;
     swg_paf hp;
-    {
-        std::string err;
-        if (!paf_open_text(in_path, &hp, &err)) {
-            set_err(c, "swg_tree_filter_paf: " + err);
-            return access(in_path, R_OK) == 0 ? SWG_ERR_RANGE : SWG_ERR_IO;
-        }
-    }
-    struct Args { swg_ctx *c; const swg_paf *hp; const char *out; u64 kn, kf; double rf; TreeResult res; bool fallback, nan; } a{c, &hp, out_path, k_nearest, k_farthest, random_fraction, {}, false, false};
-    const int rc = guarded(c, "swg_tree_filter_paf", [](void *q) {
+    if (const int orc = open_paf_text(c, "swg_tree_filter_paf", in_path, &hp)) return orc;
+    struct Args { swg_ctx *c; const swg_paf *hp; const char *out; u64 kn, kf; double rf; TreeResult res; Declines d; } a{c, &hp, out_path, k_nearest, k_farthest, random_fraction, {}, {}};
+    int rc = guarded(c, "swg_tree_filter_paf", [](void *q) {
         Args *a = (Args *)q;
         SWG_CUDA(cudaSetDevice(a->c->device));
-        try { a->res = tree_filter_device(a->c, *a->hp, a->out, a->kn, a->kf, a->rf); }
-        catch (const FrontEndFallback &) { a->fallback = true; }
-        catch (const NanError &) { a->nan = true; }
+        a->d.run([&] { a->res = tree_filter_device(a->c, *a->hp, a->out, a->kn, a->kf, a->rf); });
     }, &a);
+    if (rc == SWG_OK) rc = a.d.rc(c, "swg_tree_filter_paf", "NaN identity");
     if (rc != SWG_OK) return rc;
-    if (a.nan) { set_err(c, "swg_tree_filter_paf: NaN identity (the reference panics here)"); return SWG_ERR_RANGE; }
-    if (a.fallback) { set_err(c, "swg_tree_filter_paf: input not supported by the device front end (> 64 GiB, or a sequence-name hash collision)"); return SWG_ERR_UNSUPPORTED; }
     if (n_kept) *n_kept = a.res.n_kept;
     if (n_pairs_selected) *n_pairs_selected = a.res.n_selected;
     return SWG_OK;

@@ -17,25 +17,32 @@
 //   5. output: per-record output length -> scan -> one warp per kept record copies the line and writes the tags
 // Anything outside the plain grammar (numbers with more than 19 digits, inf/nan or long decimal dv values) is not
 // guessed on the device: the line is listed and the host's reference-exact line parser (paf_parse_line) patches it.
+//
+// The three PAF readers on the device (this filter front end, and the ANI and tree readers of ani_device.cuh) share
+// what is not their own policy: the line grammar (line_len_raw / strip_cr, name_field, u64_field, count_records /
+// raise_maxlen), the counter block (TC_*) and line kinds (TK_*), the column list (TokCols, for_each_col) with
+// take_cols / take_records, and the host patch step for the listed lines (patch_lines).  Each reader keeps its own
+// columns and tags.
 #pragma once
 
 #include <atomic>
 #include <thread>
+#include <type_traits>
 
 #include <fcntl.h>
 #include <unistd.h>
 
 namespace swg {
 
-struct t_tok_fixgather; struct t_tok_patch; struct t_name_assign; struct t_out_bounds;
+struct t_fixgather; struct t_patch; struct t_name_assign; struct t_out_bounds;
 
 __constant__ double c_pow10[23] = {1e0,  1e1,  1e2,  1e3,  1e4,  1e5,  1e6,  1e7,  1e8,  1e9,  1e10, 1e11,
                                    1e12, 1e13, 1e14, 1e15, 1e16, 1e17, 1e18, 1e19, 1e20, 1e21, 1e22};
 
 enum : u8 { TK_SKIP = 0, TK_OK = 1, TK_ERR_RANGE = 2, TK_ERR_ORDER = 3, TK_FIX = 4, TK_LONG = 5 };
-enum { TC_OK = 0, TC_ERRLINE, TC_NFIX, TC_NLONG, TC_MAXLEN, TC_COLLISION, TC_DISTINCT, TC_TABLE_FULL, TC_COUNT };
+enum { TC_OK = 0, TC_ERRLINE, TC_NFIX, TC_NLONG, TC_MAXLEN, TC_COLLISION, TC_DISTINCT, TC_TABLE_FULL, TC_INTER, TC_NAN, TC_NONINT, TC_COUNT };
 
-struct TokCols { // per line, then per record
+struct TokCols { // per line, then per record; a reader has only the columns it uses (take_cols)
     u64 *off;
     u32 *len;
     u32 *qs, *qe, *ts, *te, *blen, *matches;
@@ -43,7 +50,23 @@ struct TokCols { // per line, then per record
     u8 *strand, *kind;
     u64 *qh, *th;
     u32 *qlen, *trel, *tlen;
+    double *m, *b; // ANI: final matches, block length
+    u64 *ql, *tl;  // ANI: sequence lengths (columns 2 and 7); tree: matches, block length (columns 10 and 11)
 };
+
+// The readers, as a mask of which of them use a column.
+enum : u32 { RD_FILTER = 1, RD_ANI = 2, RD_TREE = 4 };
+
+// Every column of TokCols once, with the readers that use it: f(readers, c.column...) for the same column of each c.
+#pragma nv_exec_check_disable
+template <class F, class... C> __host__ __device__ __forceinline__ void for_each_col(F &&f, C &...c) {
+    constexpr u32 ALL = RD_FILTER | RD_ANI | RD_TREE;
+    f(ALL, c.off...); f(RD_FILTER | RD_TREE, c.len...);
+    f(RD_FILTER, c.qs...); f(RD_FILTER, c.qe...); f(RD_FILTER, c.ts...); f(RD_FILTER, c.te...);
+    f(RD_FILTER, c.blen...); f(RD_FILTER, c.matches...); f(RD_FILTER, c.identity...); f(RD_FILTER, c.strand...);
+    f(ALL, c.kind...); f(ALL, c.qh...); f(ALL, c.th...); f(ALL, c.qlen...); f(ALL, c.trel...); f(ALL, c.tlen...);
+    f(RD_ANI, c.m...); f(RD_ANI, c.b...); f(RD_ANI | RD_TREE, c.ql...); f(RD_ANI | RD_TREE, c.tl...);
+}
 
 struct TokHead {
     u64 qs, qe, ts, te, mt, bl;
@@ -58,6 +81,59 @@ __device__ __forceinline__ u64 name_hash_finish(u64 h, u32 len) {
     return h == NONE64 ? h - 1 : h;
 }
 
+// ---- the line grammar of every reader ------------------------------------------------------------
+// Length of line l without its '\n', clamped: a line of 4 GiB still trips the host's longest-line check (front-end fallback).
+__device__ __forceinline__ u32 line_len_raw(const u64 *__restrict__ line_start, u32 l) {
+    return (u32)min(line_start[l + 1] - 1 - line_start[l], (u64)0xFFFFFFF0u);
+}
+__device__ __forceinline__ u32 strip_cr(const char *line, u32 len) { // BufRead::lines strips "\r\n"
+    if (len > 0 && line[len - 1] == '\r') len--;
+    return len;
+}
+
+// The name field that starts at a: FNV-1a over its bytes, finished with its length.  b: advanced to the end of the field.
+__device__ __forceinline__ u64 name_field(const char *line, u32 a, u32 &b, u32 len) {
+    u64 hh = 0xcbf29ce484222325ull;
+    while (b < len) {
+        const u8 ch = (u8)line[b];
+        if (ch == '\t') break;
+        hh = (hh ^ ch) * 0x100000001B3ull;
+        b++;
+    }
+    return name_hash_finish(hh, b - a);
+}
+
+// str::parse::<u64>().unwrap_or(dflt) of the field that starts at a (paf_filter.rs:308-317).  More than 19 digits may or
+// may not overflow u64: fix is set and the host decides.  b: advanced to the end of the field.
+__device__ __forceinline__ u64 u64_field(const char *line, u32 a, u32 &b, u32 len, u64 dflt, bool &fix) {
+    u64 v = 0;
+    u32 nd = 0;
+    bool bad = false;
+    while (b < len) {
+        const u8 ch = (u8)line[b];
+        if (ch == '\t') break;
+        if (!(b == a && ch == '+')) {
+            const u32 d = (u32)ch - '0';
+            if (d > 9) bad = true;
+            else { if (nd < 19) v = v * 10 + d; nd++; }
+        }
+        b++;
+    }
+    if (bad || nd == 0) return dflt;
+    if (nd > 19) fix = true;
+    return v;
+}
+
+// End of a per-line parse kernel's block: the lines that became records (ok) are counted, the longest line raised.
+__device__ __forceinline__ void count_records(bool ok, u64 *__restrict__ tc) {
+    const u32 nok = __syncthreads_count(ok);
+    if (threadIdx.x == 0 && nok) atomicAdd((unsigned long long *)&tc[TC_OK], (unsigned long long)nok);
+}
+__device__ __forceinline__ void raise_maxlen(u32 len, u64 *__restrict__ tc) {
+    const u32 mx = __reduce_max_sync(0xFFFFFFFFu, len);
+    if (lane_id() == 0 && mx > (u32)tc[TC_MAXLEN]) atomicMax((unsigned long long *)&tc[TC_MAXLEN], (unsigned long long)mx);
+}
+
 // First 11 fields of a line.  false: fewer than 11 fields (the line is skipped, paf_filter.rs:302-304).
 __device__ __forceinline__ bool tok_parse_head(const char *__restrict__ line, u32 len, TokHead &h) {
     u32 a = 0;
@@ -68,34 +144,11 @@ __device__ __forceinline__ bool tok_parse_head(const char *__restrict__ line, u3
     for (int nf = 0; nf < 11; nf++) {
         u32 b = a;
         if (nf == 0 || nf == 5) {
-            u64 hh = 0xcbf29ce484222325ull;
-            while (b < len) {
-                const u8 ch = (u8)line[b];
-                if (ch == '\t') break;
-                hh = (hh ^ ch) * 0x100000001B3ull;
-                b++;
-            }
-            hh = name_hash_finish(hh, b - a);
+            const u64 hh = name_field(line, a, b, len);
             if (nf == 0) { h.qh = hh; h.qlen = b - a; }
             else { h.th = hh; h.trel = a; h.tlen = b - a; }
         } else if (nf == 2 || nf == 3 || nf >= 7) {
-            // str::parse::<u64>().unwrap_or(default), paf_filter.rs:308-317
-            u64 v = 0;
-            u32 nd = 0;
-            bool bad = false;
-            while (b < len) {
-                const u8 ch = (u8)line[b];
-                if (ch == '\t') break;
-                if (!(b == a && ch == '+')) {
-                    const u32 d = (u32)ch - '0';
-                    if (d > 9) bad = true;
-                    else { if (nd < 19) v = v * 10 + d; nd++; }
-                }
-                b++;
-            }
-            const u64 dflt = nf == 10 ? 1 : 0;
-            if (bad || nd == 0) v = dflt;
-            else if (nd > 19) h.fix = true; // may or may not overflow u64: the host decides
+            const u64 v = u64_field(line, a, b, len, nf == 10 ? 1 : 0, h.fix);
             const int slot = nf == 2 ? 0 : nf == 3 ? 1 : nf - 5; // 7,8,9,10 -> 2,3,4,5
             num[slot] = v;
         } else {
@@ -221,10 +274,8 @@ __global__ void __launch_bounds__(256) k_tok_parse(const char *__restrict__ text
     u32 len = 0;
     if (l < n_lines) {
         const u64 s = line_start[l];
-        const u64 e = line_start[l + 1] - 1;
-        len = (u32)min(e - s, (u64)0xFFFFFFF0u); // a line of 4 GiB trips the host's longest-line check (front-end fallback)
         const char *line = text + s;
-        if (len > 0 && line[len - 1] == '\r') len--; // BufRead::lines strips "\r\n"
+        len = strip_cr(line, line_len_raw(line_start, l));
         L.off[l] = s;
         L.len[l] = len;
         if (len > long_thresh) {
@@ -288,10 +339,8 @@ __global__ void __launch_bounds__(256) k_tok_parse(const char *__restrict__ text
             }
         }
     }
-    const u32 nok = __syncthreads_count(ok);
-    const u32 mx = __reduce_max_sync(0xFFFFFFFFu, len);
-    if (threadIdx.x == 0 && nok) atomicAdd((unsigned long long *)&tc[TC_OK], (unsigned long long)nok);
-    if (lane_id() == 0 && mx > (u32)tc[TC_MAXLEN]) atomicMax((unsigned long long *)&tc[TC_MAXLEN], (unsigned long long)mx);
+    count_records(ok, tc);
+    raise_maxlen(len, tc);
 }
 
 // One warp per long line: lane 0 reads the head, the warp walks the tags 32 bytes at a time.
@@ -607,6 +656,61 @@ static DevLines load_lines(swg_ctx *c, const swg_paf &hp) {
     return dl;
 }
 
+// Columns for n lines or records: the ones READER uses (for_each_col), the others nullptr.
+template <u32 READER> static TokCols take_cols(Arena &A, u32 n) {
+    TokCols C{};
+    for_each_col([&](u32 used, auto *&col) { col = (used & READER) ? A.take<std::remove_reference_t<decltype(*col)>>(n) : nullptr; }, C);
+    return C;
+}
+
+// Records = the lines of kind TK_OK, in line order: L itself when every line is one, else the columns of L compacted into
+// new ones.  rank (when not nullptr) then receives a column with the line of each record; it stays untouched otherwise.
+template <u32 READER> static TokCols take_records(swg_ctx *c, const DevLines &dl, const TokCols &L, u32 n, u32 **rank = nullptr) {
+    if (n == dl.n_lines) return L;
+    const TokCols R = take_cols<READER>(c->io, std::max<u32>(n, 1));
+    u32 *rk = rank ? (*rank = c->io.take<u32>(std::max<u32>(n, 1))) : nullptr;
+    scan_apply([=] __device__(u32 l) -> u32 { return L.kind[l] == TK_OK ? 1u : 0u; },
+               [=] __device__(u32 l, u32 r, u32 v) {
+                   if (!v) return;
+                   if (rk) rk[r] = l;
+                   for_each_col([&](u32 used, auto *dst, auto *src) { if (used & READER) dst[r] = src[l]; }, R, L);
+               },
+               dl.n_lines, dl.bsum, dl.d_cnt, c->stream, c->lc);
+    return R;
+}
+
+// The lines the device does not decide (fix_list, nfix entries) go to the host reader: reparse(line, len, p) fills the
+// patch record p of one line (p.line is set) and says whether the line is a record; one kernel then applies every record
+// with apply(p).  The host reads the same bytes as the device: from line_start, without a final '\r'.  Returns how many
+// of the lines are records.
+template <class P, class Apply>
+static u32 patch_lines(swg_ctx *c, const swg_paf &hp, const DevLines &dl, const u32 *fix_list, u32 nfix,
+                       bool (*reparse)(const char *line, size_t len, P &p), Apply apply) {
+    cudaStream_t st = c->stream;
+    std::vector<u32> lines(nfix);
+    std::vector<u64> se(2 * (size_t)nfix);
+    u64 *d_se = c->io.take<u64>(2 * (size_t)nfix);
+    const u64 *ls = dl.line_start;
+    launch_for<t_fixgather>(nfix, st, c->lc, [=] __device__(u32 i) { const u32 l = fix_list[i]; d_se[2 * i] = ls[l]; d_se[2 * i + 1] = ls[l + 1] - 1; });
+    SWG_CUDA(cudaMemcpyAsync(lines.data(), fix_list, (size_t)nfix * 4, cudaMemcpyDeviceToHost, st));
+    SWG_CUDA(cudaMemcpyAsync(se.data(), d_se, (size_t)nfix * 16, cudaMemcpyDeviceToHost, st));
+    SWG_CUDA(cudaStreamSynchronize(st));
+    std::vector<P> patches(nfix);
+    u32 n_ok = 0;
+    for (u32 i = 0; i < nfix; i++) {
+        size_t len = (size_t)(se[2 * i + 1] - se[2 * i]);
+        const char *line = hp.text + se[2 * i];
+        if (len > 0 && line[len - 1] == '\r') len--;
+        patches[i].line = lines[i];
+        if (reparse(line, len, patches[i])) n_ok++;
+    }
+    P *d_p = c->io.take<P>(nfix);
+    SWG_CUDA(cudaMemcpyAsync(d_p, patches.data(), sizeof(P) * nfix, cudaMemcpyHostToDevice, st));
+    launch_for<t_patch>(nfix, st, c->lc, [=] __device__(u32 i) { const P p = d_p[i]; apply(p); });
+    SWG_CUDA(cudaStreamSynchronize(st)); // patches lives on this stack frame
+    return n_ok;
+}
+
 struct NameTable { // result of intern_names
     u32 *qid = nullptr, *tid = nullptr;
     u32 n_seq = 0;
@@ -693,21 +797,10 @@ static void tokenize_device(swg_ctx *c, const swg_paf &hp, DevPaf &dp) {
     const u32 n_lines = dl.n_lines;
     dp.n_lines = n_lines;
     const u64 *line_start = dl.line_start;
-    u32 *bsum = dl.bsum, *d_cnt = dl.d_cnt;
+    u32 *d_cnt = dl.d_cnt;
 
     // ---- 2./3. per-line parse --------------------------------------------------------------------
-    auto take_cols = [&](u32 n) {
-        TokCols L;
-        L.off = A.take<u64>(n); L.len = A.take<u32>(n);
-        L.qs = A.take<u32>(n); L.qe = A.take<u32>(n); L.ts = A.take<u32>(n); L.te = A.take<u32>(n);
-        L.blen = A.take<u32>(n); L.matches = A.take<u32>(n);
-        L.identity = A.take<double>(n);
-        L.strand = A.take<u8>(n); L.kind = A.take<u8>(n);
-        L.qh = A.take<u64>(n); L.th = A.take<u64>(n);
-        L.qlen = A.take<u32>(n); L.trel = A.take<u32>(n); L.tlen = A.take<u32>(n);
-        return L;
-    };
-    TokCols L = take_cols(n_lines);
+    const TokCols L = take_cols<RD_FILTER>(A, n_lines);
     u32 *long_list = A.take<u32>(n_lines), *fix_list = A.take<u32>(n_lines);
     u64 *tc = A.take<u64>(TC_COUNT);
     u64 h_tc[TC_COUNT];
@@ -722,70 +815,33 @@ static void tokenize_device(swg_ctx *c, const swg_paf &hp, DevPaf &dp) {
         lc.n++;
         tok_read(c, tc, h_tc);
     }
-    u64 n_ok = h_tc[TC_OK];
-    // ---- lines the device does not decide: the host's reference-exact parser patches them -----------
-    if (h_tc[TC_NFIX]) {
-        const u32 nfix = (u32)h_tc[TC_NFIX];
-        std::vector<u32> lines(nfix);
-        std::vector<u64> offs(nfix);
-        std::vector<u32> lens(nfix);
-        u64 *d_off = A.take<u64>(nfix);
-        u32 *d_len = A.take<u32>(nfix);
-        launch_for<t_tok_fixgather>(nfix, st, lc, [=] __device__(u32 i) { const u32 l = fix_list[i]; d_off[i] = L.off[l]; d_len[i] = L.len[l]; });
-        SWG_CUDA(cudaMemcpyAsync(lines.data(), fix_list, nfix * 4, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaMemcpyAsync(offs.data(), d_off, nfix * 8, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaMemcpyAsync(lens.data(), d_len, nfix * 4, cudaMemcpyDeviceToHost, st));
-        SWG_CUDA(cudaStreamSynchronize(st));
-        std::vector<Patch> patches(nfix);
-        for (u32 i = 0; i < nfix; i++) {
-            PafLine pl;
-            const PafLine::Kind k = paf_parse_line(hp.text + offs[i], lens[i], &pl);
-            Patch &p = patches[i];
-            p.line = lines[i];
-            p.qs = pl.qs; p.qe = pl.qe; p.ts = pl.ts; p.te = pl.te; p.blen = pl.blen; p.matches = pl.matches;
-            p.identity = pl.identity;
-            u8 kind = k == PafLine::SKIP ? TK_SKIP : TK_OK; // range / order problems ride along as impossible intervals
-            p.kind_strand = (u32)kind | ((u32)pl.strand << 8);
-            if (kind == TK_OK) n_ok++;
-        }
-        Patch *d_p = A.take<Patch>(nfix);
-        SWG_CUDA(cudaMemcpyAsync(d_p, patches.data(), sizeof(Patch) * nfix, cudaMemcpyHostToDevice, st));
-        launch_for<t_tok_patch>(nfix, st, lc, [=] __device__(u32 i) {
-            const Patch p = d_p[i];
-            const u32 l = p.line;
-            L.kind[l] = (u8)(p.kind_strand & 0xFF);
-            L.qs[l] = p.qs; L.qe[l] = p.qe; L.ts[l] = p.ts; L.te[l] = p.te; L.blen[l] = p.blen; L.matches[l] = p.matches;
-            L.identity[l] = p.identity;
-            L.strand[l] = (u8)(p.kind_strand >> 8);
-        });
-        SWG_CUDA(cudaStreamSynchronize(st)); // patches lives on this stack frame
-    }
     if (h_tc[TC_MAXLEN] > ((u64)256 << 20)) throw FrontEndFallback{"a line longer than 256 MiB"};
     c->tok_maxlen = (u32)h_tc[TC_MAXLEN];
+    u64 n_ok = h_tc[TC_OK];
+    // ---- lines the device does not decide: the host's reference-exact parser patches them -----------
+    if (h_tc[TC_NFIX])
+        n_ok += patch_lines<Patch>(
+            c, hp, dl, fix_list, (u32)h_tc[TC_NFIX],
+            [](const char *line, size_t len, Patch &p) {
+                PafLine pl;
+                const bool ok = paf_parse_line(line, len, &pl) != PafLine::SKIP; // range / order problems ride along as impossible intervals
+                p.qs = pl.qs; p.qe = pl.qe; p.ts = pl.ts; p.te = pl.te; p.blen = pl.blen; p.matches = pl.matches;
+                p.identity = pl.identity;
+                p.kind_strand = (u32)(ok ? TK_OK : TK_SKIP) | ((u32)pl.strand << 8);
+                return ok;
+            },
+            [=] __device__(const Patch &p) {
+                const u32 l = p.line;
+                L.kind[l] = (u8)(p.kind_strand & 0xFF);
+                L.qs[l] = p.qs; L.qe[l] = p.qe; L.ts[l] = p.ts; L.te[l] = p.te; L.blen[l] = p.blen; L.matches[l] = p.matches;
+                L.identity[l] = p.identity;
+                L.strand[l] = (u8)(p.kind_strand >> 8);
+            });
 
     // ---- records = lines that parsed (compaction only when some line did not) ----------------------
     const u32 n = (u32)n_ok;
     dp.n = n;
-    TokCols R = L;
-    if (n != n_lines) {
-        R = take_cols(std::max<u32>(n, 1));
-        dp.rank = A.take<u32>(std::max<u32>(n, 1));
-        u32 *rank = dp.rank;
-        const TokCols Rc = R;
-        scan_apply([=] __device__(u32 l) -> u32 { return L.kind[l] == TK_OK ? 1u : 0u; },
-                   [=] __device__(u32 l, u32 r, u32 v) {
-                       if (!v) return;
-                       rank[r] = l;
-                       Rc.off[r] = L.off[l]; Rc.len[r] = L.len[l];
-                       Rc.qs[r] = L.qs[l]; Rc.qe[r] = L.qe[l]; Rc.ts[r] = L.ts[l]; Rc.te[r] = L.te[l];
-                       Rc.blen[r] = L.blen[l]; Rc.matches[r] = L.matches[l];
-                       Rc.identity[r] = L.identity[l];
-                       Rc.strand[r] = L.strand[l]; Rc.kind[r] = TK_OK;
-                       Rc.qh[r] = L.qh[l]; Rc.th[r] = L.th[l];
-                       Rc.qlen[r] = L.qlen[l]; Rc.trel[r] = L.trel[l]; Rc.tlen[r] = L.tlen[l];
-                   },
-                   n_lines, bsum, d_cnt, st, lc);
-    }
+    const TokCols R = take_records<RD_FILTER>(c, dl, L, n, &dp.rank);
     dp.rec = R;
     if (n == 0) { SWG_CUDA(cudaStreamSynchronize(st)); return; }
 

@@ -79,24 +79,28 @@ static bool cigar_eq_count(const char *s, size_t len, uint64_t *out) {
     return true;
 }
 
+// Splits the first 11 tab-separated fields of a line into fs / fl.  Returns the offset of the tags (len + 1 when there
+// are none), or 0 when the line has fewer than 11 fields.
+static size_t split_fields(const char *line, size_t len, const char *fs[11], size_t fl[11]) {
+    size_t a = 0;
+    for (int nf = 0; nf < 11; nf++) {
+        const char *tab = (const char *)memchr(line + a, '\t', len - a);
+        const size_t b = tab ? (size_t)(tab - line) : len;
+        fs[nf] = line + a;
+        fl[nf] = b - a;
+        if (!tab) return nf == 10 ? len + 1 : 0;
+        a = b + 1;
+    }
+    return a;
+}
+
 } // namespace
 
 swg::PafLine::Kind swg::paf_parse_line(const char *line, size_t len, PafLine *out) {
     const char *fs[11];
     size_t fl[11];
-    // split the first 11 fields
-    int nf = 0;
-    size_t a = 0;
-    while (nf < 11) {
-        const char *tab = (const char *)memchr(line + a, '\t', len - a);
-        size_t b = tab ? (size_t)(tab - line) : len;
-        fs[nf] = line + a;
-        fl[nf] = b - a;
-        nf++;
-        if (!tab) { a = len + 1; break; }
-        a = b + 1;
-    }
-    if (nf < 11) return PafLine::SKIP; // fewer than 11 fields: skipped, still consumes a rank
+    size_t a = split_fields(line, len, fs, fl);
+    if (a == 0) return PafLine::SKIP; // fewer than 11 fields: skipped, still consumes a rank
     uint64_t qs, qe, ts, te, mt, bl;
     parse_u64_field(fs[2], fl[2], 0, &qs);
     parse_u64_field(fs[3], fl[3], 0, &qe);
@@ -149,18 +153,8 @@ bool swg::paf_ani_line(const char *line, size_t len, AniLine *out) {
     if (len == 0 || line[0] == '#') return false; // main.rs:414-416
     const char *fs[11];
     size_t fl[11];
-    int nf = 0;
-    size_t a = 0;
-    while (nf < 11) {
-        const char *tab = (const char *)memchr(line + a, '\t', len - a);
-        size_t b = tab ? (size_t)(tab - line) : len;
-        fs[nf] = line + a;
-        fl[nf] = b - a;
-        nf++;
-        if (!tab) { a = len + 1; break; }
-        a = b + 1;
-    }
-    if (nf < 11) return false;
+    size_t a = split_fields(line, len, fs, fl);
+    if (a == 0) return false;
     out->qname = fs[0]; out->qname_len = fl[0];
     out->tname = fs[5]; out->tname_len = fl[5];
     if (!rust_parse_u64(fs[1], fl[1], &out->qlen)) out->qlen = 0;
@@ -188,18 +182,7 @@ bool swg::paf_tree_line(const char *line, size_t len, AniLine *out, uint64_t *ma
     if (len == 0 || line[0] == '#') return false; // tree_filter.rs:221-223
     const char *fs[11];
     size_t fl[11];
-    int nf = 0;
-    size_t a = 0;
-    while (nf < 11) {
-        const char *tab = (const char *)memchr(line + a, '\t', len - a);
-        size_t b = tab ? (size_t)(tab - line) : len;
-        fs[nf] = line + a;
-        fl[nf] = b - a;
-        nf++;
-        if (!tab) break;
-        a = b + 1;
-    }
-    if (nf < 11) return false;
+    if (split_fields(line, len, fs, fl) == 0) return false;
     out->qname = fs[0]; out->qname_len = fl[0];
     out->tname = fs[5]; out->tname_len = fl[5];
     if (!rust_parse_u64(fs[9], fl[9], matches)) *matches = 0;
