@@ -1,5 +1,6 @@
-"""Helpers of the batch tests (tests/test_batch_cpu.py, tests/test_batch_gpu.py): the union of independent tables with
-disjoint ids, built in numpy, and the per-table renumbering of a result on that union.  Pure numpy."""
+"""Helpers of the batch tests (tests/test_batch_cpu.py, tests/test_batch_gpu.py, tests/test_scale_gpu.py): the union of
+independent tables with disjoint ids, built in numpy, the per-table renumbering of a result on that union, and the check of a
+batch against the single calls."""
 import os
 
 import numpy as np
@@ -90,3 +91,26 @@ def reference_paf_table():
     """The table of the committed front-end vector (tests/golden/frontend.paf), parsed by the oracle."""
     import oracle_lib
     return oracle_lib.parse_paf(os.path.join(HERE, "golden", "frontend.paf"))
+
+
+def check_batch(ctx, cfg, tables, oracle=True, what=""):
+    """ctx.filter_batch(cfg, tables) against ctx.filter of every table alone (and the oracle): status, chain numbers and the
+    per-table counts; the call's stats against the sums of the counts."""
+    import oracle_lib
+    import sweepga_b200 as swg
+    res, counts, bstats = ctx.filter_batch(cfg, tables)
+    assert len(res) == len(tables) and counts.shape == (len(tables), swg.TC_COUNT)
+    for k, t in enumerate(tables):
+        s, c, st = ctx.filter(cfg, t)
+        assert np.array_equal(res[k][0], s), f"{what} table {k}: status differs from the single call"
+        assert np.array_equal(res[k][1], c), f"{what} table {k}: chain id differs from the single call"
+        want = [st.n_stage1, int((s != 0).sum()), int((s == swg.SCAFFOLD).sum()), int((s == swg.RESCUED).sum()), st.n_chains_kept]
+        assert counts[k].tolist() == want, f"{what} table {k}: counts {counts[k].tolist()} != {want}"
+        assert st.n_chains_kept == (int(c.max()) if t.n else 0)
+        if oracle and t.n:
+            os_, oc, _ = oracle_lib.apply_filters(cfg, oracle_table(t))
+            assert np.array_equal(s, os_) and np.array_equal(c, oc), f"{what} table {k}: the single call differs from the oracle"
+    assert bstats.n_input == sum(t.n for t in tables)
+    assert bstats.n_stage1 == int(counts[:, swg.TC_STAGE1].sum())
+    assert bstats.n_chains_kept == int(counts[:, swg.TC_CHAINS_KEPT].sum())
+    return res, counts, bstats

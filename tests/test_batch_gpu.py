@@ -9,7 +9,7 @@ import oracle_lib
 import sweepga_b200 as swg
 from sweepga_b200 import synth, with_ids16
 
-from batch_util import CONFIGS, oracle_table, reference_paf_table, self_only, split, union
+from batch_util import CONFIGS, check_batch, reference_paf_table, self_only, split, union
 
 pytestmark = pytest.mark.gpu
 
@@ -38,29 +38,10 @@ def _mixed_tables():
     ]
 
 
-def _check_batch(ctx, cfg, tables, oracle=True, what=""):
-    res, counts, bstats = ctx.filter_batch(cfg, tables)
-    assert len(res) == len(tables) and counts.shape == (len(tables), swg.TC_COUNT)
-    for k, t in enumerate(tables):
-        s, c, st = ctx.filter(cfg, t)
-        assert np.array_equal(res[k][0], s), f"{what} table {k}: status differs from the single call"
-        assert np.array_equal(res[k][1], c), f"{what} table {k}: chain id differs from the single call"
-        want = [st.n_stage1, int((s != 0).sum()), int((s == swg.SCAFFOLD).sum()), int((s == swg.RESCUED).sum()), st.n_chains_kept]
-        assert counts[k].tolist() == want, f"{what} table {k}: counts {counts[k].tolist()} != {want}"
-        assert st.n_chains_kept == (int(c.max()) if t.n else 0)
-        if oracle and t.n:
-            os_, oc, _ = oracle_lib.apply_filters(cfg, oracle_table(t))
-            assert np.array_equal(s, os_) and np.array_equal(c, oc), f"{what} table {k}: the single call differs from the oracle"
-    assert bstats.n_input == sum(t.n for t in tables)
-    assert bstats.n_stage1 == int(counts[:, swg.TC_STAGE1].sum())
-    assert bstats.n_chains_kept == int(counts[:, swg.TC_CHAINS_KEPT].sum())
-    return res, counts, bstats
-
-
 @pytest.mark.parametrize("name", list(CONFIGS))
 def test_batch_equals_single_calls_and_oracle(ctx, name):
     cfg = swg.FilterConfig.from_cli(**CONFIGS[name])
-    _check_batch(ctx, cfg, _mixed_tables(), what=name)
+    check_batch(ctx, cfg, _mixed_tables(), what=name)
 
 
 def test_position_independence(ctx):
@@ -83,7 +64,7 @@ def test_batch_paths(ctx, monkeypatch, knob, name):
     """The host-log re-rank and the wide-key path, each set for the batch and for the single calls alike."""
     monkeypatch.setenv(*knob)
     cfg = swg.FilterConfig.from_cli(**CONFIGS[name])
-    _, _, st = _check_batch(ctx, cfg, _mixed_tables(), oracle=False, what=f"{knob[0]} {name}")
+    _, _, st = check_batch(ctx, cfg, _mixed_tables(), oracle=False, what=f"{knob[0]} {name}")
     if knob[0] == "SWG_EXACT_SCORES":
         assert st.exact_rerank == 1
 
@@ -96,7 +77,7 @@ def test_fixpoint_inside_a_batch(ctx, monkeypatch):
     tiny = [synth.yeast_like(150, seed=40 + k) for k in range(4)]
     tables = tiny[:2] + [pile] + tiny[2:]
     for cfg in (swg.FilterConfig(), swg.FilterConfig.from_cli(scaffold_dist="20k")):
-        _check_batch(ctx, cfg, tables, what="fixpoint")
+        check_batch(ctx, cfg, tables, what="fixpoint")
 
 
 def test_many_small_tables(ctx):
@@ -127,7 +108,7 @@ def test_errors_and_context_state(ctx):
     with pytest.raises(swg.SwgError) as e:
         ctx.filter_batch(cfg, good[:3] + [bad] + good[4:])
     assert e.value.code == swg._lib.ERR_RANGE
-    _check_batch(ctx, cfg, good, oracle=False, what="after a range error")
+    check_batch(ctx, cfg, good, oracle=False, what="after a range error")
     # score in some tables only
     scored = copy.copy(good[1])
     scored.score = oracle_lib.score_column(scored.query_start, scored.query_end, scored.identity)

@@ -1,8 +1,9 @@
 """Parity proper: the CUDA path (through the C ABI) against the CPU oracle on the same seeded inputs.
 
 Bit-exact bar: identical status byte and chain number for every record.  Sizes are chosen so that the
-oracle finishes in seconds; full-size behaviour is covered by size-independent properties
-(idempotence, determinism, shard-invariance) in test_properties_gpu.py.
+single-threaded oracle finishes in seconds.  Full-size parity (20 M and 40 M records, every mode that changes which kernels
+run, against the oracle spread over genome-pair units on all host threads) lives in test_scale_gpu.py; size-independent
+properties (idempotence, determinism, shard-invariance) are in test_properties_gpu.py.
 """
 import numpy as np
 import pytest
