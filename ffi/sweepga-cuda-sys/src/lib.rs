@@ -201,6 +201,9 @@ extern "C" {
     pub fn swg_paf_write(p: *const swg_paf, out_path: *const c_char, status: *const u8, chain_id: *const u32) -> c_int;
     pub fn swg_paf_parse_device(ctx: *mut swg_ctx, path: *const c_char) -> *mut swg_paf;
     pub fn swg_filter_paf(ctx: *mut swg_ctx, cfg: *const swg_config, in_path: *const c_char, out_path: *const c_char, stats: *mut swg_stats) -> c_int;
+    /// `PafFilter::filter_paf` over many independent PAF files in one call (`file_counts`: `n_files` rows of `SWG_TC_COUNT`, may be null).
+    pub fn swg_filter_paf_batch(ctx: *mut swg_ctx, cfg: *const swg_config, n_files: u64, in_paths: *const *const c_char,
+                                out_paths: *const *const c_char, file_counts: *mut u64, stats: *mut swg_stats) -> c_int;
     pub fn swg_filter_paf_host(ctx: *mut swg_ctx, cfg: *const swg_config, in_path: *const c_char, out_path: *const c_char, stats: *mut swg_stats) -> c_int;
     pub fn swg_filter_file(ctx: *mut swg_ctx, cfg: *const swg_config, in_path: *const c_char, out_path: *const c_char, keep_self: c_int, stats: *mut swg_stats) -> c_int;
     pub fn swg_aln_to_paf(aln_path: *const c_char, paf_path: *const c_char, threads: c_int) -> c_int;

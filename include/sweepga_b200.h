@@ -344,6 +344,26 @@ swg_paf *swg_paf_parse_device(swg_ctx *ctx, const char *path);
  * upload, ms_tokenize, ms_device = the filter, ms_write.  SWG_PAF_FRONTEND=host selects swg_filter_paf_host. */
 int swg_filter_paf(swg_ctx *ctx, const swg_config *cfg, const char *in_path, const char *out_path,
                    swg_stats *stats);
+/* PafFilter::filter_paf over many independent PAF files in one call: out_paths[k] receives byte for byte what
+ * swg_filter_paf(ctx, cfg, in_paths[k], out_paths[k], NULL) writes, chain numbers from chain_1 in every file, whatever else
+ * shares the call.  Consecutive files travel as one union through the device front end, the filter and the writer (one
+ * upload, one kernel chain, one assembled output for the group), so a loop of small files stops paying the per-call floor.
+ * Files are independent tables: a sequence name that appears in two files is two sequences, and keep_self, the genome
+ * prefix rules and chain numbering work per file.  Inputs are opened as swg_filter_paf opens them (plain, .gz, .bgz); every
+ * out_paths[k] is created or truncated, also for an empty input.  A group stays below the limits of one file (2^31 lines,
+ * 64 GiB of text), the device memory free at the start of the call and the open-file limit; SWG_PAF_BATCH_BYTES=<n> caps
+ * a group's text.  A file that alone exceeds a limit is filtered as swg_filter_paf filters it; a group the device declines
+ * (name-hash collision, a line over 256 MiB, too many names), and every group under SWG_PAF_FRONTEND=host, runs
+ * swg_paf_parse, swg_filter_batch and swg_paf_write.  Results do not depend on the grouping.
+ * file_counts (may be NULL): n_files rows of SWG_TC_COUNT u64 in the layout of swg_filter_batch's table_counts.  stats (may be
+ * NULL) describes the whole call: summed stage counts, gpu_launches, ms_h2d (text upload), ms_tokenize, ms_device, ms_write.
+ * n_files == 0: SWG_OK.  A NULL array or entry, or two equal out_paths strings: SWG_ERR_ARG.  An input that cannot be
+ * opened: SWG_ERR_IO before any output is created; an output that cannot be created: SWG_ERR_IO; a range error in any file
+ * fails the call with SWG_ERR_RANGE.  swg_last_error names the file.  On an error, the outputs of groups that already
+ * finished may exist.  The context stays usable; outstanding prefetches stay outstanding; afterwards the last-call chain
+ * queries report no chains.  */
+int swg_filter_paf_batch(swg_ctx *ctx, const swg_config *cfg, uint64_t n_files, const char *const *in_paths,
+                         const char *const *out_paths, uint64_t *file_counts, swg_stats *stats);
 /* Same call with the multi-threaded host parser and writer around swg_filter. */
 int swg_filter_paf_host(swg_ctx *ctx, const swg_config *cfg, const char *in_path, const char *out_path,
                         swg_stats *stats);

@@ -107,6 +107,7 @@ SYMBOLS = [
     ("swg_tree_filter_paf", C.c_int, [_vp, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint64, C.c_double, u64p, u64p]),
     ("swg_paf_parse_device", _vp, [_vp, C.c_char_p]),
     ("swg_filter_paf", C.c_int, [_vp, _cfgp, C.c_char_p, C.c_char_p, _statp]),
+    ("swg_filter_paf_batch", C.c_int, [_vp, _cfgp, C.c_uint64, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), u64p, _statp]),
     ("swg_filter_paf_host", C.c_int, [_vp, _cfgp, C.c_char_p, C.c_char_p, _statp]),
     ("swg_filter_file", C.c_int, [_vp, _cfgp, C.c_char_p, C.c_char_p, C.c_int, _statp]),
     ("swg_aln_to_paf", C.c_int, [C.c_char_p, C.c_char_p, C.c_int]),

@@ -291,6 +291,22 @@ class Context:
         self._check(lib.swg_filter_batch(self._h, C.byref(cc), k, cms, outs, _ptr(counts, C.c_uint64), C.byref(stats)))
         return results, counts, stats
 
+    def filter_paf_batch(self, cfg: FilterConfig, in_paths, out_paths):
+        """Many independent PAF files in one call (swg_filter_paf_batch): out_paths[k] receives what swg_filter_paf writes for
+        in_paths[k] alone.  Returns (counts, stats): counts = uint64 (K, TC_COUNT) as in filter_batch; stats describes the call."""
+        ins = [os.fsencode(p) for p in in_paths]
+        outs = [os.fsencode(p) for p in out_paths]
+        if len(ins) != len(outs):
+            raise ValueError("filter_paf_batch: in_paths and out_paths differ in length")
+        k = len(ins)
+        cin = (C.c_char_p * max(k, 1))(*ins)
+        cout = (C.c_char_p * max(k, 1))(*outs)
+        counts = np.zeros((k, _lib.TC_COUNT), np.uint64)
+        stats = _lib.swg_stats()
+        cc = cfg.to_c()
+        self._check(lib.swg_filter_paf_batch(self._h, C.byref(cc), k, cin, cout, _ptr(counts, C.c_uint64), C.byref(stats)))
+        return counts, stats
+
     def prefetch(self, table: MappingTable):
         """Start uploading `table` now (swg_prefetch); the next filter() of the same table (same arrays) finds it on the device."""
         cm = table.to_c()

@@ -144,7 +144,7 @@ static bool tree_reparse(const char *line, size_t len, AniPatch &p) {
 // compaction, and the names interned (*nt).  tc: the zeroed TC_COUNT counter block.  Returns 0 records (nothing else
 // is set) when no line is an alignment.
 template <int MODE>
-static u32 ani_records(swg_ctx *c, const swg_paf &hp, const DevLines &dl, u64 *tc, TokCols *R, NameTable *nt) {
+static u32 ani_records(swg_ctx *c, const PafText &tx, const DevLines &dl, u64 *tc, TokCols *R, NameTable *nt) {
     constexpr u32 READER = MODE == 0 ? RD_ANI : RD_TREE;
     const TokCols L = take_cols<READER>(c->io, dl.n_lines);
     u32 *fix_list = c->io.take<u32>(dl.n_lines);
@@ -157,7 +157,7 @@ static u32 ani_records(swg_ctx *c, const swg_paf &hp, const DevLines &dl, u64 *t
     u64 n_ok = h_tc[TC_OK];
     if (h_tc[TC_NFIX]) // numbers outside the plain grammar: the host's line reader decides
         n_ok += patch_lines<AniPatch>(
-            c, hp, dl, fix_list, (u32)h_tc[TC_NFIX],
+            c, tx, dl, fix_list, (u32)h_tc[TC_NFIX],
             MODE == 0 ? ani_reparse : tree_reparse,
             [=] __device__(const AniPatch &p) {
                 L.kind[p.line] = (u8)p.kind;
@@ -167,7 +167,7 @@ static u32 ani_records(swg_ctx *c, const swg_paf &hp, const DevLines &dl, u64 *t
     const u32 n = (u32)n_ok;
     if (n == 0) return 0;
     *R = take_records<READER>(c, dl, L, n);
-    *nt = intern_names(c, dl.text, hp.text, *R, n, tc, dl.d_cnt);
+    *nt = intern_names(c, dl.text, tx, *R, n, tc, dl.d_cnt);
     return n;
 }
 
@@ -191,7 +191,8 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
     LaunchCounter &lc = c->lc;
     Arena &A = c->io;
     AniResult res;
-    const DevLines dl = load_lines(c, hp);
+    const PafText tx(hp);
+    const DevLines dl = load_lines(c, tx);
     if (hp.text_len == 0) return res;
     u32 *bsum = dl.bsum, *d_cnt = dl.d_cnt;
     u64 *tc = A.take<u64>(TC_COUNT);
@@ -199,7 +200,7 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
     SWG_CUDA(cudaMemsetAsync(tc, 0, sizeof(u64) * TC_COUNT, st));
     TokCols R;
     NameTable nt;
-    const u32 n = ani_records<0>(c, hp, dl, tc, &R, &nt);
+    const u32 n = ani_records<0>(c, tx, dl, tc, &R, &nt);
     if (n == 0) return res;
     const u32 n_seq = nt.n_seq;
     std::vector<std::string> genomes;
@@ -390,19 +391,20 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
     LaunchCounter &lc = c->lc;
     Arena &A = c->io;
     TreeResult res;
-    const DevLines dl = load_lines(c, hp);
+    const PafText tx(hp);
+    const DevLines dl = load_lines(c, tx);
     DevPaf dp;
     dp.text = dl.text;
-    dp.text_len = hp.text_len;
-    if (hp.text_len == 0) { write_device(c, dp, nullptr, nullptr, out_path); return res; }
+    dp.text_len = tx.bytes;
+    if (tx.bytes == 0) { write_device(c, dp, nullptr, nullptr, {out_path}); return res; }
     u32 *bsum = dl.bsum, *d_cnt = dl.d_cnt;
     u64 *tc = A.take<u64>(TC_COUNT);
     u64 h_tc[TC_COUNT];
     SWG_CUDA(cudaMemsetAsync(tc, 0, sizeof(u64) * TC_COUNT, st));
     TokCols R;
     NameTable nt;
-    const u32 n = ani_records<1>(c, hp, dl, tc, &R, &nt);
-    if (n == 0) { write_device(c, dp, nullptr, nullptr, out_path); return res; }
+    const u32 n = ani_records<1>(c, tx, dl, tc, &R, &nt);
+    if (n == 0) { write_device(c, dp, nullptr, nullptr, {out_path}); return res; }
     const u32 n_seq = nt.n_seq;
     // genome of every sequence under extract_genome_prefix (tree_filter.rs:15-25, the P2 rule)
     std::vector<std::string> genomes;
@@ -438,7 +440,7 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
     SWG_CUDA(cudaMemsetAsync(chain, 0, sizeof(u32) * (size_t)n, st));
     dp.n = n;
     dp.rec = R;
-    if (n_inter == 0) { write_device(c, dp, status, chain, out_path); return res; }
+    if (n_inter == 0) { write_device(c, dp, status, chain, {out_path}); return res; }
     u32 *gid = A.take<u32>(n_inter), *seg_start = A.take<u32>(n_inter);
     {
         const u64 *pkc = pk;
@@ -496,7 +498,7 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
     }
     SWG_CUDA(cudaStreamSynchronize(st)); // sel lives on this stack frame
     for (u32 p = 0; p < n_pairs; p++) res.n_selected += sel[p];
-    write_device(c, dp, status, chain, out_path);
+    write_device(c, dp, status, chain, {out_path});
     // kept lines: the records of the selected pairs
     {
         u32 *d_kept = d_cnt + 1;

@@ -23,15 +23,7 @@ struct BatchTable {
 constexpr u32 BATCH_SMEM_TABLES = 8192; // record offsets held in shared memory up to this many tables (32 KB)
 
 // table of union position i: the largest k < K with off[k] <= i (off[0] = 0 <= i < off[K]; empty tables are skipped)
-__device__ __forceinline__ u32 batch_table_of(const u32 *off, u32 K, u32 i) {
-    u32 lo = 0, hi = K;
-    while (hi - lo > 1) {
-        const u32 mid = (lo + hi) >> 1;
-        if (off[mid] <= i) lo = mid;
-        else hi = mid;
-    }
-    return lo;
-}
+__device__ __forceinline__ u32 batch_table_of(const u32 *off, u32 K, u32 i) { return file_at<u32>(off, K, i); }
 // the K + 1 record offsets in shared memory when they fit, else read from global memory
 __device__ __forceinline__ const u32 *batch_offsets(const u32 *rec_off, u32 K, u32 *s_off) {
     if (K + 1 > BATCH_SMEM_TABLES) return rec_off;
@@ -330,6 +322,201 @@ static void do_filter_batch(void *p) {
     F.d2h_bytes = d2h;
     F.gpu_launches = c->lc.n - launches0;
     if (a->stats) *a->stats = F;
+}
+
+// ---- many PAF files in one call (swg_filter_paf_batch, DESIGN §6b) ----------------------------------------------------------
+// Consecutive files form one union (PafText): one upload, one newline scan, one parse, one name table with a namespace per
+// file, one run of the filter, the per-file renumbering above, and one writer that sends every piece of the union's output to
+// the files it overlaps.  Launches grow with the data, not with the number of files.
+
+static void add_stats(swg_stats &a, const swg_stats &b) {
+    a.n_input += b.n_input; a.n_stage1 += b.n_stage1; a.n_after_sweep += b.n_after_sweep; a.n_chains += b.n_chains;
+    a.n_chains_after_mass += b.n_chains_after_mass; a.n_chains_kept += b.n_chains_kept; a.n_anchors += b.n_anchors;
+    a.n_rescued += b.n_rescued; a.n_kept += b.n_kept; a.score_near_ties += b.score_near_ties; a.gpu_launches += b.gpu_launches;
+    a.ms_h2d += b.ms_h2d; a.ms_device += b.ms_device; a.ms_d2h += b.ms_d2h; a.ms_sort_passes += b.ms_sort_passes;
+    a.n_sort_passes += b.n_sort_passes; a.n_sort_pairs += b.n_sort_pairs; a.ms_tokenize += b.ms_tokenize; a.ms_write += b.ms_write;
+    a.exact_rerank |= b.exact_rerank; a.h2d_bytes += b.h2d_bytes; a.d2h_bytes += b.d2h_bytes; a.n_dirty_groups += b.n_dirty_groups;
+    a.ms_prefilter += b.ms_prefilter; a.n_unsorted_groups += b.n_unsorted_groups;
+    if (b.sort_bytes_per_pair) a.sort_bytes_per_pair = b.sort_bytes_per_pair;
+    if (b.prefilter_bytes_per_record) a.prefilter_bytes_per_record = b.prefilter_bytes_per_record;
+}
+
+// A text (one file, or a union of files) through the device front end, the filter and the writer; out_paths[k] receives the
+// output of file k.  counts (K rows of SWG_TC_COUNT, or nullptr for a plain swg_filter_paf): the union's chains are renumbered
+// per file and every file's counts tallied.  FrontEndFallback: the device declines the text, and nothing was written.
+static void filter_paf_device(swg_ctx *c, const swg_config &cfg, const PafText &tx, const std::vector<const char *> &out_paths, u64 *counts,
+                              swg_stats &S) {
+    cudaStream_t st = c->stream;
+    const u64 launches0 = c->lc.n;
+    DevPaf dp;
+    tokenize_device(c, tx, dp);
+    std::memset(&S, 0, sizeof S);
+    const u32 n = dp.n, K = tx.K();
+    u8 *status = c->io.take<u8>(std::max<u32>(n, 1));
+    u32 *chain = c->io.take<u32>(std::max<u32>(n, 1));
+    u64 *d_counts = counts ? c->io.take<u64>((size_t)K * SWG_TC_COUNT) : nullptr;
+    if (counts) SWG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(u64) * SWG_TC_COUNT * (size_t)K, st));
+    if (n) {
+        SWG_CUDA(cudaEventRecord(c->ev[1], st));
+        run_filter_exact(c, cfg, devin_of(dp), status, chain, &S, nullptr, nullptr);
+        if (counts) { // c->last_flags lives in the scratch arena, which write_device takes from: tally first
+            u32 *rec_off = dp.rec_off;
+            if (!rec_off) {
+                rec_off = c->io.take<u32>(K + 1);
+                SWG_CUDA(cudaMemcpyAsync(rec_off, dp.file_rec.data(), sizeof(u32) * (K + 1), cudaMemcpyHostToDevice, st));
+            }
+            u32 *chain_off = c->io.take<u32>(K + 1);
+            const size_t smem = K + 1 <= BATCH_SMEM_TABLES ? sizeof(u32) * (K + 1) : 0;
+            k_batch_chain_off<<<cdiv(K + 1, 256), 256, 0, st>>>(K, rec_off, c->last_keyA, c->last_keyA ? (u32)c->last_n_chains : 0u, chain_off, d_counts);
+            k_batch_finish<<<(u32)c->sm_count * 8, 256, smem, st>>>(n, K, rec_off, chain_off, c->last_flags, status, chain, d_counts);
+            c->lc.n += 2;
+        }
+        SWG_CUDA(cudaEventRecord(c->ev[2], st));
+        SWG_CUDA(cudaStreamSynchronize(st));
+        float ms = 0;
+        SWG_CUDA(cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]));
+        S.ms_device = ms;
+    }
+    if (counts) {
+        SWG_CUDA(cudaMemcpyAsync(counts, d_counts, sizeof(u64) * SWG_TC_COUNT * (size_t)K, cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaStreamSynchronize(st));
+    }
+    const auto t0 = std::chrono::steady_clock::now();
+    write_device(c, dp, status, chain, out_paths);
+    S.ms_write = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    S.ms_h2d = dp.ms_upload;
+    S.ms_tokenize = dp.ms_tokenize;
+    S.gpu_launches = c->lc.n - launches0;
+}
+
+struct PafBatchArgs {
+    swg_ctx *c; const swg_config *cfg; u64 K; const char *const *in; const char *const *out; u64 *counts; swg_stats *stats;
+};
+
+static std::string file_name(const PafBatchArgs &a, u64 k) { return "file " + std::to_string(k) + " (" + a.in[k] + ")"; }
+
+// The files [first, first + K) on the host route: swg_paf_parse per file, one swg_filter_batch, swg_paf_write per file.
+static void filter_paf_host_group(const PafBatchArgs &a, u64 first, u32 K, u64 *counts, swg_stats &S) {
+    std::vector<swg_paf *> ps(K, nullptr);
+    struct Free { std::vector<swg_paf *> &p; ~Free() { for (swg_paf *x : p) swg_paf_free(x); } } free_all{ps};
+    std::vector<swg_mappings> maps(K);
+    for (u32 k = 0; k < K; k++) {
+        char err[256];
+        err[0] = 0;
+        ps[k] = swg_paf_parse(a.in[first + k], err, sizeof err);
+        if (!ps[k]) throw IoError{file_name(a, first + k) + ": " + err};
+        swg_paf_view(ps[k], &maps[k]);
+    }
+    std::vector<std::vector<u8>> status(K);
+    std::vector<std::vector<u32>> chain(K);
+    std::vector<swg_result> res(K);
+    for (u32 k = 0; k < K; k++) {
+        status[k].resize(maps[k].n);
+        chain[k].resize(maps[k].n);
+        res[k] = swg_result{status[k].data(), chain[k].data()};
+    }
+    BatchArgs ba{a.c, a.cfg, K, maps.data(), res.data(), counts, &S};
+    do_filter_batch(&ba);
+    const auto t0 = std::chrono::steady_clock::now();
+    for (u32 k = 0; k < K; k++)
+        if (swg_paf_write(ps[k], a.out[first + k], status[k].data(), chain[k].data()) != SWG_OK)
+            throw IoError{file_name(a, first + k) + ": cannot write " + a.out[first + k]};
+    S.ms_write = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+}
+
+// One group: the files [first, first + group.size()), already open.  The device route, or the host route when the device
+// declines (or SWG_PAF_FRONTEND=host).  A union with more lines than mem_budget allows is split, and its two halves are
+// filtered one after the other.  A range error of a union is located by filtering its files one at a time: the first file
+// that fails alone fails the call, named; when every file passes alone, their results are the call's.
+static void filter_paf_group(const PafBatchArgs &a, u64 first, std::vector<std::unique_ptr<swg_paf>> &group, u64 mem_budget, swg_stats &S) {
+    swg_ctx *c = a.c;
+    const u32 K = (u32)group.size();
+    std::vector<u64> counts((size_t)K * SWG_TC_COUNT);
+    swg_stats gs;
+    std::memset(&gs, 0, sizeof gs);
+    bool split = false, one_by_one = false;
+    try {
+        bool host = c->knobs.paf_host_frontend;
+        if (!host) {
+            std::vector<const swg_paf *> files;
+            for (auto &p : group) files.push_back(p.get());
+            PafText tx(files);
+            tx.mem_budget = mem_budget;
+            try {
+                filter_paf_device(c, *a.cfg, tx, std::vector<const char *>(a.out + first, a.out + first + K), counts.data(), gs);
+            } catch (const FrontEndFallback &) { host = true; } catch (const GroupTooLarge &) { split = true; }
+        }
+        if (host) filter_paf_host_group(a, first, K, counts.data(), gs);
+    } catch (const RangeError &e) {
+        if (K == 1) throw RangeError{file_name(a, first) + ": " + e.msg};
+        one_by_one = true;
+    }
+    if (split || one_by_one) { // nothing of this union was written; its parts are filtered instead
+        const u32 parts = split ? 2 : K;
+        for (u32 p = 0; p < parts; p++) {
+            const u32 k0 = (u32)((u64)K * p / parts), k1 = (u32)((u64)K * (p + 1) / parts);
+            std::vector<std::unique_ptr<swg_paf>> part;
+            for (u32 k = k0; k < k1; k++) part.push_back(std::move(group[k]));
+            filter_paf_group(a, first + k0, part, mem_budget, S);
+        }
+        return;
+    }
+    if (a.counts) std::memcpy(a.counts + first * SWG_TC_COUNT, counts.data(), sizeof(u64) * counts.size());
+    add_stats(S, gs);
+}
+
+static size_t arena_bytes(const Arena &A) {
+    size_t b = 0;
+    for (const auto &blk : A.blocks) b += blk.cap;
+    return b;
+}
+
+static void do_filter_paf_batch(void *p) {
+    const PafBatchArgs &a = *(const PafBatchArgs *)p;
+    swg_ctx *c = a.c;
+    SWG_CUDA(cudaSetDevice(c->device));
+    struct ForgetChains { // as after swg_filter_batch: the union's chain keys describe no file's numbering
+        swg_ctx *c;
+        ~ForgetChains() { c->last_n_chains = 0; c->last_keyA = c->last_keyB = nullptr; c->last_flags = nullptr; }
+    } forget{c};
+    swg_stats S;
+    std::memset(&S, 0, sizeof S);
+    if (a.counts) std::memset(a.counts, 0, sizeof(u64) * SWG_TC_COUNT * (size_t)a.K);
+    // limits of one group: those of a single file, the device memory free at the start of the call (plus what the context's
+    // reusable arenas hold), and open files: a group holds its inputs and its outputs open
+    size_t free_b = 0, total_b = 0;
+    SWG_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    const u64 mem_budget = c->knobs.paf_batch_memory ? c->knobs.paf_batch_memory : (u64)free_b + arena_bytes(c->io) + arena_bytes(c->arena);
+    const u64 byte_cap = std::min<u64>((1ull << 36) - 1, c->knobs.paf_batch_bytes ? c->knobs.paf_batch_bytes : ~0ull);
+    u64 file_cap = 1ull << 31;
+    {
+        struct rlimit rl;
+        if (getrlimit(RLIMIT_NOFILE, &rl) == 0 && rl.rlim_cur != RLIM_INFINITY) file_cap = std::max<u64>(1, ((u64)rl.rlim_cur - std::min<u64>(rl.rlim_cur, 64)) / 2);
+    }
+    std::vector<std::unique_ptr<swg_paf>> group;
+    u64 first = 0, G = 0;
+    for (u64 k = 0; k < a.K; k++) {
+        std::unique_ptr<swg_paf> f(new swg_paf());
+        std::string err;
+        if (!paf_open_text(a.in[k], f.get(), &err)) {
+            if (access(a.in[k], R_OK) == 0) throw RangeError{file_name(a, k) + ": " + err};
+            throw IoError{file_name(a, k) + ": " + err};
+        }
+        const u64 b = f->text_len + (f->text_len && f->text[f->text_len - 1] != '\n' ? 1 : 0);
+        // lines are estimated at 64 bytes or more (a PAF record has twelve fields); the newline scan checks the true count and
+        // a union that needs more is split then (GroupTooLarge), before anything of it is written
+        if (!group.empty() && !(group.size() < file_cap && G + b <= byte_cap && (G + b) / 64 < 0x7FFFFFF0ull &&
+                                paf_union_memory(G + b, (G + b) / 64) <= mem_budget)) {
+            filter_paf_group(a, first, group, mem_budget, S);
+            group.clear();
+            G = 0;
+        }
+        if (group.empty()) first = k;
+        G += b;
+        group.push_back(std::move(f));
+    }
+    if (!group.empty()) filter_paf_group(a, first, group, mem_budget, S);
+    if (a.stats) *a.stats = S;
 }
 
 } // namespace swg

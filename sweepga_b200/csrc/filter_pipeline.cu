@@ -20,8 +20,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "sweepga_b200.h"
@@ -32,6 +34,7 @@
 #include "sweep_tree.cuh"
 #include "paf_host.h"
 
+#include <sys/resource.h>
 #include <unistd.h>
 
 namespace swg {
@@ -133,6 +136,8 @@ struct Knobs {
     int fixpoint_max_rounds = 256;   // SWG_FIXPOINT_MAX_ROUNDS
     u32 tok_long = 4096;             // SWG_TOK_LONG
     bool paf_host_frontend = false;  // SWG_PAF_FRONTEND=host
+    u64 paf_batch_bytes = 0;         // SWG_PAF_BATCH_BYTES: cap on the text of one group of swg_filter_paf_batch (0: none)
+    u64 paf_batch_memory = 0;        // SWG_PAF_BATCH_MEMORY: device-memory budget of those groups (0: what is free at call start)
 };
 static Knobs read_knobs() {
     Knobs k;
@@ -159,6 +164,8 @@ static Knobs read_knobs() {
     if (const char *v = getenv("SWG_FIXPOINT_MAX_ROUNDS")) k.fixpoint_max_rounds = atoi(v);
     if (const char *v = getenv("SWG_TOK_LONG")) k.tok_long = (u32)atoi(v);
     if (const char *v = getenv("SWG_PAF_FRONTEND")) k.paf_host_frontend = strcmp(v, "host") == 0;
+    if (const char *v = getenv("SWG_PAF_BATCH_BYTES")) k.paf_batch_bytes = strtoull(v, nullptr, 10);
+    if (const char *v = getenv("SWG_PAF_BATCH_MEMORY")) k.paf_batch_memory = strtoull(v, nullptr, 10);
     return k;
 }
 } // namespace swg
@@ -1928,10 +1935,6 @@ static void staged_h2d_cols(swg_ctx *c, const std::vector<PinCol> &cols) {
     if (failed.load()) { cudaGetLastError(); throw CudaError{cudaErrorUnknown, __FILE__, __LINE__}; }
 }
 static void staged_h2d(swg_ctx *c, const std::vector<CopyJob> &jobs) { staged_h2d_cols(c, jobs_as_cols(jobs, true)); }
-// host text -> device, through the pinned pieces, one reader thread per piece buffer
-static void upload_text(swg_ctx *c, const char *src, int fd, size_t bytes, char *dst) {
-    staged_h2d(c, std::vector<CopyJob>{CopyJob{src, dst, bytes, fd}});
-}
 // device -> pageable host memory: DMA per piece into a pinned buffer, the team copies the slices out; returns when done.
 // The device data must be complete on c->copy_stream's view (the caller makes copy_stream wait for the producing stream).
 static void staged_d2h_cols(swg_ctx *c, const std::vector<PinCol> &cols) {
@@ -2747,7 +2750,7 @@ swg_paf *swg_paf_parse_device(swg_ctx *c, const char *path) {
         swg_paf *p = a->p;
         SWG_CUDA(cudaSetDevice(c->device));
         DevPaf dp;
-        try { tokenize_device(c, *p, dp); } catch (const FrontEndFallback &) { a->fallback = true; return; }
+        try { tokenize_device(c, PafText(*p), dp); } catch (const FrontEndFallback &) { a->fallback = true; return; }
         const size_t n = dp.n;
         p->n_lines = dp.n_lines;
         p->rank.resize(n); p->line_off.resize(n); p->line_len.resize(n);
@@ -2791,34 +2794,44 @@ int swg_filter_paf(swg_ctx *c, const swg_config *cfg, const char *in_path, const
     struct Args { swg_ctx *c; const swg_config *cfg; const swg_paf *hp; const char *out; swg_stats *stats; bool fallback; } a{c, cfg, &hp, out_path, stats, false};
     const int rc = guarded(c, "swg_filter_paf", [](void *q) {
         Args *a = (Args *)q;
-        swg_ctx *c = a->c;
-        SWG_CUDA(cudaSetDevice(c->device));
-        DevPaf dp;
-        const u64 launches0 = c->lc.n;
-        try { tokenize_device(c, *a->hp, dp); } catch (const FrontEndFallback &) { a->fallback = true; return; }
+        SWG_CUDA(cudaSetDevice(a->c->device));
         swg_stats local;
-        std::memset(&local, 0, sizeof local);
-        u8 *status = c->io.take<u8>(std::max<u32>(dp.n, 1));
-        u32 *chain = c->io.take<u32>(std::max<u32>(dp.n, 1));
-        if (dp.n) {
-            SWG_CUDA(cudaEventRecord(c->ev[1], c->stream));
-            run_filter_exact(c, *a->cfg, devin_of(dp), status, chain, &local, nullptr, nullptr);
-            SWG_CUDA(cudaEventRecord(c->ev[2], c->stream));
-            SWG_CUDA(cudaStreamSynchronize(c->stream));
-            float ms = 0;
-            SWG_CUDA(cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]));
-            local.ms_device = ms;
-        }
-        const auto t0 = std::chrono::steady_clock::now();
-        write_device(c, dp, status, chain, a->out);
-        local.ms_write = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        local.ms_h2d = dp.ms_upload;
-        local.ms_tokenize = dp.ms_tokenize;
-        local.gpu_launches = c->lc.n - launches0;
+        try { filter_paf_device(a->c, *a->cfg, PafText(*a->hp), {a->out}, nullptr, local); } catch (const FrontEndFallback &) { a->fallback = true; return; }
         if (a->stats) *a->stats = local;
     }, &a);
     if (rc == SWG_OK && a.fallback) return swg_filter_paf_host(c, cfg, in_path, out_path, stats);
     return rc;
+}
+
+int swg_filter_paf_batch(swg_ctx *c, const swg_config *cfg, uint64_t n_files, const char *const *in_paths, const char *const *out_paths,
+                         uint64_t *file_counts, swg_stats *stats) {
+    if (!c) return SWG_ERR_ARG;
+    if (!check_cfg(c, cfg)) return SWG_ERR_ARG;
+    if (n_files == 0) {
+        if (stats) std::memset(stats, 0, sizeof *stats);
+        return SWG_OK;
+    }
+    const std::string who = "swg_filter_paf_batch: ";
+    if (!in_paths || !out_paths) { set_err(c, who + "NULL path array"); return SWG_ERR_ARG; }
+    if (n_files >= (1ull << 31)) { set_err(c, who + "too many files (must be < 2^31)"); return SWG_ERR_ARG; }
+    {
+        std::unordered_map<std::string, u64> seen;
+        for (u64 k = 0; k < n_files; k++) {
+            if (!in_paths[k] || !out_paths[k]) { set_err(c, who + "file " + std::to_string(k) + ": NULL path"); return SWG_ERR_ARG; }
+            const auto ins = seen.emplace(out_paths[k], k);
+            if (!ins.second) {
+                set_err(c, who + "files " + std::to_string(ins.first->second) + " and " + std::to_string(k) + " have the same output path " + out_paths[k]);
+                return SWG_ERR_ARG;
+            }
+        }
+    }
+    for (u64 k = 0; k < n_files; k++) { // every input opens before any output is created
+        const int fd = open(in_paths[k], O_RDONLY);
+        if (fd < 0) { set_err(c, who + "file " + std::to_string(k) + ": cannot open " + in_paths[k]); return SWG_ERR_IO; }
+        close(fd);
+    }
+    PafBatchArgs a{c, cfg, n_files, in_paths, out_paths, file_counts, stats};
+    return guarded(c, "swg_filter_paf_batch", do_filter_paf_batch, &a);
 }
 
 // calculate_ani_stats (src/main.rs:334-688) with the text tokenised and the per-pair sums accumulated on the GPU.

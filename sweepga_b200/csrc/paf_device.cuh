@@ -34,7 +34,7 @@
 
 namespace swg {
 
-struct t_fixgather; struct t_patch; struct t_name_assign; struct t_out_bounds;
+struct t_fixgather; struct t_patch; struct t_name_assign; struct t_out_bounds; struct t_name_salt; struct t_file_recs;
 
 __constant__ double c_pow10[23] = {1e0,  1e1,  1e2,  1e3,  1e4,  1e5,  1e6,  1e7,  1e8,  1e9,  1e10, 1e11,
                                    1e12, 1e13, 1e14, 1e15, 1e16, 1e17, 1e18, 1e19, 1e20, 1e21, 1e22};
@@ -460,6 +460,8 @@ __global__ void __launch_bounds__(256) k_name_insert(const u64 *__restrict__ qh,
                 break;
             }
             s = (s + 1) & hmask;
+            // a table past half full is retried larger: stop probing it (once full, a missing key would walk every slot)
+            if ((probe & 31) == 31 && *(volatile const u64 *)&tc[TC_TABLE_FULL]) return;
         }
         if (tc[TC_TABLE_FULL]) return;
     }
@@ -472,13 +474,28 @@ __device__ __forceinline__ u32 name_find(const u64 *__restrict__ hk, u32 hmask, 
 }
 
 // ids + byte verification against the representative (the record / side of the first appearance)
+// file of union position o (a byte, or a record): the largest k < K with fstart[k] <= o
+template <class T> __device__ __forceinline__ u32 file_at(const T *fstart, u32 K, T o) {
+    u32 lo = 0, hi = K;
+    while (hi - lo > 1) {
+        const u32 mid = (lo + hi) >> 1;
+        if (fstart[mid] <= o) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// A union of K > 1 files (fstart: their union byte offsets) gives every file its own namespace: the hashes are salted with
+// the file, and a representative counts only when it lies in the same file, so a salted-hash collision of equal names in
+// two files is reported, never merged.
 __global__ void __launch_bounds__(256) k_name_lookup(const char *__restrict__ text, TokCols R, u32 n, const u64 *__restrict__ hk,
                                                      const u32 *__restrict__ id_of_slot, u32 hmask, const u64 *__restrict__ rep_off,
-                                                     const u32 *__restrict__ rep_len, u32 *__restrict__ qid, u32 *__restrict__ tid,
-                                                     u64 *__restrict__ tc) {
+                                                     const u32 *__restrict__ rep_len, const u64 *__restrict__ fstart, u32 K,
+                                                     u32 *__restrict__ qid, u32 *__restrict__ tid, u64 *__restrict__ tc) {
     const u32 r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= n) return;
     bool mismatch = false;
+    const u32 file = K > 1 ? file_at<u64>(fstart, K, R.off[r]) : 0;
 #pragma unroll 1
     for (int side = 0; side < 2; side++) {
         const u64 key = side ? R.th[r] : R.qh[r];
@@ -486,7 +503,7 @@ __global__ void __launch_bounds__(256) k_name_lookup(const char *__restrict__ te
         const u32 len = side ? R.tlen[r] : R.qlen[r];
         const char *mine = text + R.off[r] + (side ? R.trel[r] : 0);
         const char *rep = text + rep_off[id];
-        if (len != rep_len[id]) mismatch = true;
+        if (len != rep_len[id] || (K > 1 && file_at<u64>(fstart, K, rep_off[id]) != file)) mismatch = true;
         else if (mine != rep)
             for (u32 j = 0; j < len; j++)
                 if (mine[j] != rep[j]) { mismatch = true; break; }
@@ -556,6 +573,29 @@ __device__ __forceinline__ u32 nl_mask(u32 x) { // 0x80 in every byte of x that 
 // ==================================================================================================
 // host driver
 // ==================================================================================================
+// The text the device readers see: one file, or many laid end to end as one union (swg_filter_paf_batch).  File k starts at
+// union byte start[k]; a non-empty file that does not end in '\n' is followed by one '\n' of the union, so every file ends a
+// line and its last line parses and is written exactly as without the terminator.
+struct PafText {
+    std::vector<const swg_paf *> files;
+    std::vector<u64> start; // K + 1 entries; start[K] = bytes
+    u64 bytes = 0;
+    u64 mem_budget = 0;     // a union of K > 1 files whose lines need more device memory than this is declined (GroupTooLarge)
+    explicit PafText(std::vector<const swg_paf *> f) : files(std::move(f)), start(files.size() + 1) {
+        for (size_t k = 0; k < files.size(); k++) {
+            start[k] = bytes;
+            bytes += files[k]->text_len + (pads(k) ? 1 : 0);
+        }
+        start[files.size()] = bytes;
+    }
+    explicit PafText(const swg_paf &p) : PafText(std::vector<const swg_paf *>{&p}) {}
+    u32 K() const { return (u32)files.size(); }
+    bool pads(size_t k) const { const swg_paf &p = *files[k]; return p.text_len && p.text[p.text_len - 1] != '\n'; }
+    // the file that holds union byte o (o < bytes), and the host copy of that byte
+    u32 file_of(u64 o) const { return (u32)(std::upper_bound(start.begin(), start.end() - 1, o) - start.begin()) - 1; }
+    const char *host(u64 o) const { const u32 k = file_of(o); return files[k]->text + (o - start[k]); }
+};
+
 struct DevPaf {
     char *text = nullptr;
     u64 text_len = 0;
@@ -568,11 +608,21 @@ struct DevPaf {
     u32 *P = nullptr, *P2 = nullptr;
     std::vector<std::string> names;
     std::vector<u32> hP, hP2;
+    // per file of the text (K + 1 entries): first record and first sequence id; rec_off: device copy of file_rec (K > 1)
+    std::vector<u32> file_rec, file_seq;
+    u32 *rec_off = nullptr;
     double ms_upload = 0, ms_tokenize = 0;
 };
 
 struct Patch { u32 line, qs, qe, ts, te, blen, matches; u32 kind_strand; double identity; }; // a line re-parsed by the host
 struct FrontEndFallback { std::string why; }; // the device front end declines: the caller uses the host front end
+struct GroupTooLarge {}; // a union of files has more lines than one call may hold: the caller splits it (nothing was written)
+
+// Device memory a text of `bytes` bytes and `lines` lines needs through the front end, the filter and the writer: the text
+// twice (c->io), per line the tokeniser's line and record columns (~170 B), status and chain (5 B), k_prefilter's reserve
+// (400 B per record) and the writer's margin (48 B per record), plus the writer's 1 GiB window.
+constexpr u64 PAF_MEM_PER_BYTE = 2, PAF_MEM_PER_LINE = 640;
+static u64 paf_union_memory(u64 bytes, u64 lines) { return PAF_MEM_PER_BYTE * bytes + PAF_MEM_PER_LINE * lines + (1ull << 30); }
 
 static void tok_read(swg_ctx *c, const u64 *d_tc, u64 *h) {
     SWG_CUDA(cudaMemcpyAsync(h, d_tc, sizeof(u64) * TC_COUNT, cudaMemcpyDeviceToHost, c->stream));
@@ -586,9 +636,11 @@ struct DevLines { // the text in HBM and the start offset of every line (line_st
     u32 *bsum = nullptr, *d_cnt = nullptr; // scan scratch sized for the word scan (>= any per-line scan), 4 counters
 };
 
-// Copies hp.text to the device (c->io, which is reset) and finds the line starts.  Events c->ev[0] / c->ev[1] bracket the upload.
-static DevLines load_lines(swg_ctx *c, const swg_paf &hp) {
-    const u64 B = hp.text_len;
+// Copies the text to the device (c->io, which is reset) and finds the line starts.  Events c->ev[0] / c->ev[1] bracket the
+// upload: one column whose slices are the files (read with pread where a file is mapped) and the terminators the union adds.
+static DevLines load_lines(swg_ctx *c, const PafText &tx) {
+    static const char nl = '\n';
+    const u64 B = tx.bytes;
     cudaStream_t st = c->stream;
     LaunchCounter &lc = c->lc;
     if (B >= (1ull << 36)) throw FrontEndFallback{"input larger than 64 GiB"};
@@ -600,16 +652,22 @@ static DevLines load_lines(swg_ctx *c, const swg_paf &hp) {
     cudaEvent_t e0 = c->ev[0], e1 = c->ev[1];
     char *text = A.take<char>(B + 64);
     dl.text = text;
+    PinCol col{text, (size_t)B, {}};
+    for (u32 k = 0; k < tx.K(); k++) {
+        const swg_paf &p = *tx.files[k];
+        if (p.text_len) col.segs.push_back(PinSeg{(char *)p.text, tx.start[k], p.text_len, p.fd});
+        if (tx.pads(k)) col.segs.push_back(PinSeg{(char *)&nl, tx.start[k] + p.text_len, 1});
+    }
     SWG_CUDA(cudaEventRecord(e0, st));
     SWG_CUDA(cudaMemsetAsync(text + (B & ~(u64)15), 0, 48, st));
     SWG_CUDA(cudaEventRecord(c->ev_copy[0], st));
     SWG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_copy[0], 0));
-    upload_text(c, hp.text, hp.fd, B, text);
+    staged_h2d_cols(c, std::vector<PinCol>{col});
     SWG_CUDA(cudaEventRecord(c->ev_copy[1], c->copy_stream));
     SWG_CUDA(cudaStreamWaitEvent(st, c->ev_copy[1], 0));
     SWG_CUDA(cudaEventRecord(e1, st));
 
-    // ---- 1. line starts -----------------------------------------------------------------------
+    // ---- 1. line starts (the text ends in '\n': every line has its terminator) -------------------
     const u32 nw = (u32)((B + 15) / 16);
     u32 *bsum = A.take<u32>(scan_temp_u32(nw));
     u32 *d_cnt = A.take<u32>(4);
@@ -619,11 +677,9 @@ static DevLines load_lines(swg_ctx *c, const swg_paf &hp) {
         return __popc(nl_mask(v.x)) + __popc(nl_mask(v.y)) + __popc(nl_mask(v.z)) + __popc(nl_mask(v.w));
     };
     scan_apply(count_nl, [] __device__(u32, u32, u32) {}, nw, bsum, d_cnt, st, lc);
-    const u32 n_nl = read_u32(c, d_cnt);
-    const bool last_nl = hp.text[B - 1] == '\n';
-    const u64 n_lines64 = (u64)n_nl + (last_nl ? 0 : 1);
-    if (n_lines64 >= 0x7FFFFFF0ull) throw RangeError{"too many lines (must be < 2^31 per context)"};
-    const u32 n_lines = (u32)n_lines64;
+    const u32 n_lines = read_u32(c, d_cnt);
+    if (tx.K() > 1 && (n_lines >= 0x7FFFFFF0u || (tx.mem_budget && paf_union_memory(B, n_lines) > tx.mem_budget))) throw GroupTooLarge{};
+    if (n_lines >= 0x7FFFFFF0u) throw RangeError{"too many lines (must be < 2^31 per context)"};
     dl.n_lines = n_lines;
     if (n_lines > nw) bsum = A.take<u32>(scan_temp_u32(n_lines)); // lines shorter than 16 bytes on average: the per-line scans need more tiles
     dl.bsum = bsum;
@@ -631,7 +687,7 @@ static DevLines load_lines(swg_ctx *c, const swg_paf &hp) {
     u64 *line_start = A.take<u64>((size_t)n_lines + 2);
     dl.line_start = line_start;
     {
-        const u64 first_last[2] = {0, last_nl ? B : B + 1};
+        const u64 first_last[2] = {0, B};
         SWG_CUDA(cudaMemcpyAsync(line_start, &first_last[0], 8, cudaMemcpyHostToDevice, st));
         SWG_CUDA(cudaMemcpyAsync(line_start + n_lines, &first_last[1], 8, cudaMemcpyHostToDevice, st));
         SWG_CUDA(cudaStreamSynchronize(st)); // first_last lives on this stack frame
@@ -684,7 +740,7 @@ template <u32 READER> static TokCols take_records(swg_ctx *c, const DevLines &dl
 // with apply(p).  The host reads the same bytes as the device: from line_start, without a final '\r'.  Returns how many
 // of the lines are records.
 template <class P, class Apply>
-static u32 patch_lines(swg_ctx *c, const swg_paf &hp, const DevLines &dl, const u32 *fix_list, u32 nfix,
+static u32 patch_lines(swg_ctx *c, const PafText &tx, const DevLines &dl, const u32 *fix_list, u32 nfix,
                        bool (*reparse)(const char *line, size_t len, P &p), Apply apply) {
     cudaStream_t st = c->stream;
     std::vector<u32> lines(nfix);
@@ -699,7 +755,7 @@ static u32 patch_lines(swg_ctx *c, const swg_paf &hp, const DevLines &dl, const 
     u32 n_ok = 0;
     for (u32 i = 0; i < nfix; i++) {
         size_t len = (size_t)(se[2 * i + 1] - se[2 * i]);
-        const char *line = hp.text + se[2 * i];
+        const char *line = tx.host(se[2 * i]);
         if (len > 0 && line[len - 1] == '\r') len--;
         patches[i].line = lines[i];
         if (reparse(line, len, patches[i])) n_ok++;
@@ -715,20 +771,33 @@ struct NameTable { // result of intern_names
     u32 *qid = nullptr, *tid = nullptr;
     u32 n_seq = 0;
     std::vector<std::string> names;
+    std::vector<u32> file_seq; // first id of every file of the text (K + 1 entries)
 };
 
+__device__ __forceinline__ u64 name_salt(u64 h, u32 file) { return file ? name_hash_finish(h ^ ((u64)file * 0xD6E8FEB86659FD93ull), 0) : h; }
+
 // Names -> ids in first-appearance order (query before target within a record).  R needs off / qh / th / qlen / trel /
-// tlen; tc is the TC_COUNT counter block, d_cnt 4 scratch counters.  Memory comes from c->io.
-static NameTable intern_names(swg_ctx *c, const char *text, const char *host_text, const TokCols &R, u32 n, u64 *tc, u32 *d_cnt) {
+// tlen; tc is the TC_COUNT counter block, d_cnt 4 scratch counters.  Memory comes from c->io.  A text of K > 1 files
+// (fstart: their union offsets on the device) gets one namespace per file: the ids are file-major, file k's ids are
+// [file_seq[k], file_seq[k + 1]) in that file's own first-appearance order.
+static NameTable intern_names(swg_ctx *c, const char *text, const PafText &tx, const TokCols &R, u32 n, u64 *tc, u32 *d_cnt,
+                              const u64 *fstart = nullptr) {
     cudaStream_t st = c->stream;
     LaunchCounter &lc = c->lc;
     Arena &A = c->io;
+    const u32 K = tx.K();
     u64 h_tc[TC_COUNT];
     NameTable nt;
     u32 hcap = 1u << 16;
     u64 *hk = nullptr, *hfirst = nullptr;
     u32 D = 0;
     SWG_CUDA(cudaMemsetAsync(tc + TC_COLLISION, 0, sizeof(u64), st));
+    if (K > 1)
+        launch_for<t_name_salt>(n, st, lc, [=] __device__(u32 r) {
+            const u32 f = file_at<u64>(fstart, K, R.off[r]);
+            R.qh[r] = name_salt(R.qh[r], f);
+            R.th[r] = name_salt(R.th[r], f);
+        });
     while (true) {
         hk = A.take<u64>(hcap);
         hfirst = A.take<u64>(hcap);
@@ -766,7 +835,7 @@ static NameTable intern_names(swg_ctx *c, const char *text, const char *host_tex
     }
     nt.qid = A.take<u32>(n);
     nt.tid = A.take<u32>(n);
-    k_name_lookup<<<cdiv(n, 256), 256, 0, st>>>(text, R, n, hk, id_of_slot, hcap - 1, rep_off, rep_len, nt.qid, nt.tid, tc);
+    k_name_lookup<<<cdiv(n, 256), 256, 0, st>>>(text, R, n, hk, id_of_slot, hcap - 1, rep_off, rep_len, fstart, K, nt.qid, nt.tid, tc);
     lc.n++;
     std::vector<u64> h_off(D);
     std::vector<u32> h_len(D);
@@ -776,20 +845,29 @@ static NameTable intern_names(swg_ctx *c, const char *text, const char *host_tex
     if (h_tc[TC_COLLISION]) throw FrontEndFallback{"64-bit name hash collision"};
     nt.n_seq = D;
     nt.names.resize(D);
-    for (u32 j = 0; j < D; j++) nt.names[j].assign(host_text + h_off[j], h_len[j]);
+    nt.file_seq.assign(K + 1, 0);
+    for (u32 j = 0; j < D; j++) {
+        const u32 f = K > 1 ? tx.file_of(h_off[j]) : 0;
+        nt.names[j].assign(tx.files[f]->text + (h_off[j] - tx.start[f]), h_len[j]);
+        nt.file_seq[f + 1]++;
+    }
+    for (u32 k = 0; k < K; k++) nt.file_seq[k + 1] += nt.file_seq[k];
     return nt;
 }
 
-// Tokenise hp.text on the device.  All device memory comes from c->io and stays valid until the next front-end call.
-static void tokenize_device(swg_ctx *c, const swg_paf &hp, DevPaf &dp) {
+// Tokenise the text on the device.  All device memory comes from c->io and stays valid until the next front-end call.
+static void tokenize_device(swg_ctx *c, const PafText &tx, DevPaf &dp) {
     const u32 long_thresh = c->knobs.tok_long;
-    const u64 B = hp.text_len;
+    const u64 B = tx.bytes;
+    const u32 K = tx.K();
     cudaStream_t st = c->stream;
     LaunchCounter &lc = c->lc;
     Arena &A = c->io;
     dp = DevPaf();
     dp.text_len = B;
-    const DevLines dl = load_lines(c, hp);
+    dp.file_rec.assign(K + 1, 0);
+    dp.file_seq.assign(K + 1, 0);
+    const DevLines dl = load_lines(c, tx);
     if (B == 0) return;
     cudaEvent_t e0 = c->ev[0], e1 = c->ev[1], e2 = c->ev[2];
     char *text = dl.text;
@@ -821,7 +899,7 @@ static void tokenize_device(swg_ctx *c, const swg_paf &hp, DevPaf &dp) {
     // ---- lines the device does not decide: the host's reference-exact parser patches them -----------
     if (h_tc[TC_NFIX])
         n_ok += patch_lines<Patch>(
-            c, hp, dl, fix_list, (u32)h_tc[TC_NFIX],
+            c, tx, dl, fix_list, (u32)h_tc[TC_NFIX],
             [](const char *line, size_t len, Patch &p) {
                 PafLine pl;
                 const bool ok = paf_parse_line(line, len, &pl) != PafLine::SKIP; // range / order problems ride along as impossible intervals
@@ -845,16 +923,58 @@ static void tokenize_device(swg_ctx *c, const swg_paf &hp, DevPaf &dp) {
     dp.rec = R;
     if (n == 0) { SWG_CUDA(cudaStreamSynchronize(st)); return; }
 
+    // ---- first record of every file: its first line (the line that starts at its union offset), or the first record at or
+    // after that line when lines were dropped ----------------------------------------------------------------------------
+    u64 *fstart = nullptr;
+    if (K > 1) {
+        fstart = A.take<u64>(K + 1);
+        dp.rec_off = A.take<u32>(K + 1);
+        SWG_CUDA(cudaMemcpyAsync(fstart, tx.start.data(), sizeof(u64) * (K + 1), cudaMemcpyHostToDevice, st));
+        u32 *rec_off = dp.rec_off;
+        const u32 *rank = dp.rank;
+        launch_for<t_file_recs>(K + 1, st, lc, [=] __device__(u32 k) {
+            u32 lo = 0, hi = n_lines;
+            while (lo < hi) { const u32 mid = (lo + hi) >> 1; if (line_start[mid] < fstart[k]) lo = mid + 1; else hi = mid; }
+            const u32 line = lo;
+            if (rank) {
+                lo = 0; hi = n;
+                while (lo < hi) { const u32 mid = (lo + hi) >> 1; if (rank[mid] < line) lo = mid + 1; else hi = mid; }
+            }
+            rec_off[k] = lo;
+        });
+        SWG_CUDA(cudaMemcpyAsync(dp.file_rec.data(), rec_off, sizeof(u32) * (K + 1), cudaMemcpyDeviceToHost, st));
+    } else dp.file_rec[1] = n;
+
     // ---- 4. names -> ids in first-appearance order ------------------------------------------------
     {
-        NameTable nt = intern_names(c, text, hp.text, R, n, tc, d_cnt);
+        NameTable nt = intern_names(c, text, tx, R, n, tc, d_cnt, fstart);
         dp.qid = nt.qid;
         dp.tid = nt.tid;
         dp.n_seq = nt.n_seq;
         dp.names.swap(nt.names);
+        dp.file_seq.swap(nt.file_seq);
     }
     const u32 D = dp.n_seq;
-    paf_prefix_ids(dp.names, &dp.hP, &dp.hP2);
+    // genome prefixes P and P2 per file, the ids of file k shifted by the genomes of the files before it
+    if (K == 1) paf_prefix_ids(dp.names, &dp.hP, &dp.hP2);
+    else {
+        dp.hP.resize(D);
+        dp.hP2.resize(D);
+        u32 goff = 0;
+        std::vector<u32> p, p2;
+        for (u32 k = 0; k < K; k++) {
+            const u32 a = dp.file_seq[k], b = dp.file_seq[k + 1];
+            if (a == b) continue;
+            paf_prefix_ids(std::vector<std::string>(dp.names.begin() + a, dp.names.begin() + b), &p, &p2);
+            u32 mx = 0;
+            for (u32 j = 0; j < b - a; j++) {
+                dp.hP[a + j] = p[j] + goff;
+                dp.hP2[a + j] = p2[j] + goff;
+                mx = std::max(mx, std::max(p[j], p2[j]));
+            }
+            goff += mx + 1;
+        }
+    }
     dp.P = A.take<u32>(D);
     dp.P2 = A.take<u32>(D);
     SWG_CUDA(cudaMemcpyAsync(dp.P, dp.hP.data(), (size_t)D * 4, cudaMemcpyHostToDevice, st));
@@ -877,17 +997,24 @@ static DevIn devin_of(const DevPaf &dp) {
 }
 
 // Tagged output, assembled on the device window by window (1 GiB of input text per window keeps every offset in u32),
-// copied back through the pinned pieces and written with plain write()s.
-static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u32 *chain_id, const char *out_path) {
+// copied back through the pinned pieces and written with pwrite()s.  out_paths: one per file of the text (dp.file_rec; a
+// DevPaf without it is one file).  The outputs of the files are consecutive ranges of the union's output: a piece goes to
+// every file it overlaps, at its output position minus the file's base (the output position of the file's first record,
+// taken from the window's scan once the window that holds that record is assembled).
+static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u32 *chain_id, const std::vector<const char *> &out_paths) {
     const bool trace = c->knobs.stage_timing;
     const auto t_begin = std::chrono::steady_clock::now();
     auto lap = [&](const char *what) {
         if (trace) fprintf(stderr, "[swg write] %s at %.1f ms\n", what, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count());
     };
-    const int fd = open(out_path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    const u32 K = (u32)out_paths.size();
+    struct Closer { std::vector<int> fd; ~Closer() { for (int f : fd) if (f >= 0) close(f); } } closer{std::vector<int>(K, -1)};
+    std::vector<int> &fds = closer.fd;
+    for (u32 k = 0; k < K; k++) {
+        fds[k] = open(out_paths[k], O_WRONLY | O_CREAT | O_TRUNC, 0644);
+        if (fds[k] < 0) throw IoError{std::string("cannot create ") + out_paths[k]};
+    }
     lap("open");
-    if (fd < 0) throw IoError{std::string("cannot create ") + out_path};
-    struct Closer { int fd; ~Closer() { if (fd >= 0) close(fd); } } closer{fd};
     const u32 n = dp.n;
     if (n == 0) return;
     ensure_pinned(c);
@@ -916,7 +1043,18 @@ static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u
     u32 *d_tot = A.take<u32>(4);
     char *out = A.take<char>(std::min<u64>(W, dp.text_len) + c->tok_maxlen + (u64)48 * max_rec + 256);
     const u32 *len = dp.rec.len;
+    // the files with records, in order, and their output bases (UINT64_MAX until known)
+    const std::vector<u32> frec = dp.file_rec.empty() ? std::vector<u32>{0, n} : dp.file_rec;
+    std::vector<u32> live;
+    for (u32 k = 0; k < K; k++)
+        if (frec[k] < frec[k + 1]) live.push_back(k);
+    std::vector<u64> live_base(live.size(), UINT64_MAX);
+    std::vector<u32> h_base(K);
+    u32 *d_base = K > 1 ? A.take<u32>(K) : nullptr;
+    const u32 *rec_off = dp.rec_off;
+    size_t known = 0; // live files whose base is known
     std::atomic<int> failed{0}; // 1: CUDA, 2: write
+    std::atomic<u32> bad_file{0};
     u64 file_off = 0;
     for (u32 k = 0; k < nwin && !failed.load(); k++) {
         const u32 r0 = bounds[k], nrec = bounds[k + 1] - bounds[k];
@@ -925,12 +1063,25 @@ static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u
                        const u8 s = status[r0 + w];
                        return (s == 0 || s > OUT_PLAIN) ? 0u : len[r0 + w] + out_suffix_len(s, chain_id[r0 + w]);
                    },
-                   [=] __device__(u32 w, u32 ex, u32 v) { out_off[w] = v ? ex : NONE32; }, nrec, bsum, d_tot, st, lc);
+                   [=] __device__(u32 w, u32 ex, u32 v) {
+                       out_off[w] = v ? ex : NONE32;
+                       if (K > 1) {
+                           const u32 r = r0 + w, f = file_at<u32>(rec_off, K, r);
+                           if (rec_off[f] == r) d_base[f] = ex;
+                       }
+                   },
+                   nrec, bsum, d_tot, st, lc);
         k_out_copy<<<cdiv((u64)nrec * 32, 256), 256, 0, st>>>(dp.text, dp.rec.off, len, status, chain_id, r0, nrec, out_off, out);
         lc.n++;
+        size_t now = known;
+        while (now < live.size() && frec[live[now]] < r0 + nrec) now++;
+        if (K > 1 && now > known)
+            SWG_CUDA(cudaMemcpyAsync(h_base.data() + live[known], d_base + live[known], sizeof(u32) * (live[now - 1] + 1 - live[known]),
+                                     cudaMemcpyDeviceToHost, st));
         const u32 total = read_u32(c, d_tot); // synchronises: the window is assembled
+        for (; known < now; known++) live_base[known] = file_off + (K > 1 ? h_base[live[known]] : 0);
         lap("window assembled");
-        // device -> pinned piece -> pwrite at its file offset, one worker per piece buffer
+        // device -> pinned piece -> pwrite at its file offsets, one worker per piece buffer
         const size_t npieces = ((size_t)total + PIN_PIECE - 1) / PIN_PIECE;
         std::atomic<size_t> next{0};
         auto worker = [&](int t) {
@@ -944,11 +1095,17 @@ static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u
                     failed = 1;
                     break;
                 }
-                size_t done = 0;
-                while (done < l) {
-                    const ssize_t w = pwrite(fd, c->pin[t] + done, l - done, (off_t)(file_off + o + done));
-                    if (w <= 0) { failed = 2; break; }
-                    done += (size_t)w;
+                const u64 g0 = file_off + o, g1 = g0 + l;
+                size_t i = (size_t)(std::upper_bound(live_base.begin(), live_base.end(), g0) - live_base.begin()) - 1;
+                for (u64 g = g0; g < g1 && !failed.load(); i++) {
+                    const u64 stop = std::min(g1, i + 1 < live_base.size() ? live_base[i + 1] : UINT64_MAX);
+                    size_t done = 0;
+                    while (g + done < stop) {
+                        const ssize_t w = pwrite(fds[live[i]], c->pin[t] + (g - g0) + done, stop - g - done, (off_t)(g - live_base[i] + done));
+                        if (w <= 0) { bad_file = live[i]; failed = 2; break; }
+                        done += (size_t)w;
+                    }
+                    g = stop;
                 }
             }
         };
@@ -960,11 +1117,14 @@ static void write_device(swg_ctx *c, const DevPaf &dp, const u8 *status, const u
         file_off += total;
         lap("window written");
     }
-    closer.fd = -1;
-    const bool closed = close(fd) == 0;
+    bool closed = true;
+    for (u32 k = 0; k < K; k++) {
+        if (close(fds[k]) != 0 && closed) { closed = false; bad_file = k; }
+        fds[k] = -1;
+    }
     lap("closed");
     if (failed.load() == 1) { cudaGetLastError(); throw CudaError{cudaErrorUnknown, __FILE__, __LINE__}; }
-    if (failed.load() == 2 || !closed) throw IoError{std::string("write to ") + out_path + " failed"};
+    if (failed.load() == 2 || !closed) throw IoError{std::string("write to ") + out_paths[bad_file.load()] + " failed"};
 }
 
 } // namespace swg
