@@ -301,15 +301,17 @@ int swg_parse_ani_method(const char *s, int *method, double *percentile, int *so
  * filter (ORTHOGONAL; runs swg_filter_paf into a temp file first), or the best ones in a stable descending sort
  * until their block lengths cover `percentile` % of the genome size.  The text is tokenised on the GPU and every
  * pair's f64 sums are accumulated there in the reference's order, so *ani50 is the reference's value bit for bit
- * (NSORT_SCORE: up to ties within 1 ulp of log).  SWG_ERR_RANGE when the reference would panic on a NaN. */
+ * (NSORT_SCORE takes ln from the device's port of the host libm, so this holds whenever swg_log_matches_host()).
+ * SWG_ERR_RANGE when the reference would panic on a NaN. */
 int swg_ani_stats(swg_ctx *ctx, const char *paf_path, int method, double percentile, int sort, double *ani50,
                   uint64_t *n_pairs);
 
 /* apply_tree_filter_to_paf, src/tree_filter.rs:205-283 (`--sparsify tree:k[,f[,r]]` on an existing PAF): per genome
  * pair (extract_genome_prefix, :15-25) identity = sum(matches) / sum(block length); every genome keeps its k_nearest
  * and k_farthest neighbours, plus the pairs whose SipHash-1-3 is below random_fraction * 2^64 (select_tree_pairs,
- * :84-164); the lines of the selected pairs are written verbatim, in input order.  Tokenising, the per-pair integer
- * sums and the output assembly run on the GPU; the pair selection (thousands of pairs) on the host.  Ties in identity
+ * :84-164); the lines of the selected pairs are written verbatim, in input order.  Tokenising, the per-pair sums (the
+ * reference's f64 sums in file order, also past 2^53 and 2^64) and the output assembly run on the GPU; the pair
+ * selection (thousands of pairs) on the host.  Ties in identity
  * go by neighbour name (the reference leaves them to HashMap iteration order). */
 int swg_tree_filter_paf(swg_ctx *ctx, const char *in_path, const char *out_path, uint64_t k_nearest, uint64_t k_farthest,
                         double random_fraction, uint64_t *n_kept, uint64_t *n_pairs_selected);

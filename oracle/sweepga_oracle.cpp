@@ -968,7 +968,8 @@ int orc_ani_stats(const char *path, int method, double percentile, int sort, dou
                     double dv;
                     if (rust_parse_f64(f[k].substr(5), dv)) { fm = (1.0 - dv) * b; break; }
                 }
-            alns.push_back(Aln{qg, tg, fm, b, fm / std::max(b, 1.0)});
+            // Rust's f64::max returns the other argument when one is NaN (std::max would return the NaN), so fmax
+            alns.push_back(Aln{qg, tg, fm, b, fm / std::fmax(b, 1.0)});
         }
     }
     if (!tmp.empty()) remove(tmp.c_str());
@@ -976,11 +977,10 @@ int orc_ani_stats(const char *path, int method, double percentile, int sort, dou
     if (alns.empty()) { *ani50 = 0.0; return 0; } // :468-471 / :606-609
     size_t take = alns.size();
     if (method == 2) {
-        for (const auto &a : alns) {
-            double key = sort == 0 ? a.block : sort == 1 ? a.identity : a.identity * std::max(std::log(a.block), 1.0);
-            if (key != key) return -2;
-        }
-        auto key = [&](const Aln &a) { return sort == 0 ? a.block : sort == 1 ? a.identity : a.identity * std::max(std::log(a.block), 1.0); };
+        // f64::max again (fmax): ln of a zero, negative or NaN block length is -inf or NaN, and the key then uses 1
+        auto key = [&](const Aln &a) { return sort == 0 ? a.block : sort == 1 ? a.identity : a.identity * std::fmax(std::log(a.block), 1.0); };
+        for (const auto &a : alns)
+            if (key(a) != key(a)) return -2;
         std::stable_sort(alns.begin(), alns.end(), [&](const Aln &x, const Aln &y) { return key(x) > key(y); }); // :612-631
         double total = 0.0;
         for (const auto &kv : genome_sizes) total += (double)kv.second; // :634

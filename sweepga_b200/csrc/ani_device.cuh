@@ -10,7 +10,8 @@
 //   1. the text is tokenised on the device (k_ani_parse, built from the line grammar of paf_device.cuh; the lines it
 //      lists are patched by the host reader through patch_lines, records compacted by take_records, names interned as
 //      in the filter front end: ani_records)
-//   2. "nX": one stable radix sort on the order-preserving bit pattern of the f64 key; the cut is found from per-tile
+//   2. "nX": one stable radix sort on the order-preserving bit pattern of the f64 key (the score key takes its logarithm
+//      from the glibc port, ln_fn, so it is the reference's key bit for bit); the cut is found from per-tile
 //      integer sums (exact while the block lengths are integers, which a PAF column always is; otherwise the host
 //      walks the sorted column)
 //   3. a second stable sort by genome pair brings every pair's addends together IN ORDER; one thread per pair adds them
@@ -215,6 +216,7 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
     const u32 *qid = nt.qid, *tid = nt.tid;
     const u64 nP64 = nP;
     const bool npct = method == SWG_ANI_NPERCENTILE;
+    const bool cuda_log = c->knobs.cuda_log;
     {
         u64 *sk = skey;
         u32 *sv = sval;
@@ -226,8 +228,10 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
             bool isnan_ = false, nonint = false;
             if (inter && npct) {
                 const double m = R.m[r], b = R.b[r];
-                const double identity = __ddiv_rn(m, fmax(b, 1.0)); // main.rs:592
-                double k = sort == SWG_NSORT_LENGTH ? b : sort == SWG_NSORT_IDENTITY ? identity : __dmul_rn(identity, fmax(log(b), 1.0));
+                // main.rs:592 and :612-631; fmax is f64::max (a NaN argument yields the other one), ln_fn the host libm's
+                // bits (glibc_log.cuh): ln(b) < 1 (near 1, zero, negative, NaN) gives 1 whichever log computes it
+                const double identity = __ddiv_rn(m, fmax(b, 1.0));
+                double k = sort == SWG_NSORT_LENGTH ? b : sort == SWG_NSORT_IDENTITY ? identity : __dmul_rn(identity, fmax(ln_fn(b, cuda_log), 1.0));
                 isnan_ = k != k;
                 if (k == 0.0) k = 0.0; // -0.0 and +0.0 compare equal in partial_cmp
                 key = score_desc_key(k);
@@ -379,11 +383,14 @@ static AniResult ani_device(swg_ctx *c, const swg_paf &hp, int method, double pe
 
 // ---- tree sparsification of an existing PAF (`--sparsify tree:k[,f[,r]]`) --------------------------------------
 //   tree_filter_device  <- apply_tree_filter_to_paf   (src/tree_filter.rs:205-283)
-// Per genome pair (the P2 prefix rule) Σ matches / Σ block length over u64 columns — integers, so the sums are
-// order-free: sort by pair, warp-segmented reduction, one atomic per (warp, pair).  The pair list (thousands) goes
-// to the host, select_tree_pairs picks the k nearest / k farthest / hashed-random pairs, the flags come back, and
-// the kept lines are assembled on the device in input order (write_device, verbatim lines).
-struct t_tree_keys; struct t_tree_sums; struct t_tree_status; struct t_tree_pairout;
+// Per genome pair (the P2 prefix rule) Σ matches / Σ block length over u64 columns, which the reference adds as f64
+// in file order.  Sort by pair (stable: each pair's records stay in file order), then a warp-segmented reduction of
+// the exact integer sums, split into 32-bit halves so that nothing wraps, one atomic per (warp, pair).  While every
+// pair's totals are below 2^53 each partial f64 sum is exact and the integer total is the reference's value; past
+// that the conversions round and the order matters, so k_ani_pair_sums adds the f64 values sequentially instead.  The
+// pair list (thousands) goes to the host, select_tree_pairs picks the k nearest / k farthest / hashed-random pairs,
+// the flags come back, and the kept lines are assembled on the device in input order (write_device, verbatim lines).
+struct t_tree_keys; struct t_tree_sums; struct t_tree_f64; struct t_tree_status; struct t_tree_pairout;
 struct TreeResult { u64 n_kept = 0, n_selected = 0; };
 
 static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *out_path, u64 k_nearest, u64 k_farthest, double random_fraction) {
@@ -452,40 +459,67 @@ static TreeResult tree_filter_device(swg_ctx *c, const swg_paf &hp, const char *
                    n_inter, bsum, d_cnt, st, lc);
     }
     const u32 n_pairs = read_u32(c, d_cnt);
-    u64 *sums = A.take<u64>(2 * (size_t)n_pairs), *pkeys = A.take<u64>(n_pairs);
-    SWG_CUDA(cudaMemsetAsync(sums, 0, sizeof(u64) * 2 * (size_t)n_pairs, st));
+    // per pair: Σ of the high and Σ of the low 32-bit halves of matches and of block length; fewer than 2^32 addends,
+    // so none of the four wraps and the exact totals are rebuilt on the host
+    u64 *sums = A.take<u64>(4 * (size_t)n_pairs), *pkeys = A.take<u64>(n_pairs);
+    SWG_CUDA(cudaMemsetAsync(sums, 0, sizeof(u64) * 4 * (size_t)n_pairs, st));
     {
         const u32 *pvc = pv;
         const u64 *pkc = pk;
         launch_for<t_tree_sums>(n_inter, st, lc, [=] __device__(u32 k) {
             const u32 r = pvc[k], p = gid[k];
-            u64 m = R.ql[r], b = R.tl[r];
+            const u64 m = R.ql[r], b = R.tl[r];
+            u64 v[4] = {m >> 32, m & 0xFFFFFFFFull, b >> 32, b & 0xFFFFFFFFull};
             // runs of one pair are contiguous: segmented reduction towards the first lane of each run
             const u32 am = __activemask();
             const u32 run = __match_any_sync(am, p);
             const u32 lane = threadIdx.x & 31;
             for (u32 off = 1; off < 32; off <<= 1) {
-                const u64 tm = __shfl_down_sync(am, m, off), tb = __shfl_down_sync(am, b, off);
-                if (lane + off < 32 && ((run >> (lane + off)) & 1u)) { m += tm; b += tb; }
+                u64 t[4];
+#pragma unroll
+                for (int j = 0; j < 4; j++) t[j] = __shfl_down_sync(am, v[j], off);
+                if (lane + off < 32 && ((run >> (lane + off)) & 1u))
+#pragma unroll
+                    for (int j = 0; j < 4; j++) v[j] += t[j];
             }
-            if (lane == (u32)(__ffs(run) - 1)) {
-                atomicAdd((unsigned long long *)&sums[2 * (size_t)p], (unsigned long long)m);
-                atomicAdd((unsigned long long *)&sums[2 * (size_t)p + 1], (unsigned long long)b);
-            }
+            if (lane == (u32)(__ffs(run) - 1))
+#pragma unroll
+                for (int j = 0; j < 4; j++) atomicAdd((unsigned long long *)&sums[4 * (size_t)p + j], (unsigned long long)v[j]);
         });
         launch_for<t_tree_pairout>(n_pairs, st, lc, [=] __device__(u32 p) { pkeys[p] = pkc[seg_start[p]]; });
     }
-    std::vector<u64> h_sums(2 * (size_t)n_pairs), h_keys(n_pairs);
-    SWG_CUDA(cudaMemcpyAsync(h_sums.data(), sums, sizeof(u64) * 2 * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
+    std::vector<u64> h_sums(4 * (size_t)n_pairs), h_keys(n_pairs);
+    SWG_CUDA(cudaMemcpyAsync(h_sums.data(), sums, sizeof(u64) * 4 * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
     SWG_CUDA(cudaMemcpyAsync(h_keys.data(), pkeys, sizeof(u64) * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
     SWG_CUDA(cudaStreamSynchronize(st));
     std::vector<u32> lo(n_pairs), hi(n_pairs);
     std::vector<double> ident(n_pairs);
+    bool exact = true;
     for (u32 p = 0; p < n_pairs; p++) {
         lo[p] = (u32)(h_keys[p] / nG);
         hi[p] = (u32)(h_keys[p] % nG);
-        const double tm = (double)h_sums[2 * (size_t)p], tb = (double)h_sums[2 * (size_t)p + 1]; // tree_filter.rs:58-59: f64 sums of integers, exact below 2^53
-        ident[p] = tb > 0.0 ? tm / tb : 0.0;
+        const u64 *s = &h_sums[4 * (size_t)p];
+        const unsigned __int128 tm = ((unsigned __int128)s[0] << 32) + s[1], tb = ((unsigned __int128)s[2] << 32) + s[3];
+        // tree_filter.rs:58-59 adds `as f64` conversions in file order: below 2^53 every partial sum is exact, so the
+        // exact total is that f64 sum
+        if (tm >= ((unsigned __int128)1 << 53) || tb >= ((unsigned __int128)1 << 53)) exact = false;
+        else ident[p] = tb > 0 ? (double)tm / (double)tb : 0.0;
+    }
+    // A pair past 2^53: the conversions round and the order matters; add them sequentially in file order.  One thread per
+    // pair then walks all of that pair's records (dependent adds): a two-genome file of 20 M lines takes 1.99 s instead
+    // of 0.77 s on a B200 at 1000 W (tools/bench_tree_prepass.py --past-2p53).  Only such totals take this path.
+    if (!exact) {
+        double *ms = A.take<double>(n_inter), *bs = A.take<double>(n_inter), *d_ident = A.take<double>(n_pairs);
+        const u32 *pvc = pv;
+        launch_for<t_tree_f64>(n_inter, st, lc, [=] __device__(u32 k) {
+            const u32 r = pvc[k];
+            ms[k] = __ull2double_rn(R.ql[r]);
+            bs[k] = __ull2double_rn(R.tl[r]);
+        });
+        k_ani_pair_sums<<<cdiv(n_pairs, 128), 128, 0, st>>>(ms, bs, seg_start, n_pairs, n_inter, d_ident); // sb > 0 ? sm / sb : 0
+        lc.n++;
+        SWG_CUDA(cudaMemcpyAsync(ident.data(), d_ident, sizeof(double) * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
+        SWG_CUDA(cudaStreamSynchronize(st));
     }
     bool has_nan = false;
     std::vector<uint8_t> sel = tree_select_pairs(genomes, lo, hi, ident, k_nearest, k_farthest, random_fraction, &has_nan);
