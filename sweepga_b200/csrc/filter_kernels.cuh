@@ -18,7 +18,7 @@ constexpr u8 F_ZLQ = 2;     // zero-length query interval
 constexpr u8 F_ZLT = 4;     // zero-length target interval
 constexpr u8 F_PREMEM = 8;  // member of a chain that passed the mass/identity filter (pre_sweep_scaffold_members)
 constexpr u8 F_REV = 16;    // reverse strand (any strand byte other than '+', paf_filter.rs:311)
-constexpr u8 F_ANCHOR = 32; // status == scaffold: member of a kept chain or captured inversion (set by t_assign / t_inversion)
+constexpr u8 F_ANCHOR = 32; // status == scaffold: member of a kept chain or captured inversion (set by k_assign / t_inversion)
 
 // counters (u64 each) shared with the host
 enum {
@@ -211,19 +211,6 @@ __global__ void __launch_bounds__(256) k_unassigned(u32 n, const u8 *__restrict_
     const int slots[1] = {C_KEPT};
     const u32 vals[1] = {kept ? 1u : 0u};
     block_count_add<1>(ctr, slots, vals);
-}
-
-// final tallies for swg_stats (grid-stride, one atomic pair per CTA)
-__global__ void __launch_bounds__(256) k_count_status(u32 n, const u8 *__restrict__ status, u64 *__restrict__ ctr) {
-    u32 a = 0, r = 0;
-    for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        u8 s = status[i];
-        a += s == 1;
-        r += s == 2;
-    }
-    const int slots[2] = {C_ANCHORS, C_RESCUED};
-    const u32 vals[2] = {a, r};
-    block_count_add<2>(ctr, slots, vals);
 }
 
 // ---------------------------------------------------------------------------------------------

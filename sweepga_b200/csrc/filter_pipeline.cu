@@ -62,10 +62,16 @@ template <class Tag, class F> static inline void launch_for_dev(const u32 *n_ptr
     k_for_dev<Tag, F><<<(u32)sm_count * 8, 256, 0, st>>>(n_ptr, f);
     lc.n++;
 }
-// tags: one per element-wise stage, so that the ncu launch list reads k_for<swg::t_assign, ...> etc.
+// add the hits of the active lanes to a counter: one atomic per warp (for rare hits, e.g. the statuses of the inversion capture)
+static __device__ __forceinline__ void warp_count_add(u64 *ctr, int slot, bool hit) {
+    const u32 am = __activemask();
+    const u32 n = __popc(__ballot_sync(am, hit));
+    if (n && lane_id() == (u32)(__ffs(am) - 1)) atomicAdd((unsigned long long *)&ctr[slot], (unsigned long long)n);
+}
+// tags: one per element-wise stage, so that the ncu launch list reads k_for<swg::t_tspace, ...> etc.
 struct t_iota; struct t_maxp; struct t_scores; struct t_gkey; struct t_events; struct t_sweep_gather; struct t_sweep_keep;
 struct t_gather; struct t_chain_order; struct t_tspace; struct t_segapply; struct t_keys_c2min; struct t_keys_g2min;
-struct t_final_k; struct t_assign; struct t_invkeys; struct t_invw; struct t_invw2; struct t_invent; struct t_inversion; struct t_anchor_keys; struct t_rescue;
+struct t_final_k; struct t_invkeys; struct t_invw; struct t_invw2; struct t_invent; struct t_inversion; struct t_anchor_keys; struct t_rescue;
 
 // ---- grow-only HBM arena ----------------------------------------------------------------------
 // One block sized for the common path; a call that needs more (general sweeps, degenerate
@@ -1279,18 +1285,87 @@ static KeptChains order_chains(swg_ctx *c, const swg_config &cfg, const DevIn &i
 }
 
 // ---- K5: anchors = members of kept chains (paf_filter.rs:517-528) ---------------------------------
-static void assign_anchors(swg_ctx *c, const Ordered &O, const Chains &chains, u8 *flags, u8 *status, u32 *chain_id) {
-    const u32 *chain_of = chains.chain_of;
-    const SortedIdx sidx = O.sidx;
-    const ChainTable ct = chains.ct;
-    launch_for<t_assign>(O.n_m, c->stream, c->lc, [=] __device__(u32 p) {
-        u32 ci = chain_of[p];
-        u32 i = sidx[p];
-        u32 kk = ct.k[ci];
-        if (kk) { status[i] = 1; chain_id[i] = kk; }
-        const u8 add = (u8)((kk ? F_ANCHOR : 0) | (ct.pass[ci] ? F_PREMEM : 0));
-        if (add) flags[i] |= add;
-    });
+// One thread per four sorted positions (striped over a 1024-position block).  Counts the anchors it writes into C_ANCHORS, one
+// atomic per block.  EMIT: also appends the inversion candidates (alive, reverse strand, not an anchor) to inv_list in no
+// particular order, one atomic on *inv_n per block.  That list equals the flag scan over all N records only when every alive
+// record is a sorted position (n_m == n_alive).
+template <bool EMIT>
+__global__ void __launch_bounds__(256) k_assign(u32 n_m, const u32 *__restrict__ chain_of, SortedIdx sidx, ChainTable ct, u8 *flags,
+                                                u8 *__restrict__ status, u32 *__restrict__ chain_id, u64 *ctr, u32 *__restrict__ inv_list,
+                                                u32 *inv_n) {
+    __shared__ u32 s_w[8][4];
+    __shared__ u32 s_base;
+    const u32 lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const u32 base = blockIdx.x * 1024;
+    u32 rec[4], m[4], n_anchor = 0;
+    bool cand[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const u32 p = base + k * 256 + threadIdx.x;
+        cand[k] = false;
+        rec[k] = 0;
+        if (p < n_m) {
+            const u32 ci = chain_of[p];
+            const u32 i = sidx[p];
+            const u32 kk = ct.k[ci];
+            if (kk) { status[i] = 1; chain_id[i] = kk; n_anchor++; }
+            const u8 add = (u8)((kk ? F_ANCHOR : 0) | (ct.pass[ci] ? F_PREMEM : 0));
+            if (EMIT) {
+                const u8 fl = flags[i];
+                cand[k] = !kk && (fl & (F_ALIVE | F_REV)) == (F_ALIVE | F_REV);
+                if (add) flags[i] = fl | add;
+            } else if (add) flags[i] |= add;
+            rec[k] = i;
+        }
+        if (EMIT) {
+            m[k] = __ballot_sync(0xFFFFFFFFu, cand[k]);
+            if (lane == 0) s_w[warp][k] = __popc(m[k]);
+        }
+    }
+    const int slots[1] = {C_ANCHORS};
+    const u32 vals[1] = {n_anchor};
+    block_count_add<1>(ctr, slots, vals); // (its barriers also publish s_w)
+    if (!EMIT) return;
+    if (threadIdx.x == 0) {
+        u32 tot = 0;
+        for (int k = 0; k < 4; k++)
+            for (int w = 0; w < 8; w++) { const u32 t = s_w[w][k]; s_w[w][k] = tot; tot += t; }
+        s_base = tot ? atomicAdd(inv_n, tot) : 0;
+    }
+    __syncthreads();
+    const u32 lt = lanemask_lt();
+#pragma unroll
+    for (int k = 0; k < 4; k++)
+        if (cand[k]) inv_list[s_base + s_w[warp][k] + __popc(m[k] & lt)] = rec[k];
+}
+
+// The inversion candidates of the default path, emitted by the anchor pass (k_assign<true>); nullptr list: capture_inversions
+// compacts them itself with a flag scan over all records.
+struct InvCands { u32 *list = nullptr, *n = nullptr; };
+
+// inversion capture through the buckets of inversion_grid: a huge group (or SWG_INV_GRID=1), when its key fits 64 bits.  wb0 is the
+// widest query bucket: 2^wb0 > 2 * jump.
+static int inversion_grid_wb0(const swg_config &cfg) { return std::max(17, bits_for(2 * cfg.scaffold_gap + 1)); }
+static bool takes_inversion_grid(const swg_ctx *c, const swg_config &cfg, const Prefiltered &P, u32 n_huge) {
+    const int wb0 = inversion_grid_wb0(cfg);
+    return (n_huge > 0 || c->knobs.inv_grid) && 2 * P.sb + (P.cb > wb0 ? P.cb - wb0 : 1) + 1 <= 64;
+}
+
+static InvCands assign_anchors(swg_ctx *c, const Ordered &O, const Chains &chains, u8 *flags, u8 *status, u32 *chain_id, bool emit_candidates) {
+    const u32 n_m = O.n_m;
+    InvCands inv;
+    if (emit_candidates) {
+        inv.list = c->arena.take<u32>(n_m);
+        inv.n = c->arena.take<u32>(1);
+        SWG_CUDA(cudaMemsetAsync(inv.n, 0, sizeof(u32), c->stream));
+        k_assign<true><<<cdiv(n_m, 1024), 256, 0, c->stream>>>(n_m, chains.chain_of, O.sidx, chains.ct, flags, status, chain_id, c->d_ctr,
+                                                             inv.list, inv.n);
+    } else {
+        k_assign<false><<<cdiv(n_m, 1024), 256, 0, c->stream>>>(n_m, chains.chain_of, O.sidx, chains.ct, flags, status, chain_id, c->d_ctr,
+                                                              nullptr, nullptr);
+    }
+    c->lc.n++;
+    return inv;
 }
 
 // ---- K6: inversion capture (paf_filter.rs:535-597) ------------------------------------------------
@@ -1314,6 +1389,7 @@ static void inversion_grid(swg_ctx *c, const swg_config &cfg, const DevIn &in, c
     const Knobs &K = c->knobs;
     const u32 N = in.n;
     u8 *flags = P.flags;
+    u64 *ctr = c->d_ctr;
     const int sb = P.sb, cb = P.cb;
     stage_mark(c, "inversion_grid");
     const u64 G = cfg.scaffold_gap;
@@ -1443,6 +1519,7 @@ static void inversion_grid(swg_ctx *c, const swg_config &cfg, const DevIn &in, c
             }
         }
         if (best != NONE32) { status[i] = 1; chain_id[i] = best + 1; flags[i] |= F_ANCHOR; }
+        warp_count_add(ctr, C_ANCHORS, best != NONE32);
         if (dbg) { atomicAdd(&inv_dbg[0], (unsigned long long)n_walk); atomicAdd(&inv_dbg[1], (unsigned long long)n_cells); atomicMax(&inv_dbg[2], (unsigned long long)n_walk); if (best != NONE32) atomicAdd(&inv_dbg[3], 1ull); }
     });
     if (dbg) {
@@ -1457,11 +1534,12 @@ static void inversion_grid(swg_ctx *c, const swg_config &cfg, const DevIn &in, c
 // final order groups the chains by chromosome pair, so a pair's chains are one run of u: the table below maps a pair to the start
 // of its run (atomicMin of u).
 static void capture_inversions(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Prefiltered &P, u32 n_huge, const KeptChains &kc,
-                               u8 *status, u32 *chain_id) {
+                               const InvCands &cands, u8 *status, u32 *chain_id) {
     cudaStream_t st = c->stream; LaunchCounter &lc = c->lc; Arena &A = c->arena;
     const u32 N = in.n, C2 = kc.C2;
     u8 *flags = P.flags;
-    const int sb = P.sb, cb = P.cb;
+    u64 *ctr = c->d_ctr;
+    const int sb = P.sb;
     const u32 *t_qs = kc.t_qs, *t_qe = kc.t_qe, *t_ts = kc.t_ts;
     const u64 *t_c2key = kc.t_c2key;
     const u8 *t_fwd = kc.t_fwd;
@@ -1485,34 +1563,38 @@ static void capture_inversions(swg_ctx *c, const swg_config &cfg, const DevIn &i
             hash_insert_min(hk4, hv4, hmask4, c2, u);
         });
     }
-    // a huge group (or SWG_INV_GRID=1) takes the buckets of inversion_grid
-    const int wb0 = std::max(17, bits_for(2 * cfg.scaffold_gap + 1)); // widest bucket: 2^wb0 > 2 * jump
-    if ((n_huge > 0 || c->knobs.inv_grid) && 2 * sb + (cb > wb0 ? cb - wb0 : 1) + 1 <= 64) {
-        inversion_grid(c, cfg, in, P, C2, ik, u_qs, u_qe, u_ts, wb0, status, chain_id);
+    if (takes_inversion_grid(c, cfg, P, n_huge)) {
+        inversion_grid(c, cfg, in, P, C2, ik, u_qs, u_qe, u_ts, inversion_grid_wb0(cfg), status, chain_id);
         return;
     }
-    // the candidates (reverse strand, alive, not yet an anchor: a few per cent of the records) are compacted first, in
-    // no particular order (each is judged on its own); a candidate looks its chromosome pair up and walks the pair's run
-    // of chains in chain_N order — the reference's loop over the kept '+' chains "in order", first hit wins
-    // (paf_filter.rs:553-596)
+    // the candidates (reverse strand, alive, not yet an anchor: a few per cent of the records) come as a list in no particular
+    // order (each is judged on its own): from the anchor pass, else compacted here; a candidate looks its chromosome pair up
+    // and walks the pair's run of chains in chain_N order — the reference's loop over the kept '+' chains "in order", first
+    // hit wins (paf_filter.rs:553-596)
     const u64 G = cfg.scaffold_gap;
     const u64 *ikc = ik;
-    u32 *inv_list = A.take<u32>(N);
-    u32 *d_ninv = A.take<u32>(1);
-    u32 *bsum = A.take<u32>(scan_temp_u32(N));
-    scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & (F_ALIVE | F_REV | F_ANCHOR)) == (F_ALIVE | F_REV); },
-               [=] __device__(u32 i, u32 slot, u32 v) { if (v) inv_list[slot] = i; }, N, bsum, d_ninv, st, lc);
+    u32 *inv_list = cands.list, *d_ninv = cands.n;
+    if (!inv_list) {
+        inv_list = A.take<u32>(N);
+        d_ninv = A.take<u32>(1);
+        u32 *bsum = A.take<u32>(scan_temp_u32(N));
+        scan_flags([=] __device__(u32 i) -> bool { return (flags[i] & (F_ALIVE | F_REV | F_ANCHOR)) == (F_ALIVE | F_REV); },
+                   [=] __device__(u32 i, u32 slot, u32 v) { if (v) inv_list[slot] = i; }, N, bsum, d_ninv, st, lc);
+    }
     launch_for_dev<t_inversion>(d_ninv, c->sm_count, st, lc, [=] __device__(u32 x0) {
         const u32 i = inv_list[x0];
         const u64 key = ((u64)in.qid[i] << sb) | in.tid[i];
         const u32 u0 = hash_lookup(hk4, hv4, hmask4, key);
-        if (u0 == NONE32) return;
-        u64 mqs = in.qs[i], mqe = in.qe[i], mts = in.ts[i], mte = in.te[i];
-        u64 qc = (mqs + mqe) / 2, tc = (mts + mte) / 2;
-        for (u32 u = u0; u < C2 && u_c2[u] == key; u++) {
-            if (ikc[u] == NONE64) continue; // a '-' chain
-            if (inversion_hit(mqs, mqe, qc, tc, u_qs[u], u_qe[u], u_ts[u], G)) { status[i] = 1; chain_id[i] = u + 1; flags[i] |= F_ANCHOR; break; }
+        bool hit = false;
+        if (u0 != NONE32) {
+            u64 mqs = in.qs[i], mqe = in.qe[i], mts = in.ts[i], mte = in.te[i];
+            u64 qc = (mqs + mqe) / 2, tc = (mts + mte) / 2;
+            for (u32 u = u0; u < C2 && u_c2[u] == key; u++) {
+                if (ikc[u] == NONE64) continue; // a '-' chain
+                if (inversion_hit(mqs, mqe, qc, tc, u_qs[u], u_qe[u], u_ts[u], G)) { status[i] = 1; chain_id[i] = u + 1; flags[i] |= F_ANCHOR; hit = true; break; }
+            }
         }
+        warp_count_add(ctr, C_ANCHORS, hit);
     });
 }
 
@@ -1522,6 +1604,7 @@ static void rescue(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Pre
     const Knobs &K = c->knobs;
     const u32 N = in.n;
     u8 *flags = P.flags;
+    u64 *ctr = c->d_ctr;
     const int sb = P.sb, cb = P.cb;
     const u64 D = cfg.scaffold_max_deviation;
     // anchor list (status == 1) ordered by (chromosome pair, query center); one sort when the key fits 64 bits,
@@ -1638,6 +1721,7 @@ static void rescue(swg_ctx *c, const swg_config &cfg, const DevIn &in, const Pre
             visit(x, qd);
         }
         if (best_a != NONE32) { status[i] = 2; chain_id[i] = chain_id[best_a]; }
+        warp_count_add(ctr, C_RESCUED, best_a != NONE32);
     });
 }
 
@@ -1682,15 +1766,18 @@ static void run_filter(swg_ctx *c, const swg_config &cfg, const DevIn &in, u8 *s
     const KeptChains kc = order_chains(c, cfg, in, P, chains, exact_host, S);
 
     stage_mark(c, "assign+inversion+rescue");
-    assign_anchors(c, O, chains, P.flags, status, chain_id);
-    if (!cfg.scaffolds_only && kc.C2 > 0) {
-        capture_inversions(c, cfg, in, P, chained.n_huge, kc, status, chain_id);
+    // The anchor pass hands the inversion capture its candidates when it visits every alive record (every alive record is a
+    // sorted position) and the capture walks the chains of a pair (not the buckets of inversion_grid, which sorts them itself).
+    const bool capture = !cfg.scaffolds_only && kc.C2 > 0;
+    const bool fused_candidates = capture && O.n_m == P.n_alive && !takes_inversion_grid(c, cfg, P, chained.n_huge);
+    const InvCands cands = assign_anchors(c, O, chains, P.flags, status, chain_id, fused_candidates);
+    if (capture) {
+        capture_inversions(c, cfg, in, P, chained.n_huge, kc, cands, status, chain_id);
         if (cfg.scaffold_max_deviation > 0) rescue(c, cfg, in, P, status, chain_id);
     }
 
+    // k_assign, the inversion capture and rescue have counted the statuses they wrote (C_ANCHORS, C_RESCUED)
     stage_mark(c, "stats");
-    k_count_status<<<std::min<u32>(cdiv(N, 256), (u32)c->sm_count * 8), 256, 0, c->stream>>>(N, status, c->d_ctr);
-    c->lc.n++;
     read_counters(c);
     S.n_anchors = c->h_ctr[C_ANCHORS];
     S.n_rescued = c->h_ctr[C_RESCUED];
