@@ -317,8 +317,10 @@ __device__ __forceinline__ void bb_best_successor(const uint4 *__restrict__ srec
 // for the resolve kernels / the fixed-point iteration; no claims.
 constexpr u32 RES_SMALL = 16;
 constexpr u32 RES_THREAD_MAX = 16; // dirty groups up to this size are walked by one thread (from registers), larger ones by a warp
+// 8 CTAs per SM (32 registers): the window scan is a chain of dependent loads, hidden only by resident warps; the bound costs one
+// 4 B spill of the loop index per position, outside the scan (40 registers without it: 268 against 220 us per 20 M positions)
 template <bool LIST>
-__global__ void __launch_bounds__(256)
+__global__ void __launch_bounds__(256, 8)
 k_chain_candidates(const uint4 *__restrict__ srec, const u64 *__restrict__ skey, const u32 *__restrict__ gid,
                    const u32 *__restrict__ gstart, u32 n_groups, u32 n_m, int cb, u64 G, Cand *__restrict__ cand,
                    u32 *pred, u32 *grp_dirty, const u32 *__restrict__ list, const u32 *__restrict__ n_list_ptr, u32 fx_min = 0,
@@ -739,12 +741,16 @@ k_chain_work_estimate(const uint4 *__restrict__ rec4, SortedIdx sidx, const u32 
 // P2c: union-find roots and dense chain numbers in ONE pass over pred[] (union_find.rs:25-41: every union hangs the
 // singleton j under find(pred[j]), so the root of a set is its head and pred[] is a forest of paths with pred[j] < j;
 // chains are numbered by ascending head position, union_find.rs:52-63).
-// A CTA takes a tile of 2048 consecutive sorted positions (tile ids in scheduling order): pointer jumping in shared memory
-// resolves every position to a head inside the tile or to an ancestor in an EARLIER tile; heads are numbered by a
-// decoupled look-back over the tiles' head counts; positions whose ancestor lies in an earlier tile wait for that
-// position's published chain number (its tile is resident or done: the wait only ever points backwards).
-// chain_of[] must be NONE32 everywhere on entry.  PRESET: root[] already holds the final root of some positions (huge
-// groups chained by the fixed-point iteration), NONE32 elsewhere.
+// A CTA takes a tile of 2048 consecutive sorted positions (tile ids in scheduling order); heads are numbered by a decoupled
+// look-back over the tiles' head counts.  Every position is resolved to a head inside the tile or to an ancestor in an
+// EARLIER tile without block-wide rounds: each warp owns 256 consecutive positions and walks them as 8 chunks of 32 in
+// order; an ancestor inside the current chunk is followed by pointer jumping in registers (5 shuffle rounds cover 32 hops),
+// one in an earlier chunk of the warp is read once from the warp's resolved slice in shared memory.  After one barrier, a
+// position pointing into an earlier warp's range hops over those slices (at most 7 hops, each to an earlier warp).
+// A position whose ancestor a lies in an earlier tile gets chain_of[p] = 0x80000000 | a (positions are < 2^31) instead of
+// waiting for that tile: k_chain_aggregate, which runs after this kernel, follows such marks to a number and writes it back.
+// Every chain_of[] entry is written.  PRESET: root[] already holds the final root of some positions (huge groups chained by
+// the fixed-point iteration), NONE32 elsewhere.
 struct ChainDense { // per-chain aggregates, rows indexed by chain number
     u32 *qmin, *qmax, *tmin, *tmax; // = ChainTable qs / qe / ts / te
     u64 *sum_matches, *sum_block;
@@ -752,42 +758,55 @@ struct ChainDense { // per-chain aggregates, rows indexed by chain number
 };
 constexpr int CR_THREADS = 256, CR_ITEMS = 8, CR_TILE = CR_THREADS * CR_ITEMS;
 static_assert(CR_THREADS == SC_THREADS, "k_chain_number uses the 256-thread block scan of scan.cuh");
+// 8 CTAs per SM (32 registers): a tile is a short chain of latencies (tile id, loads, scan, look-back), so resident tiles are
+// what hides them; 20 B of spills in the row-clearing loop, once per CTA (48 registers without the bound: 145 against 117 us)
 template <bool PRESET>
-__global__ void __launch_bounds__(CR_THREADS)
-k_chain_number(const u32 *__restrict__ pred, const u32 *__restrict__ root_preset, u32 n_m, u32 *chain_of, u32 *__restrict__ head_pos,
+__global__ void __launch_bounds__(CR_THREADS, 8)
+k_chain_number(const u32 *__restrict__ pred, const u32 *__restrict__ root_preset, u32 n_m, u32 *__restrict__ chain_of, u32 *__restrict__ head_pos,
                u64 *status, u32 *tile_counter, u32 *n_chains_out, ChainDense cd) {
     __shared__ u32 anc[CR_TILE];
     __shared__ u32 ws[CR_THREADS / 32];
     __shared__ u32 s_tile, s_excl;
-    const u32 tid = threadIdx.x, lane = tid & 31;
+    const u32 full = 0xFFFFFFFFu;
+    const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) s_tile = atomicAdd(tile_counter, 1u);
     __syncthreads();
     const u32 tile = s_tile;
     const u32 base = tile * CR_TILE;
-    // load (striped: coalesced), ancestor = predecessor or the position itself (a head)
+    const u32 wl = warp * (32 * CR_ITEMS); // the warp's range [wl, wl + 256) of the tile; chunk k = [wl + 32 k, wl + 32 k + 32)
+    // load (chunk k of the warp at lane: coalesced), ancestor = predecessor, preset root or the position itself (a head)
+    u32 a[CR_ITEMS], hcnt = 0; // hcnt: heads of the warp's range
 #pragma unroll
     for (int k = 0; k < CR_ITEMS; k++) {
-        const u32 l = k * CR_THREADS + tid, p = base + l;
-        u32 a = p;
+        const u32 p = base + wl + 32 * k + lane;
+        a[k] = p;
         if (p < n_m) {
             const u32 pr = pred[p];
-            if (pr != NONE32) a = pr;
-            if (PRESET) { const u32 r = root_preset[p]; if (r != NONE32) a = r; }
+            if (pr != NONE32) a[k] = pr;
+            if (PRESET) { const u32 r = root_preset[p]; if (r != NONE32) a[k] = r; }
         }
-        anc[l] = a;
+        hcnt += __popc(__ballot_sync(full, p < n_m && a[k] == p));
     }
-    __syncthreads();
-    // heads of the tile in position order (blocked), published before anything can wait
-    u32 hflag = 0, hcnt = 0;
+    // resolve inside the warp's range, chunk by chunk: afterwards a[k] is a head of the range or an ancestor before it
 #pragma unroll
     for (int k = 0; k < CR_ITEMS; k++) {
-        const u32 l = tid * CR_ITEMS + k, p = base + l;
-        const bool h = p < n_m && anc[l] == p;
-        hflag |= (h ? 1u : 0u) << k;
-        hcnt += h;
+        const u32 c0 = base + wl + 32 * k;
+        u32 x = a[k];
+#pragma unroll
+        for (int r = 0; r < 5; r++) { // pred < position: a chunk holds at most 31 hops
+            const bool in = x >= c0 && x < c0 + 32;
+            const u32 y = __shfl_sync(full, x, in ? x - c0 : lane);
+            if (in) x = y;
+        }
+        if (x >= base + wl && x < c0) x = anc[x - base]; // an earlier chunk of this warp: already resolved
+        a[k] = x;
+        anc[wl + 32 * k + lane] = x;
+        __syncwarp();
     }
+    // heads of the tile in position order: lane 0 of each warp enters the warp's head count, so its exclusive prefix is the
+    // number of heads before the warp's range
     u32 tot;
-    const u32 ex_local = block_exclusive_scan_256(hcnt, ws, tot);
+    const u32 ex_local = block_exclusive_scan_256(lane == 0 ? hcnt : 0u, ws, tot); // its barriers also publish every warp's slice of anc[]
     if (tid < 32) {
         if (lane == 0) st_relaxed_u64(&status[tile], (tile == 0 ? SC_FLAG_INCL : SC_FLAG_AGG) | tot);
         u32 excl = 0;
@@ -812,31 +831,32 @@ k_chain_number(const u32 *__restrict__ pred, const u32 *__restrict__ root_preset
             if ((u64)(tile + 1) * CR_TILE >= n_m) *n_chains_out = excl + tot;
         }
     }
-    // pointer jumping inside the tile (a racing read sees an older or a newer ancestor: both are ancestors)
-    while (true) {
-        bool changed = false;
+    // an ancestor in an earlier warp's range: hop over the resolved slices (each hop lands on a head or goes to an earlier
+    // warp) until a head of the tile or a position before the tile
 #pragma unroll
-        for (int k = 0; k < CR_ITEMS; k++) {
-            const u32 l = k * CR_THREADS + tid;
-            const u32 a = anc[l];
-            if (a >= base && a != base + l) {
-                const u32 a2 = anc[a - base];
-                if (a2 != a) { anc[l] = a2; changed = true; }
-            }
+    for (int k = 0; k < CR_ITEMS; k++) {
+        u32 x = a[k];
+        while (x >= base && x < base + wl) {
+            const u32 y = anc[x - base];
+            if (y == x) break;
+            x = y;
         }
-        if (!__syncthreads_or(changed)) break;
+        a[k] = x;
     }
-    // heads get their numbers (s_excl is visible: the loop above ended in a barrier)
+    __syncthreads(); // every read of the resolved slices is done, and s_excl is visible
+    // heads get their numbers, in position order
     {
-        u32 ex = s_excl + ex_local;
+        u32 ex = s_excl + __shfl_sync(full, ex_local, 0); // heads of the tile before this warp's range
 #pragma unroll
         for (int k = 0; k < CR_ITEMS; k++) {
-            if ((hflag >> k) & 1u) {
-                const u32 l = tid * CR_ITEMS + k;
-                head_pos[ex] = base + l;
-                anc[l] = 0x80000000u | ex; // marks "this entry now holds a chain number" (positions are < 2^31)
-                ex++;
+            const u32 p = base + wl + 32 * k + lane;
+            const u32 hmask = __ballot_sync(full, p < n_m && a[k] == p); // a head resolves to itself, nothing else does
+            if ((hmask >> lane) & 1u) {
+                const u32 r = ex + __popc(hmask & lanemask_lt());
+                head_pos[r] = p;
+                anc[wl + 32 * k + lane] = 0x80000000u | r; // marks "this entry now holds a chain number" (positions are < 2^31)
             }
+            ex += __popc(hmask);
         }
     }
     // the tile's chains are the consecutive rows s_excl .. s_excl + tot of the aggregate table: they start empty (the host does
@@ -846,19 +866,13 @@ k_chain_number(const u32 *__restrict__ pred, const u32 *__restrict__ root_preset
         cd.sum_matches[r] = 0; cd.sum_block[r] = 0; cd.k[r] = 0;
     }
     __syncthreads();
-    // every position: chain number of its head (inside the tile) or of its ancestor in an earlier tile
+    // every position: chain number of its head (inside the tile) or the mark of its ancestor in an earlier tile
 #pragma unroll
     for (int k = 0; k < CR_ITEMS; k++) {
-        const u32 l = k * CR_THREADS + tid, p = base + l;
+        const u32 p = base + wl + 32 * k + lane;
         if (p >= n_m) continue;
-        const u32 a = anc[l];
-        u32 ci;
-        if (a & 0x80000000u) ci = a & 0x7FFFFFFFu;
-        else if (a >= base) ci = anc[a - base] & 0x7FFFFFFFu; // its head: numbered above
-        else {
-            do { ci = ld_volatile_u32(chain_of + a); } while (ci == NONE32);
-        }
-        st_volatile_u32(chain_of + p, ci);
+        const u32 x = a[k];
+        chain_of[p] = x >= base ? anc[x - base] & 0x7FFFFFFFu : 0x80000000u | x;
     }
 }
 
@@ -866,9 +880,12 @@ k_chain_number(const u32 *__restrict__ pred, const u32 *__restrict__ root_preset
 // by atomicAdd; runs of one chain inside a warp are reduced first (one set of atomics per run).  Every position also feeds
 // its group's min original index (the first appearance of the group in the input).  The table rows are pre-set to
 // (max, 0, max, 0, 0, 0).
+// A marked chain_of[p] (0x80000000 | ancestor, left by k_chain_number) is followed to a number, which is written back for
+// k_assign.  Marks only ever point backwards and are only ever replaced by their number, so a racing reader sees the mark
+// or the number: both lead to the same chain, in at most as many hops as the chain spans tiles.
 __global__ void __launch_bounds__(256)
 k_chain_aggregate(const uint4 *__restrict__ srec, const u32 *__restrict__ blen, const u32 *__restrict__ matches, SortedIdx sidx,
-                  const u32 *__restrict__ gid, const u32 *__restrict__ chain_of, u32 n_m, ChainDense cd, u32 *__restrict__ grp_minidx) {
+                  const u32 *__restrict__ gid, u32 *chain_of, u32 n_m, ChainDense cd, u32 *__restrict__ grp_minidx) {
     const u32 full = 0xFFFFFFFFu;
     const u32 lane = lane_id();
     const u32 p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -880,6 +897,10 @@ k_chain_aggregate(const uint4 *__restrict__ srec, const u32 *__restrict__ blen, 
         g = gid[p];
         idx = sidx[p];
         ci = chain_of[p];
+        if (ci & 0x80000000u) {
+            do { ci = chain_of[ci & 0x7FFFFFFFu]; } while (ci & 0x80000000u);
+            chain_of[p] = ci;
+        }
         a = srec[p];
         m = make_uint2(__ldg(&blen[idx]), __ldg(&matches[idx])); // gathered by input index (a separate sorted copy cost 16 B more per record)
     }

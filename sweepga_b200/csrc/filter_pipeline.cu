@@ -1054,7 +1054,7 @@ static Chains chain_table(swg_ctx *c, const swg_config &cfg, const DevIn &in, co
     stage_mark(c, "ch_number");
     // The table is sized for the worst case (every position its own chain) and each row is cleared by the kernel that numbers
     // its chain, so the aggregate pass can start before the host knows the chain count (it reads it while that pass runs).
-    u32 *chain_of = A.take<u32>(n_m);  // chain number of every sorted position
+    u32 *chain_of = A.take<u32>(n_m);  // chain number of every sorted position (cross-tile marks resolved by the aggregate pass)
     u32 *head_pos = A.take<u32>(n_m);  // compacted head positions (C of them)
     u32 *grp_minidx = A.take<u32>(O.n_groups); // per GROUP: min original index over its members (first appearance of the group)
     u32 *d_cnt = A.take<u32>(2);       // [0] chains, [1] passing chains
@@ -1072,7 +1072,6 @@ static Chains chain_table(swg_ctx *c, const swg_config &cfg, const DevIn &in, co
         u32 *cn_ctr = A.take<u32>(2);
         SWG_CUDA(cudaMemsetAsync(cn_status, 0, sizeof(u64) * (size_t)(tiles + 1), st));
         SWG_CUDA(cudaMemsetAsync(cn_ctr, 0, 2 * sizeof(u32), st));
-        SWG_CUDA(cudaMemsetAsync(chain_of, 0xFF, sizeof(u32) * (size_t)n_m, st));
         if (chained.root_preset) k_chain_number<true><<<tiles, CR_THREADS, 0, st>>>(chained.pred, chained.root_preset, n_m, chain_of, head_pos, cn_status, cn_ctr, d_cnt, cd);
         else k_chain_number<false><<<tiles, CR_THREADS, 0, st>>>(chained.pred, nullptr, n_m, chain_of, head_pos, cn_status, cn_ctr, d_cnt, cd);
         lc.n++;
