@@ -410,7 +410,8 @@ static void sweep_piles_n1(swg_ctx *c, const u32 *sitem, const SweepItem *sdata,
                [=] __device__(u32 b, u32 ex, u32) { boff[b] = ex; }, n_big, tmp, d_tot, st, lc);
     const u32 nb = read_u32(c, d_tot);
     if (nb == 0) return;
-    if (nb >= (1u << 30)) throw RangeError{"plane sweep: more than 2^30 mappings in deep piles"};
+    // the event sort below holds 2 * nb pairs, and the radix sort is exact up to 2^30 - 1 pairs (30-bit tile status counts)
+    if (nb >= (1u << 29)) throw RangeError{"plane sweep: 2^29 or more mappings in deep piles (the sort of their two events each holds at most 2^30 - 1)"};
     u32 *bitem = A.take<u32>(nb), *bgrp = A.take<u32>(nb);
     k_pile_expand<<<cdiv(nb, 256), 256, 0, st>>>(big_list, boff, n_big, nb, gstart, bitem, bgrp);
     u64 *ek = A.take<u64>(2 * (size_t)nb), *ek2 = A.take<u64>(2 * (size_t)nb), *rk = A.take<u64>(nb), *rk2 = A.take<u64>(nb);
